@@ -3,6 +3,13 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched per rank by torch.distributed.run)
   python bench.py --impl reference ...                      (the reference's CPU arithmetic: the oracle port)
+  python bench.py ... --dump-outputs DIR                    (also write the last timed step's outputs as .npy files)
+
+--dump-outputs writes boxes.npy and cls_logits.npy for every image of the step, and masks.npy and seg_logits.npy for
+a fixed seeded sample of at most DUMP_MAP_IMAGES of them, all float32.  It is what the pipeline returns to a caller on
+one GPU; with N>1 it is rank 0's own slice of the global batch (the gathered masks / boxes / logits on rank 0 are
+these slices side by side, which tests/test_dist_gpu.py checks bit for bit against a 1-GPU run).  With --impl
+reference it is the oracle port's outputs for its --cpu-sample images, under the same names.
 
 A step is one pass of the whole path over this rank's batch of synthetic 224x224 images (default 256 per GPU,
 run as micro-batches of 128 — BASELINE.json configs[3]/[4]: 512 images on 2 GPUs, 2048 on 8), followed for N>1 by
@@ -34,6 +41,7 @@ sys.path.insert(0, ROOT)
 METRIC = "seg+crop+cls images/sec"
 UNIT = "images/s"
 FLOP_PER_IMAGE = 81.53e9   # SURVEY.md §8d: live algorithmic FLOPs of the whole path per image
+DUMP_MAP_IMAGES = 64       # --dump-outputs: images whose masks / logit maps are written (2 x 12.8 MB as float32)
 
 
 def _peaks():
@@ -154,7 +162,7 @@ def run_reference_arm(args, rank):
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
     sample = args.cpu_sample
-    usd, gsd = fixtures.trained_unet_state(), fixtures.trained_googlenet_state()   # same weights as the GPU arm
+    usd, gsd = _fixture_weights()   # same weights as the GPU arm
     imgs, _, _ = fixtures.synth_images(sample, seed=1234)
     x = torch.from_numpy(imgs)
 
@@ -162,16 +170,21 @@ def run_reference_arm(args, rank):
         with torch.no_grad():
             logits = unet_ref.unet_forward(usd, x)
             masks = unet_ref.mask_from_logits(logits)[:, 0].numpy()
-            crops = np.stack([roi_ref.roi_tensor(imgs[i], masks[i])[0] for i in range(sample)])
-            return googlenet_ref.googlenet_forward(gsd, torch.from_numpy(crops))
+            rois = [roi_ref.roi_tensor(imgs[i], masks[i]) for i in range(sample)]
+            cls = googlenet_ref.googlenet_forward(gsd, torch.from_numpy(np.stack([r[0] for r in rois])))
+            boxes = torch.tensor([r[1] for r in rois], dtype=torch.int32)
+            return {"masks": torch.from_numpy(masks), "boxes": boxes, "cls_logits": cls, "seg_logits": logits}
 
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        out = step()
     dt = time.perf_counter() - t0
     v = sample * args.steps / dt
+    if args.dump_outputs and args.steps:                      # same names as the GPU arm's dump
+        dump_outputs(args.dump_outputs, sample, {k: out[k] for k in ("boxes", "cls_logits")},
+                     {k: out[k] for k in ("masks", "seg_logits")})
     desc = f"{sample} images/step of the same synthetic workload, fp32, oracle port of the reference path"
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -189,7 +202,7 @@ def cpu_baseline(sample, budget_s=20.0):
     from oracle import fixtures, googlenet_ref, roi_ref, unet_ref
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
-    usd, gsd = fixtures.trained_unet_state(), fixtures.trained_googlenet_state()   # same weights as the GPU arm
+    usd, gsd = _fixture_weights()   # same weights as the GPU arm
     imgs, _, _ = fixtures.synth_images(sample, seed=1234)
     x = torch.from_numpy(imgs)
 
@@ -219,9 +232,8 @@ def gpu_eager_yardstick(dev, iters=3):
     channels_last, UNet at B=64 and GoogLeNet at B=256, compute only (no mask -> bbox -> crop step, which the
     reference does on the host).  images/s = 1 / (t_unet / 64 + t_googlenet / 256)."""
     import torch
-    from oracle import fixtures, googlenet_ref, unet_ref
-    usd = {k: v.to(dev) for k, v in fixtures.trained_unet_state().items()}
-    gsd = {k: v.to(dev) for k, v in fixtures.trained_googlenet_state().items()}
+    from oracle import googlenet_ref, unet_ref
+    usd, gsd = ({k: v.to(dev) for k, v in sd.items()} for sd in _fixture_weights())
     xu = torch.rand((64, 3, 224, 224), device=dev)
     xg = torch.rand((256, 3, 224, 224), device=dev)
     out = {}
@@ -256,8 +268,22 @@ def gpu_eager_yardstick(dev, iters=3):
     return out
 
 
+def dump_outputs(out_dir, batch, per_image, maps=None):
+    """--dump-outputs: every array as float32 DIR/<name>.npy.  `per_image` arrays ([B, ...], small) are written whole;
+    the per-pixel `maps` ([B, ...], 200 KB an image as float32) only for a fixed seeded sample of the batch, so that a
+    dump stays well under 64 MB and two runs with the same arguments compare array for array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    sample = np.sort(np.random.default_rng(0).permutation(batch)[:DUMP_MAP_IMAGES])
+    arrays = {name: t.float().cpu().numpy() for name, t in per_image.items()}
+    arrays.update({name: t.float().cpu().numpy()[sample] for name, t in (maps or {}).items()})
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _fixture_weights():
-    """Briefly-trained reference-format state_dicts (cached under tests/_cache, regenerated on this GPU if absent)."""
+    """Briefly-trained reference-format state_dicts, trained deterministically on this GPU if no cached copy exists
+    (oracle/fixtures.py; the cache lives outside the source tree).  CPU tensors."""
     import torch
     from oracle import fixtures
     dev = "cuda" if torch.cuda.is_available() else "cpu"
@@ -308,6 +334,12 @@ def run_stage_alone(args, dev, rank):
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
     v = B * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        if args.workload == "unet":
+            dump_outputs(args.dump_outputs, B, {"boxes": ws["boxes"]},
+                         {"masks": ws["mask"], "seg_logits": ws["logits"]})
+        else:
+            dump_outputs(args.dump_outputs, B, {"cls_logits": ws["cls_logits"]})
     if rank == 0:
         print(json.dumps({"metric": f"{args.workload} images/sec (stage alone)", "value": v, "unit": UNIT, "n_gpus": 1,
                           "steps": args.steps, "warmup": W, "ms_per_step": ms / args.steps, "higher_is_better": True,
@@ -343,6 +375,10 @@ def main():
     ap.add_argument("--yardstick", action="store_true", help=argparse.SUPPRESS)   # (round-1 flag: now the default)
     ap.add_argument("--collective", default="gather", choices=["gather", "all_gather"],
                     help="gather: masks/boxes/logits to rank 0 on a side stream (default); all_gather: round 1's form")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed on rank 0 as DIR/<name>.npy "
+                         f"(float32; per-pixel maps for a fixed seeded sample of at most {DUMP_MAP_IMAGES} images)")
+    ap.add_argument("--breakdown", metavar="FILE", help="write the per-op time breakdown of the pipeline as JSON")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -473,6 +509,9 @@ def main():
     sampler.mark_end()
     launches = eng.launch_count - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:                        # before the host-fed loop below reuses the buffers
+        dump_outputs(args.dump_outputs, PB, {"boxes": ws["boxes"], "cls_logits": ws["cls_logits"]},
+                     {"masks": ws["mask"], "seg_logits": ws["logits"]})
     value = world * PB * args.steps / (ms / 1e3)
     gathered_ok = None
     if gather is not None:
@@ -571,19 +610,19 @@ def main():
             line["cpu_baseline"] = cpu_baseline(args.cpu_sample)
         if world == 1 and not args.no_yardstick:
             line["gpu_eager_yardstick"] = gpu_eager_yardstick(dev)
-        # per-op breakdown for profiles/ (not part of the contract line)
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        kinds = {}
-        for t, d in zip(per_op_ms, prog.descs):
-            kinds[type(d).__name__] = kinds.get(type(d).__name__, 0.0) + t
-        with open(os.path.join(ROOT, "gpurun_out", f"bench_breakdown_n{world}.json"), "w") as f:
-            json.dump({"per_kind_ms_per_step": kinds, "images_per_step": PB, "micro_batch": MB,
-                       "per_op": [{"i": i, "kind": type(d).__name__, "ms": t, "gflop": fl / 1e9,
-                                   "tflops": (fl / (t / 1e3) / 1e12) if fl and t > 0 else None,
-                                   "shape": ([d.B, d.H, d.W, d.Cin, d.N, d.R] if isinstance(d, E.ConvDesc) else
-                                             ([d.B, d.H, d.W, 3, 64, 3 if d.kind == 0 else 7]
-                                              if isinstance(d, E.StemDesc) else None))}
-                                  for i, (t, d, fl) in enumerate(zip(per_op_ms, prog.descs, per_op_flop))]}, f, indent=1)
+        if args.breakdown:                                     # per-op breakdown for profiles/ (not part of the line)
+            kinds = {}
+            for t, d in zip(per_op_ms, prog.descs):
+                kinds[type(d).__name__] = kinds.get(type(d).__name__, 0.0) + t
+            with open(args.breakdown, "w") as f:
+                json.dump({"per_kind_ms_per_step": kinds, "images_per_step": PB, "micro_batch": MB,
+                           "per_op": [{"i": i, "kind": type(d).__name__, "ms": t, "gflop": fl / 1e9,
+                                       "tflops": (fl / (t / 1e3) / 1e12) if fl and t > 0 else None,
+                                       "shape": ([d.B, d.H, d.W, d.Cin, d.N, d.R] if isinstance(d, E.ConvDesc) else
+                                                 ([d.B, d.H, d.W, 3, 64, 3 if d.kind == 0 else 7]
+                                                  if isinstance(d, E.StemDesc) else None))}
+                                      for i, (t, d, fl) in enumerate(zip(per_op_ms, prog.descs, per_op_flop))]},
+                          f, indent=1)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -8,10 +8,19 @@
   (logits ~ 0 everywhere) and no bf16 implementation, including the reference under autocast, reaches the
   99.9 % mask-agreement gate.  Training uses the differentiable oracle (oracle/unet_ref.py,
   oracle/googlenet_ref.py) with AdamW and 0.5*BCE + 0.5*soft-Dice, a MONAI-free restatement of the reference's
-  DC_and_BCE_loss (分割/util/loss.py:64-86); results are cached under tests/_cache/ (git-ignored).
+  DC_and_BCE_loss (分割/util/loss.py:64-86).  On a GPU the training runs with deterministic cuDNN algorithms and
+  TF32 off, so every run on the same GPU model and software stack yields the same weights bit for bit.  Results are
+  cached outside the source tree, so that a read-only checkout works: in UGNET_FIXTURE_CACHE if set, else in
+  $XDG_CACHE_HOME/ugnet_fixtures (~/.cache/ugnet_fixtures), else in a per-user directory under the system temporary
+  directory; a directory is used only if the current user owns it and nobody else may write to it.  The cache key
+  holds the oracle's source code, the torch / CUDA / cuDNN versions and the device name, so a change of any of them
+  retrains instead of reusing weights trained under other conditions.
 """
+import hashlib
 import math
 import os
+import stat
+import tempfile
 
 import numpy as np
 import torch
@@ -19,7 +28,10 @@ import torch.nn.functional as F
 
 from . import googlenet_ref, roi_ref, unet_ref
 
-CACHE_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "_cache")
+_XDG = os.environ.get("XDG_CACHE_HOME") or os.path.join(os.path.expanduser("~"), ".cache")
+CACHE_DIRS = ([os.environ["UGNET_FIXTURE_CACHE"]] if os.environ.get("UGNET_FIXTURE_CACHE") else
+              [os.path.join(_XDG, "ugnet_fixtures"),
+               os.path.join(tempfile.gettempdir(), f"ugnet_fixtures_{os.getuid()}")])
 
 
 # ------------------------------------------------------------------------------------------------ images
@@ -101,18 +113,74 @@ def _bce_dice(logits, target):
     return 0.5 * F.binary_cross_entropy_with_logits(logits, target) + 0.5 * dice.mean()
 
 
+class _DeterministicGpu:
+    """Deterministic cuDNN algorithms, no autotuning and no TF32 while a fixture trains, previous settings restored."""
+
+    FLAGS = ((torch.backends.cudnn, "deterministic", True), (torch.backends.cudnn, "benchmark", False),
+             (torch.backends.cudnn, "allow_tf32", False), (torch.backends.cuda.matmul, "allow_tf32", False))
+
+    def __enter__(self):
+        self.prev = [getattr(mod, name) for mod, name, _ in self.FLAGS]
+        for mod, name, value in self.FLAGS:
+            setattr(mod, name, value)
+
+    def __exit__(self, *a):
+        for (mod, name, _), value in zip(self.FLAGS, self.prev):
+            setattr(mod, name, value)
+
+
 def _train(sd, loss_fn, batches, lr, device):
     params = {k: v.to(device).clone().requires_grad_(v.is_floating_point() and "running" not in k)
               for k, v in sd.items()}
     opt = torch.optim.AdamW([p for p in params.values() if p.requires_grad], lr=lr)
     last = None
-    for batch in batches:
-        opt.zero_grad(set_to_none=True)
-        loss = loss_fn(params, batch)
-        loss.backward()
-        opt.step()
-        last = float(loss.detach())
+    with _DeterministicGpu():
+        for batch in batches:
+            opt.zero_grad(set_to_none=True)
+            loss = loss_fn(params, batch)
+            loss.backward()
+            opt.step()
+            last = float(loss.detach())
     return {k: v.detach() for k, v in params.items()}, last
+
+
+def _cache_dir():
+    """The first of CACHE_DIRS that exists or can be made, is owned by this user and is writable by nobody else; None
+    (no caching) if there is none."""
+    for d in CACHE_DIRS:
+        try:
+            os.makedirs(d, mode=0o700, exist_ok=True)
+            st = os.stat(d)
+        except OSError:
+            continue
+        if st.st_uid == os.getuid() and not st.st_mode & (stat.S_IWGRP | stat.S_IWOTH) and os.access(d, os.W_OK):
+            return d
+    return None
+
+
+def _fingerprint(device):
+    """What the trained weights depend on besides the arguments: the oracle's code, the software stack, the device."""
+    h = hashlib.sha256()
+    here = os.path.dirname(os.path.abspath(__file__))
+    for fn in ("fixtures.py", "unet_ref.py", "googlenet_ref.py", "roi_ref.py"):
+        with open(os.path.join(here, fn), "rb") as f:
+            h.update(f.read())
+    dev = torch.device(device)
+    name = torch.cuda.get_device_name(dev) if dev.type == "cuda" else "cpu"
+    h.update(f"{torch.__version__}|{torch.version.cuda}|{torch.backends.cudnn.version()}|{name}".encode())
+    return h.hexdigest()[:16]
+
+
+def _cache_path(name, device):
+    d = _cache_dir()
+    return os.path.join(d, f"{name}_{torch.device(device).type}_{_fingerprint(device)}.pt") if d else None
+
+
+def _save_cache(state, path):
+    """Write-then-rename, so that a concurrent reader never sees a partial file."""
+    tmp = f"{path}.{os.getpid()}.tmp"
+    torch.save({"net": state}, tmp)
+    os.replace(tmp, path)
 
 
 def _reparam_bn_stats(sd, seed, eps):
@@ -141,8 +209,8 @@ def trained_unet_state(device="cpu", steps=120, batch=4, seed=1234, lr=3e-4, cac
     BN stays in eval mode throughout (running stats from the procedural init are part of the function), which
     keeps the trained function identical between train and eval; afterwards the BN statistics are
     re-parameterised to non-trivial values without changing the function (_reparam_bn_stats)."""
-    path = os.path.join(CACHE_DIR, f"unet_trained_s{seed}_n{steps}_b{batch}.pt")
-    if cache and os.path.exists(path):
+    path = _cache_path(f"unet_trained_s{seed}_n{steps}_b{batch}", device)
+    if cache and path and os.path.exists(path):
         return torch.load(path, map_location="cpu")["net"]
     sd = procedural_state(unet_template(), seed)
     # start from identity-like BN so that activations are well scaled at step 0
@@ -166,9 +234,8 @@ def trained_unet_state(device="cpu", steps=120, batch=4, seed=1234, lr=3e-4, cac
 
     out, _ = _train(sd, loss_fn, batches(), lr, device)
     out = _reparam_bn_stats({k: v.cpu() for k, v in out.items()}, seed + 1, unet_ref.BN_EPS)
-    if cache:
-        os.makedirs(CACHE_DIR, exist_ok=True)
-        torch.save({"net": out}, path)
+    if cache and path:
+        _save_cache(out, path)
     return out
 
 
@@ -178,8 +245,8 @@ def roi_crops_from_masks(imgs, masks):
 
 
 def trained_googlenet_state(device="cpu", steps=300, batch=16, seed=4321, lr=1e-3, cache=True, verbose=False):
-    path = os.path.join(CACHE_DIR, f"googlenet_trained_s{seed}_n{steps}_b{batch}.pt")
-    if cache and os.path.exists(path):
+    path = _cache_path(f"googlenet_trained_s{seed}_n{steps}_b{batch}", device)
+    if cache and path and os.path.exists(path):
         return torch.load(path, map_location="cpu")["net"]
     sd = procedural_state(googlenet_template(), seed)
     for k in sd:
@@ -203,7 +270,6 @@ def trained_googlenet_state(device="cpu", steps=300, batch=16, seed=4321, lr=1e-
 
     out, _ = _train(sd, loss_fn, batches(), lr, device)
     out = _reparam_bn_stats({k: v.cpu() for k, v in out.items()}, seed + 1, googlenet_ref.BN_EPS)
-    if cache:
-        os.makedirs(CACHE_DIR, exist_ok=True)
-        torch.save({"net": out}, path)
+    if cache and path:
+        _save_cache(out, path)
     return out

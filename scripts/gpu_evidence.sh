@@ -9,8 +9,7 @@ set -x
 if [ "$2" != "ncu" ]; then
 python -m pytest tests -m gpu -q -x --tb=short -p no:cacheprovider -rP > $O/${TAG}_gputests.log 2>&1; echo "pytest rc=$?"; tail -5 $O/${TAG}_gputests.log
 python -c "import __graft_entry__ as g; g.smoke()" > $O/${TAG}_smoke.log 2>&1; echo "smoke rc=$?"; tail -2 $O/${TAG}_smoke.log
-python bench.py --steps 20 --warmup 3 > $O/${TAG}_bench.log 2>&1; echo "bench rc=$?"; tail -c 3800 $O/${TAG}_bench.log
-cp $O/bench_breakdown_n1.json $O/${TAG}_per_op.json
+python bench.py --steps 20 --warmup 3 --breakdown $O/${TAG}_per_op.json > $O/${TAG}_bench.log 2>&1; echo "bench rc=$?"; tail -c 3800 $O/${TAG}_bench.log
 fi
 if [ "$2" != "quick" ] && [ "$2" != "ncu" ]; then
 python bench.py --steps 20 --warmup 3 --no-cpu-baseline --no-yardstick --source-size 512 > $O/${TAG}_bench_src512.log 2>&1; tail -c 900 $O/${TAG}_bench_src512.log

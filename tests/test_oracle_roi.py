@@ -1,12 +1,13 @@
-"""CPU: pin the ROI oracle (oracle/roi_ref.py) against PIL itself and against golden vectors produced by the
-reference's own process_and_augment_roi (tests/golden/roi_golden.npz, see oracle/make_golden.py)."""
+"""CPU: pin the ROI oracle (oracle/roi_ref.py) against PIL itself and against golden vectors of the reference's
+process_and_augment_roi and CDDataAugmentation.transform (tests/golden/roi_golden.npz, roi_random_golden.npz,
+frontend_golden.npz; see oracle/make_golden.py)."""
 import os
 
 import numpy as np
 import pytest
 from PIL import Image
 
-from oracle import fixtures, roi_ref
+from oracle import fixtures, make_golden, roi_ref
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "roi_golden.npz")
 
@@ -54,65 +55,30 @@ def test_roi_matches_reference_golden():
         assert np.array_equal(got, rois[i]), f"case {i}"
 
 
-@pytest.mark.skipif(not __import__("oracle.ref_import", fromlist=["x"]).available(),
-                    reason="reference tree only exists in the build container")
+def _check_sampled_golden(name, k, got_u8):
+    """Case k of a sampled golden file: the stored output rows bit for bit, and the SHA-256 of the whole output."""
+    g = np.load(os.path.join(os.path.dirname(GOLD), name))
+    rows = make_golden.golden_rows()
+    assert np.array_equal(got_u8[rows], g["rows"][k]), f"{name} case {k}: sampled rows differ"
+    assert np.array_equal(make_golden.digest(got_u8), g["sha256"][k]), f"{name} case {k}: output digest differs"
+
+
 def test_roi_oracle_matches_live_reference_on_random_masks():
-    """The reference's own process_and_augment_roi (分类/util/roi.py:12-51, through a stub segmentation model that
-    returns prescribed logits) against the restatement, on random blob / border / single-pixel / empty masks."""
-    import torch
-    from oracle import ref_import
-    proc, Aug = ref_import.reference_roi()
-    aug = Aug(img_size=224, ori_size=224, crop=None, p_hflip=0.0, p_vflip=0.0, color_jitter_params=None,
-              long_mask=True)                                     # as 分类/test.py:113-116 constructs it
-
-    class Stub(torch.nn.Module):
-        def __init__(self, mask):
-            super().__init__()
-            self.mask = mask
-
-        def forward(self, x):
-            return (torch.from_numpy(self.mask).float() * 8.0 - 4.0)[None, None]
-
-    rng = np.random.default_rng(123)
-    masks = [np.zeros((224, 224), np.uint8)]
-    for _ in range(9):
-        m = np.zeros((224, 224), np.uint8)
-        kind = rng.integers(0, 3)
-        if kind == 0:                                             # a rectangle anywhere, possibly touching the border
-            y0, x0 = rng.integers(0, 220, 2)
-            m[y0:y0 + rng.integers(1, 120), x0:x0 + rng.integers(1, 120)] = 1
-        elif kind == 1:                                           # a few isolated pixels
-            for _ in range(rng.integers(1, 4)):
-                m[rng.integers(0, 224), rng.integers(0, 224)] = 1
-        else:                                                     # an ellipse
-            yy, xx = np.mgrid[:224, :224]
-            cy, cx, a, b = rng.integers(40, 184), rng.integers(40, 184), rng.integers(5, 80), rng.integers(5, 80)
-            m[((yy - cy) / a) ** 2 + ((xx - cx) / b) ** 2 <= 1.0] = 1
-        masks.append(m)
-    imgs = rng.random((len(masks), 3, 224, 224), dtype=np.float32)
+    """The reference's process_and_augment_roi (分类/util/roi.py:12-51, through a stub segmentation model that returns
+    prescribed logits) on random blob / border / single-pixel / empty masks, stored in
+    tests/golden/roi_random_golden.npz by oracle/make_golden.py, against the restatement."""
+    masks, imgs = make_golden.random_roi_cases()
     for i, m in enumerate(masks):
-        roi, se = proc(Stub(m), torch.from_numpy(imgs[i]), torch.device("cpu"), aug, f"{i}.png")
         want, box = roi_ref.roi_tensor(imgs[i], m)
-        assert tuple(roi.shape) == (3, 224, 224)
-        assert np.array_equal(np.round(roi.numpy() * 255).astype(np.uint8), np.round(want * 255).astype(np.uint8)), \
-            f"case {i}, box {box}"
-        assert np.abs(roi.numpy() - want).max() < 1e-6
+        assert want.shape == (3, 224, 224)
+        _check_sampled_golden("roi_random_golden.npz", i, np.round(want * 255).astype(np.uint8).transpose(1, 2, 0))
 
 
-@pytest.mark.skipif(not __import__("oracle.ref_import", fromlist=["x"]).available(),
-                    reason="reference tree only exists in the build container")
-@pytest.mark.parametrize("hs,ws", [(512, 512), (300, 400), (224, 224), (97, 131), (1000, 640)])
+@pytest.mark.parametrize("hs,ws", make_golden.FRONTEND_SIZES)
 def test_frontend_oracle_matches_live_reference_transform(hs, ws):
     """SURVEY §8(f) rank 1: the reference's CDDataAugmentation.transform in its inference configuration
-    (分类/util/data_utils.py:92-148; test.py:113-116) on a uint8 HWC source of any size == the oracle's Pillow
-    restatement followed by /255 (to_tensor), bit for bit."""
-    from oracle import ref_import
-    _, Aug = ref_import.reference_roi()
-    aug = Aug(img_size=224, ori_size=224, crop=None, p_hflip=0.0, p_vflip=0.0, color_jitter_params=None,
-              long_mask=True)
-    rng = np.random.default_rng(hs * 7 + ws)
-    src = rng.integers(0, 256, (hs, ws, 3), dtype=np.uint8)
-    ref = aug.transform(src).numpy()                                # float32 [3,224,224]
-    u8 = roi_ref.pil_resize_bilinear_u8(src, 224)                  # uint8 [224,224,3]
-    want = np.transpose(u8, (2, 0, 1)).astype(np.float32) / np.float32(255)
-    assert ref.shape == (3, 224, 224) and np.array_equal(ref, want)
+    (分类/util/data_utils.py:92-148; test.py:113-116) on a uint8 HWC source of any size, stored in
+    tests/golden/frontend_golden.npz by oracle/make_golden.py, == the oracle's Pillow restatement followed by /255
+    (to_tensor), bit for bit."""
+    u8 = roi_ref.pil_resize_bilinear_u8(make_golden.frontend_source(hs, ws), 224)     # uint8 [224,224,3]
+    _check_sampled_golden("frontend_golden.npz", make_golden.FRONTEND_SIZES.index((hs, ws)), u8)
