@@ -54,9 +54,9 @@ def transform_input(x):
 
 
 def googlenet_forward(sd, x, prefix="googlenet.", training=False):
-    """fp32 NCHW [B,3,224,224] in [0,1] -> logits [B, num_classes]."""
+    """fp32 NCHW [B,3,224,224] in [0,1] -> logits [B, num_classes] (a float64 input is evaluated in float64)."""
     g = {k[len(prefix):]: v for k, v in sd.items() if k.startswith(prefix)}
-    x = transform_input(x.float())
+    x = transform_input(x if x.dtype == torch.float64 else x.float())
     x = basic_conv(x, g, "conv1", stride=2, padding=3, training=training)
     x = F.max_pool2d(x, 3, stride=2, ceil_mode=True)
     x = basic_conv(x, g, "conv2", training=training)
