@@ -239,6 +239,47 @@ typedef struct ug_wavelet_desc {
   int B, H, W;
 } ug_wavelet_desc;
 
+/* Ragged batches: B images of different sizes packed back to back in one uint8 buffer, described by a device table of
+ * B entries (16 bytes each).  Image i's grayscale bytes start at byte px_offset of the packed buffer, its HWC RGB bytes
+ * at byte 3 * px_offset, so one table describes the gray input of ug_wavelet_ragged, its RGB output and the RGB input
+ * of ug_resize_ragged.  The table is input from outside the library (a plan image's host fills it): every kernel
+ * checks each entry before touching memory.  An entry with a negative offset, a side out of range or an extent past the
+ * buffer's capacity is "bad": the kernel reads nothing for it and sets status[i] = 1 (status[i] = 0 otherwise; status
+ * is an optional int32 [B]).  Packing, validation and chunking live in unet-goolenet_b200/util/ragged.py. */
+typedef struct ug_ragged_image {
+  long long px_offset;
+  int H, W;
+} ug_ragged_image;
+
+/* ug_resize_desc over a ragged batch of uint8 HWC sources: image i is index[i].H x index[i].W at src + 3*px_offset,
+ * 1 <= H, W <= 8*S, and 3*(px_offset + H*W) <= src_bytes.  Same arithmetic and outputs as ug_resize_desc (one launch,
+ * launch geometry sized for the largest source the descriptor allows, so it does not depend on the table).  A bad entry
+ * writes zeros to image i's outputs. */
+typedef struct ug_resize_ragged_desc {
+  const unsigned char* src;
+  const ug_ragged_image* index; /* device, [B] */
+  int* status;                  /* optional int32 [B] */
+  float* out_f32;
+  unsigned char* out_u8;
+  long long src_bytes;
+  int B, S;
+} ug_resize_ragged_desc;
+
+/* ug_wavelet_desc over a ragged batch of grayscale images: image i is index[i].H x index[i].W (H, W in [2, 32768]) at
+ * gray + px_offset with px_offset + H*W <= capacity_px; its pseudo-RGB result goes to out_u8 + 3*px_offset (out_u8
+ * holds 3*capacity_px bytes).  workspace: at least ug_wavelet_ragged_workspace_bytes(B, capacity_px) bytes.  A bad entry
+ * has no trustworthy destination: nothing is written for it except its status. */
+typedef struct ug_wavelet_ragged_desc {
+  const unsigned char* gray;
+  const ug_ragged_image* index; /* device, [B] */
+  int* status;                  /* optional int32 [B] */
+  unsigned char* out_u8;
+  void* workspace;
+  size_t workspace_bytes;
+  long long capacity_px;
+  int B;
+} ug_wavelet_ragged_desc;
+
 /* AdaptiveAvgPool2d(1) + Linear(C, ncls): in NHWC bf16 [B][HW][C], w fp32 [ncls][C], logits fp32 [B][ncls]. */
 typedef struct ug_head_desc {
   const void* in;
@@ -262,7 +303,9 @@ enum {
   UG_OP_STEM = 12,
   UG_OP_RESIZE = 13,
   UG_OP_WAVELET = 14,
-  UG_OP_S2D = 15
+  UG_OP_S2D = 15,
+  UG_OP_RESIZE_RAGGED = 16,
+  UG_OP_WAVELET_RAGGED = 17
 };
 
 typedef struct ug_op {
@@ -282,6 +325,8 @@ typedef struct ug_op {
     ug_resize_desc resize;
     ug_wavelet_desc wavelet;
     ug_s2d_desc s2d;
+    ug_resize_ragged_desc resize_ragged; /* both smaller than ug_conv_desc: sizeof(ug_op) is unchanged */
+    ug_wavelet_ragged_desc wavelet_ragged;
   } u;
 } ug_op;
 
@@ -306,7 +351,10 @@ int ug_stem(ug_handle h, const ug_stem_desc* d, void* stream);
 int ug_resize_u8(ug_handle h, const ug_resize_desc* d, void* stream);
 int ug_wavelet(ug_handle h, const ug_wavelet_desc* d, void* stream);
 int ug_s2d_pack(ug_handle h, const ug_s2d_desc* d, void* stream);
+int ug_resize_ragged(ug_handle h, const ug_resize_ragged_desc* d, void* stream);
+int ug_wavelet_ragged(ug_handle h, const ug_wavelet_ragged_desc* d, void* stream);
 size_t ug_wavelet_workspace_bytes(int B, int H, int W);
+size_t ug_wavelet_ragged_workspace_bytes(int B, long long capacity_px);
 
 /* Programs: a validated op list with tensor maps and launch geometry prepared once; run = launches only. */
 int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out);
@@ -351,7 +399,9 @@ int ug_program_run_host_pipelined(ug_handle h, ug_program p, const ug_copy* h2d,
  *   "cls_logits" / "logits" / "u8") -> ug_plan_destroy.     (examples/run_plan.c is exactly this.)
  * Named io buffers of a pipeline plan: "x_in" f32 [B,3,224,224] (or "src_u8" u8 [B,Hs,Ws,3] for plans with the device
  * front-end), "logits" f32 [B,1,224,224], "mask" u8 [B,224,224], "boxes" i32 [B,4], "u8" u8 [B,224,224,3] (the ROI
- * crops), "cls_logits" f32 [B,6]. */
+ * crops), "cls_logits" f32 [B,6].  A ragged plan (export_plan(B, source="ragged", capacity=P)) takes packed sources
+ * instead: "src_u8" u8 [P*3] (images back to back, HWC), "src_index" ug_ragged_image [B] and reports "src_status"
+ * i32 [B] (1 = the table entry was rejected and the image's outputs are those of a zero input). */
 typedef struct ug_plan_s* ug_plan;
 /* Parses the image (host memory, may be freed afterwards), allocates ONE device arena for every buffer of the plan
  * (ug_plan_device_bytes), uploads the constants, relocates the op list and prepares the program. */

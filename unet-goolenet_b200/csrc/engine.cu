@@ -53,6 +53,8 @@ static int run_simple(ug_engine* h, const ug_op* op, cudaStream_t s) {
     case UG_OP_RESIZE: return launch_resize_u8(h, &op->u.resize, s);
     case UG_OP_WAVELET: return launch_wavelet(h, &op->u.wavelet, s);
     case UG_OP_S2D: return launch_s2d_pack(h, &op->u.s2d, s);
+    case UG_OP_RESIZE_RAGGED: return launch_resize_ragged(h, &op->u.resize_ragged, s);
+    case UG_OP_WAVELET_RAGGED: return launch_wavelet_ragged(h, &op->u.wavelet_ragged, s);
     default: return set_error(h, UG_EINVAL, "unknown op kind %d", op->kind);
   }
 }
@@ -135,6 +137,8 @@ UG_SIMPLE_ENTRY(ug_head, ug_head_desc, launch_head)
 UG_SIMPLE_ENTRY(ug_resize_u8, ug_resize_desc, launch_resize_u8)
 UG_SIMPLE_ENTRY(ug_wavelet, ug_wavelet_desc, launch_wavelet)
 UG_SIMPLE_ENTRY(ug_s2d_pack, ug_s2d_desc, launch_s2d_pack)
+UG_SIMPLE_ENTRY(ug_resize_ragged, ug_resize_ragged_desc, launch_resize_ragged)
+UG_SIMPLE_ENTRY(ug_wavelet_ragged, ug_wavelet_ragged_desc, launch_wavelet_ragged)
 
 int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out) {
   if (!h || !ops || n_ops <= 0 || !out) return UG_EINVAL;
@@ -162,7 +166,7 @@ int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out)
         delete p;
         return rc;
       }
-    } else if (po.kind < UG_OP_CONV || po.kind > UG_OP_S2D) {
+    } else if (po.kind < UG_OP_CONV || po.kind > UG_OP_WAVELET_RAGGED) {
       delete p;
       return set_error(h, UG_EINVAL, "op %d: unknown kind %d", i, po.kind);
     }

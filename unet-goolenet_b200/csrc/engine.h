@@ -21,7 +21,7 @@ struct ug_engine {
   // "already raised" flags are per handle (= per device), not process-wide
   bool attr_gemm = false, attr_multi = false, attr_pair = false, attr_stem = false, attr_attn = false;
   int max_pairs = -1;  // co-resident clusters of two ~200 KB CTAs on this device (cudaOccupancyMaxActiveClusters), -1 = not queried
-  size_t attr_resize = 0, attr_crop = 0;
+  size_t attr_resize = 0, attr_crop = 0, attr_ragged = 0;
 };
 
 namespace ug {
@@ -165,5 +165,7 @@ int launch_head(ug_engine* h, const ug_head_desc* d, cudaStream_t s);
 int launch_resize_u8(ug_engine* h, const ug_resize_desc* d, cudaStream_t s);
 int launch_wavelet(ug_engine* h, const ug_wavelet_desc* d, cudaStream_t s);
 int launch_s2d_pack(ug_engine* h, const ug_s2d_desc* d, cudaStream_t s);
+int launch_resize_ragged(ug_engine* h, const ug_resize_ragged_desc* d, cudaStream_t s);
+int launch_wavelet_ragged(ug_engine* h, const ug_wavelet_ragged_desc* d, cudaStream_t s);
 
 }  // namespace ug

@@ -729,6 +729,7 @@ __device__ __forceinline__ int clip8(int v) {
 // One block per (group of R output rows, image): the horizontal pass of the source rows those output rows need is
 // kept in shared memory as uint8 (exactly Pillow's intermediate image), the vertical pass reads it from there.
 static constexpr int kRsMaxTaps = 17;   // support <= 8: source side up to 8 * S
+static constexpr int kRsMaxSide = 8;    // (kRsMaxTaps - 1) / 2
 static constexpr int kRsRows = 8;       // output rows per block
 
 struct RsCoef {
@@ -767,12 +768,20 @@ __device__ void pil_coef_general(int in_size, int out_size, int xx, RsCoef* c) {
   }
 }
 
-// kCrop = false: source = uint8 HWC images (ug_resize_desc).  kCrop = true: source = the box (x0,y0,x1,y1) of an fp32
+// Source modes.  kUniform: uint8 HWC images of one size (ug_resize_desc).  kCrop: the box (x0,y0,x1,y1) of an fp32
 // NCHW image in [0,1], quantised as (x*255).astype(uint8) with the channel order reversed (roi.py:39-44), i.e. the
-// ROI stage (ug_cropresize_desc); d.src is unused, `img` / `boxes` / `IH` / `IW` describe the float image.
-template <bool kCrop>
+// ROI stage (ug_cropresize_desc); d.src is unused, `img` / `boxes` / `IH` / `IW` describe the float image.  kRagged:
+// uint8 HWC images of different sizes (ug_resize_ragged_desc); image n's size and offset come from rg.index[n].
+enum { kUniform = 0, kCrop = 1, kRagged = 2 };
+struct RaggedSrc {
+  const ug_ragged_image* index;
+  int* status;
+  long long src_bytes;
+};
+
+template <int kMode>
 __global__ void __launch_bounds__(256) resize_u8_kernel(ug_resize_desc d, int max_src_rows, const float* __restrict__ img,
-                                                        const int* __restrict__ boxes, int IH, int IW) {
+                                                        const int* __restrict__ boxes, int IH, int IW, RaggedSrc rg) {
   pdl_wait();  // programmatic dependent launch: see common.cuh
   pdl_launch_dependents();
   extern __shared__ unsigned char rs_smem[];
@@ -783,25 +792,49 @@ __global__ void __launch_bounds__(256) resize_u8_kernel(ug_resize_desc d, int ma
   const int oy0 = blockIdx.x * kRsRows;
   const int rows = min(kRsRows, d.S - oy0);
   int bx0 = 0, by0 = 0;
-  if (kCrop) {
+  long long src_off = (long long)n * d.Hs * d.Ws * 3;
+  if (kMode == kCrop) {
     bx0 = boxes[n * 4 + 0];
     by0 = boxes[n * 4 + 1];
     d.Ws = boxes[n * 4 + 2] - bx0;
     d.Hs = boxes[n * 4 + 3] - by0;
+  }
+  if (kMode == kRagged) {
+    // the table comes from outside the library: check the entry before reading a byte of the image
+    const ug_ragged_image e = rg.index[n];
+    const int smax = kRsMaxSide * d.S;
+    const bool ok = e.px_offset >= 0 && e.H >= 1 && e.W >= 1 && e.H <= smax && e.W <= smax &&
+                    e.px_offset <= rg.src_bytes / 3 && (long long)e.H * e.W * 3 <= rg.src_bytes - 3 * e.px_offset;
+    if (rg.status && blockIdx.x == 0 && threadIdx.x == 0) rg.status[n] = ok ? 0 : 1;
+    if (!ok) {  // this block's output rows of a rejected image are zeros
+      for (int t = threadIdx.x; t < rows * d.S; t += blockDim.x) {
+        const int oy = oy0 + t / d.S, ox = t % d.S;
+        if (d.out_u8) {
+          unsigned char* o = d.out_u8 + (((long long)n * d.S + oy) * d.S + ox) * 3;
+          o[0] = o[1] = o[2] = 0;
+        }
+        if (d.out_f32)
+          for (int c = 0; c < 3; ++c) d.out_f32[(((long long)n * 3 + c) * d.S + oy) * d.S + ox] = 0.0f;
+      }
+      return;
+    }
+    d.Hs = e.H;
+    d.Ws = e.W;
+    src_off = 3 * e.px_offset;
   }
   for (int i = threadIdx.x; i < d.S; i += blockDim.x) pil_coef_general(d.Ws, d.S, i, &s_h[i]);
   if (threadIdx.x < rows) pil_coef_general(d.Hs, d.S, oy0 + threadIdx.x, &s_v[threadIdx.x]);
   __syncthreads();
   const int sy0 = s_v[0].xmin;                                          // first / one-past-last source row needed
   const int sy1 = s_v[rows - 1].xmin + s_v[rows - 1].n;
-  const unsigned char* src = kCrop ? nullptr : d.src + (long long)n * d.Hs * d.Ws * 3;
-  const float* fimg = kCrop ? img + (long long)n * 3 * IH * IW : nullptr;
+  const unsigned char* src = kMode == kCrop ? nullptr : d.src + src_off;
+  const float* fimg = kMode == kCrop ? img + (long long)n * 3 * IH * IW : nullptr;
   const int row_elems = d.S * 3;
   for (int t = threadIdx.x; t < (sy1 - sy0) * d.S; t += blockDim.x) {   // horizontal pass (one output pixel, 3 ch)
     const int r = t / d.S, ox = t - r * d.S;
     const RsCoef& hc = s_h[ox];
     int a0 = 1 << (kPrecBits - 1), a1 = a0, a2 = a0;
-    if (kCrop) {
+    if (kMode == kCrop) {
       // (roi*255).astype(uint8): fp32 multiply, truncate; output channel c reads plane 2-c (cv2.COLOR_BGR2RGB)
       const float* p0 = fimg + ((long long)(by0 + sy0 + r)) * IW + bx0 + hc.xmin;
       const long long plane = (long long)IH * IW;
@@ -865,13 +898,36 @@ int launch_resize_u8(ug_engine* h, const ug_resize_desc* d, cudaStream_t s) {
   const size_t smem = (size_t)(d->S + kRsRows) * sizeof(RsCoef) + (size_t)max_rows * d->S * 3;
   if (smem > h->attr_resize) {
     if (smem > 200 * 1024) return set_error(h, UG_EUNSUPPORTED, "resize: shared memory request %zu too large", smem);
-    cudaError_t e = cudaFuncSetAttribute((const void*)resize_u8_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute((const void*)resize_u8_kernel<kUniform>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(resize_u8_kernel)");
     h->attr_resize = smem;
   }
-  launch_pdl(h, resize_u8_kernel<false>, dim3(cdiv(d->S, kRsRows), d->B), 256, smem, s, *d, max_rows, nullptr, nullptr, 0, 0);
+  launch_pdl(h, resize_u8_kernel<kUniform>, dim3(cdiv(d->S, kRsRows), d->B), 256, smem, s, *d, max_rows, nullptr, nullptr,
+             0, 0, RaggedSrc{});
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "resize_u8 launch");
+}
+
+// Ragged front-end: the uniform kernel with per-image sizes from the table.  Shared memory and grid are sized for the
+// largest source the descriptor admits (sides up to kRsMaxSide * S), so the launch does not depend on the table.
+int launch_resize_ragged(ug_engine* h, const ug_resize_ragged_desc* d, cudaStream_t s) {
+  if (!d->src || !d->index || (!d->out_f32 && !d->out_u8) || d->B <= 0 || d->S <= 0 || d->S > 512 || d->src_bytes < 0)
+    return set_error(h, UG_EINVAL, "resize_ragged: bad args (S <= 512)");
+  const double sc = kRsMaxSide;
+  const int max_rows = (int)ceil((kRsRows - 1) * sc + 2.0 * sc + 3.0);
+  const size_t smem = (size_t)(d->S + kRsRows) * sizeof(RsCoef) + (size_t)max_rows * d->S * 3;
+  if (smem > h->attr_ragged) {
+    if (smem > 200 * 1024) return set_error(h, UG_EUNSUPPORTED, "resize_ragged: shared memory request %zu too large", smem);
+    cudaError_t e = cudaFuncSetAttribute((const void*)resize_u8_kernel<kRagged>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(resize_u8_kernel<ragged>)");
+    h->attr_ragged = smem;
+  }
+  ug_resize_desc r;
+  r.src = d->src; r.out_f32 = d->out_f32; r.out_u8 = d->out_u8; r.B = d->B; r.Hs = 0; r.Ws = 0; r.S = d->S;
+  launch_pdl(h, resize_u8_kernel<kRagged>, dim3(cdiv(d->S, kRsRows), d->B), 256, smem, s, r, max_rows, nullptr, nullptr,
+             0, 0, RaggedSrc{d->index, d->status, d->src_bytes});
+  h->launches++;
+  return check_cuda(h, cudaGetLastError(), "resize_ragged launch");
 }
 
 // ROI stage (roi.py:39-44 + data_utils.py:102,146-147): the same two-pass kernel reading the box of the float image.
@@ -886,13 +942,14 @@ int launch_cropresize(ug_engine* h, const ug_cropresize_desc* d, cudaStream_t s)
   const size_t smem = (size_t)(d->S + kRsRows) * sizeof(RsCoef) + (size_t)max_rows * d->S * 3;
   if (smem > h->attr_crop) {
     if (smem > 200 * 1024) return set_error(h, UG_EUNSUPPORTED, "cropresize: shared memory request %zu too large", smem);
-    cudaError_t e = cudaFuncSetAttribute((const void*)resize_u8_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute((const void*)resize_u8_kernel<kCrop>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(resize_u8_kernel<crop>)");
     h->attr_crop = smem;
   }
   ug_resize_desc r;
   r.src = nullptr; r.out_f32 = nullptr; r.out_u8 = d->out_u8; r.B = d->B; r.Hs = d->H; r.Ws = d->W; r.S = d->S;
-  launch_pdl(h, resize_u8_kernel<true>, dim3(cdiv(d->S, kRsRows), d->B), 256, smem, s, r, max_rows, d->img, d->boxes, d->H, d->W);
+  launch_pdl(h, resize_u8_kernel<kCrop>, dim3(cdiv(d->S, kRsRows), d->B), 256, smem, s, r, max_rows, d->img, d->boxes,
+             d->H, d->W, RaggedSrc{});
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "cropresize launch");
 }

@@ -9,6 +9,7 @@
 //                              INTER_LINEAR restated bit-exactly: half-pixel centres, replicated border, fused lerp)
 //   K3 wavelet_up_kernel<1>    recomputes the up-sampling, applies the reference's normalize()
 //                              ((x - min) / max(x - min) * 255 truncated to uint8) and writes HWC
+// The wavelet_ragged_* kernels run the same per-image functions over a ragged batch (ug_wavelet_ragged_desc).
 // All three are memory-light (one 8-bit image in, three out).  Non-negative floats are reduced with integer atomics
 // on their bit patterns (order-preserving for x >= 0; every value here is >= 0).
 #include <cfloat>
@@ -43,29 +44,25 @@ __device__ __forceinline__ void block_minmax(float mn, float mx, unsigned* gmn, 
   }
 }
 
+// The per-image arithmetic below is shared by the uniform kernels (one [B][H][W] batch) and the ragged ones (image n
+// described by a table entry); each __global__ kernel only locates image n and calls it.
+
 // min / max of the gray image (needed first: the reference rescales by 255 when max <= 1)
-__global__ void __launch_bounds__(256) wavelet_gray_stats_kernel(const unsigned char* __restrict__ gray, WvStats* st,
-                                                                 int HW) {
-  const int n = blockIdx.y;
-  const unsigned char* g = gray + (long long)n * HW;
+__device__ __forceinline__ void wv_gray_minmax(const unsigned char* __restrict__ g, int HW, WvStats* st) {
   float mn = FLT_MAX, mx = 0.0f;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < HW; i += gridDim.x * blockDim.x) {
     const float v = (float)g[i];
     mn = fminf(mn, v);
     mx = fmaxf(mx, v);
   }
-  block_minmax(mn, mx, &st[n].gmin, &st[n].gmax);
+  block_minmax(mn, mx, &st->gmin, &st->gmax);
 }
 
-__global__ void __launch_bounds__(256) wavelet_dwt_kernel(const unsigned char* __restrict__ gray, const WvStats* st,
-                                                          float* __restrict__ cA, float* __restrict__ hf, int H, int W,
-                                                          int h2, int w2) {
-  const int n = blockIdx.y;
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= h2 * w2) return;
+// half-resolution pixel i of cA and of the detail magnitude
+__device__ __forceinline__ void wv_dwt_px(const unsigned char* __restrict__ g, const WvStats* st, float* __restrict__ cA,
+                                          float* __restrict__ hf, int H, int W, int w2, int i) {
   const int oy = i / w2, ox = i - oy * w2;
-  const float sc = __uint_as_float(st[n].gmax) <= 1.0f ? 255.0f : 1.0f;  // `if gray_img.max() <= 1.0: *= 255`
-  const unsigned char* g = gray + (long long)n * H * W;
+  const float sc = __uint_as_float(st->gmax) <= 1.0f ? 255.0f : 1.0f;  // `if gray_img.max() <= 1.0: *= 255`
   const int y0 = 2 * oy, y1 = min(2 * oy + 1, H - 1), x0 = 2 * ox, x1 = min(2 * ox + 1, W - 1);  // symmetric extension
   const float p00 = __fmul_rn((float)g[y0 * W + x0], sc), p01 = __fmul_rn((float)g[y0 * W + x1], sc);
   const float p10 = __fmul_rn((float)g[y1 * W + x0], sc), p11 = __fmul_rn((float)g[y1 * W + x1], sc);
@@ -79,10 +76,9 @@ __global__ void __launch_bounds__(256) wavelet_dwt_kernel(const unsigned char* _
   const float ad = __fadd_rn(__fmul_rn(-kHaar, a_x1), __fmul_rn(kHaar, a_x0));
   const float da = __fadd_rn(__fmul_rn(kHaar, d_x1), __fmul_rn(kHaar, d_x0));
   const float dd = __fadd_rn(__fmul_rn(-kHaar, d_x1), __fmul_rn(kHaar, d_x0));
-  const long long o = (long long)n * h2 * w2 + i;
-  cA[o] = aa;
+  cA[i] = aa;
   // np.sqrt(cH**2 + cV**2 + cD**2) with cH = da, cV = ad, cD = dd
-  hf[o] = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(da, da), __fmul_rn(ad, ad)), __fmul_rn(dd, dd)));
+  hf[i] = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(da, da), __fmul_rn(ad, ad)), __fmul_rn(dd, dd)));
 }
 
 // cv2.resize INTER_LINEAR coordinate (OpenCV 4.x): fx = (d + 0.5) * scale - 0.5 in double; s = floor(fx); the
@@ -114,24 +110,22 @@ __device__ __forceinline__ float cv_bilinear(const float* __restrict__ m, int w2
   return __fmaf_rn(__fsub_rn(r1, r0), wy, r0);                           // vertical pass
 }
 
+// kWrite = false: min / max of the two up-sampled maps into st.  kWrite = true: normalise and write HWC to out.
 template <bool kWrite>
-__global__ void __launch_bounds__(256) wavelet_up_kernel(const unsigned char* __restrict__ gray, WvStats* st,
-                                                         const float* __restrict__ cA, const float* __restrict__ hf,
-                                                         unsigned char* __restrict__ out, int H, int W, int h2, int w2) {
-  const int n = blockIdx.y;
+__device__ __forceinline__ void wv_up(const unsigned char* __restrict__ g, WvStats* st, const float* __restrict__ a,
+                                      const float* __restrict__ hh, unsigned char* __restrict__ out, int H, int W, int h2,
+                                      int w2) {
   const double sx = 1.0 / ((double)W / w2), sy = 1.0 / ((double)H / h2);  // cv2: scale = 1 / (dsize / ssize)
-  const float* a = cA + (long long)n * h2 * w2;
-  const float* hh = hf + (long long)n * h2 * w2;
   float lmn = FLT_MAX, lmx = 0.0f, hmn = FLT_MAX, hmx = 0.0f;
   float gmin = 0.f, gmax = 0.f, lmin = 0.f, lmax = 0.f, hmin = 0.f, hmax = 0.f, gsc = 1.0f;
   if (kWrite) {
-    gsc = __uint_as_float(st[n].gmax) <= 1.0f ? 255.0f : 1.0f;
-    gmin = __fmul_rn(__uint_as_float(st[n].gmin), gsc);
-    gmax = __fmul_rn(__uint_as_float(st[n].gmax), gsc);
-    lmin = __uint_as_float(st[n].lmin);
-    lmax = __uint_as_float(st[n].lmax);
-    hmin = __uint_as_float(st[n].hmin);
-    hmax = __uint_as_float(st[n].hmax);
+    gsc = __uint_as_float(st->gmax) <= 1.0f ? 255.0f : 1.0f;
+    gmin = __fmul_rn(__uint_as_float(st->gmin), gsc);
+    gmax = __fmul_rn(__uint_as_float(st->gmax), gsc);
+    lmin = __uint_as_float(st->lmin);
+    lmax = __uint_as_float(st->lmax);
+    hmin = __uint_as_float(st->hmin);
+    hmax = __uint_as_float(st->hmax);
   }
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < H * W; i += gridDim.x * blockDim.x) {
     const int y = i / W, x = i - y * W;
@@ -148,10 +142,10 @@ __global__ void __launch_bounds__(256) wavelet_up_kernel(const unsigned char* __
       hmx = fmaxf(hmx, hi);
     } else {
       // normalize(): x = x - min; if max(x) != 0: x = x / max(x); (x * 255).astype(uint8)   (fp32, truncation)
-      const float g = __fmul_rn((float)gray[(long long)n * H * W + i], gsc);
-      float v[3] = {__fadd_rn(g, -gmin), __fadd_rn(lo, -lmin), __fadd_rn(hi, -hmin)};
+      const float gv = __fmul_rn((float)g[i], gsc);
+      float v[3] = {__fadd_rn(gv, -gmin), __fadd_rn(lo, -lmin), __fadd_rn(hi, -hmin)};
       const float mx[3] = {__fadd_rn(gmax, -gmin), __fadd_rn(lmax, -lmin), __fadd_rn(hmax, -hmin)};
-      unsigned char* o = out + ((long long)n * H * W + i) * 3;
+      unsigned char* o = out + (long long)i * 3;
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
         if (mx[c] != 0.0f) v[c] = __fdiv_rn(v[c], mx[c]);
@@ -160,9 +154,102 @@ __global__ void __launch_bounds__(256) wavelet_up_kernel(const unsigned char* __
     }
   }
   if (!kWrite) {
-    block_minmax(lmn, lmx, &st[n].lmin, &st[n].lmax);
-    block_minmax(hmn, hmx, &st[n].hmin, &st[n].hmax);
+    block_minmax(lmn, lmx, &st->lmin, &st->lmax);
+    block_minmax(hmn, hmx, &st->hmin, &st->hmax);
   }
+}
+
+// ---------------------------------------------------------------- uniform batch [B][H][W]
+__global__ void __launch_bounds__(256) wavelet_gray_stats_kernel(const unsigned char* __restrict__ gray, WvStats* st,
+                                                                 int HW) {
+  const int n = blockIdx.y;
+  wv_gray_minmax(gray + (long long)n * HW, HW, &st[n]);
+}
+
+__global__ void __launch_bounds__(256) wavelet_dwt_kernel(const unsigned char* __restrict__ gray, const WvStats* st,
+                                                          float* __restrict__ cA, float* __restrict__ hf, int H, int W,
+                                                          int h2, int w2) {
+  const int n = blockIdx.y;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= h2 * w2) return;
+  const long long o = (long long)n * h2 * w2;
+  wv_dwt_px(gray + (long long)n * H * W, &st[n], cA + o, hf + o, H, W, w2, i);
+}
+
+template <bool kWrite>
+__global__ void __launch_bounds__(256) wavelet_up_kernel(const unsigned char* __restrict__ gray, WvStats* st,
+                                                         const float* __restrict__ cA, const float* __restrict__ hf,
+                                                         unsigned char* __restrict__ out, int H, int W, int h2, int w2) {
+  const int n = blockIdx.y;
+  const long long o = (long long)n * h2 * w2;
+  wv_up<kWrite>(gray + (long long)n * H * W, &st[n], cA + o, hf + o, kWrite ? out + (long long)n * H * W * 3 : nullptr, H,
+                W, h2, w2);
+}
+
+// ---------------------------------------------------------------- ragged batch (ug_wavelet_ragged_desc)
+// Image n: gray + off, out + 3*off, and its cA / detail maps at workspace offset `off` (h2*w2 <= H*W, so the slices of
+// disjoint images are disjoint).  The table is checked entry by entry; a bad entry is skipped by every kernel.
+static constexpr int kWvMaxSide = 32768;
+
+struct WvRagged {
+  const ug_ragged_image* index;
+  int* status;
+  long long capacity_px;
+};
+
+__device__ __forceinline__ bool wv_entry(const WvRagged& rg, int n, ug_ragged_image* e) {
+  *e = rg.index[n];
+  return e->px_offset >= 0 && e->H >= 2 && e->W >= 2 && e->H <= kWvMaxSide && e->W <= kWvMaxSide &&
+         e->px_offset <= rg.capacity_px && (long long)e->H * e->W <= rg.capacity_px - e->px_offset;
+}
+
+__global__ void wavelet_ragged_init_kernel(WvStats* st, WvRagged rg, int B) {
+  pdl_wait();  // programmatic dependent launch: see common.cuh
+  pdl_launch_dependents();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < B) {
+    st[i].gmin = st[i].lmin = st[i].hmin = 0x7F7FFFFFu;  // FLT_MAX
+    st[i].gmax = st[i].lmax = st[i].hmax = 0u;
+    ug_ragged_image e;
+    const bool ok = wv_entry(rg, i, &e);
+    if (rg.status) rg.status[i] = ok ? 0 : 1;
+  }
+}
+
+__global__ void __launch_bounds__(256) wavelet_ragged_gray_stats_kernel(const unsigned char* __restrict__ gray,
+                                                                        WvStats* st, WvRagged rg) {
+  pdl_wait();
+  pdl_launch_dependents();
+  const int n = blockIdx.y;
+  ug_ragged_image e;
+  if (!wv_entry(rg, n, &e)) return;
+  wv_gray_minmax(gray + e.px_offset, e.H * e.W, &st[n]);
+}
+
+__global__ void __launch_bounds__(256) wavelet_ragged_dwt_kernel(const unsigned char* __restrict__ gray,
+                                                                 const WvStats* st, float* __restrict__ cA,
+                                                                 float* __restrict__ hf, WvRagged rg) {
+  pdl_wait();
+  pdl_launch_dependents();
+  const int n = blockIdx.y;
+  ug_ragged_image e;
+  if (!wv_entry(rg, n, &e)) return;
+  const int h2 = (e.H + 1) / 2, w2 = (e.W + 1) / 2;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < h2 * w2; i += gridDim.x * blockDim.x)
+    wv_dwt_px(gray + e.px_offset, &st[n], cA + e.px_offset, hf + e.px_offset, e.H, e.W, w2, i);
+}
+
+template <bool kWrite>
+__global__ void __launch_bounds__(256) wavelet_ragged_up_kernel(const unsigned char* __restrict__ gray, WvStats* st,
+                                                                const float* __restrict__ cA, const float* __restrict__ hf,
+                                                                unsigned char* __restrict__ out, WvRagged rg) {
+  pdl_wait();
+  pdl_launch_dependents();
+  const int n = blockIdx.y;
+  ug_ragged_image e;
+  if (!wv_entry(rg, n, &e)) return;
+  wv_up<kWrite>(gray + e.px_offset, &st[n], cA + e.px_offset, hf + e.px_offset, kWrite ? out + 3 * e.px_offset : nullptr,
+                e.H, e.W, (e.H + 1) / 2, (e.W + 1) / 2);
 }
 
 static inline int cdivw(long long a, long long b) { return (int)((a + b - 1) / b); }
@@ -187,10 +274,43 @@ int launch_wavelet(ug_engine* h, const ug_wavelet_desc* d, cudaStream_t s) {
   return check_cuda(h, cudaGetLastError(), "wavelet launch");
 }
 
+int launch_wavelet_ragged(ug_engine* h, const ug_wavelet_ragged_desc* d, cudaStream_t s) {
+  if (!d->gray || !d->index || !d->out_u8 || !d->workspace || d->B <= 0 || d->capacity_px <= 0)
+    return set_error(h, UG_EINVAL, "wavelet_ragged: bad args");
+  const size_t need = ug_wavelet_ragged_workspace_bytes(d->B, d->capacity_px);
+  if (d->workspace_bytes < need)
+    return set_error(h, UG_EINVAL, "wavelet_ragged: workspace too small (%zu < %zu)", d->workspace_bytes, need);
+  WvStats* st = static_cast<WvStats*>(d->workspace);
+  float* cA = reinterpret_cast<float*>(st + ((d->B + 3) / 4) * 4);
+  float* hf = cA + d->capacity_px;
+  const WvRagged rg{d->index, d->status, d->capacity_px};
+  // The table lives on the device, so the grid is sized from the capacity (a bound on the largest image) and every
+  // kernel strides over its image; blocks past an image's extent do no work.
+  const dim3 grid(std::min(cdivw(d->capacity_px, 256), 64), d->B);
+  int rc = check_cuda(h, launch_pdl(h, wavelet_ragged_init_kernel, cdivw(d->B, 128), 128, 0, s, st, rg, d->B), "wavelet_ragged init");
+  if (rc == UG_OK)
+    rc = check_cuda(h, launch_pdl(h, wavelet_ragged_gray_stats_kernel, grid, 256, 0, s, d->gray, st, rg), "wavelet_ragged stats");
+  if (rc == UG_OK)
+    rc = check_cuda(h, launch_pdl(h, wavelet_ragged_dwt_kernel, grid, 256, 0, s, d->gray, st, cA, hf, rg), "wavelet_ragged dwt");
+  if (rc == UG_OK)
+    rc = check_cuda(h, launch_pdl(h, wavelet_ragged_up_kernel<false>, grid, 256, 0, s, d->gray, st, cA, hf, nullptr, rg),
+                    "wavelet_ragged up");
+  if (rc == UG_OK)
+    rc = check_cuda(h, launch_pdl(h, wavelet_ragged_up_kernel<true>, grid, 256, 0, s, d->gray, st, cA, hf, d->out_u8, rg),
+                    "wavelet_ragged up");
+  h->launches += 5;
+  return rc;
+}
+
 }  // namespace ug
 
 extern "C" size_t ug_wavelet_workspace_bytes(int B, int H, int W) {
   if (B <= 0 || H <= 0 || W <= 0) return 0;
   const size_t h2 = (H + 1) / 2, w2 = (W + 1) / 2;
   return (size_t)((B + 3) / 4) * 4 * sizeof(ug::WvStats) + 2 * (size_t)B * h2 * w2 * sizeof(float);
+}
+
+extern "C" size_t ug_wavelet_ragged_workspace_bytes(int B, long long capacity_px) {
+  if (B <= 0 || capacity_px <= 0) return 0;
+  return (size_t)((B + 3) / 4) * 4 * sizeof(ug::WvStats) + 2 * (size_t)capacity_px * sizeof(float);
 }

@@ -21,6 +21,7 @@ EPI_STORE, EPI_ADD, EPI_GATE, EPI_OUTC = 0, 1, 2, 3
 # (2 and 10 were round 1's stand-alone im2col packs; the numbers stay retired, see ugnet.h)
 OP_CONV, OP_POOL, OP_LAYERNORM, OP_ATTN, OP_CHANSTATS, OP_GATE, OP_BBOX, OP_CROPRESIZE = 1, 3, 4, 5, 6, 7, 8, 9
 OP_HEAD, OP_STEM, OP_RESIZE, OP_WAVELET, OP_S2D = 11, 12, 13, 14, 15
+OP_RESIZE_RAGGED, OP_WAVELET_RAGGED = 16, 17
 
 _vp, _i, _f, _ll = C.c_void_p, C.c_int, C.c_float, C.c_longlong
 
@@ -93,11 +94,22 @@ class S2dDesc(C.Structure):
     _fields_ = [("in_u8", _vp), ("in_f32", _vp), ("out", _vp), ("B", _i), ("S", _i)]
 
 
+class ResizeRaggedDesc(C.Structure):
+    _fields_ = [("src", _vp), ("index", _vp), ("status", _vp), ("out_f32", _vp), ("out_u8", _vp), ("src_bytes", _ll),
+                ("B", _i), ("S", _i)]
+
+
+class WaveletRaggedDesc(C.Structure):
+    _fields_ = [("gray", _vp), ("index", _vp), ("status", _vp), ("out_u8", _vp), ("workspace", _vp),
+                ("workspace_bytes", C.c_size_t), ("capacity_px", _ll), ("B", _i)]
+
+
 class _OpUnion(C.Union):
     _fields_ = [("conv", ConvDesc), ("pool", PoolDesc), ("ln", LayerNormDesc),
                 ("attn", AttnDesc), ("stats", ChanStatsDesc), ("gate", GateDesc), ("bbox", BBoxDesc),
                 ("crop", CropResizeDesc), ("head", HeadDesc), ("stem", StemDesc),
-                ("resize", ResizeDesc), ("wavelet", WaveletDesc), ("s2d", S2dDesc)]
+                ("resize", ResizeDesc), ("wavelet", WaveletDesc), ("s2d", S2dDesc),
+                ("resize_ragged", ResizeRaggedDesc), ("wavelet_ragged", WaveletRaggedDesc)]
 
 
 class Op(C.Structure):
@@ -110,21 +122,25 @@ class Copy(C.Structure):
 
 _KIND_FIELD = {OP_CONV: "conv", OP_POOL: "pool", OP_LAYERNORM: "ln", OP_ATTN: "attn",
                OP_CHANSTATS: "stats", OP_GATE: "gate", OP_BBOX: "bbox", OP_CROPRESIZE: "crop",
-               OP_HEAD: "head", OP_STEM: "stem", OP_RESIZE: "resize", OP_WAVELET: "wavelet", OP_S2D: "s2d"}
+               OP_HEAD: "head", OP_STEM: "stem", OP_RESIZE: "resize", OP_WAVELET: "wavelet", OP_S2D: "s2d",
+               OP_RESIZE_RAGGED: "resize_ragged", OP_WAVELET_RAGGED: "wavelet_ragged"}
 _DESC_KIND = {ConvDesc: OP_CONV, PoolDesc: OP_POOL, LayerNormDesc: OP_LAYERNORM,
               AttnDesc: OP_ATTN, ChanStatsDesc: OP_CHANSTATS, GateDesc: OP_GATE, BBoxDesc: OP_BBOX,
               CropResizeDesc: OP_CROPRESIZE, HeadDesc: OP_HEAD, StemDesc: OP_STEM,
-              ResizeDesc: OP_RESIZE, WaveletDesc: OP_WAVELET, S2dDesc: OP_S2D}
+              ResizeDesc: OP_RESIZE, WaveletDesc: OP_WAVELET, S2dDesc: OP_S2D,
+              ResizeRaggedDesc: OP_RESIZE_RAGGED, WaveletRaggedDesc: OP_WAVELET_RAGGED}
 _SINGLE_ENTRY = {OP_CONV: "ug_conv", OP_POOL: "ug_pool",
                  OP_LAYERNORM: "ug_layernorm", OP_ATTN: "ug_attention", OP_CHANSTATS: "ug_chanstats",
                  OP_GATE: "ug_gate", OP_BBOX: "ug_bbox", OP_CROPRESIZE: "ug_cropresize",
                  OP_HEAD: "ug_head", OP_STEM: "ug_stem",
-                 OP_RESIZE: "ug_resize_u8", OP_WAVELET: "ug_wavelet", OP_S2D: "ug_s2d_pack"}
+                 OP_RESIZE: "ug_resize_u8", OP_WAVELET: "ug_wavelet", OP_S2D: "ug_s2d_pack",
+                 OP_RESIZE_RAGGED: "ug_resize_ragged", OP_WAVELET_RAGGED: "ug_wavelet_ragged"}
 
 EXPORTED_SYMBOLS = ["ug_version", "ug_create", "ug_destroy", "ug_last_error", "ug_launch_count",
                     *_SINGLE_ENTRY.values(), "ug_program_create", "ug_program_run", "ug_program_num_launches",
                     "ug_program_destroy", "ug_program_run_host", "ug_program_run_host_pipelined",
                     "ug_program_run_timed", "ug_program_autotune", "ug_wavelet_workspace_bytes",
+                    "ug_wavelet_ragged_workspace_bytes",
                     "ug_plan_load", "ug_plan_num_io", "ug_plan_io_name", "ug_plan_io", "ug_plan_device_bytes",
                     "ug_plan_program", "ug_plan_copy_in", "ug_plan_copy_out", "ug_plan_run", "ug_plan_destroy"]
 DEV_SYMBOLS = ["ug_conv_profile", "ug_conv_profile16", "ug_mma_microbench", "ug_mma_microbench2",
@@ -165,6 +181,8 @@ def load_library():
     lib.ug_program_run_timed.argtypes = [_vp, _vp, _vp, C.POINTER(C.c_float)]
     lib.ug_wavelet_workspace_bytes.argtypes = [_i, _i, _i]
     lib.ug_wavelet_workspace_bytes.restype = C.c_size_t
+    lib.ug_wavelet_ragged_workspace_bytes.argtypes = [_i, _ll]
+    lib.ug_wavelet_ragged_workspace_bytes.restype = C.c_size_t
     lib.ug_program_autotune.argtypes = [_vp, _vp, _vp, C.POINTER(_i)]
     lib.ug_program_destroy.argtypes = [_vp, _vp]
     lib.ug_program_run_host.argtypes = [_vp, _vp, _vp, _i, _vp, _i, _vp]

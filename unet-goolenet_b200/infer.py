@@ -56,13 +56,20 @@ def inference_all_seg(model, test_loader, device, save_dir=None):
 
 @torch.no_grad()
 def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256):
-    """The whole of 分类/test.py:122-134 + :74-96 on the device for a list of grayscale images of one size:
+    """The whole of 分类/test.py:122-134 + :74-96 on the device for a batch of grayscale images:
     cv2.imread(path, 0) output (uint8 [H, W]) -> wavelet_enhance -> resize 224 + to_tensor -> UNet -> mask -> bbox ->
     ROI crop/resize -> GoogLeNet -> argmax; returns the sorted "<name> <class>" records (and writes result.txt).
 
-    pipeline: pipeline.TwoStagePipeline (or lower.PipelineRunner); gray_images: uint8 array / tensor [N, H, W]."""
+    pipeline: pipeline.TwoStagePipeline (or lower.PipelineRunner); gray_images: uint8 array / tensor [N, H, W], or a
+    list of uint8 [H, W] images of any sizes (2 <= H, W <= 8*224), as the reference reads a directory.  A list runs as
+    ragged batches (util/ragged.py): per chunk of the pipeline, one copy of the packed gray bytes and one of the table,
+    the wavelet step writing its RGB output straight into the plan's source buffer, then the program; batch_size is
+    not used (the pipeline's own chunking applies)."""
     from .util.wavelet import wavelet_enhance_batch
     runner = getattr(pipeline, "runner", pipeline)
+    if isinstance(gray_images, (list, tuple)):
+        records = _grade_ragged(runner, gray_images, filenames)
+        return _write_records(records, save_dir)
     g = torch.as_tensor(np.ascontiguousarray(gray_images) if isinstance(gray_images, np.ndarray) else gray_images)
     records = []
     for s in range(0, g.shape[0], batch_size):
@@ -71,6 +78,28 @@ def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256
         pred = torch.argmax(torch.softmax(cls, dim=1), dim=1).cpu().numpy()  # test.py:86
         for i, name in enumerate(filenames[s:s + batch_size]):
             records.append(f"{name.replace('.png', '')} {int(pred[i])}")
+    return _write_records(records, save_dir)
+
+
+def _grade_ragged(runner, gray_images, filenames):
+    from .util import ragged
+    from .util.wavelet import wavelet_ragged_into
+    packed = ragged.pack(gray_images, 1, min_side=ragged.WAVELET_MIN_SIDE, max_side=ragged.MAX_RATIO * 224)
+    records = []
+    for s, c in runner._chunks(len(gray_images)):
+        part = ragged.chunk(packed, s, s + c)
+        ws = runner.plan(c, source="ragged", capacity=part.n_px)
+        gray = part.data.to(runner.dev, non_blocking=True)
+        ws["src_index"].copy_(ragged.table_tensor(part.table))
+        wavelet_ragged_into(gray, ws["src_index"], ws["src_u8"], c)         # test.py:128-129, into the plan's input
+        ws["program"].run()                                                  # test.py:130-131 and :82-84
+        pred = torch.argmax(torch.softmax(ws["cls_logits"], dim=1), dim=1).cpu().numpy()  # test.py:86
+        for i, name in enumerate(filenames[s:s + c]):
+            records.append(f"{name.replace('.png', '')} {int(pred[i])}")
+    return records
+
+
+def _write_records(records, save_dir):
     records.sort(key=lambda x: int(x.split()[0].replace(".jpg", "").replace(".png", "")))
     if save_dir is not None:
         os.makedirs(save_dir, exist_ok=True)

@@ -17,6 +17,7 @@ import torch
 
 from . import engine as E
 from . import pack
+from .util import ragged
 
 IMG = 224
 # UG_AUTOTUNE=1: measured kernel-variant choice at plan time (ug_program_autotune).  Off by default: on the B200 it
@@ -745,14 +746,21 @@ class PipelineRunner:
         for b in [m for m in self._gpools if m not in liveb]:
             del self._gpools[b]
 
-    def plan(self, B, source=None, slot=0):
+    def plan(self, B, source=None, slot=0, capacity=None):
         """Program for a batch of B images; B must be <= micro_batch or a multiple of it.  With `source` =
         (Hs, Ws) the program starts with the device front-end (PIL-exact resize of uint8 HWC sources + to_tensor,
         util/data_utils.py) writing the UNet input, and `ws["src_u8"]` is the program's input buffer.
+        With source = "ragged" the sources have different sizes: `ws["src_u8"]` holds `capacity` pixels of packed HWC
+        images (capacity is rounded up to a power of two, so batches of similar total size share a plan) and
+        `ws["src_index"]` their table (util/ragged.py); `ws["src_status"]` receives 1 for a rejected table entry.
         `slot` selects one of several programs of the same shape with their OWN input / output buffers (x_in, src_u8,
         logits, mask, boxes, u8) over the SAME activation workspaces: a host-fed serving loop alternates slots so that
         the H2D copy of step i+1 lands in place while step i computes (Program.run_host_pipelined(direct=True))."""
-        key = (B, slot) if source is None else (B, slot) + tuple(source)
+        if source == "ragged":
+            capacity = ragged.capacity(capacity or 0)
+            key = (B, slot, "ragged", capacity)
+        else:
+            key = (B, slot) if source is None else (B, slot) + tuple(source)
 
         def build():
             mb = min(B, self.micro_batch)
@@ -765,7 +773,14 @@ class PipelineRunner:
                       boxes=torch.empty((B, 4), device=dev, dtype=torch.int32),
                       u8=torch.empty((B, IMG, IMG, 3), device=dev, dtype=torch.uint8))
             ops = []
-            if source is not None:
+            if source == "ragged":
+                ws["src_u8"] = torch.empty((capacity * 3,), device=dev, dtype=torch.uint8)
+                ws["src_index"] = torch.zeros((B, 4), device=dev, dtype=torch.int32)
+                ws["src_status"] = torch.zeros((B,), device=dev, dtype=torch.int32)
+                ops.append(E.ResizeRaggedDesc(ws["src_u8"].data_ptr(), ws["src_index"].data_ptr(),
+                                              ws["src_status"].data_ptr(), ws["x_in"].data_ptr(), None, capacity * 3, B,
+                                              IMG))
+            elif source is not None:
                 ws["src_u8"] = torch.empty((B, source[0], source[1], 3), device=dev, dtype=torch.uint8)
                 ops.append(E.ResizeDesc(ws["src_u8"].data_ptr(), ws["x_in"].data_ptr(), None, B, source[0], source[1],
                                         IMG))
@@ -786,13 +801,15 @@ class PipelineRunner:
             return _finish(self.engine, ops, ws, ua + ga + [v for v in ws.values() if isinstance(v, torch.Tensor)])
         return self.plans.get_or_build(key, build)
 
-    def export_plan(self, B, source=None):
+    def export_plan(self, B, source=None, capacity=None):
         """The whole two-stage program for a batch of B images as a relocatable plan image (bytes): op list, device
         memory layout, BN-folded packed weights of both networks.  A host in any language runs it through the C ABI
-        alone (ug_plan_load / ug_plan_copy_in / ug_plan_run / ug_plan_copy_out, include/ugnet.h; examples/run_plan.c)."""
-        ws = self.plan(B, source=source)
+        alone (ug_plan_load / ug_plan_copy_in / ug_plan_run / ug_plan_copy_out, include/ugnet.h; examples/run_plan.c).
+        source / capacity as for plan(); a ragged plan's inputs are "src_u8" and "src_index"."""
+        ws = self.plan(B, source=source, capacity=capacity)
         prog = ws["program"]
-        io = {k: ws[k] for k in ("x_in", "src_u8", "logits", "mask", "boxes", "u8", "cls_logits") if k in ws}
+        io = {k: ws[k] for k in ("x_in", "src_u8", "src_index", "src_status", "logits", "mask", "boxes", "u8",
+                                 "cls_logits") if k in ws}
         tensors = list(prog.keepalive) + list(io.values()) + [(self.unet.w_blob, True), (self.gnet.w_blob, True)]
         return E.export_plan(prog.descs, io, tensors)
 
@@ -807,17 +824,33 @@ class PipelineRunner:
             out.append((s, n - s))
         return out
 
+    def feed_ragged(self, part):
+        """The ragged plan for one chunk (a ragged.Packed of HWC images, at most one plan's batch) with its packed
+        sources and table copied in (one copy each)."""
+        ws = self.plan(len(part.table), source="ragged", capacity=part.n_px)
+        ws["src_u8"][:part.data.numel()].copy_(part.data, non_blocking=True)
+        ws["src_index"].copy_(ragged.table_tensor(part.table))
+        return ws
+
     @torch.no_grad()
     def __call__(self, imgs, return_logits=False):
         """imgs: float [B,3,224,224] CUDA, or uint8 [B,Hs,Ws,3] CUDA source images of any size (resized on the
-        device exactly as the reference's PIL transform does) ->
+        device exactly as the reference's PIL transform does), or a list of uint8 [H,W,3] images of different sizes
+        (CUDA tensors or numpy arrays, sides up to 8*224; one ragged batch, util/ragged.py) ->
         (masks u8 [B,224,224], boxes i32 [B,4], cls_logits f32 [B,6])."""
         masks, boxes, cls, seg = [], [], [], []
-        from_u8 = imgs.dtype == torch.uint8
+        packed = None
+        if isinstance(imgs, (list, tuple)):
+            packed = ragged.pack(imgs, 3, max_side=ragged.MAX_RATIO * IMG)
+            n, from_u8 = len(imgs), False
+        else:
+            n, from_u8 = imgs.shape[0], imgs.dtype == torch.uint8
         if from_u8 and (imgs.dim() != 4 or imgs.shape[3] != 3):
             raise ValueError(f"uint8 input must be HWC [B,H,W,3], got {tuple(imgs.shape)}")
-        for s, c in self._chunks(imgs.shape[0]):
-            if from_u8:
+        for s, c in self._chunks(n):
+            if packed is not None:
+                ws = self.feed_ragged(ragged.chunk(packed, s, s + c))
+            elif from_u8:
                 ws = self.plan(c, source=(imgs.shape[1], imgs.shape[2]))
                 ws["src_u8"].copy_(imgs[s:s + c])
             else:

@@ -21,7 +21,8 @@ class TwoStagePipeline:
     @torch.no_grad()
     def __call__(self, imgs, return_logits=False):
         """imgs: float [B,3,224,224] on the pipeline's device, or uint8 HWC sources [B,Hs,Ws,3] of any size (resized
-        on the device like the reference's CDDataAugmentation.transform: PIL bilinear + to_tensor) ->
+        on the device like the reference's CDDataAugmentation.transform: PIL bilinear + to_tensor), or a list of uint8
+        [H,W,3] images of different sizes (CUDA tensors or numpy arrays; run as ragged batches, util/ragged.py) ->
         (masks uint8 [B,224,224], boxes int32 [B,4] = (x0,y0,x1,y1), class logits float32 [B,6])."""
         return self.runner(imgs, return_logits=return_logits)
 

@@ -10,12 +10,18 @@ import numpy as np
 import torch
 
 from .. import engine as E
+from . import ragged
 
 
 @torch.no_grad()
 def resize_to_tensor(src_u8, img_size=224, out=None, return_u8=False):
     """src_u8: uint8 [B,Hs,Ws,3] CUDA tensor -> float32 [B,3,img_size,img_size] in [0,1] (to_tensor of the
-    PIL-resized image).  With return_u8 also returns the resized uint8 HWC image."""
+    PIL-resized image).  With return_u8 also returns the resized uint8 HWC image.
+
+    src_u8 may also be a list of uint8 [H,W,3] images of different sizes (numpy arrays or tensors, sides up to
+    8*img_size): they are packed into one ragged batch (util/ragged.py) and resized in one launch."""
+    if isinstance(src_u8, (list, tuple)):
+        return _resize_ragged(src_u8, img_size, out, return_u8)
     if src_u8.device.type != "cuda":
         raise RuntimeError("ugnet: input must be a CUDA tensor (no CPU path)")
     if src_u8.dtype != torch.uint8 or src_u8.dim() != 4 or src_u8.shape[3] != 3:
@@ -27,6 +33,21 @@ def resize_to_tensor(src_u8, img_size=224, out=None, return_u8=False):
         out = torch.empty((B, 3, img_size, img_size), dtype=torch.float32, device=src.device)
     u8 = torch.empty((B, img_size, img_size, 3), dtype=torch.uint8, device=src.device) if return_u8 else None
     eng.run_op(E.ResizeDesc(src.data_ptr(), out.data_ptr(), E.ptr(u8), B, Hs, Ws, img_size))
+    return (out, u8) if return_u8 else out
+
+
+def _resize_ragged(images, img_size, out, return_u8):
+    packed = ragged.pack(images, 3, max_side=ragged.MAX_RATIO * img_size)
+    dev = packed.data.device if packed.data.is_cuda else torch.device("cuda", torch.cuda.current_device())
+    src = packed.data.to(dev, non_blocking=True)
+    index = ragged.table_tensor(packed.table, dev)
+    B = len(images)
+    eng = E.Engine.get(dev)
+    if out is None:
+        out = torch.empty((B, 3, img_size, img_size), dtype=torch.float32, device=dev)
+    u8 = torch.empty((B, img_size, img_size, 3), dtype=torch.uint8, device=dev) if return_u8 else None
+    eng.run_op(E.ResizeRaggedDesc(src.data_ptr(), index.data_ptr(), None, out.data_ptr(), E.ptr(u8), src.numel(), B,
+                                  img_size))
     return (out, u8) if return_u8 else out
 
 

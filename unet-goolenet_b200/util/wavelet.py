@@ -9,10 +9,24 @@ import numpy as np
 import torch
 
 from .. import engine as E
+from . import ragged
 
 
 @torch.no_grad()
 def wavelet_enhance_batch(gray_u8):
+    """gray_u8: uint8 [B,H,W] CUDA tensor -> uint8 [B,H,W,3] CUDA tensor.
+
+    gray_u8 may also be a list of uint8 [H,W] images of different sizes (numpy arrays or tensors, sides >= 2): the
+    result is then a ragged.Packed of the pseudo-RGB images (one device buffer, image i's HWC bytes at
+    3 * table[i].px_offset; ragged.unpack gives [H,W,3] views), computed in one pass of five launches."""
+    if isinstance(gray_u8, (list, tuple)):
+        packed = ragged.pack(gray_u8, 1, min_side=ragged.WAVELET_MIN_SIDE, max_side=ragged.WAVELET_MAX_SIDE)
+        dev = packed.data.device if packed.data.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        gray = packed.data.to(dev, non_blocking=True)
+        index = ragged.table_tensor(packed.table, dev)
+        out = torch.empty((gray.numel() * 3,), dtype=torch.uint8, device=dev)
+        wavelet_ragged_into(gray, index, out, len(gray_u8))
+        return ragged.Packed(out, packed.table, 3)
     if gray_u8.device.type != "cuda":
         raise RuntimeError("ugnet: input must be a CUDA tensor (no CPU path)")
     if gray_u8.dtype != torch.uint8 or gray_u8.dim() != 3:
@@ -25,6 +39,19 @@ def wavelet_enhance_batch(gray_u8):
     out = torch.empty((B, H, W, 3), dtype=torch.uint8, device=g.device)
     eng.run_op(E.WaveletDesc(g.data_ptr(), out.data_ptr(), ws.data_ptr(), nbytes, B, H, W))
     return out
+
+
+def wavelet_ragged_into(gray, index, out_u8, B, status=None):
+    """One ug_wavelet_ragged op: packed gray bytes `gray` (uint8 CUDA, its length is the capacity in pixels) with the
+    device table `index` (ragged.table_tensor) -> pseudo-RGB HWC bytes into out_u8 at 3 * px_offset per image."""
+    eng = E.Engine.get(gray.device)
+    cap = gray.numel()
+    if out_u8.numel() < 3 * cap:
+        raise ValueError(f"output buffer of {out_u8.numel()} bytes is smaller than 3 x {cap}")
+    nbytes = eng.lib.ug_wavelet_ragged_workspace_bytes(B, cap)
+    ws = torch.empty((nbytes,), dtype=torch.uint8, device=gray.device)
+    eng.run_op(E.WaveletRaggedDesc(gray.data_ptr(), index.data_ptr(), E.ptr(status), out_u8.data_ptr(), ws.data_ptr(),
+                                   nbytes, cap, B))
 
 
 def wavelet_enhance(gray_img, wavelet="haar", level=1, device="cuda"):
