@@ -179,22 +179,19 @@ typedef struct ug_cropresize_desc {
 /* Stem convolution fused with its im2col (no im2col matrix in HBM), N = 64 output channels, folded BN + ReLU:
  *   kind 0: UNet inc (basicUnet.py:409; ConvBatchNorm :25-40): 3x3 s1 p1 on in_f32 = fp32 NCHW [B,3,H,W]
  *           (also performs x.float(), :408); w = bf16 [64][64], column (r*3+s)*3+c, columns 27.. zero.
- *   kind 1: GoogLeNet conv1 (torchvision BasicConv2d 7x7 s2 p3; 分类/test.py:68-73) on in_u8 = uint8 HWC
- *           [B,H,W,3] (the ROI crop) or, if in_f32 is non-NULL, a float NCHW [B,3,H,W] image in [0,1];
- *           to_tensor (/255) and _transform_input are applied before the zero padding;
- *           w = bf16 [64][192], column r*22 + s*3 + c (column r*22+21 and columns 154.. zero).
- * out: bf16 NHWC [B,OH,OW,out_cstride], channels [0,64); OH,OW = H,W (kind 0) or H/2,W/2 (kind 1). */
+ * Any other kind is rejected with UG_EINVAL (GoogLeNet conv1 runs as ug_s2d_pack + a row-tap conv).
+ * out: bf16 NHWC [B,H,W,out_cstride], channels [0,64). */
 typedef struct ug_stem_desc {
   int kind;
   const float* in_f32;
-  const unsigned char* in_u8;
+  const unsigned char* in_u8;   /* unused */
   const void* w;
   const float* scale;
   const float* bias;
   void* out;
   int out_cstride;
   int B, H, W;
-  void* pool_out;   /* optional (kind 0, H and W even): also write nn.MaxPool2d(2) of the output (DownBlock,
+  void* pool_out;   /* optional (H and W even): also write nn.MaxPool2d(2) of the output (DownBlock,
                        basicUnet.py:47) to bf16 NHWC [B,H/2,W/2,pool_cstride], fused into the epilogue */
   int pool_cstride;
 } ug_stem_desc;
@@ -360,10 +357,6 @@ size_t ug_wavelet_ragged_workspace_bytes(int B, long long capacity_px);
 int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out);
 int ug_program_run(ug_handle h, ug_program p, void* stream);
 int ug_program_num_launches(ug_program p);
-/* Measured kernel-variant choice for every conv op created with variant 0 (auto): each kernel structure that accepts
- * the op is timed on the op's own buffers (which are overwritten; call before the first real run) and the fastest
- * is kept.  Synchronizes the stream.  n_changed (optional) receives the number of switched ops. */
-int ug_program_autotune(ug_handle h, ug_program p, void* stream, int* n_changed);
 /* Profiling aid: run with a CUDA event pair around every op, synchronize, and return the device time of each
  * op in milliseconds (ms_per_op has ug_program_num_launches(p) entries). */
 int ug_program_run_timed(ug_handle h, ug_program p, void* stream, float* ms_per_op);

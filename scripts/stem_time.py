@@ -1,4 +1,4 @@
-"""Time the two stem convolutions alone (inc at B=128 with the fused pool, conv1 at B=256): python scripts/stem_time.py"""
+"""Time the stem convolution alone (inc at B=128 with the fused pool): python scripts/stem_time.py"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -30,9 +30,3 @@ pool = torch.empty((B, 112, 112, 64), device="cuda", dtype=torch.bfloat16)
 d0 = E.StemDesc(0, x.data_ptr(), None, wp.data_ptr(), sc.data_ptr(), bi.data_ptr(), out.data_ptr(), 64, B, 224, 224,
                 pool.data_ptr(), 64)
 print(f"inc B={B} +pool: {timeit(d0):.4f} ms")
-B = 256
-u8 = torch.randint(0, 256, (B, 224, 224, 3), generator=g, device="cuda", dtype=torch.uint8)
-wp1 = pack.pack_linear_weight(torch.randn((64, 154), generator=g, device="cuda"), 64)
-out1 = torch.empty((B, 112, 112, 64), device="cuda", dtype=torch.bfloat16)
-d1 = E.StemDesc(1, None, u8.data_ptr(), wp1.data_ptr(), sc.data_ptr(), bi.data_ptr(), out1.data_ptr(), 64, B, 224, 224)
-print(f"conv1 B={B}: {timeit(d1):.4f} ms")

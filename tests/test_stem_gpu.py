@@ -1,6 +1,6 @@
-"""GPU parity of the fused stem convolutions (ug_stem, csrc/stem_conv.cu) against torch fp32 on the same
-bf16-rounded operands: UNet inc (3x3 on fp32 NCHW, basicUnet.py:409) and GoogLeNet conv1 (7x7 s2 on the uint8
-crop or a float image, with to_tensor + _transform_input folded in before the zero padding)."""
+"""GPU parity of the stem convolutions against torch fp32 on the same bf16-rounded operands: UNet inc (ug_stem,
+csrc/stem_conv.cu: 3x3 on fp32 NCHW, basicUnet.py:409) and GoogLeNet conv1 (ug_s2d_pack + a row-tap conv: 7x7 s2 on
+the uint8 crop or a float image, with to_tensor + _transform_input folded in before the zero padding)."""
 import pytest
 import torch
 import torch.nn.functional as F
@@ -46,40 +46,6 @@ def test_stem_inc(engine, B, H, W, extra, pool):
     _check(out[..., :64].float(), ref.permute(0, 2, 3, 1))
     if extra:
         assert (out[..., 64:] == 7.0).all()
-
-
-def _pack_conv1(wt):
-    from ugnet_b200 import pack
-    gemm = torch.zeros(64, 7, 22, device=wt.device)
-    gemm[:, :, :21] = wt.permute(0, 2, 3, 1).reshape(64, 7, 21)
-    return pack.pack_linear_weight(gemm.reshape(64, 154), 64)
-
-
-@pytest.mark.parametrize("B,S,src", [(1, 224, "u8"), (5, 224, "u8"), (2, 224, "f32"), (3, 64, "u8"), (40, 32, "f32")])
-def test_stem_conv1(engine, B, S, src):
-    from ugnet_b200 import engine as E
-    g = torch.Generator(device="cuda").manual_seed(B * 77 + S)
-    wt = torch.randn((64, 3, 7, 7), generator=g, device="cuda") * 0.1
-    scale = torch.rand((64,), generator=g, device="cuda") + 0.5
-    bias = torch.randn((64,), generator=g, device="cuda")
-    wp = _pack_conv1(wt)
-    out, o_intact = guarded((B, S // 2, S // 2, 64), 7.0, torch.bfloat16)
-    if src == "u8":
-        u8 = torch.randint(0, 256, (B, S, S, 3), generator=g, device="cuda", dtype=torch.uint8)
-        xf = (u8.float() / 255.0).permute(0, 3, 1, 2)
-        d = E.StemDesc(1, None, u8.data_ptr(), wp.data_ptr(), scale.data_ptr(), bias.data_ptr(), out.data_ptr(), 64,
-                       B, S, S)
-    else:
-        xf = torch.rand((B, 3, S, S), generator=g, device="cuda")
-        d = E.StemDesc(1, xf.data_ptr(), None, wp.data_ptr(), scale.data_ptr(), bias.data_ptr(), out.data_ptr(), 64,
-                       B, S, S)
-    engine.run_op(d)
-    torch.cuda.synchronize()
-    o_intact()
-    xt = xf * _SC.cuda()[None, :, None, None] + _SH.cuda()[None, :, None, None]   # GoogLeNet._transform_input
-    xq, wq = xt.to(torch.bfloat16).float(), wt.to(torch.bfloat16).float()
-    ref = torch.relu(F.conv2d(xq, wq, stride=2, padding=3) * scale[None, :, None, None] + bias[None, :, None, None])
-    _check(out.float(), ref.permute(0, 2, 3, 1))
 
 
 @pytest.mark.parametrize("B,S,src", [(1, 224, "u8"), (5, 224, "u8"), (2, 224, "f32"), (3, 64, "u8"), (40, 32, "f32")])
@@ -134,3 +100,6 @@ def test_stem_rejects_bad_args(engine):
         engine.run_op(E.StemDesc(0, None, None, w.data_ptr(), None, None, out.data_ptr(), 64, 1, 8, 8))
     with pytest.raises(RuntimeError):
         engine.run_op(E.StemDesc(2, out.data_ptr(), None, w.data_ptr(), None, None, out.data_ptr(), 64, 1, 8, 8))
+    x = torch.zeros((1, 3, 8, 8), device="cuda")
+    with pytest.raises(RuntimeError):     # kind 1 (the former GoogLeNet conv1 stem) is rejected like any other kind
+        engine.run_op(E.StemDesc(1, x.data_ptr(), None, w.data_ptr(), None, None, out.data_ptr(), 64, 1, 8, 8))

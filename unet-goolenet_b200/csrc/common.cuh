@@ -166,9 +166,90 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
   d |= static_cast<uint64_t>(2) << 61;
   return d;
 }
+// The same with an explicit stride-byte offset: the distance of consecutive 8-row groups (halo tiles: pitch * 128 B).
+__device__ __forceinline__ uint64_t umma_desc_sw128_sbo(uint32_t smem_addr, uint32_t sbo_bytes) {
+  uint64_t d = 0;
+  d |= static_cast<uint64_t>((smem_addr & 0x3FFFF) >> 4);
+  d |= static_cast<uint64_t>(1) << 16;
+  d |= static_cast<uint64_t>(sbo_bytes >> 4) << 32;
+  d |= static_cast<uint64_t>(1) << 46;
+  d |= static_cast<uint64_t>(2) << 61;
+  return d;
+}
 // kind::f16 instruction descriptor: D=f32, A=B=bf16, both K-major, M x N.
 __device__ __forceinline__ uint32_t umma_idesc_bf16(uint32_t M, uint32_t N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
+
+// ---------------------------------------------------------------- CTA pairs (clusters of two, tcgen05 cta_group::2)
+// The leader CTA (cluster rank 0) issues M = 256 MMAs that read both CTAs' shared memory and write both TMEMs; its
+// barriers collect the TMA bytes of both CTAs.
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// shared::cluster address of `p` (a shared-memory object of this CTA) in the leader CTA
+__device__ __forceinline__ uint32_t leader_addr(const void* p) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(0u));
+  return r;
+}
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
+}
+// TMA loads into this CTA's shared memory whose completion is signalled on the barrier at `bar_cluster_addr`, which may
+// belong to the peer CTA (callers map it once with leader_addr, outside their load loops)
+__device__ __forceinline__ void tma_load_4d_pair(void* dst, const CUtensorMap* m, uint32_t bar_cluster_addr, int c0, int c1,
+                                                 int c2, int c3) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], "
+      "[%2];" ::"r"(smem_u32(dst)),
+      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+      : "memory");
+}
+__device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* m, uint32_t bar_cluster_addr, int c0, int c1) {
+  asm volatile(
+      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1)
+      : "memory");
+}
+// The same with the barrier given by this CTA's pointer to it and mapped to the leader CTA inside the load: the
+// multi-issuer kernel's weight loops are scheduled with the mapping there (a separate leader_addr call before the load
+// compiles to a different register allocation)
+__device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* m, const uint64_t* leader_bar, int c0, int c1) {
+  asm volatile(
+      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(leader_addr(leader_bar)), "r"(c0), "r"(c1)
+      : "memory");
+}
+__device__ __forceinline__ void tmem_alloc_pair(uint32_t* dst_smem, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols)
+               : "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void umma_bf16_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                               uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// arrive on the barrier at this shared-memory offset in BOTH CTAs once the MMAs issued so far have completed
+__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+                   smem_u32(bar)),
+               "h"((uint16_t)3)
+               : "memory");
 }
 
 // ---------------------------------------------------------------- small math / packing helpers
@@ -182,6 +263,10 @@ __device__ __forceinline__ uint32_t pack_bf16x2_relu(float lo, float hi) {
   uint32_t r;
   asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
   return r;
+}
+__device__ __forceinline__ uint32_t bf16x2_max(uint32_t a, uint32_t b) {
+  __nv_bfloat162 r = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a), *reinterpret_cast<__nv_bfloat162*>(&b));
+  return *reinterpret_cast<uint32_t*>(&r);
 }
 __device__ __forceinline__ float bf16_lo(uint32_t w) { return __uint_as_float(w << 16); }
 __device__ __forceinline__ float bf16_hi(uint32_t w) { return __uint_as_float(w & 0xFFFF0000u); }

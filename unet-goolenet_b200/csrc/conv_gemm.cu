@@ -16,7 +16,6 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
-#include <cstdlib>
 #include "conv_common.cuh"
 
 namespace ug {
@@ -508,10 +507,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_persistent_kernel(const
 
 // ------------------------------------------------------------------------------------------ host side
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 EncodeTiledFn get_encode_fn() {
   static EncodeTiledFn fn = nullptr;
   if (fn) return fn;
@@ -524,7 +519,13 @@ EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
+int encode_bf16_sw128(CUtensorMap* m, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                      const cuuint32_t* box, CUtensorMapL2promotion promo) {
+  const cuuint32_t es[4] = {1, 1, 1, 1};
+  return (int)get_encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), dims, strides,
+                              box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, promo,
+                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+}
 
 // Pick the pixel-tile rectangle with the best fill of the 128 MMA rows.
 void choose_tile(int B, int H, int W, int* TW, int* TH, int* TN) {
@@ -551,8 +552,7 @@ void choose_tile(int B, int H, int W, int* TW, int* TH, int* TN) {
 }
 
 int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return set_error(h, UG_ECUDA, "cuTensorMapEncodeTiled entry point unavailable");
+  if (!get_encode_fn()) return set_error(h, UG_ECUDA, "cuTensorMapEncodeTiled entry point unavailable");
   if (!d->in || !d->w) return set_error(h, UG_EINVAL, "conv: null in/w pointer");
   if (d->B <= 0 || d->H <= 0 || d->W <= 0 || d->Cin <= 0 || d->N <= 0)
     return set_error(h, UG_EINVAL, "conv: non-positive shape");
@@ -612,9 +612,7 @@ int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   // (conv_pair.cu, tcgen05.mma.cta_group::2) — profiles/r02_pair_kernel.txt: 64->64 0.221 -> 0.201 ms, + outc 0.208 ->
   // 0.176, 128->64 0.451 -> 0.359, 256->64 at 112x112 0.218 -> 0.188 per 64 images.  The CoordAtt3 combine on 64 input
   // channels is bound by its epilogue, not by the MMA, and stays on the multi-issuer kernel (0.277 against 0.291 ms).
-  // UG_PAIR=0 turns the rule off.
-  static const int use_pair = [] { const char* e = getenv("UG_PAIR"); return e ? atoi(e) : 1; }();
-  if (use_pair && d->variant == 0 && d->R == 3 && up == 1 && d->N <= 64 && d->H * d->W >= 112 * 112 &&
+  if (d->variant == 0 && d->R == 3 && up == 1 && d->N <= 64 && d->H * d->W >= 112 * 112 &&
       !(d->mode == UG_EPI_GATE && d->Cin <= 64)) {
     const int rc = conv_pair_prepare(h, d, L);
     if (rc == UG_OK) return rc;
@@ -632,11 +630,9 @@ int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   // 0.172 -> 0.148 ms (1600 TFLOP/s), 56x56 256->256 0.185 -> 0.164, 28x28 512->512 0.182 -> 0.169, 1024->256 0.204 ->
   // 0.186; the 256-image step +4.9 %.  Not routed: 64 input channels (resident weights, bound by the epilogue: 0.094 ->
   // 0.112 ms; GoogLeNet conv3 64->192 neutral).  The CoordAtt3 combine runs in pair mode with its residual sub-tiles
-  // TMA-loaded by an extra warp (UG_RESID_TMA128, profiles/r02_resid_tma128.txt): 112x112 128->128 0.197 -> 0.165 ms.
+  // TMA-loaded by an extra warp (profiles/r02_resid_tma128.txt): 112x112 128->128 0.197 -> 0.165 ms.
   // GoogLeNet's 3x3 layers with N >= 128 (ragged last n-tile) gain 8-13 % each, the stage 2.151 -> 2.124 ms.
-  // UG_PAIR128=0 turns the rule off.
-  static const int use_pair128 = [] { const char* e = getenv("UG_PAIR128"); return e ? atoi(e) : 1; }();
-  if (use_pair128 && d->variant == 0 && d->R == 3 && up == 1 && d->H * d->W >= 196 && !d->stats_sum && d->N >= 128 &&
+  if (d->variant == 0 && d->R == 3 && up == 1 && d->H * d->W >= 196 && !d->stats_sum && d->N >= 128 &&
       ((d->mode == UG_EPI_STORE && d->Cin > 64) || (d->mode == UG_EPI_GATE && d->Cin >= 128))) {
     const int rc = conv_multi_prepare(h, d, 128, L, 1);
     if (rc == UG_OK) return rc;
@@ -673,9 +669,8 @@ int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   // kernel (two CTAs per SM, 2-4 stages) is latency-bound: >= 1024 m-tiles -> multi-issuer kernel when K = 64
   // (one chunk), persistent otherwise; >= 296 m-tiles with BN > 64 -> persistent; else one tile per CTA.
   const int m_tiles_total = ceil_div(d->W, TW) * ceil_div(d->H, TH) * ceil_div(d->B, TN);
-  static const int gemm_rule = [] { const char* e = getenv("UG_GEMM_RULE"); return e ? atoi(e) : 1; }();
   int auto_persistent = BN == 256;
-  if (gemm_rule && d->variant == 0 && d->R == 1 && d->S == 1 && up == 1 && d->mode != UG_EPI_OUTC) {
+  if (d->variant == 0 && d->R == 1 && d->S == 1 && up == 1 && d->mode != UG_EPI_OUTC) {
     if (m_tiles_total >= 1024 && kchunks == 1 && (n_tiles == 1 || BN % 64 == 0) && !split) {
       const int rc = conv_multi_prepare(h, d, BN, L);
       if (rc == UG_OK) return rc;
@@ -686,19 +681,19 @@ int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
     if (boxes_ok && (m_tiles_total >= 1024 || (m_tiles_total >= 296 && BN > 64))) auto_persistent = 1;
   }
   if (split && d->n_split % BN) auto_persistent = 1;  // the one-tile kernel needs whole n-tiles on either side of n_split
-  const int variant = d->variant == 1 ? 1 : (d->variant == 2 ? 0 : (auto_persistent ? 0 : 1));
-  if (split && variant == 1 && d->n_split % BN)
+  const bool persistent = d->variant == 2 || (d->variant != 1 && auto_persistent);
+  if (split && !persistent && d->n_split % BN)
     return set_error(h, UG_EINVAL, "conv: split GEMM on the one-tile kernel needs BN to divide n_split (BN = 64)");
-  const int tma_store = (variant == 0 && up == 1 && d->mode != UG_EPI_OUTC) ? 1 : 0;
-  const int stage_copy = (variant == 0 && up == 2) ? 1 : 0;
+  const int tma_store = (persistent && up == 1 && d->mode != UG_EPI_OUTC) ? 1 : 0;
+  const int stage_copy = (persistent && up == 2) ? 1 : 0;
   const int n_sub = ceil_div(BN, 64);
   const int obuf_bytes = (tma_store || stage_copy) ? n_sub * kABytesPerStage : 0;
   const int acc_stages = std::max(1, std::min(4, 512 / BN));
   const int npad = n_tiles * BN;
-  int obufs = (variant == 0 && (tma_store || stage_copy)) ? 2 : 0;
+  int obufs = (persistent && (tma_store || stage_copy)) ? 2 : 0;
   int stages = d->stages;
   const int per_stage = kABytesPerStage + BN * 128;
-  if (variant == 1) {
+  if (!persistent) {
     if (stages <= 0) {
       stages = (108 * 1024) / per_stage;  // two CTAs per SM
       stages = std::max(2, std::min(stages, 8));
@@ -740,12 +735,12 @@ int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   p.gate = d->gate; p.outc_w = d->outc_w; p.outc_b = d->outc_b;
   p.logits = d->logits; p.mask = d->mask;
   p.m_tiles = m_tiles_total; p.n_tiles = n_tiles; p.acc_stages = acc_stages;
-  static const int m_major_on = [] { const char* e = getenv("UG_M_MAJOR"); return e ? atoi(e) : 1; }();
-  p.m_major = (m_major_on && n_tiles > 1) ? 1 : 0;
+  p.m_major = n_tiles > 1 ? 1 : 0;
   p.tma_store = tma_store; p.obufs = obufs; p.npad = npad; p.stage_copy = stage_copy;
   p.out2 = d->out2; p.out2_cstride = d->out2_cstride; p.n_split = split ? d->n_split : 0; p.n1 = d->n1;
-  L->variant = variant;
-  if (variant == 0) {
+  L->kernel = persistent ? ConvKernel::Persistent : ConvKernel::OneTile;
+  L->block = kThreads;
+  if (persistent) {
     int tcols = 32;
     while (tcols < acc_stages * BN) tcols <<= 1;
     p.tmem_cols = tcols;
@@ -755,20 +750,15 @@ int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
     cuuint64_t strides[3] = {(cuuint64_t)d->out_cstride * 2, (cuuint64_t)d->W * d->out_cstride * 2,
                              (cuuint64_t)d->H * d->W * d->out_cstride * 2};
     cuuint32_t box[4] = {64, (cuuint32_t)TW, (cuuint32_t)TH, (cuuint32_t)TN};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    CUresult r = encode(&L->tmO, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, d->out, dims, strides, box, es,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(h, UG_ECUDA, "conv: output tensor map encode failed (%d)", (int)r);
+    int r = encode_bf16_sw128(&L->tmO, d->out, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+    if (r) return set_error(h, UG_ECUDA, "conv: output tensor map encode failed (%d)", r);
     memset(&L->tmO2, 0, sizeof(L->tmO2));
     if (split) {
       cuuint64_t dims2[4] = {(cuuint64_t)(d->N - d->n_split), (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->B};
       cuuint64_t strides2[3] = {(cuuint64_t)d->out2_cstride * 2, (cuuint64_t)d->W * d->out2_cstride * 2,
                                 (cuuint64_t)d->H * d->W * d->out2_cstride * 2};
-      r = encode(&L->tmO2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, d->out2, dims2, strides2, box, es,
-                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return set_error(h, UG_ECUDA, "conv: second output tensor map encode failed (%d)", (int)r);
+      r = encode_bf16_sw128(&L->tmO2, d->out2, 4, dims2, strides2, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+      if (r) return set_error(h, UG_ECUDA, "conv: second output tensor map encode failed (%d)", r);
     }
   } else {
     memset(&L->tmO, 0, sizeof(L->tmO));
@@ -780,23 +770,17 @@ int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
     cuuint64_t strides[3] = {(cuuint64_t)d->in_cstride * 2, (cuuint64_t)d->W * d->in_cstride * 2,
                              (cuuint64_t)d->H * d->W * d->in_cstride * 2};
     cuuint32_t box[4] = {64, (cuuint32_t)TW, (cuuint32_t)TH, (cuuint32_t)TN};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    CUresult r = encode(&L->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(d->in), dims, strides, box, es,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(h, UG_ECUDA, "conv: activation tensor map encode failed (%d)", (int)r);
+    const int r = encode_bf16_sw128(&L->tmA, d->in, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+    if (r) return set_error(h, UG_ECUDA, "conv: activation tensor map encode failed (%d)", r);
   }
   {
     cuuint64_t dims[2] = {(cuuint64_t)ktot, (cuuint64_t)n_tiles * BN};
     cuuint64_t strides[1] = {(cuuint64_t)ktot * 2};
     cuuint32_t box[2] = {64, (cuuint32_t)BN};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = encode(&L->tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(d->w), dims, strides, box, es,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(h, UG_ECUDA, "conv: weight tensor map encode failed (%d)", (int)r);
+    const int r = encode_bf16_sw128(&L->tmB, d->w, 2, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+    if (r) return set_error(h, UG_ECUDA, "conv: weight tensor map encode failed (%d)", r);
   }
-  if (variant == 1) {
+  if (!persistent) {
     L->grid = dim3((unsigned)(p.tiles_x * p.tiles_y * tiles_n), (unsigned)n_tiles, 1);
     L->smem = 1024 + (size_t)stages * per_stage + 8 * (2 * stages + 1) + 8 + 2 * BN * sizeof(float);
   } else {
@@ -824,21 +808,24 @@ int conv_launch(ug_engine* h, const ConvLaunch* L, cudaStream_t s) {
     if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(conv_gemm kernels)");
     h->attr_gemm = true;
   }
-  if (L->variant == 5) return conv_multi_launch(h, L, s);
-  if (L->variant == 6) return conv_pair_launch(h, L, s);
   const int act = L->p.act;
-  cudaError_t le;
-  if (L->variant == 1) {
-    if (act == UG_ACT_RELU) le = launch_pdl(h, conv_gemm_kernel<UG_ACT_RELU>, L->grid, kThreads, L->smem, s, L->tmA, L->tmB, L->p);
-    else if (act == UG_ACT_GELU) le = launch_pdl(h, conv_gemm_kernel<UG_ACT_GELU>, L->grid, kThreads, L->smem, s, L->tmA, L->tmB, L->p);
-    else le = launch_pdl(h, conv_gemm_kernel<UG_ACT_NONE>, L->grid, kThreads, L->smem, s, L->tmA, L->tmB, L->p);
-  } else {
-    if (act == UG_ACT_RELU)
-      le = launch_pdl(h, conv_gemm_persistent_kernel<UG_ACT_RELU>, L->grid, kThreads, L->smem, s, L->tmA, L->tmB, L->tmO, L->tmO2, L->p);
-    else if (act == UG_ACT_GELU)
-      le = launch_pdl(h, conv_gemm_persistent_kernel<UG_ACT_GELU>, L->grid, kThreads, L->smem, s, L->tmA, L->tmB, L->tmO, L->tmO2, L->p);
-    else
-      le = launch_pdl(h, conv_gemm_persistent_kernel<UG_ACT_NONE>, L->grid, kThreads, L->smem, s, L->tmA, L->tmB, L->tmO, L->tmO2, L->p);
+  cudaError_t le = cudaErrorInvalidValue;
+  switch (L->kernel) {
+    case ConvKernel::Multi:
+    case ConvKernel::MultiPair: return conv_multi_launch(h, L, s);
+    case ConvKernel::Pair: return conv_pair_launch(h, L, s);
+    case ConvKernel::OneTile: {
+      auto fn = act == UG_ACT_RELU ? conv_gemm_kernel<UG_ACT_RELU>
+                : act == UG_ACT_GELU ? conv_gemm_kernel<UG_ACT_GELU> : conv_gemm_kernel<UG_ACT_NONE>;
+      le = launch_pdl(fn, L->grid, L->block, L->smem, s, L->tmA, L->tmB, L->p);
+      break;
+    }
+    case ConvKernel::Persistent: {
+      auto fn = act == UG_ACT_RELU ? conv_gemm_persistent_kernel<UG_ACT_RELU>
+                : act == UG_ACT_GELU ? conv_gemm_persistent_kernel<UG_ACT_GELU> : conv_gemm_persistent_kernel<UG_ACT_NONE>;
+      le = launch_pdl(fn, L->grid, L->block, L->smem, s, L->tmA, L->tmB, L->tmO, L->tmO2, L->p);
+      break;
+    }
   }
   h->launches++;
   return check_cuda(h, le != cudaSuccess ? le : cudaGetLastError(), "conv_gemm kernel launch");

@@ -57,17 +57,12 @@
 // sub-tiles by TMA too: the weight warp is busy streaming, so ONE EXTRA WARP (warp 12, 416 threads) produces them.
 #include <cfloat>
 #include <cstring>
-#include <cstdlib>
 #include <algorithm>
 #include "conv_common.cuh"
 
-#ifndef UG_EPI_UNROLL
-#define UG_EPI_UNROLL 1
-#endif
-
 namespace ug {
 
-static constexpr int kEpiUnroll = UG_EPI_UNROLL;   // unroll factor of the epilogue chunk loop
+static constexpr int kEpiUnroll = 1;   // unroll factor of the epilogue chunk loop (see there)
 static constexpr int kMI = 2;           // tile streams per CTA (each with its own epilogue warpgroup)
 // threads per CTA: 384 (kKS = 1) / 448 (kKS = 2); + one warp (residual producer) for the TMA-residual pair kernels, whose
 // weight warp is busy streaming
@@ -82,124 +77,20 @@ static constexpr int kMAllocWarp = 4 * kMI;          // 8: TMEM allocator + weig
 static constexpr int kMProducerWarp = 4 * kMI + 1;   // 9: activation (A) producer
 static constexpr int kMIssuerWarp0 = 4 * kMI + 2;    // 10 ..: issuer of (stream i, K-half h) is warp 10 + i*kKS + h
 
-__device__ __forceinline__ uint64_t umma_desc_sw128_sbo(uint32_t smem_addr, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr & 0x3FFFF) >> 4);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>(sbo_bytes >> 4) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(2) << 61;
-  return d;
-}
-
-// Division by a launch-time constant as multiply + shift (exact for n < 2^24): the role loops decode a tile index
-// into (image, tile row, tile column) once per tile, and on the short K=64 / N=64 tiles that decode (four integer
-// divisions, ~25 instructions each) was a third of the epilogue time.
-struct FastDiv {
-  unsigned mul, shift;
-  __device__ __forceinline__ int div(int n) const {
-    return (int)(((unsigned long long)(unsigned)n * mul) >> shift);
-  }
-};
-static FastDiv make_fastdiv(int d) {
-  FastDiv f;
-  int s = 0;
-  while ((1 << s) < d) ++s;
-  f.shift = 24 + s;
-  f.mul = (unsigned)(((1ULL << f.shift) + d - 1) / d);
-  return f;
-}
-
-struct MultiParams {
-  int TH;             // output rows per tile (tile = 8 x TH pixels)
-  int a_stage_bytes;  // bytes of one activation stage
-  int sa, sb;         // activation stages per issuer / shared weight stages
-  int b_resident;     // whole weight matrix kept in smem (requires n_tiles == 1)
-  int m_super;        // ceil(m_tiles / kMI): pixel tiles are handed out in groups of kMI
-  FastDiv d_msuper, d_tx, d_ty;   // dividers by m_super, tiles_x, tiles_y
-  int m_major;        // work item s -> (pixel-tile group s / n_tiles, n-tile s % n_tiles): the n-tiles of one pixel-tile group
-                      // run on neighbouring CTAs at the same time, so the activation tile comes from HBM once and from L2
-                      // for the other n-tiles (n-major order re-read the whole input from HBM once per n-tile)
-  FastDiv d_nt;       // divider by n_tiles
-  int pitch;          // halo pixels per stage row: kMPitch (8-pixel-wide tiles) or W + 2 (row-strip tiles)
-  int sbo;            // byte distance of consecutive 8-row groups of the A operand: pitch * 128 (tiles) or 1024 (strips)
-  int strip;          // row-strip tiles (see the header comment); TH is then the number of image rows per tile
-  FastDiv d_pitch;    // divider by pitch (strip mode: MMA row -> (image row, x))
-  int rowtaps;        // 1x1 tiles: k-chunk kc is ROW TAP kc of an overlapping-window input.  1: one A box per tap (at row
-                      // y0 + kc); 2: ONE box of TH + R - 1 rows per tile, tap kc reads it TW * 128 * kc bytes further in
-                      // (a "row halo": the window rows of neighbouring taps are the same bytes)
-  int resid_tma;      // kRT kernels: residual tiles arrive by TMA in the staging buffers (see the header comment)
-  int debug;          // ablation switches for profiling (results are wrong when set): 1 = no TMEM loads,
-                      // 2 = no staging stores / TMA store, 4 = activation TMA loads only for the first stages,
-                      // 16 = no residual loads (ADD / GATE epilogues)
-};
-
-__device__ __forceinline__ uint32_t bf16x2_max(uint32_t a, uint32_t b) {
-  __nv_bfloat162 r = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a), *reinterpret_cast<__nv_bfloat162*>(&b));
-  return *reinterpret_cast<uint32_t*>(&r);
-}
 static constexpr int kPoolBytes = 4096;
 
-// ---- CTA-pair (cta_group::2) forms
-__device__ __forceinline__ uint32_t mp_rank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void mp_cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t mp_leader_addr(const void* p) {   // shared::cluster address of `p` in the leader CTA
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(0u));
-  return r;
-}
-__device__ __forceinline__ void mp_arrive_leader(const void* bar) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(mp_leader_addr(bar)) : "memory");
-}
-__device__ __forceinline__ void mp_tma_load_4d(void* dst, const CUtensorMap* m, const void* leader_bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], "
-      "[%2];" ::"r"(smem_u32(dst)),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(mp_leader_addr(leader_bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void mp_tma_load_2d(void* dst, const CUtensorMap* m, const void* leader_bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(mp_leader_addr(leader_bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
+// tcgen05.mma / commit of one CTA or (kPair) of a CTA pair; pair commits arrive on the barrier at `bar`'s offset in
+// BOTH CTAs
 template <int kPair>
 __device__ __forceinline__ void mp_umma(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  if constexpr (kPair) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-  } else {
-    umma_bf16(d_tmem, adesc, bdesc, idesc, accumulate);
-  }
+  if constexpr (kPair) umma_bf16_pair(d_tmem, adesc, bdesc, idesc, accumulate);
+  else umma_bf16(d_tmem, adesc, bdesc, idesc, accumulate);
 }
-// arrive on `bar` once the MMAs issued so far have completed; pairs: on the barrier at that offset in BOTH CTAs
 template <int kPair>
 __device__ __forceinline__ void mp_commit(uint64_t* bar) {
-  if constexpr (kPair) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                     smem_u32(bar)),
-                 "h"((uint16_t)3)
-                 : "memory");
-  } else {
-    umma_commit(bar);
-  }
-}   // pooled sub-tile staging: 4 x TH/2 <= 32 pixels x 64 channels bf16
-
-struct StoreMaps {  // output maps: [0] for plain stores, [q] = quadrant (dy,dx) of a ConvTranspose 2x2 s2 scatter;
-  CUtensorMap m[5];  // [4] = load map of the residual tensor (kRT)
-};
+  if constexpr (kPair) umma_commit_pair(bar);
+  else umma_commit(bar);
+}
 
 template <int kAct, int kTaps, int kMode, int kKS, int kRT, int kPair>
 __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_multi_kernel(const __grid_constant__ CUtensorMap tmA,
@@ -235,7 +126,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
   const int warp = uniform_warp_idx();
   const int lane = threadIdx.x & 31;
   const int total_super = hp.m_super * p.n_tiles;
-  const uint32_t rank = kPair ? mp_rank() : 0u;                         // CTA of the pair (0 = leader: issues every MMA)
+  const uint32_t rank = kPair ? cluster_ctarank() : 0u;                        // CTA of the pair (0 = leader: issues every MMA)
   const int cta0 = kPair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;     // first work item / stride of the persistent loops
   const int ncta = kPair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
   // pixel tile of (group ms, stream i): pairs interleave the two CTAs; tiles past the end stay in the loops of a pair
@@ -286,8 +177,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
   }
   if (warp == kMAllocWarp) {
     if constexpr (kPair) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr)), "r"(p.tmem_cols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+      tmem_alloc_pair(tmem_ptr, p.tmem_cols);
     } else {
       tmem_alloc(tmem_ptr, p.tmem_cols);
       tmem_relinquish();
@@ -299,7 +189,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
   }
   tc_fence_before();
   __syncthreads();
-  if constexpr (kPair) mp_cluster_sync();   // the barriers of both CTAs exist before any remote arrive / TMA signal
+  if constexpr (kPair) cluster_sync();   // the barriers of both CTAs exist before any remote arrive / TMA signal
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   // Everything above touched only kernel parameters and constant weights; from here on the roles read activations /
@@ -375,7 +265,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
           if (elect_one_sync()) {
             if constexpr (kPair) {   // the leader's barrier collects the bytes of both CTAs' loads
               if (rank == 0) mbar_arrive_expect_tx(&a_full[slot], 2 * a_tx);
-              mp_tma_load_4d(sA + slot * hp.a_stage_bytes, &tmA, &a_full[slot], kc * 64, x0 - 1, y0 - 1, n);
+              tma_load_4d_pair(sA + slot * hp.a_stage_bytes, &tmA, leader_addr(&a_full[slot]), kc * 64, x0 - 1, y0 - 1, n);
             } else if ((hp.debug & 4) && s >= (int)gridDim.x * 2) {
               mbar_arrive(&a_full[slot]);
             } else {
@@ -410,8 +300,8 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
           if (rank == 0) mbar_arrive_expect_tx(&b_full[0], (uint32_t)(2 * kTaps * p.kchunks * b_tile_bytes));
           for (int kc = 0; kc < p.kchunks; ++kc)
             for (int tap = 0; tap < kTaps; ++tap)
-              mp_tma_load_2d(sB + (kc * kTaps + tap) * b_tile_bytes, &tmB, &b_full[0], (tap * p.kchunks + kc) * 64,
-                             (int)rank * (p.BN / 2));
+              tma_load_2d_pair(sB + (kc * kTaps + tap) * b_tile_bytes, &tmB, &b_full[0],
+                               (tap * p.kchunks + kc) * 64, (int)rank * (p.BN / 2));
         } else {
           mbar_arrive_expect_tx(&b_full[0], (uint32_t)(kTaps * p.kchunks * b_tile_bytes));
           for (int kc = 0; kc < p.kchunks; ++kc)
@@ -438,8 +328,8 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
             if (elect_one_sync()) {
               if constexpr (kPair) {
                 if (rank == 0) mbar_arrive_expect_tx(&b_full[bs], (uint32_t)(2 * b_tile_bytes));
-                mp_tma_load_2d(sB + bs * b_tile_bytes, &tmB, &b_full[bs], (tap * p.kchunks + kc) * 64,
-                               nt * p.BN + (int)rank * (p.BN / 2));
+                tma_load_2d_pair(sB + bs * b_tile_bytes, &tmB, &b_full[bs], (tap * p.kchunks + kc) * 64,
+                                 nt * p.BN + (int)rank * (p.BN / 2));
               } else {
                 mbar_arrive_expect_tx(&b_full[bs], (uint32_t)b_tile_bytes);
                 tma_load_2d(sB + bs * b_tile_bytes, &tmB, &b_full[bs], (tap * p.kchunks + kc) * 64, nt * p.BN);
@@ -676,9 +566,10 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
           if (p.prof) e_wobuf += clock64() - tw0;
         }
         uint8_t* so_row = sOi + obuf * obuf_bytes + srow * 128;
-        // unroll factor of the chunk loop (UG_EPI_UNROLL, default see below): the epilogue warps of an SMSP share its
-        // 6 KB L0 instruction cache with an MMA issuer / producer warp; with run-time epilogue modes a 4x larger loop
-        // body measurably slowed the MMA issue (0.24 -> 0.29 ms), so round 1 did not unroll at all
+        // the chunk loop is not unrolled (kEpiUnroll): the epilogue warps of an SMSP share its 6 KB L0 instruction
+        // cache with an MMA issuer / producer warp; with run-time epilogue modes a 4x larger loop body measurably slowed
+        // the MMA issue (0.24 -> 0.29 ms), and x2 / x4 unrolling of this loop measured neutral / slower
+        // (profiles/r02_epilogue_unroll.txt)
         const long long tl0 = p.prof ? clock64() : 0;
 #pragma unroll kEpiUnroll
         for (int cc = 0; cc < 4; ++cc) {
@@ -783,7 +674,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
           tc_fence_before();
           __syncwarp();
           if (lane == 0) {
-            if (kPair && rank != 0) mp_arrive_leader(&acc_empty[i * p.acc_stages + acc]);
+            if (kPair && rank != 0) mbar_arrive_cluster(leader_addr(&acc_empty[i * p.acc_stages + acc]));
             else mbar_arrive(&acc_empty[i * p.acc_stages + acc]);
           }
         }
@@ -876,7 +767,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
         tc_fence_before();
         __syncwarp();
         if (lane == 0) {
-          if (kPair && rank != 0) mp_arrive_leader(&acc_empty[i * p.acc_stages + acc]);
+          if (kPair && rank != 0) mbar_arrive_cluster(leader_addr(&acc_empty[i * p.acc_stages + acc]));
           else mbar_arrive(&acc_empty[i * p.acc_stages + acc]);
         }
         if (valid) {
@@ -908,36 +799,46 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
   tc_fence_before();
   __syncthreads();
   if constexpr (kPair) {
-    mp_cluster_sync();   // the leader's MMAs write the peer's tensor memory until both CTAs are done
-    if (warp == kMAllocWarp)
-      asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols) : "memory");
+    cluster_sync();   // the leader's MMAs write the peer's tensor memory until both CTAs are done
+    if (warp == kMAllocWarp) tmem_dealloc_pair(tmem_base, p.tmem_cols);
   } else {
     if (warp == kMAllocWarp) tmem_dealloc(tmem_base, p.tmem_cols);
   }
 }
 
 // ------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
-static inline int cdiv_m(int a, int b) { return (a + b - 1) / b; }
-
 void choose_tile(int B, int H, int W, int* TW, int* TH, int* TN);  // conv_gemm.cu
 
-static int encode_map(EncodeTiledFn encode, CUtensorMap* m, void* base, int rank, const cuuint64_t* dims,
-                      const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapL2promotion promo) {
-  cuuint32_t es[4] = {1, 1, 1, 1};
-  return (int)encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-}
+// The instantiated (activation, taps, epilogue mode, K-split, TMA residual, CTA pair) combinations; conv_multi_prepare
+// admits exactly these.
+struct MultiInstance {
+  int act, taps, mode, ks, rt, pair;
+  MultiKernelFn fn;
+};
+#define UG_MULTI_CASE(A, T, M, K, RT, P) {A, T, M, K, RT, P, conv_multi_kernel<A, T, M, K, RT, P>},
+static const MultiInstance kMultiInstances[] = {
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_STORE, 1, 0, 0)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_STORE, 2, 0, 0)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_ADD, 1, 0, 0)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 1, 0, 0)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 2, 0, 0)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 2, 1, 0)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_OUTC, 1, 0, 0)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_OUTC, 2, 0, 0)
+    UG_MULTI_CASE(UG_ACT_NONE, 1, UG_EPI_STORE, 1, 0, 0)
+    UG_MULTI_CASE(UG_ACT_RELU, 1, UG_EPI_STORE, 1, 0, 0)
+    UG_MULTI_CASE(UG_ACT_GELU, 1, UG_EPI_STORE, 1, 0, 0)
+    UG_MULTI_CASE(UG_ACT_NONE, 1, UG_EPI_ADD, 1, 0, 0)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_STORE, 1, 0, 1)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 1, 0, 1)
+    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 1, 1, 1)
+};
+#undef UG_MULTI_CASE
 
 // Fills L for the multi-issuer kernel: 3x3 pad-1 convolutions (halo tiles) and 1x1 convolutions / linear layers /
 // ConvTranspose 2x2 s2 (plain pixel tiles).  Returns UG_EUNSUPPORTED when the shape does not fit it.
 int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* L, int pair) {
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return set_error(h, UG_ECUDA, "cuTensorMapEncodeTiled entry point unavailable");
+  if (!get_encode_fn()) return set_error(h, UG_ECUDA, "cuTensorMapEncodeTiled entry point unavailable");
   const int up = d->up == 2 ? 2 : 1;
   // row taps (see ug_conv_desc.in_rstride): R x 1 "valid" convolution over an overlapping-window input, one 64-element
   // window per tap: runs as a 1x1 tile whose R k-chunks are the taps
@@ -959,22 +860,21 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
   int strip = 0, pitch = kMPitch;
   if (taps == 9) {
     TW = 8;
-    TH = cdiv_m(d->H, cdiv_m(d->H, 16));  // <= 16 rows per tile, no wasted tile rows
+    TH = ceil_div(d->H, ceil_div(d->H, 16));  // <= 16 rows per tile, no wasted tile rows
     TN = 1;
     // row-strip tiles (SR full image rows per tile) when they put more output pixels on the 128 MMA rows than the
-    // 8-pixel-wide tiles do: 28-wide maps (87.5 % instead of 76.6 %).  UG_STRIP=0 turns them off.
-    static const int strip_on = [] { const char* e = getenv("UG_STRIP"); return e ? atoi(e) : 1; }();
+    // 8-pixel-wide tiles do: 28-wide maps (87.5 % instead of 76.6 %)
     const int sr_max = 128 / (d->W + 2);
-    if (strip_on && sr_max >= 1 && !d->stats_sum) {
+    if (sr_max >= 1 && !d->stats_sum) {
       int sr = std::min(sr_max, d->H);
       if (d->pool_out) sr &= ~1;                                   // pooled tiles need an even number of rows
       if (sr >= 1) {
-        sr = cdiv_m(d->H, cdiv_m(d->H, sr));                       // no wasted tile rows
+        sr = ceil_div(d->H, ceil_div(d->H, sr));                   // no wasted tile rows
         if (d->pool_out && (sr & 1)) sr = 0;
       }
       if (sr >= 1) {
-        const double fill_strip = (double)d->H * d->W / ((double)cdiv_m(d->H, sr) * 128.0);
-        const double fill_tile = (double)d->H * d->W / ((double)cdiv_m(d->W, 8) * cdiv_m(d->H, TH) * 128.0);
+        const double fill_strip = (double)d->H * d->W / ((double)ceil_div(d->H, sr) * 128.0);
+        const double fill_tile = (double)d->H * d->W / ((double)ceil_div(d->W, 8) * ceil_div(d->H, TH) * 128.0);
         if (fill_strip > fill_tile + 1e-6) {
           strip = 1;
           pitch = d->W + 2;
@@ -987,9 +887,9 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
     choose_tile(d->B, d->H, d->W, &TW, &TH, &TN);
     if (TW > 256 || TH > 256 || TN > 256) return set_error(h, UG_EUNSUPPORTED, "conv(multi): tile exceeds the TMA box limits");
   }
-  const int cin_pad = cdiv_m(d->Cin, 64) * 64;
+  const int cin_pad = ceil_div(d->Cin, 64) * 64;
   const int kchunks = rowtaps ? d->R : cin_pad / 64;
-  const int n_tiles = cdiv_m(d->N, BN);
+  const int n_tiles = ceil_div(d->N, BN);
   const int npad = n_tiles * BN;
   const long long ktot = rowtaps ? (long long)d->R * 64 : (long long)taps * cin_pad;
   const int tma_store = d->mode != UG_EPI_OUTC;
@@ -1004,13 +904,12 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
                !(d->mode == UG_EPI_STORE || d->mode == UG_EPI_GATE)))
     return set_error(h, UG_EUNSUPPORTED, "conv(multi, pairs): 3x3 layers with 128-column n-tiles, STORE / GATE epilogue");
   if (stats && (taps != 9 || d->mode != UG_EPI_STORE || !d->stats_max ||
-                d->stats_tiles != cdiv_m(d->W, 8) * cdiv_m(d->H, TH)))
+                d->stats_tiles != ceil_div(d->W, 8) * ceil_div(d->H, TH)))
     return set_error(h, UG_EUNSUPPORTED, "conv(multi): fused channel statistics need a 3x3 STORE conv and stats_tiles == %d",
-                     cdiv_m(d->W, 8) * cdiv_m(d->H, TH));
+                     ceil_div(d->W, 8) * ceil_div(d->H, TH));
   const int obuf_bytes = tma_store ? kABytesPerStage + (pool ? kPoolBytes : 0) : 0;  // per staging buffer, for sizing
-  // K-split: two issuing warps per tile stream for narrow 3x3 tiles (see the header comment); UG_KSPLIT=0 turns it off
-  static const int ksplit_on = [] { const char* e = getenv("UG_KSPLIT"); return e ? atoi(e) : 1; }();
-  const int ks = (taps == 9 && BN <= 64 && !pair && ksplit_on && d->act == UG_ACT_RELU && d->mode != UG_EPI_ADD) ? 2 : 1;
+  // K-split: two issuing warps per tile stream for narrow 3x3 tiles (see the header comment)
+  const int ks = (taps == 9 && BN <= 64 && !pair && d->act == UG_ACT_RELU && d->mode != UG_EPI_ADD) ? 2 : 1;
   // instantiated (activation, taps, epilogue) combinations: 3x3 = ReLU with any epilogue; 1x1 = plain stores with any
   // activation, residual add without activation
   if (taps == 9 && d->act != UG_ACT_RELU)
@@ -1020,34 +919,31 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
   const int acc_stages = std::max(1, std::min(4, 512 / (kMI * ks * BN)));
   // TMA residual (see the header comment): CoordAtt3 combine layers with one 64-column n-tile and resident weights.
   // Needs two staging buffers per stream next to the weights: tiles of <= 14 rows make room (the layer is bound by its
-  // epilogue, not by the 12.5 % of MMA rows this leaves empty).  UG_RESID_TMA=0 turns it off.
-  static const int rt_on = [] { const char* e = getenv("UG_RESID_TMA"); return e ? atoi(e) : 1; }();
-  int rt = (rt_on && !pair && taps == 9 && !strip && ks == 2 && d->mode == UG_EPI_GATE && d->N <= 64 && BN == 64 && d->add_bstride > 0 &&
+  // epilogue, not by the 12.5 % of MMA rows this leaves empty).
+  int rt = (!pair && taps == 9 && !strip && ks == 2 && d->mode == UG_EPI_GATE && d->N <= 64 && BN == 64 && d->add_bstride > 0 &&
             !pool && !stats) ? 1 : 0;
   // pair mode: the residual of every 64-column sub-tile by TMA (an extra warp produces them: the weight warp is streaming);
   // costs the second staging buffer per stream, i.e. four of the 8 KB weight-ring slots
-  static const int rt128_on = [] { const char* e = getenv("UG_RESID_TMA128"); return e ? atoi(e) : 1; }();
-  const int rt_pair = (rt_on && rt128_on && pair && d->mode == UG_EPI_GATE && d->add_bstride > 0 && d->add_cstride % 8 == 0 &&
+  const int rt_pair = (pair && d->mode == UG_EPI_GATE && d->add_bstride > 0 && d->add_cstride % 8 == 0 &&
                        !(reinterpret_cast<uintptr_t>(d->add) & 15)) ? 1 : 0;
   if (rt_pair) rt = 1;
   if (rt && !pair) {
-    const int th2 = cdiv_m(d->H, cdiv_m(d->H, 14));
+    const int th2 = ceil_div(d->H, ceil_div(d->H, 14));
     const long long need = (long long)taps * kchunks * BN * 128 + kMI * 2LL * (((kMPitch * (th2 + 2) * 128) + 1023) / 1024 * 1024) +
                            kMI * 2LL * kABytesPerStage + 4096;
     if (need <= 227LL * 1024) TH = th2;
     else rt = 0;
   }
   // row halo (rowtaps 2): one box of TH + R - 1 rows per tile instead of R boxes of TH rows; needs whole 1024-byte swizzle
-  // atoms per tile row (TW % 8 == 0) and one image per tile.  UG_ROW_HALO=0 keeps one box per tap.
-  static const int row_halo_on = [] { const char* e = getenv("UG_ROW_HALO"); return e ? atoi(e) : 1; }();
-  const int row_halo = (rowtaps && row_halo_on && TW % 8 == 0 && TN == 1) ? 1 : 0;
+  // atoms per tile row (TW % 8 == 0) and one image per tile; otherwise one box per tap
+  const int row_halo = (rowtaps && TW % 8 == 0 && TN == 1) ? 1 : 0;
   const int a_bytes = taps == 9 ? pitch * (TH + 2) * 128 : TW * (TH + (row_halo ? d->R - 1 : 0)) * TN * 128;
   // strip mode: MMA row 127 of tap (2,2) reads halo position 127 + 2*pitch + 2, past the loaded box (garbage rows only)
   const int a_span = strip ? std::max(a_bytes, (128 + 2 * pitch + 2) * 128) : a_bytes;
   const int a_stage = ((a_span + 1023) / 1024) * 1024;
   const int b_tile = (pair ? BN / 2 : BN) * 128;   // pairs: each CTA holds half of the rows of a weight tile
 
-  MultiParams hp;
+  MultiParams& hp = L->mp;
   memset(&hp, 0, sizeof(hp));
   hp.TH = TH;
   hp.a_stage_bytes = a_stage;
@@ -1089,8 +985,8 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
   memset(&p, 0, sizeof(p));
   p.H = d->H; p.W = d->W; p.B = d->B;
   p.TW = TW; p.TH = TH; p.TN = TN;
-  p.tiles_x = cdiv_m(d->W, TW);
-  p.tiles_y = cdiv_m(d->H, TH);
+  p.tiles_x = ceil_div(d->W, TW);
+  p.tiles_y = ceil_div(d->H, TH);
   p.R = d->R; p.S = d->S; p.pad = d->pad;
   p.kchunks = kchunks; p.num_k = taps * kchunks;
   p.N = d->N; p.BN = BN; p.stages = hp.sa;
@@ -1106,20 +1002,23 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
   p.add = d->add; p.add_bstride = d->add_bstride; p.add_cstride = d->add_cstride;
   p.gate = d->gate; p.outc_w = d->outc_w; p.outc_b = d->outc_b;
   p.logits = d->logits; p.mask = d->mask;
-  p.m_tiles = p.tiles_x * p.tiles_y * cdiv_m(d->B, TN); p.n_tiles = n_tiles; p.acc_stages = acc_stages;
+  p.m_tiles = p.tiles_x * p.tiles_y * ceil_div(d->B, TN); p.n_tiles = n_tiles; p.acc_stages = acc_stages;
   p.tma_store = tma_store; p.obufs = obufs; p.npad = npad; p.pool = pool;
   p.stats_sum = d->stats_sum; p.stats_max = d->stats_max;
-  hp.m_super = cdiv_m(p.m_tiles, kMI * (pair ? 2 : 1));
-  L->variant = 5;
-  L->halo_pair = pair;
-  L->halo_mode = taps;
-  L->halo_TH = TH; L->halo_a_stage = a_stage; L->halo_copy = hp.m_super;
-  L->halo_sa = hp.sa; L->halo_sb = hp.sb; L->halo_bres = hp.b_resident;
-  L->halo_debug = d->stages >= 100 ? d->stages - 100 : 0;  // profiling ablations (scripts/conv_prof.py)
-  L->halo_ks = ks;
-  L->halo_rt = rt;
-  L->halo_rowtaps = hp.rowtaps;
-  L->halo_strip = strip; L->halo_pitch = pitch;
+  hp.m_super = ceil_div(p.m_tiles, kMI * (pair ? 2 : 1));
+  hp.d_msuper = make_fastdiv(hp.m_super);
+  hp.d_tx = make_fastdiv(p.tiles_x);
+  hp.d_ty = make_fastdiv(p.tiles_y);
+  hp.m_major = n_tiles > 1 ? 1 : 0;
+  hp.d_nt = make_fastdiv(n_tiles);
+  hp.d_pitch = make_fastdiv(pitch);
+  hp.debug = d->stages >= 100 ? d->stages - 100 : 0;  // profiling ablations (scripts/conv_prof.py)
+  L->kernel = pair ? ConvKernel::MultiPair : ConvKernel::Multi;
+  L->multi_fn = nullptr;
+  for (const MultiInstance& k : kMultiInstances)
+    if (k.act == d->act && k.taps == taps && k.mode == d->mode && k.ks == ks && k.rt == rt && k.pair == pair) L->multi_fn = k.fn;
+  if (!L->multi_fn) return set_error(h, UG_EUNSUPPORTED, "conv(multi): no kernel instantiated for this layer");
+  L->block = kMultiThreads(ks, rt && pair);
 
   {
     const long long in_h = d->H + (rowtaps ? d->R - 1 : 0);
@@ -1130,8 +1029,7 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
     cuuint64_t strides[3] = {(cuuint64_t)d->in_cstride * 2, (cuuint64_t)rs * 2, (cuuint64_t)bs * 2};
     cuuint32_t box9[4] = {64, (cuuint32_t)pitch, (cuuint32_t)(TH + 2), 1};
     cuuint32_t box1[4] = {64, (cuuint32_t)TW, (cuuint32_t)(TH + (row_halo ? d->R - 1 : 0)), (cuuint32_t)TN};
-    const int r = encode_map(encode, &L->tmA, const_cast<void*>(d->in), 4, dims, strides, taps == 9 ? box9 : box1,
-                             CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+    const int r = encode_bf16_sw128(&L->tmA, d->in, 4, dims, strides, taps == 9 ? box9 : box1, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
     if (r) return set_error(h, UG_ECUDA, "conv(multi): activation tensor map encode failed (%d)", r);
   }
   {
@@ -1140,17 +1038,15 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
     cuuint64_t dims[2] = {(cuuint64_t)ktot, (cuuint64_t)d->N};
     cuuint64_t strides[1] = {(cuuint64_t)ktot * 2};
     cuuint32_t box[2] = {64, (cuuint32_t)(pair ? BN / 2 : BN)};
-    const int r = encode_map(encode, &L->tmB, const_cast<void*>(d->w), 2, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+    const int r = encode_bf16_sw128(&L->tmB, d->w, 2, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
     if (r) return set_error(h, UG_ECUDA, "conv(multi): weight tensor map encode failed (%d)", r);
   }
-  memset(L->tmQ, 0, sizeof(L->tmQ));
-  memset(&L->tmO, 0, sizeof(L->tmO));
-  memset(&L->tmR, 0, sizeof(L->tmR));
+  memset(&L->maps, 0, sizeof(L->maps));
   if (rt) {  // load map of the residual tensor, same box as the output store
     cuuint64_t dims[4] = {(cuuint64_t)d->N, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->B};
     cuuint64_t strides[3] = {(cuuint64_t)d->add_cstride * 2, (cuuint64_t)d->W * d->add_cstride * 2, (cuuint64_t)d->add_bstride * 2};
     cuuint32_t box[4] = {64, (cuuint32_t)TW, (cuuint32_t)TH, (cuuint32_t)TN};
-    const int r = encode_map(encode, &L->tmR, const_cast<void*>(d->add), 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+    const int r = encode_bf16_sw128(&L->maps.m[4], d->add, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
     if (r) return set_error(h, UG_ECUDA, "conv(multi): residual tensor map encode failed (%d)", r);
   }
   if (tma_store) {
@@ -1159,7 +1055,7 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
       cuuint64_t dims[4] = {(cuuint64_t)d->N, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->B};
       cuuint64_t strides[3] = {(cuuint64_t)d->out_cstride * 2, (cuuint64_t)d->W * d->out_cstride * 2,
                                (cuuint64_t)d->H * d->W * d->out_cstride * 2};
-      const int r = encode_map(encode, &L->tmO, d->out, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+      const int r = encode_bf16_sw128(&L->maps.m[0], d->out, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
       if (r) return set_error(h, UG_ECUDA, "conv(multi): output tensor map encode failed (%d)", r);
       if (pool) {  // fused nn.MaxPool2d(2): pooled tile = 4 x TH/2 pixels of the half-resolution map
         const long long pcs = d->pool_cstride;
@@ -1167,7 +1063,7 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
         cuuint64_t pstrides[3] = {(cuuint64_t)(pcs * 2), (cuuint64_t)((d->W / 2) * pcs * 2),
                                   (cuuint64_t)((long long)(d->H / 2) * (d->W / 2) * pcs * 2)};
         cuuint32_t pbox[4] = {64, (cuuint32_t)(TW / 2), (cuuint32_t)(TH / 2), 1};
-        const int rp = encode_map(encode, &L->tmQ[0], d->pool_out, 4, pdims, pstrides, pbox, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+        const int rp = encode_bf16_sw128(&L->maps.m[1], d->pool_out, 4, pdims, pstrides, pbox, CU_TENSOR_MAP_L2_PROMOTION_NONE);
         if (rp) return set_error(h, UG_ECUDA, "conv(multi): pooled output tensor map encode failed (%d)", rp);
       }
     } else {
@@ -1179,8 +1075,7 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
         void* base = static_cast<char*>(d->out) + ((long long)dy * OW + dx) * cs * 2;
         cuuint64_t dims[4] = {(cuuint64_t)d->convt_cout, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->B};
         cuuint64_t strides[3] = {(cuuint64_t)(2 * cs * 2), (cuuint64_t)(2 * OW * cs * 2), (cuuint64_t)(OH * OW * cs * 2)};
-        CUtensorMap* m = q == 0 ? &L->tmO : &L->tmQ[q - 1];
-        const int r = encode_map(encode, m, base, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+        const int r = encode_bf16_sw128(&L->maps.m[q], base, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
         if (r) return set_error(h, UG_ECUDA, "conv(multi): ConvTranspose output tensor map encode failed (%d)", r);
       }
     }
@@ -1197,100 +1092,18 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
   return UG_OK;
 }
 
-template <int kAct, int kTaps, int kMode, int kKS, int kRT = 0, int kPair = 0>
-static cudaError_t launch_one(ug_engine* h, const ConvLaunch* L, const StoreMaps& maps, const MultiParams& hp,
-                              cudaStream_t s, bool set_attr) {
-  auto fn = conv_multi_kernel<kAct, kTaps, kMode, kKS, kRT, kPair>;
-  if (set_attr) return cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-  if constexpr (kPair) {   // clusters of two CTAs (+ programmatic dependent launch)
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(std::min(L->grid.x, 2u * (unsigned)max_cluster_pairs(h)));   // persistent loops: any even grid works
-    cfg.blockDim = dim3(kMultiThreads(kKS, kRT && kPair));
-    cfg.dynamicSmemBytes = L->smem;
-    cfg.stream = s;
-    cudaLaunchAttribute at[2];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = h->pdl ? 2 : 1;
-    return cudaLaunchKernelEx(&cfg, fn, L->tmA, L->tmB, maps, L->p, hp);
-  } else {
-    return launch_pdl(h, fn, L->grid, kMultiThreads(kKS), L->smem, s, L->tmA, L->tmB, maps, L->p, hp);
-  }
-}
-
-// Dispatch over the instantiated (activation, taps, epilogue mode, K-split) combinations (conv_multi_prepare rejects the
-// others).  set_attr = true raises the dynamic shared memory limit of every instantiation instead of launching.
-static cudaError_t dispatch_multi(ug_engine* h, const ConvLaunch* L, const StoreMaps& maps, const MultiParams& hp,
-                                  cudaStream_t s, bool set_attr) {
-  cudaError_t e = cudaSuccess;
-  const int act = L->p.act, mode = L->p.mode, taps = L->halo_mode, ks = L->halo_ks;
-  if (set_attr) {
-    if (e == cudaSuccess) e = launch_one<UG_ACT_RELU, 9, UG_EPI_GATE, 2, 1>(h, L, maps, hp, s, true);
-    if (e == cudaSuccess) e = launch_one<UG_ACT_RELU, 9, UG_EPI_STORE, 1, 0, 1>(h, L, maps, hp, s, true);
-    if (e == cudaSuccess) e = launch_one<UG_ACT_RELU, 9, UG_EPI_GATE, 1, 0, 1>(h, L, maps, hp, s, true);
-    if (e == cudaSuccess) e = launch_one<UG_ACT_RELU, 9, UG_EPI_GATE, 1, 1, 1>(h, L, maps, hp, s, true);
-  } else if (L->halo_pair) {   // CTA pairs: three instantiations (conv_multi_prepare admits exactly these)
-    if (mode == UG_EPI_GATE && L->halo_rt) return launch_one<UG_ACT_RELU, 9, UG_EPI_GATE, 1, 1, 1>(h, L, maps, hp, s, false);
-    if (mode == UG_EPI_GATE) return launch_one<UG_ACT_RELU, 9, UG_EPI_GATE, 1, 0, 1>(h, L, maps, hp, s, false);
-    return launch_one<UG_ACT_RELU, 9, UG_EPI_STORE, 1, 0, 1>(h, L, maps, hp, s, false);
-  } else if (L->halo_rt) {  // TMA residual: the only instantiation (conv_multi_prepare sets rt for exactly this case)
-    return launch_one<UG_ACT_RELU, 9, UG_EPI_GATE, 2, 1>(h, L, maps, hp, s, false);
-  }
-#define UG_MULTI_CASE(A, T, M, K)                                                        \
-  if (set_attr) {                                                                        \
-    if (e == cudaSuccess) e = launch_one<A, T, M, K>(h, L, maps, hp, s, true);           \
-  } else if (act == A && taps == T && mode == M && ks == K) {                            \
-    return launch_one<A, T, M, K>(h, L, maps, hp, s, false);                             \
-  }
-  UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_STORE, 1)
-  UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_STORE, 2)
-  UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_ADD, 1)
-  UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 1)
-  UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 2)
-  UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_OUTC, 1)
-  UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_OUTC, 2)
-  UG_MULTI_CASE(UG_ACT_NONE, 1, UG_EPI_STORE, 1)
-  UG_MULTI_CASE(UG_ACT_RELU, 1, UG_EPI_STORE, 1)
-  UG_MULTI_CASE(UG_ACT_GELU, 1, UG_EPI_STORE, 1)
-  UG_MULTI_CASE(UG_ACT_NONE, 1, UG_EPI_ADD, 1)
-#undef UG_MULTI_CASE
-  return set_attr ? e : cudaErrorInvalidValue;
-}
-
 int conv_multi_launch(ug_engine* h, const ConvLaunch* L, cudaStream_t s) {
-  MultiParams hp;
-  memset(&hp, 0, sizeof(hp));
-  hp.TH = L->halo_TH; hp.a_stage_bytes = L->halo_a_stage;
-  hp.sa = L->halo_sa; hp.sb = L->halo_sb; hp.b_resident = L->halo_bres; hp.m_super = L->halo_copy;
-  hp.debug = L->halo_debug;
-  hp.resid_tma = L->halo_rt;
-  hp.rowtaps = L->halo_rowtaps;
-  hp.strip = L->halo_strip; hp.pitch = L->halo_pitch;
-  hp.sbo = hp.strip ? 1024 : hp.pitch * 128;
-  hp.d_pitch = make_fastdiv(hp.pitch);
-  hp.d_msuper = make_fastdiv(hp.m_super);
-  static const int m_major_on = [] { const char* e = getenv("UG_M_MAJOR"); return e ? atoi(e) : 1; }();
-  hp.m_major = (m_major_on && L->p.n_tiles > 1) ? 1 : 0;
-  hp.d_nt = make_fastdiv(L->p.n_tiles);
-  hp.d_tx = make_fastdiv(L->p.tiles_x);
-  hp.d_ty = make_fastdiv(L->p.tiles_y);
-  StoreMaps maps;
-  maps.m[0] = L->tmO;
-  maps.m[1] = L->tmQ[0];
-  maps.m[2] = L->tmQ[1];
-  maps.m[3] = L->tmQ[2];
-  maps.m[4] = L->tmR;
   if (!h->attr_multi) {
-    const cudaError_t e = dispatch_multi(h, L, maps, hp, s, true);
-    if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(conv_multi_kernel)");
+    for (const MultiInstance& k : kMultiInstances) {
+      const cudaError_t e = cudaFuncSetAttribute((const void*)k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+      if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(conv_multi_kernel)");
+    }
     h->attr_multi = true;
   }
-  const cudaError_t e = dispatch_multi(h, L, maps, hp, s, false);
+  const cudaError_t e =
+      L->kernel == ConvKernel::MultiPair
+          ? launch_pairs(h, L->multi_fn, L->grid.x, L->block, L->smem, s, L->tmA, L->tmB, L->maps, L->p, L->mp)
+          : launch_pdl(L->multi_fn, L->grid, L->block, L->smem, s, L->tmA, L->tmB, L->maps, L->p, L->mp);
   h->launches++;
   return check_cuda(h, e != cudaSuccess ? e : cudaGetLastError(), "conv_multi_kernel launch");
 }

@@ -24,11 +24,9 @@
 //     two-chain rate of profiles/r02_mma_pair.txt, and the epilogue of such a layer is 1/4 of its MMA time);
 //   * the CoordAtt3 combine (GATE epilogue, kRT) uses the residual-by-TMA protocol of conv_multi.cu: the weight warp
 //     loads the residual tile of the NEXT tile into the free staging buffer, the epilogue combines in place.
-#include <cfloat>
 #include <cstdio>
-#include <cstring>
 #include <cstdlib>
-#include <algorithm>
+#include <cstring>
 #include "conv_common.cuh"
 
 namespace ug {
@@ -40,91 +38,6 @@ static constexpr int kPPitch = 10;      // halo pitch: 8 output pixels + one bor
 static constexpr int kPAllocWarp = 8, kPProducerWarp = 9, kPIssuerWarp0 = 10;
 static constexpr int kPAcc = 2;         // accumulator stages per (stream, K-half): 2 x 2 x 2 x 64 = 512 TMEM columns
 static constexpr int kPPoolBytes = 4096;
-
-struct PairDiv {
-  unsigned mul, shift;
-  __device__ __forceinline__ int div(int n) const { return (int)(((unsigned long long)(unsigned)n * mul) >> shift); }
-};
-static PairDiv make_pairdiv(int d) {
-  PairDiv f;
-  int s = 0;
-  while ((1 << s) < d) ++s;
-  f.shift = 24 + s;
-  f.mul = (unsigned)(((1ULL << f.shift) + d - 1) / d);
-  return f;
-}
-
-struct PairParams {
-  int TH, a_stage_bytes, sa, n_quads;   // rows per tile, bytes of one activation stage, stages per stream, tile groups
-  int streams;                          // tile streams per CTA: 2, or 1 when the resident weights leave room for one
-  PairDiv d_tx, d_ty;
-};
-
-struct PairMaps {
-  CUtensorMap out, pool, resid;
-};
-
-__device__ __forceinline__ uint32_t pair_rank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void pair_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cluster address of `p` (a shared-memory object of this CTA) in the CTA with cluster rank `rank`
-__device__ __forceinline__ uint32_t pair_map(const void* p, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA loads whose completion may be signalled on the barrier of the PEER CTA of the pair
-__device__ __forceinline__ void tma_load_4d_pair(void* dst, const CUtensorMap* m, uint32_t bar_cluster_addr, int c0, int c1,
-                                                 int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], "
-      "[%2];" ::"r"(smem_u32(dst)),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* m, uint32_t bar_cluster_addr, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void umma_bf16_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrive on the barrier at this shared-memory offset in BOTH CTAs once the MMAs issued so far have completed
-__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"((uint16_t)3)
-               : "memory");
-}
-__device__ __forceinline__ uint64_t pair_desc_sbo(uint32_t smem_addr, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr & 0x3FFFF) >> 4);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>(sbo_bytes >> 4) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(2) << 61;
-  return d;
-}
-__device__ __forceinline__ uint32_t pair_bf16x2_max(uint32_t a, uint32_t b) {
-  __nv_bfloat162 r = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a), *reinterpret_cast<__nv_bfloat162*>(&b));
-  return *reinterpret_cast<uint32_t*>(&r);
-}
 
 template <int kMode, int kRT>
 __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_constant__ CUtensorMap tmA,
@@ -155,7 +68,7 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
 
   const int warp = uniform_warp_idx();
   const int lane = threadIdx.x & 31;
-  const uint32_t rank = pair_rank();
+  const uint32_t rank = cluster_ctarank();
   const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
 
   if (warp == kPProducerWarp && lane == 0) {
@@ -182,8 +95,7 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
     fence_mbar_init();
   }
   if (warp == kPAllocWarp) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tmem_alloc_pair(tmem_ptr, 512);
   }
   for (int i = threadIdx.x; i < 64; i += kPThreads) {
     sScale[i] = (i < p.N) ? (p.scale ? p.scale[i] : 1.0f) : 0.0f;
@@ -191,7 +103,7 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
   }
   tc_fence_before();
   __syncthreads();
-  pair_sync();                 // barriers of both CTAs are initialised before any remote arrive / TMA signal
+  cluster_sync();              // barriers of both CTAs are initialised before any remote arrive / TMA signal
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   if (warp != kPAllocWarp) pdl_wait();
@@ -223,7 +135,7 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
           mbar_wait(&a_empty[slot], aph[i] ^ 1);
           if (elect_one_sync()) {
             if (rank == 0) mbar_arrive_expect_tx(&a_full[slot], 2 * a_tx);
-            tma_load_4d_pair(sA + slot * hp.a_stage_bytes, &tmA, pair_map(&a_full[slot], 0), kc * 64, cx[i] - 1, cy[i] - 1, cn[i]);
+            tma_load_4d_pair(sA + slot * hp.a_stage_bytes, &tmA, leader_addr(&a_full[slot]), kc * 64, cx[i] - 1, cy[i] - 1, cn[i]);
           }
           __syncwarp();
           if (++as[i] == hp.sa) {
@@ -237,7 +149,7 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
     // ------------------------------------------------------------------ weights: this CTA's 32 rows of every (chunk, tap) tile
     if (elect_one_sync()) {
       if (rank == 0) mbar_arrive_expect_tx(b_full, (uint32_t)(2 * nb_tiles * kBTile));
-      const uint32_t bar = pair_map(b_full, 0);
+      const uint32_t bar = leader_addr(b_full);
       for (int kc = 0; kc < p.kchunks; ++kc)
         for (int tap = 0; tap < 9; ++tap)
           tma_load_2d_pair(sB + (kc * 9 + tap) * kBTile, &tmB, bar, (tap * p.kchunks + kc) * 64, (int)rank * 32);
@@ -288,7 +200,7 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
         for (int kc = 0; kc < p.kchunks; ++kc) {
           mbar_wait(&a_full[i * hp.sa + as], aph);
           tc_fence_after();
-          const uint64_t ad0 = pair_desc_sbo(smem_u32(sA + (i * hp.sa + as) * hp.a_stage_bytes), kPPitch * 128);
+          const uint64_t ad0 = umma_desc_sw128_sbo(smem_u32(sA + (i * hp.sa + as) * hp.a_stage_bytes), kPPitch * 128);
 #pragma unroll 3
           for (int tap = 0; tap < 9; ++tap) {
             const int item = kc * 9 + tap;
@@ -417,14 +329,14 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
           if (p.pool) {
             // fused nn.MaxPool2d(2): the 2x2 window of pixel (tx, ty) lives in lanes ^1 (x) and ^8 (y) of this warp
             uint4 m = o;
-            m.x = pair_bf16x2_max(m.x, __shfl_xor_sync(0xffffffffu, m.x, 1));
-            m.y = pair_bf16x2_max(m.y, __shfl_xor_sync(0xffffffffu, m.y, 1));
-            m.z = pair_bf16x2_max(m.z, __shfl_xor_sync(0xffffffffu, m.z, 1));
-            m.w = pair_bf16x2_max(m.w, __shfl_xor_sync(0xffffffffu, m.w, 1));
-            m.x = pair_bf16x2_max(m.x, __shfl_xor_sync(0xffffffffu, m.x, 8));
-            m.y = pair_bf16x2_max(m.y, __shfl_xor_sync(0xffffffffu, m.y, 8));
-            m.z = pair_bf16x2_max(m.z, __shfl_xor_sync(0xffffffffu, m.z, 8));
-            m.w = pair_bf16x2_max(m.w, __shfl_xor_sync(0xffffffffu, m.w, 8));
+            m.x = bf16x2_max(m.x, __shfl_xor_sync(0xffffffffu, m.x, 1));
+            m.y = bf16x2_max(m.y, __shfl_xor_sync(0xffffffffu, m.y, 1));
+            m.z = bf16x2_max(m.z, __shfl_xor_sync(0xffffffffu, m.z, 1));
+            m.w = bf16x2_max(m.w, __shfl_xor_sync(0xffffffffu, m.w, 1));
+            m.x = bf16x2_max(m.x, __shfl_xor_sync(0xffffffffu, m.x, 8));
+            m.y = bf16x2_max(m.y, __shfl_xor_sync(0xffffffffu, m.y, 8));
+            m.z = bf16x2_max(m.z, __shfl_xor_sync(0xffffffffu, m.z, 8));
+            m.w = bf16x2_max(m.w, __shfl_xor_sync(0xffffffffu, m.w, 8));
             if (((tx | ty) & 1) == 0) {
               const int pr = (ty >> 1) * 4 + (tx >> 1);
               *reinterpret_cast<uint4*>(sP + (i * p.obufs + obuf) * kPPoolBytes + pr * 128 + ((chunk ^ (pr & 7)) << 4)) = m;
@@ -438,7 +350,7 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
       __syncwarp();
       if (lane == 0) {
         if (rank == 0) mbar_arrive(&acc_empty[i * kPAcc + acc]);
-        else mbar_arrive_cluster(pair_map(&acc_empty[i * kPAcc + acc], 0));
+        else mbar_arrive_cluster(leader_addr(&acc_empty[i * kPAcc + acc]));
       }
       if constexpr (kMode == UG_EPI_OUTC) {
         if (valid) {
@@ -468,32 +380,17 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
 
   tc_fence_before();
   __syncthreads();
-  pair_sync();     // the peer's accumulators are still written by MMAs issued from the leader until both are done
-  if (warp == kPAllocWarp)
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+  cluster_sync();  // the peer's accumulators are still written by MMAs issued from the leader until both are done
+  if (warp == kPAllocWarp) tmem_dealloc_pair(tmem_base, 512);
 }
 
 // ------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
-static inline int cdiv_p(int a, int b) { return (a + b - 1) / b; }
-
-static int encode_pair(EncodeTiledFn encode, CUtensorMap* m, void* base, int rank, const cuuint64_t* dims,
-                       const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapL2promotion promo) {
-  cuuint32_t es[4] = {1, 1, 1, 1};
-  return (int)encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-}
 
 // Fills L for the CTA-pair kernel.  UG_EUNSUPPORTED when the layer is not one it takes (the caller falls back to
 // conv_multi_prepare): 3x3 pad 1, ReLU, <= 64 output channels in one 64-column n-tile, STORE (optionally with the fused
 // 2x2 pool), OUTC or GATE epilogue, weights resident at 36 KB per 64 input channels per CTA, an even number of SMs.
 int conv_pair_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return set_error(h, UG_ECUDA, "cuTensorMapEncodeTiled entry point unavailable");
+  if (!get_encode_fn()) return set_error(h, UG_ECUDA, "cuTensorMapEncodeTiled entry point unavailable");
   if (!(d->R == 3 && d->S == 3 && d->pad == 1 && d->up != 2) || d->act != UG_ACT_RELU || d->N > 64 || d->N % 8 ||
       !(d->mode == UG_EPI_STORE || d->mode == UG_EPI_OUTC || d->mode == UG_EPI_GATE) || d->stats_sum || d->out2 ||
       d->in_rstride || d->in_bstride || (h->num_sms & 1))
@@ -502,7 +399,7 @@ int conv_pair_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   if (gate && (!d->add || !d->gate || d->add_bstride <= 0 || d->add_cstride % 8 || (reinterpret_cast<uintptr_t>(d->add) & 15) ||
                d->pool_out))
     return set_error(h, UG_EUNSUPPORTED, "conv(pair): the GATE epilogue needs a per-image residual tensor (16-byte aligned rows)");
-  const int cin_pad = cdiv_p(d->Cin, 64) * 64;
+  const int cin_pad = ceil_div(d->Cin, 64) * 64;
   const int kchunks = cin_pad / 64;
   const long long ktot = 9LL * cin_pad;
   const int tma_store = d->mode != UG_EPI_OUTC;
@@ -512,7 +409,7 @@ int conv_pair_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   const long long fixed = 1024 + 3 * 64 * sizeof(float) + 64 * sizeof(float) + 8 * (2 * kPI * 3 + 1 + 2 * kPI * kPAcc + 4 * kPI) + 16;
   // shared-memory plan, first fit: two tile streams with two activation stages each; else ONE stream with up to three
   // stages (resident weights of 192 / 256 input channels).  GATE needs both staging buffers (residual one tile ahead).
-  const int TH = cdiv_p(d->H, cdiv_p(d->H, 16));
+  const int TH = ceil_div(d->H, ceil_div(d->H, 16));
   const int a_stage = ((kPPitch * (TH + 2) * 128 + 1023) / 1024) * 1024;
   static const int cand[6][3] = {{2, 2, 2}, {2, 2, 1}, {1, 3, 2}, {1, 3, 1}, {1, 2, 2}, {1, 2, 1}};   // streams, stages, staging buffers
   int streams = 0, sa = 0, obufs = 0;
@@ -535,8 +432,8 @@ int conv_pair_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   memset(&p, 0, sizeof(p));
   p.H = d->H; p.W = d->W; p.B = d->B;
   p.TW = 8; p.TH = TH; p.TN = 1;
-  p.tiles_x = cdiv_p(d->W, 8);
-  p.tiles_y = cdiv_p(d->H, TH);
+  p.tiles_x = ceil_div(d->W, 8);
+  p.tiles_y = ceil_div(d->H, TH);
   p.R = 3; p.S = 3; p.pad = 1;
   p.kchunks = kchunks; p.num_k = 9 * kchunks;
   p.N = d->N; p.BN = 64; p.stages = sa; p.tmem_cols = 512;
@@ -548,35 +445,40 @@ int conv_pair_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   p.add = d->add; p.add_bstride = d->add_bstride; p.add_cstride = d->add_cstride; p.gate = d->gate;
   p.m_tiles = p.tiles_x * p.tiles_y * d->B; p.n_tiles = 1; p.acc_stages = kPAcc;
   p.tma_store = tma_store; p.obufs = obufs; p.npad = 64; p.pool = pool;
-  L->variant = 6;
-  L->halo_TH = TH; L->halo_a_stage = a_stage; L->halo_sa = sa;
-  L->halo_copy = cdiv_p(p.m_tiles, 2 * streams);   // tile groups: streams x 2 CTAs
-  L->halo_mode = streams;
-  L->halo_rt = gate;
+  PairParams& hp = L->pp;
+  memset(&hp, 0, sizeof(hp));
+  hp.TH = TH; hp.a_stage_bytes = a_stage; hp.sa = sa;
+  hp.n_quads = ceil_div(p.m_tiles, 2 * streams);   // tile groups: streams x 2 CTAs
+  hp.streams = streams;
+  hp.d_tx = make_fastdiv(p.tiles_x);
+  hp.d_ty = make_fastdiv(p.tiles_y);
+  L->kernel = ConvKernel::Pair;
+  L->pair_fn = d->mode == UG_EPI_OUTC ? conv_pair_kernel<UG_EPI_OUTC, 0>
+               : gate                 ? conv_pair_kernel<UG_EPI_GATE, 1>
+                                      : conv_pair_kernel<UG_EPI_STORE, 0>;
+  L->block = kPThreads;
 
   {
     cuuint64_t dims[4] = {(cuuint64_t)d->Cin, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->B};
     cuuint64_t strides[3] = {(cuuint64_t)d->in_cstride * 2, (cuuint64_t)d->W * d->in_cstride * 2,
                              (cuuint64_t)d->H * d->W * d->in_cstride * 2};
     cuuint32_t box[4] = {64, (cuuint32_t)kPPitch, (cuuint32_t)(TH + 2), 1};
-    const int r = encode_pair(encode, &L->tmA, const_cast<void*>(d->in), 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+    const int r = encode_bf16_sw128(&L->tmA, d->in, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
     if (r) return set_error(h, UG_ECUDA, "conv(pair): activation tensor map encode failed (%d)", r);
   }
   {
     cuuint64_t dims[2] = {(cuuint64_t)ktot, (cuuint64_t)d->N};   // rows beyond N are zero-filled
     cuuint64_t strides[1] = {(cuuint64_t)ktot * 2};
     cuuint32_t box[2] = {64, 32};
-    const int r = encode_pair(encode, &L->tmB, const_cast<void*>(d->w), 2, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+    const int r = encode_bf16_sw128(&L->tmB, d->w, 2, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
     if (r) return set_error(h, UG_ECUDA, "conv(pair): weight tensor map encode failed (%d)", r);
   }
-  memset(L->tmQ, 0, sizeof(L->tmQ));
-  memset(&L->tmO, 0, sizeof(L->tmO));
-  memset(&L->tmR, 0, sizeof(L->tmR));
+  memset(&L->pmaps, 0, sizeof(L->pmaps));
   if (gate) {  // load map of the residual tensor, same box as the output store
     cuuint64_t dims[4] = {(cuuint64_t)d->N, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->B};
     cuuint64_t strides[3] = {(cuuint64_t)d->add_cstride * 2, (cuuint64_t)d->W * d->add_cstride * 2, (cuuint64_t)d->add_bstride * 2};
     cuuint32_t box[4] = {64, 8, (cuuint32_t)TH, 1};
-    const int r = encode_pair(encode, &L->tmR, const_cast<void*>(d->add), 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+    const int r = encode_bf16_sw128(&L->pmaps.resid, d->add, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
     if (r) return set_error(h, UG_ECUDA, "conv(pair): residual tensor map encode failed (%d)", r);
   }
   if (tma_store) {
@@ -584,7 +486,7 @@ int conv_pair_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
     cuuint64_t dims[4] = {(cuuint64_t)d->N, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->B};
     cuuint64_t strides[3] = {(cuuint64_t)d->out_cstride * 2, (cuuint64_t)d->W * d->out_cstride * 2,
                              (cuuint64_t)d->H * d->W * d->out_cstride * 2};
-    const int r = encode_pair(encode, &L->tmO, d->out, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+    const int r = encode_bf16_sw128(&L->pmaps.out, d->out, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
     if (r) return set_error(h, UG_ECUDA, "conv(pair): output tensor map encode failed (%d)", r);
     if (pool) {
       const long long pcs = d->pool_cstride;
@@ -592,12 +494,11 @@ int conv_pair_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
       cuuint64_t pstrides[3] = {(cuuint64_t)(pcs * 2), (cuuint64_t)((d->W / 2) * pcs * 2),
                                 (cuuint64_t)((long long)(d->H / 2) * (d->W / 2) * pcs * 2)};
       cuuint32_t pbox[4] = {64, 4, (cuuint32_t)(TH / 2), 1};
-      const int rp = encode_pair(encode, &L->tmQ[0], d->pool_out, 4, pdims, pstrides, pbox, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+      const int rp = encode_bf16_sw128(&L->pmaps.pool, d->pool_out, 4, pdims, pstrides, pbox, CU_TENSOR_MAP_L2_PROMOTION_NONE);
       if (rp) return set_error(h, UG_ECUDA, "conv(pair): pooled output tensor map encode failed (%d)", rp);
     }
   }
-  const int quads = L->halo_copy;
-  const int pairs = std::min(quads, h->num_sms / 2);
+  const int pairs = std::min(hp.n_quads, h->num_sms / 2);
   L->grid = dim3((unsigned)(2 * pairs), 1, 1);
   L->smem = (size_t)smem;
   return UG_OK;
@@ -608,17 +509,9 @@ int max_cluster_pairs(ug_engine* h) {
   int pairs = h->num_sms / 2;
   cudaError_t e = cudaFuncSetAttribute((const void*)conv_pair_kernel<UG_EPI_STORE, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(2 * (h->num_sms / 2)));
-    cfg.blockDim = dim3(kPThreads);
-    cfg.dynamicSmemBytes = 200 * 1024;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
+    cudaLaunchAttribute at[2];
+    cudaLaunchConfig_t cfg = pair_config(at, 2 * (h->num_sms / 2), kPThreads, 200 * 1024, 0);
+    cfg.numAttrs = 1;   // (the cluster shape only)
     int n = 0;
     e = cudaOccupancyMaxActiveClusters(&n, (const void*)conv_pair_kernel<UG_EPI_STORE, 0>, &cfg);
     if (e == cudaSuccess && n > 0) pairs = std::min(pairs, n);
@@ -631,42 +524,13 @@ int max_cluster_pairs(ug_engine* h) {
 
 int conv_pair_launch(ug_engine* h, const ConvLaunch* L, cudaStream_t s) {
   if (!h->attr_pair) {
-    cudaError_t e = cudaFuncSetAttribute((const void*)conv_pair_kernel<UG_EPI_STORE, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute((const void*)conv_pair_kernel<UG_EPI_OUTC, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute((const void*)conv_pair_kernel<UG_EPI_GATE, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(conv_pair_kernel)");
+    for (PairKernelFn fn : {conv_pair_kernel<UG_EPI_STORE, 0>, conv_pair_kernel<UG_EPI_OUTC, 0>, conv_pair_kernel<UG_EPI_GATE, 1>}) {
+      const cudaError_t e = cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+      if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(conv_pair_kernel)");
+    }
     h->attr_pair = true;
   }
-  PairParams hp;
-  memset(&hp, 0, sizeof(hp));
-  hp.TH = L->halo_TH; hp.a_stage_bytes = L->halo_a_stage; hp.sa = L->halo_sa; hp.n_quads = L->halo_copy;
-  hp.streams = L->halo_mode;
-  hp.d_tx = make_pairdiv(L->p.tiles_x);
-  hp.d_ty = make_pairdiv(L->p.tiles_y);
-  PairMaps maps;
-  maps.out = L->tmO;
-  maps.pool = L->tmQ[0];
-  maps.resid = L->tmR;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(std::min(L->grid.x, 2u * (unsigned)max_cluster_pairs(h)));   // persistent loops: any even grid works
-  cfg.blockDim = dim3(kPThreads);
-  cfg.dynamicSmemBytes = L->smem;
-  cfg.stream = s;
-  cudaLaunchAttribute at[2];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = h->pdl ? 2 : 1;
-  cudaError_t e;
-  if (L->p.mode == UG_EPI_OUTC) e = cudaLaunchKernelEx(&cfg, conv_pair_kernel<UG_EPI_OUTC, 0>, L->tmA, L->tmB, maps, L->p, hp);
-  else if (L->p.mode == UG_EPI_GATE) e = cudaLaunchKernelEx(&cfg, conv_pair_kernel<UG_EPI_GATE, 1>, L->tmA, L->tmB, maps, L->p, hp);
-  else e = cudaLaunchKernelEx(&cfg, conv_pair_kernel<UG_EPI_STORE, 0>, L->tmA, L->tmB, maps, L->p, hp);
+  const cudaError_t e = launch_pairs(h, L->pair_fn, L->grid.x, L->block, L->smem, s, L->tmA, L->tmB, L->pmaps, L->p, L->pp);
   h->launches++;
   return check_cuda(h, e != cudaSuccess ? e : cudaGetLastError(), "conv_pair_kernel launch");
 }

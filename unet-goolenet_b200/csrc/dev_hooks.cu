@@ -14,7 +14,7 @@ int ug_conv_profile(ug_handle h, const ug_conv_desc* d, void* stream, double* ou
   ConvLaunch L;
   int rc = conv_prepare(h, d, &L);
   if (rc != UG_OK) return rc;
-  if (L.variant != 0) return set_error(h, UG_EINVAL, "conv_profile: persistent variant only");
+  if (L.kernel != ConvKernel::Persistent) return set_error(h, UG_EINVAL, "conv_profile: persistent variant only");
   const int ctas = (int)L.grid.x;
   long long* dev = nullptr;
   rc = check_cuda(h, cudaMalloc(&dev, sizeof(long long) * 8 * ctas), "cudaMalloc(prof)");
@@ -44,7 +44,8 @@ int ug_conv_profile16(ug_handle h, const ug_conv_desc* d, void* stream, double* 
   ConvLaunch L;
   int rc = conv_prepare(h, d, &L);
   if (rc != UG_OK) return rc;
-  if (L.variant != 5) return set_error(h, UG_EINVAL, "conv_profile16: multi-issuer variant only");
+  if (L.kernel != ConvKernel::Multi && L.kernel != ConvKernel::MultiPair)
+    return set_error(h, UG_EINVAL, "conv_profile16: multi-issuer variant only");
   const int ctas = (int)L.grid.x;
   long long* dev = nullptr;
   rc = check_cuda(h, cudaMalloc(&dev, sizeof(long long) * 16 * ctas), "cudaMalloc(prof)");
@@ -62,7 +63,7 @@ int ug_conv_profile16(ug_handle h, const ug_conv_desc* d, void* stream, double* 
     double a = 0;
     for (int c = 0; c < ctas; ++c) a += (double)host[c * 16 + j];
     // (CTA pairs: only the leader CTAs have issuers, slots 4-11)
-    out16[j] = a / ((L.halo_pair && j >= 4 && j < 12) ? ctas / 2 : ctas);
+    out16[j] = a / ((L.kernel == ConvKernel::MultiPair && j >= 4 && j < 12) ? ctas / 2 : ctas);
   }
   return UG_OK;
 }

@@ -4,7 +4,6 @@
 #include <cstring>
 #include <new>
 #include "engine.h"
-#include <cstdlib>
 
 namespace ug {
 
@@ -81,7 +80,6 @@ int ug_create(int device, ug_handle* out) {
   if (!h) return UG_ENOMEM;
   h->device = device;
   h->num_sms = prop.multiProcessorCount;
-  if (const char* e = getenv("UG_PDL")) h->pdl = atoi(e) != 0;
   *out = h;
   return UG_OK;
 }
@@ -209,57 +207,6 @@ int ug_program_run_timed(ug_handle h, ug_program p, void* stream, float* ms_per_
   if (rc == UG_OK)
     for (size_t i = 0; i < n; ++i) cudaEventElapsedTime(&ms_per_op[i], ev[i], ev[i + 1]);
   for (auto& e : ev) cudaEventDestroy(e);
-  return rc;
-}
-
-// Measured kernel-variant choice: every conv op of the program is timed on its own buffers with each kernel
-// structure that accepts it (one tile per CTA, persistent, multi-issuer, the two CTA-pair forms) and keeps the fastest.  All conv ops are
-// pure functions of their inputs, so re-running them before the first real run is harmless.
-int ug_program_autotune(ug_handle h, ug_program p, void* stream, int* n_changed) {
-  if (!h || !p) return UG_EINVAL;
-  DeviceGuard guard(h);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  cudaEvent_t e0, e1;
-  if (cudaEventCreate(&e0) != cudaSuccess || cudaEventCreate(&e1) != cudaSuccess)
-    return set_error(h, UG_ECUDA, "cudaEventCreate failed");
-  auto time_launch = [&](const ConvLaunch& L, float* ms) -> int {
-    int rc = UG_OK;
-    for (int i = 0; i < 2 && rc == UG_OK; ++i) rc = conv_launch(h, &L, s);
-    cudaEventRecord(e0, s);
-    for (int i = 0; i < 4 && rc == UG_OK; ++i) rc = conv_launch(h, &L, s);
-    cudaEventRecord(e1, s);
-    if (rc == UG_OK) rc = check_cuda(h, cudaStreamSynchronize(s), "autotune sync");
-    if (rc == UG_OK) cudaEventElapsedTime(ms, e0, e1);
-    return rc;
-  };
-  int changed = 0, rc = UG_OK;
-  const long long launches_before = h->launches;
-  for (size_t i = 0; i < p->ops.size() && rc == UG_OK; ++i) {
-    PreparedOp& po = p->ops[i];
-    if (po.kind != UG_OP_CONV || po.op.u.conv.variant != 0) continue;  // explicit variants are left alone
-    float best = 0.f;
-    rc = time_launch(po.conv, &best);
-    if (rc != UG_OK) break;
-    const int variants[5] = {1, 2, 5, 6, 7};
-    for (int v : variants) {
-      ug_conv_desc d = po.op.u.conv;
-      d.variant = v;
-      ConvLaunch L;
-      if (conv_prepare(h, &d, &L) != UG_OK) continue;  // this structure does not take the shape
-      float ms = 0.f;
-      rc = time_launch(L, &ms);
-      if (rc != UG_OK) break;
-      if (ms < 0.97f * best) {  // switch only for a clear win (timing noise)
-        best = ms;
-        po.conv = L;
-        ++changed;
-      }
-    }
-  }
-  h->launches = launches_before;  // tuning launches are not part of any step
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  if (n_changed) *n_changed = changed;
   return rc;
 }
 

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <string>
 #include <vector>
 #include "../../include/ugnet.h"
@@ -16,7 +17,6 @@ struct ug_engine {
   cudaEvent_t ev_h2d[2] = {nullptr, nullptr};   // staging slot filled (recorded on the copy stream)
   cudaEvent_t ev_free[2] = {nullptr, nullptr};  // staging slot consumed (recorded on the compute stream)
   long long pipelined_steps = 0;
-  int pdl = 1;  // launch kernels with programmatic stream serialization (UG_PDL=0 turns it off)
   // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) applies to the device that is current at the call, so the
   // "already raised" flags are per handle (= per device), not process-wide
   bool attr_gemm = false, attr_multi = false, attr_pair = false, attr_stem = false, attr_attn = false;
@@ -75,30 +75,100 @@ struct ConvKParams {
   long long* prof;  // optional per-CTA cycle counters [grid][8] (debug / profiling builds of the plan)
 };
 
-// A fully prepared launch of the implicit-GEMM kernel.
+// Division by a launch-time constant as multiply + shift (exact for n < 2^24): the role loops decode a tile index
+// into (image, tile row, tile column) once per tile, and on the short K=64 / N=64 tiles that decode (four integer
+// divisions, ~25 instructions each) was a third of the epilogue time.
+struct FastDiv {
+  unsigned mul, shift;
+  __device__ __forceinline__ int div(int n) const {
+    return (int)(((unsigned long long)(unsigned)n * mul) >> shift);
+  }
+};
+inline FastDiv make_fastdiv(int d) {
+  FastDiv f;
+  int s = 0;
+  while ((1 << s) < d) ++s;
+  f.shift = 24 + s;
+  f.mul = (unsigned)(((1ULL << f.shift) + d - 1) / d);
+  return f;
+}
+
+// Parameter block of the multi-issuer kernel (csrc/conv_multi.cu).
+struct MultiParams {
+  int TH;             // output rows per tile (tile = 8 x TH pixels)
+  int a_stage_bytes;  // bytes of one activation stage
+  int sa, sb;         // activation stages per issuer / shared weight stages
+  int b_resident;     // whole weight matrix kept in smem (requires n_tiles == 1)
+  int m_super;        // ceil(m_tiles / kMI): pixel tiles are handed out in groups of kMI
+  FastDiv d_msuper, d_tx, d_ty;   // dividers by m_super, tiles_x, tiles_y
+  int m_major;        // work item s -> (pixel-tile group s / n_tiles, n-tile s % n_tiles): the n-tiles of one pixel-tile group
+                      // run on neighbouring CTAs at the same time, so the activation tile comes from HBM once and from L2
+                      // for the other n-tiles (n-major order re-read the whole input from HBM once per n-tile)
+  FastDiv d_nt;       // divider by n_tiles
+  int pitch;          // halo pixels per stage row: kMPitch (8-pixel-wide tiles) or W + 2 (row-strip tiles)
+  int sbo;            // byte distance of consecutive 8-row groups of the A operand: pitch * 128 (tiles) or 1024 (strips)
+  int strip;          // row-strip tiles (see the header comment); TH is then the number of image rows per tile
+  FastDiv d_pitch;    // divider by pitch (strip mode: MMA row -> (image row, x))
+  int rowtaps;        // 1x1 tiles: k-chunk kc is ROW TAP kc of an overlapping-window input.  1: one A box per tap (at row
+                      // y0 + kc); 2: ONE box of TH + R - 1 rows per tile, tap kc reads it TW * 128 * kc bytes further in
+                      // (a "row halo": the window rows of neighbouring taps are the same bytes)
+  int resid_tma;      // kRT kernels: residual tiles arrive by TMA in the staging buffers (see the header comment)
+  int debug;          // ablation switches for profiling (results are wrong when set): 1 = no TMEM loads,
+                      // 2 = no staging stores / TMA store, 4 = activation TMA loads only for the first stages,
+                      // 16 = no residual loads (ADD / GATE epilogues)
+};
+
+struct StoreMaps {  // output maps: [0] for plain stores, [q] = quadrant (dy,dx) of a ConvTranspose 2x2 s2 scatter;
+  CUtensorMap m[5];  // [1] = pooled output (fused max-pool); [4] = load map of the residual tensor (kRT)
+};
+
+// Parameter block of the CTA-pair kernel (csrc/conv_pair.cu).
+struct PairParams {
+  int TH, a_stage_bytes, sa, n_quads;   // rows per tile, bytes of one activation stage, stages per stream, tile groups
+  int streams;                          // tile streams per CTA: 2, or 1 when the resident weights leave room for one
+  FastDiv d_tx, d_ty;
+};
+
+struct PairMaps {
+  CUtensorMap out, pool, resid;
+};
+
+// Which kernel a prepared conv launches.
+enum class ConvKernel {
+  OneTile,     // conv_gemm_kernel: one output tile per CTA
+  Persistent,  // conv_gemm_persistent_kernel
+  Multi,       // conv_multi_kernel: two MMA issuers per CTA
+  MultiPair,   // conv_multi_kernel on clusters of two CTAs (128-column n-tiles)
+  Pair,        // conv_pair_kernel: clusters of two CTAs, <= 64 output channels
+};
+
+typedef void (*MultiKernelFn)(CUtensorMap, CUtensorMap, StoreMaps, ConvKParams, MultiParams);
+typedef void (*PairKernelFn)(CUtensorMap, CUtensorMap, PairMaps, ConvKParams, PairParams);
+
+// A fully prepared launch of one of the conv kernels: the prepare functions fill the kernel's parameter blocks and
+// tensor maps, the launch functions only launch.
 struct ConvLaunch {
   alignas(64) CUtensorMap tmA;
   alignas(64) CUtensorMap tmB;
-  alignas(64) CUtensorMap tmO;  // output map for the TMA-store epilogues
-  alignas(64) CUtensorMap tmO2;    // persistent GEMM kernel: TMA-store map of the second destination (split 1x1 GEMM)
-  alignas(64) CUtensorMap tmR;     // multi-issuer kernel: TMA load map of the residual tensor (kRT kernels)
-  alignas(64) CUtensorMap tmQ[3];  // multi-issuer kernel, ConvTranspose: output views of quadrants 1..3 (tmO = quadrant 0)
+  alignas(64) CUtensorMap tmO;   // persistent GEMM kernel: output map (TMA-store epilogue)
+  alignas(64) CUtensorMap tmO2;  // persistent GEMM kernel: second destination of a split 1x1 GEMM
+  StoreMaps maps;                // multi-issuer kernel
+  PairMaps pmaps;                // CTA-pair kernel
   ConvKParams p;
+  MultiParams mp;                // multi-issuer kernel
+  PairParams pp;                 // CTA-pair kernel
+  ConvKernel kernel;
+  MultiKernelFn multi_fn;        // the conv_multi_kernel instantiation (activation, taps, epilogue, K-split, ...)
+  PairKernelFn pair_fn;          // the conv_pair_kernel instantiation (epilogue)
   dim3 grid;
+  unsigned block;
   size_t smem;
-  int variant;  // 0 = persistent, 1 = one tile per CTA, 5 = multi-issuer kernel (halo_mode = taps: 9 or 1), 6 = CTA-pair kernel
-  int halo_mode, halo_TH, halo_a_stage, halo_copy, halo_sa, halo_sb, halo_bres, halo_debug;
-  int halo_strip, halo_pitch;  // multi-issuer kernel: row-strip tiles (full image rows per tile) and their halo pitch
-  int halo_rt;  // multi-issuer kernel: residual tiles by TMA into the staging buffers (CoordAtt3 combine, 64 channels)
-  int halo_rowtaps;  // multi-issuer kernel, 1x1 tiles: the k-chunks are R row taps of an overlapping-window input
-  int halo_ks;  // multi-issuer kernel: issuing warps per tile stream (K-split), 1 or 2
-  int halo_pair;  // multi-issuer kernel: clusters of two CTAs issuing tcgen05.mma.cta_group::2 (128-column n-tiles)
 };
 
 // Stem convolution (csrc/stem_conv.cu): kernel parameters and a prepared launch.
 struct StemParams {
   const float* in_f32;
-  const unsigned char* in_u8;
+  const unsigned char* in_u8;   // (not read by the inc kernel)
   const float* scale;
   const float* bias;
   int B, H, W;  // source image
@@ -109,10 +179,8 @@ struct StemParams {
 struct StemLaunch {
   alignas(64) CUtensorMap tmB;
   alignas(64) CUtensorMap tmO;
-  alignas(64) CUtensorMap tmP;  // pooled output (kind 0 with pool_out)
+  alignas(64) CUtensorMap tmP;  // pooled output (pool_out)
   StemParams p;
-  int kind;
-  int groups;   // warpgroups (independent tile pipelines) per CTA
   unsigned grid;
   size_t smem;
 };
@@ -120,12 +188,23 @@ struct StemLaunch {
 int set_error(ug_engine* h, int code, const char* fmt, ...);
 int check_cuda(ug_engine* h, cudaError_t e, const char* what);
 
-// Launch `kernel` on `s`; with h->pdl the launch carries the programmatic-stream-serialization attribute, so the kernel
-// may start its prologue while the previous kernel of the stream drains.  ONLY for kernels that execute pdl_wait()
-// (common.cuh) before their first access to memory written by earlier kernels.
+inline int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
+
+// Driver entry point cuTensorMapEncodeTiled (nullptr when unavailable) and the one map format the kernels use: bf16
+// elements, 128-byte swizzle (boxes with an inner extent of 64 elements), no interleave, zero fill.  Returns the CUresult.
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn get_encode_fn();
+int encode_bf16_sw128(CUtensorMap* m, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                      const cuuint32_t* box, CUtensorMapL2promotion promo);
+
+// Launch `kernel` on `s` with the programmatic-stream-serialization attribute, so the kernel may start its prologue
+// while the previous kernel of the stream drains.  ONLY for kernels that execute pdl_wait() (common.cuh) before their
+// first access to memory written by earlier kernels.
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(const ug_engine* h, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
-                              cudaStream_t s, Args&&... args) {
+inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s,
+                              Args&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
@@ -135,8 +214,28 @@ inline cudaError_t launch_pdl(const ug_engine* h, void (*kernel)(KArgs...), dim3
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = (h && h->pdl) ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+
+// Launch configuration of a grid of CTA pairs (clusters of two CTAs along x), attribute 0 = the cluster shape,
+// attribute 1 = programmatic stream serialization (as in launch_pdl); `at` holds the attributes.
+inline cudaLaunchConfig_t pair_config(cudaLaunchAttribute (&at)[2], unsigned grid_x, unsigned block, size_t smem,
+                                      cudaStream_t s) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid_x);
+  cfg.blockDim = dim3(block);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = s;
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = 2;
+  at[0].val.clusterDim.y = 1;
+  at[0].val.clusterDim.z = 1;
+  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[1].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 2;
+  return cfg;
 }
 
 int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* out);
@@ -150,6 +249,15 @@ int conv_pair_launch(ug_engine* h, const ConvLaunch* l, cudaStream_t s);
 // the persistent pair kernels must not launch more, or the surplus clusters would run as a second wave.  Usually
 // num_sms / 2; fewer when a GPC has an odd number of usable SMs.
 int max_cluster_pairs(ug_engine* h);
+
+// Launch a persistent CTA-pair kernel (pair_config) on at most max_cluster_pairs(h) pairs: its loops take any even grid.
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_pairs(ug_engine* h, void (*kernel)(KArgs...), unsigned grid_x, unsigned block, size_t smem,
+                                cudaStream_t s, Args&&... args) {
+  cudaLaunchAttribute at[2];
+  const cudaLaunchConfig_t cfg = pair_config(at, std::min(grid_x, 2u * (unsigned)max_cluster_pairs(h)), block, smem, s);
+  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
 
 int stem_prepare(ug_engine* h, const ug_stem_desc* d, StemLaunch* out);
 int stem_launch(ug_engine* h, const StemLaunch* l, cudaStream_t s);

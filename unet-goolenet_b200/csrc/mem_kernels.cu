@@ -9,15 +9,8 @@
 
 namespace ug {
 
-static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
-
 // ------------------------------------------------------------------------------------------------
 // max pooling: one thread per (output pixel, 8-channel group); channel groups vary fastest.
-__device__ __forceinline__ uint32_t bf16x2_max(uint32_t a, uint32_t b) {
-  __nv_bfloat162 r = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a), *reinterpret_cast<__nv_bfloat162*>(&b));
-  return *reinterpret_cast<uint32_t*>(&r);
-}
-
 __global__ void __launch_bounds__(256) pool_kernel(const __nv_bfloat16* __restrict__ in, __nv_bfloat16* __restrict__ out,
                                                    ug_pool_desc d) {
   pdl_wait();  // programmatic dependent launch: see common.cuh
@@ -213,35 +206,34 @@ int launch_pool(ug_engine* h, const ug_pool_desc* d, cudaStream_t s) {
     return set_error(h, UG_EINVAL, "pool: bad args (C and strides must be multiples of 8)");
   if ((d->OH - 1) * d->stride - d->pad >= d->H || (d->OW - 1) * d->stride - d->pad >= d->W)
     return set_error(h, UG_EINVAL, "pool: last window starts outside the input");
-  // UG_POOL_BLOCK=0: the previous kernels (generic for stride 2, sliding rows for stride 1) for A/B runs.  Block forms
-  // (profiles/r02_pool_s2.txt): maxpool1 0.1505 -> 0.107 ms per 256 images (4.8 TB/s of DRAM traffic), maxpool2 0.118 ->
+  // Block forms for 3x3 windows (profiles/r02_pool_s2.txt, against the generic kernel for stride 2 and sliding rows for
+  // stride 1): maxpool1 0.1505 -> 0.107 ms per 256 images (4.8 TB/s of DRAM traffic), maxpool2 0.118 ->
   // 0.086, the branch-4 pools on 28x28 / 14x14 maps 0.074 / 0.042 -> 0.058 / 0.033; the 7x7 maps stay on sliding rows
   // (0.015 against 0.0195 ms).
-  static const int pool_block = [] { const char* e = getenv("UG_POOL_BLOCK"); return e ? atoi(e) : 1; }();
-  if (pool_block && d->k == 3 && d->stride == 1 && d->pad == 1 && d->OH == d->H && d->OW == d->W && d->H * d->W >= 196) {
+  if (d->k == 3 && d->stride == 1 && d->pad == 1 && d->OH == d->H && d->OW == d->W && d->H * d->W >= 196) {
     const long long total = (long long)d->B * ((d->H + 1) / 2) * ((d->W + 1) / 2) * (d->C / 8);
-    launch_pdl(h, pool3x3s1_block_kernel, cdiv(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
-                                                            reinterpret_cast<__nv_bfloat16*>(d->out), *d);
+    launch_pdl(pool3x3s1_block_kernel, ceil_div(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
+                                                         reinterpret_cast<__nv_bfloat16*>(d->out), *d);
     h->launches++;
     return check_cuda(h, cudaGetLastError(), "pool3x3s1 launch");
   }
   if (d->k == 3 && d->stride == 1 && d->pad == 1 && d->OH == d->H && d->OW == d->W) {
     const long long total = (long long)d->B * d->H * (d->C / 8);
-    launch_pdl(h, pool3x3s1_kernel, cdiv(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
-                                                      reinterpret_cast<__nv_bfloat16*>(d->out), *d);
+    launch_pdl(pool3x3s1_kernel, ceil_div(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
+                                                   reinterpret_cast<__nv_bfloat16*>(d->out), *d);
     h->launches++;
     return check_cuda(h, cudaGetLastError(), "pool3x3s1 launch");
   }
-  if (pool_block && d->k == 3 && d->stride == 2 && d->pad == 0 && 2 * (d->OH - 1) < d->H && 2 * (d->OW - 1) < d->W) {
+  if (d->k == 3 && d->stride == 2 && d->pad == 0 && 2 * (d->OH - 1) < d->H && 2 * (d->OW - 1) < d->W) {
     const long long total = (long long)d->B * ((d->OH + 1) / 2) * ((d->OW + 1) / 2) * (d->C / 8);
-    launch_pdl(h, pool3x3s2_kernel, cdiv(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
-                                                      reinterpret_cast<__nv_bfloat16*>(d->out), *d);
+    launch_pdl(pool3x3s2_kernel, ceil_div(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
+                                                   reinterpret_cast<__nv_bfloat16*>(d->out), *d);
     h->launches++;
     return check_cuda(h, cudaGetLastError(), "pool3x3s2 launch");
   }
   const long long total = (long long)d->B * d->OH * d->OW * (d->C / 8);
-  launch_pdl(h, pool_kernel, cdiv(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
-                                               reinterpret_cast<__nv_bfloat16*>(d->out), *d);
+  launch_pdl(pool_kernel, ceil_div(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
+                                            reinterpret_cast<__nv_bfloat16*>(d->out), *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "pool launch");
 }
@@ -333,14 +325,14 @@ int launch_layernorm(ug_engine* h, const ug_layernorm_desc* d, cudaStream_t s) {
       (reinterpret_cast<uintptr_t>(d->in) & 15) || (reinterpret_cast<uintptr_t>(d->out) & 15))
     return set_error(h, UG_EINVAL, "layernorm: in / out / gamma / beta must be 16-byte aligned");
   const long long warps = ((long long)d->M + kLnTok - 1) / kLnTok;
-  const dim3 grid(cdiv(warps * 32, 256));
+  const dim3 grid(ceil_div(warps * 32, 256));
   const __nv_bfloat16* in = reinterpret_cast<const __nv_bfloat16*>(d->in);
   __nv_bfloat16* out = reinterpret_cast<__nv_bfloat16*>(d->out);
   switch (d->C / 256) {
-    case 1: launch_pdl(h, layernorm_kernel<1>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
-    case 2: launch_pdl(h, layernorm_kernel<2>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
-    case 3: launch_pdl(h, layernorm_kernel<3>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
-    default: launch_pdl(h, layernorm_kernel<4>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
+    case 1: launch_pdl(layernorm_kernel<1>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
+    case 2: launch_pdl(layernorm_kernel<2>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
+    case 3: launch_pdl(layernorm_kernel<3>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
+    default: launch_pdl(layernorm_kernel<4>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
   }
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "layernorm launch");
@@ -495,7 +487,7 @@ int launch_attention(ug_engine* h, const ug_attn_desc* d, cudaStream_t s) {
     h->attr_attn = true;
   }
   const size_t smem = (size_t)(kAttnSP * kAttnKPitch + kAttnSP * kAttnVPitch) * sizeof(__nv_bfloat16);
-  launch_pdl(h, attention_mma_kernel, d->B * d->heads, 128, smem, s, *d);
+  launch_pdl(attention_mma_kernel, d->B * d->heads, 128, smem, s, *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "attention launch");
 }
@@ -559,7 +551,7 @@ int launch_chanstats(ug_engine* h, const ug_chanstats_desc* d, cudaStream_t s) {
   if (!d->in || !d->psum || !d->pmax || d->C % 8 || d->C > 512 || d->C < 8 || (256 % (d->C / 8)) || d->splits <= 0 ||
       d->in_cstride % 8)
     return set_error(h, UG_EINVAL, "chanstats: C must be 8*2^k <= 512");
-  launch_pdl(h, chanstats_kernel, dim3(d->splits, d->B), 256, 0, s, *d);
+  launch_pdl(chanstats_kernel, dim3(d->splits, d->B), 256, 0, s, *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "chanstats launch");
 }
@@ -628,8 +620,8 @@ int launch_gate(ug_engine* h, const ug_gate_desc* d, cudaStream_t s) {
   if (!d->psum || !d->pmax || !d->w1 || !d->w2 || !d->w3 || !d->b1 || !d->b2 || !d->b3 || !d->g || !d->hid ||
       d->C > 512 || d->C % 2 || d->HW <= 0 || d->splits <= 0)
     return set_error(h, UG_EINVAL, "gate: bad args (C <= 512, hid scratch required)");
-  launch_pdl(h, gate_hidden_kernel, dim3(kGateSplit, d->B), 256, 0, s, *d, d->hid);
-  launch_pdl(h, gate_out_kernel, dim3(kGateSplit, d->B), 256, 0, s, *d, d->hid);
+  launch_pdl(gate_hidden_kernel, dim3(kGateSplit, d->B), 256, 0, s, *d, d->hid);
+  launch_pdl(gate_out_kernel, dim3(kGateSplit, d->B), 256, 0, s, *d, d->hid);
   h->launches += 2;
   return check_cuda(h, cudaGetLastError(), "gate launch");
 }
@@ -706,7 +698,7 @@ __global__ void __launch_bounds__(1024) bbox_kernel(const unsigned char* __restr
 
 int launch_bbox(ug_engine* h, const ug_bbox_desc* d, cudaStream_t s) {
   if (!d->mask || !d->boxes || d->B <= 0 || d->H <= 0 || d->W <= 0) return set_error(h, UG_EINVAL, "bbox: bad args");
-  launch_pdl(h, bbox_kernel, d->B, 1024, 0, s, d->mask, d->boxes, d->H, d->W, d->padding);
+  launch_pdl(bbox_kernel, d->B, 1024, 0, s, d->mask, d->boxes, d->H, d->W, d->padding);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "bbox launch");
 }
@@ -902,7 +894,7 @@ int launch_resize_u8(ug_engine* h, const ug_resize_desc* d, cudaStream_t s) {
     if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(resize_u8_kernel)");
     h->attr_resize = smem;
   }
-  launch_pdl(h, resize_u8_kernel<kUniform>, dim3(cdiv(d->S, kRsRows), d->B), 256, smem, s, *d, max_rows, nullptr, nullptr,
+  launch_pdl(resize_u8_kernel<kUniform>, dim3(ceil_div(d->S, kRsRows), d->B), 256, smem, s, *d, max_rows, nullptr, nullptr,
              0, 0, RaggedSrc{});
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "resize_u8 launch");
@@ -924,7 +916,7 @@ int launch_resize_ragged(ug_engine* h, const ug_resize_ragged_desc* d, cudaStrea
   }
   ug_resize_desc r;
   r.src = d->src; r.out_f32 = d->out_f32; r.out_u8 = d->out_u8; r.B = d->B; r.Hs = 0; r.Ws = 0; r.S = d->S;
-  launch_pdl(h, resize_u8_kernel<kRagged>, dim3(cdiv(d->S, kRsRows), d->B), 256, smem, s, r, max_rows, nullptr, nullptr,
+  launch_pdl(resize_u8_kernel<kRagged>, dim3(ceil_div(d->S, kRsRows), d->B), 256, smem, s, r, max_rows, nullptr, nullptr,
              0, 0, RaggedSrc{d->index, d->status, d->src_bytes});
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "resize_ragged launch");
@@ -948,7 +940,7 @@ int launch_cropresize(ug_engine* h, const ug_cropresize_desc* d, cudaStream_t s)
   }
   ug_resize_desc r;
   r.src = nullptr; r.out_f32 = nullptr; r.out_u8 = d->out_u8; r.B = d->B; r.Hs = d->H; r.Ws = d->W; r.S = d->S;
-  launch_pdl(h, resize_u8_kernel<kCrop>, dim3(cdiv(d->S, kRsRows), d->B), 256, smem, s, r, max_rows, d->img, d->boxes,
+  launch_pdl(resize_u8_kernel<kCrop>, dim3(ceil_div(d->S, kRsRows), d->B), 256, smem, s, r, max_rows, d->img, d->boxes,
              d->H, d->W, RaggedSrc{});
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "cropresize launch");
@@ -1008,7 +1000,7 @@ int launch_s2d_pack(ug_engine* h, const ug_s2d_desc* d, cudaStream_t s) {
     return set_error(h, UG_EINVAL, "s2d_pack: bad args (even image side, 16-byte aligned output)");
   const int Q = d->S / 2 + 3;
   const long long total = (long long)d->B * Q * Q;
-  launch_pdl(h, s2d_pack_kernel, cdiv(total, 256), 256, 0, s, *d);
+  launch_pdl(s2d_pack_kernel, ceil_div(total, 256), 256, 0, s, *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "s2d_pack launch");
 }
@@ -1045,7 +1037,7 @@ __global__ void __launch_bounds__(256) head_kernel(ug_head_desc d) {
 int launch_head(ug_engine* h, const ug_head_desc* d, cudaStream_t s) {
   if (!d->in || !d->w || !d->b || !d->logits || d->C > 1024 || d->C % 2 || d->HW <= 0 || d->ncls <= 0)
     return set_error(h, UG_EINVAL, "head: bad args (C <= 1024)");
-  launch_pdl(h, head_kernel, d->B, 256, 0, s, *d);
+  launch_pdl(head_kernel, d->B, 256, 0, s, *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "head launch");
 }

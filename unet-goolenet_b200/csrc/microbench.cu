@@ -110,15 +110,6 @@ __global__ void __launch_bounds__(128) mma_bench2_kernel(int N, int n_acc, int i
 // Third form: a CTA PAIR (cluster of 2) issuing tcgen05.mma.cta_group::2 (M = 256 across the two SMs, each CTA supplies
 // its own 128 A rows and N/2 of the B rows).  `issuers` warps of the LEADER CTA each run their own chain into their own
 // accumulator.  Answers what MMA rate a 2-CTA conv kernel could reach for N = 64 / 128 tiles.
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 __global__ void __launch_bounds__(128) mma_bench_pair_kernel(int N, int issuers, int iters, long long* out) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -135,13 +126,12 @@ __global__ void __launch_bounds__(128) mma_bench_pair_kernel(int N, int issuers,
   int cols = 32;
   while (cols < issuers * N) cols <<= 1;
   if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_ptr)), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tmem_alloc_pair(&tmem_ptr, cols);
   }
   fence_proxy_async_smem();
   tc_fence_before();
   __syncthreads();
-  cluster_sync_all();
+  cluster_sync();
   tc_fence_after();
   const uint32_t tmem_base = tmem_ptr;
   if (rank == 0 && warp < issuers && lane == 0) {
@@ -152,13 +142,7 @@ __global__ void __launch_bounds__(128) mma_bench_pair_kernel(int N, int issuers,
     const long long t0 = clock64();
     for (int it = 0; it < iters; ++it) {
 #pragma unroll
-      for (int k = 0; k < 4; ++k)
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "setp.ne.b32 p, %4, 0;\n\t"
-            "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d0),
-            "l"(ad + 2 * k), "l"(bd + 2 * k), "r"(idesc), "r"(1u)
-            : "memory");
+      for (int k = 0; k < 4; ++k) umma_bf16_pair(d0, ad + 2 * k, bd + 2 * k, idesc, 1u);
     }
     asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(&bar[warp])) : "memory");
     mbar_wait(&bar[warp], 0);
@@ -167,8 +151,8 @@ __global__ void __launch_bounds__(128) mma_bench_pair_kernel(int N, int issuers,
   }
   tc_fence_before();
   __syncthreads();
-  cluster_sync_all();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(cols) : "memory");
+  cluster_sync();
+  if (warp == 0) tmem_dealloc_pair(tmem_base, cols);
 }
 
 }  // namespace ug

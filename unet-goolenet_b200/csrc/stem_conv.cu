@@ -1,51 +1,40 @@
-// Stem convolutions (the two 3-input-channel layers) as fused implicit GEMMs on tcgen05: the im2col tile is
-// built directly in shared memory from the source image, so no im2col matrix ever reaches HBM.
+// Stem convolution (the UNet's 3-input-channel layer) as a fused implicit GEMM on tcgen05: the im2col tile is built
+// directly in shared memory from the source image, so no im2col matrix ever reaches HBM.
 //
 //   kind 0  UNet `inc`  (basicUnet.py:409, ConvBatchNorm :25-40): 3x3, stride 1, pad 1 on fp32 NCHW [B,3,H,W]
 //           K index = (r*3+s)*3+c, 27 real columns, two K=16 MMAs (columns 27..31 are written as zeros).
-//   kind 1  GoogLeNet `conv1` (torchvision BasicConv2d 7x7, stride 2, pad 3) on the uint8 HWC crop (or a float
-//           NCHW image), with to_tensor (/255) and _transform_input applied before the zero padding.
-//           K index = r*22 + s*3 + c (each filter row is a run of 21 contiguous source values padded to 22 so
-//           that runs stay 4-byte aligned), 154 columns, ten K=16 MMAs.
+// (GoogLeNet's conv1 runs as ug_s2d_pack + a row-tap implicit GEMM on the multi-issuer kernel, see lower.py.)
 //
 // One warpgroup (128 threads) = one 16x8 tile of output pixels (thread t <-> pixel row t of the MMA <-> TMEM lane t),
-// N = 64 output channels.  A CTA holds kGroups independent warpgroups (own A tile, patch, accumulator and named
-// barrier, one shared copy of the weights): conv1's 48 KB A tile + 24 KB weights allowed only two 128-thread CTAs per
-// SM (8 warps, latency-bound); three warpgroups in one CTA share the weights and fit.  Per tile: (kind 1: stage the transformed bf16 source patch in smem) -> every thread
-// writes its im2col row into the 128B-swizzled K-major A tile -> one thread issues the MMAs -> all threads read
-// their accumulator row from TMEM, apply folded BN + ReLU, stage the bf16 tile in swizzled smem -> TMA store.
-// The phases of one warpgroup are serial; the co-resident warpgroups of an SM (6 for inc, 3 for conv1) overlap them.
-// Both layers are bound by the 64-channel output write (128 B per pixel), not by the tensor pipe.
-#include <cstdlib>
+// N = 64 output channels.  A CTA holds kGroups = 6 independent warpgroups (own A tile, patch, accumulator and named
+// barrier, one shared copy of the weights) at 80 registers per thread: 0.296 -> 0.263 ms per 128 images against five
+// single-warpgroup CTAs per SM.  Per tile: every thread writes its im2col row into the 128B-swizzled K-major A tile ->
+// one thread issues the MMAs -> all threads read their accumulator row from TMEM, apply folded BN + ReLU, stage the
+// bf16 tile in swizzled smem -> TMA store.  The phases of one warpgroup are serial; the co-resident warpgroups of an SM
+// overlap them.  The layer is bound by the 64-channel output write (128 B per pixel), not by the tensor pipe.
 #include <cstring>
 #include "conv_common.cuh"
 
 namespace ug {
 
 static constexpr int kStemTW = 16, kStemTH = 8;          // output tile
-static constexpr int kG1PatchW = 2 * kStemTW + 5;        // 37 source pixels
-static constexpr int kG1PatchH = 2 * kStemTH + 5;        // 21 source rows
+static constexpr int kStemGroups = 6;                    // warpgroups per CTA
 static constexpr int kIncPatchH = kStemTH + 2, kIncPatchW = kStemTW + 2;   // 10 x 18 source pixels per channel
 static constexpr int kIncPatchPitch = 48;                // floats per patch row: the two tile rows of a warp (ty, ty+1)
                                                          // then read banks [tx+s, ..] and [16+tx+s, ..]: no conflicts
-static constexpr int kG1PatchPitch = 112;                // bf16 elements per patch row (111 used); 56 words keeps
-                                                         // the 4-byte run copies of a warp on distinct banks
-
-__device__ __forceinline__ uint32_t stem_bf16x2_max(uint32_t a, uint32_t b) {
-  __nv_bfloat162 r = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a), *reinterpret_cast<__nv_bfloat162*>(&b));
-  return *reinterpret_cast<uint32_t*>(&r);
-}
 static constexpr int kStemPoolBytes = 4096;  // pooled tile staging: 8 x 4 pixels x 64 channels bf16
 
+// (instantiated as stem_conv_kernel<0, kStemGroups> only: kind 0 = inc)
 template <int kKind, int kGroups>
 __global__ void __launch_bounds__(128 * kGroups) stem_conv_kernel(const __grid_constant__ CUtensorMap tmB,
                                                         const __grid_constant__ CUtensorMap tmO,
                                                         const __grid_constant__ CUtensorMap tmP, const StemParams p) {
-  constexpr int kAtoms = kKind == 0 ? 1 : 3;             // 64-column swizzle atoms of the A / B tiles
-  constexpr int kKSteps = kKind == 0 ? 2 : 10;           // K=16 MMAs per tile
+  static_assert(kKind == 0, "stem kind 0 (inc) only");
+  constexpr int kAtoms = 1;                              // 64-column swizzle atoms of the A / B tiles
+  constexpr int kKSteps = 2;                             // K=16 MMAs per tile
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);  // keeps the shared address space
-  constexpr int kPatchBytes = kKind == 0 ? 3 * kIncPatchH * kIncPatchPitch * 4 : kG1PatchH * kG1PatchPitch * 2;
+  constexpr int kPatchBytes = 3 * kIncPatchH * kIncPatchPitch * 4;
   constexpr int kPatchAlloc = (kPatchBytes + 1023) / 1024 * 1024;
   constexpr uint32_t kTmemCols = kGroups == 1 ? 64 : (kGroups == 2 ? 128 : (kGroups <= 4 ? 256 : 512));
   const int grp = threadIdx.x >> 7;                      // warpgroup: an independent tile pipeline
@@ -57,8 +46,7 @@ __global__ void __launch_bounds__(128 * kGroups) stem_conv_kernel(const __grid_c
   uint8_t* sO = sA;                                      // output staging [128 rows][128 B] reuses the first A atom:
                                                          // the A tile is dead once the MMAs of the tile completed
   uint8_t* sPool = sA + kAtoms * kABytesPerStage;        // pooled tile staging (4 KB, 1024-aligned) when p.pool
-  __nv_bfloat16* sPatch = reinterpret_cast<__nv_bfloat16*>(sPool + (p.pool ? kStemPoolBytes : 0));   // kind 1: bf16 patch
-  float* sPatchF = reinterpret_cast<float*>(sPatch);                                  // kind 0: fp32 patch
+  float* sPatchF = reinterpret_cast<float*>(sPool + (p.pool ? kStemPoolBytes : 0));   // fp32 source patch
   uint8_t* tail = sB + kAtoms * 64 * 128 + kGroups * group_bytes;
   float* sScale = reinterpret_cast<float*>(tail);       // 16-byte aligned: read as float4
   float* sBias = sScale + 64;
@@ -81,9 +69,6 @@ __global__ void __launch_bounds__(128 * kGroups) stem_conv_kernel(const __grid_c
   if (threadIdx.x < 32) {
     tmem_alloc(tmem_ptr, kTmemCols);
     tmem_relinquish();
-  }
-  if constexpr (kKind == 1) {  // element 111 of every patch row is read (times a zero weight) but never staged
-    if (tid < kG1PatchH) sPatch[tid * kG1PatchPitch + kG1PatchPitch - 1] = __float2bfloat16_rn(0.0f);
   }
   if (threadIdx.x < 64) {
     sScale[threadIdx.x] = p.scale ? p.scale[threadIdx.x] : 1.0f;
@@ -128,114 +113,47 @@ __global__ void __launch_bounds__(128 * kGroups) stem_conv_kernel(const __grid_c
       inc_raw[k] = inb ? __ldg(xn + ((long long)c * p.H + iy) * p.W + ix) : 0.0f;
     }
   };
-  // conv1: one source pixel (3 channels) per thread and step, fetched one tile ahead like the inc patch
-  constexpr int kG1Pix = kG1PatchW * kG1PatchH;
-  constexpr int kG1Steps = (kG1Pix + 127) / 128;
-  float g1_raw[kG1Steps][3];
-  unsigned g1_mask = 0;
-  auto load_g1_patch = [&](int t2) {
-    const int qx0 = 2 * ((t2 % p.tiles_x) * kStemTW) - 3, qy0 = 2 * (((t2 / p.tiles_x) % p.tiles_y) * kStemTH) - 3;
-    const int n2 = t2 / (p.tiles_x * p.tiles_y);
-    g1_mask = 0;
-#pragma unroll
-    for (int k = 0; k < kG1Steps; ++k) {
-      const int idx = tid + k * 128;
-      const int r = idx / kG1PatchW, px = idx - r * kG1PatchW;
-      const int iy = qy0 + r, ix = qx0 + px;
-      const bool inb = idx < kG1Pix && iy >= 0 && iy < p.H && ix >= 0 && ix < p.W;
-      g1_mask |= (inb ? 1u : 0u) << k;
-      if (p.in_f32) {
-        const float* src = p.in_f32 + ((long long)n2 * 3 * p.H + iy) * p.W + ix;
-#pragma unroll
-        for (int c = 0; c < 3; ++c) g1_raw[k][c] = inb ? __ldg(src + (long long)c * p.H * p.W) : 0.0f;
-      } else {
-        const unsigned char* src = p.in_u8 + (((long long)n2 * p.H + iy) * p.W + ix) * 3;
-#pragma unroll
-        for (int c = 0; c < 3; ++c) g1_raw[k][c] = inb ? (float)__ldg(src + c) / 255.0f : 0.0f;
-      }
-    }
-  };
   const int t_first = blockIdx.x * kGroups + grp, t_stride = gridDim.x * kGroups;
-  if (t_first < p.total_tiles) {
-    if constexpr (kKind == 0) load_inc_patch(t_first);
-    else load_g1_patch(t_first);
-  }
+  if (t_first < p.total_tiles) load_inc_patch(t_first);
 
   for (int t = t_first; t < p.total_tiles; t += t_stride) {
     const int x0 = (t % p.tiles_x) * kStemTW;
     const int y0 = ((t / p.tiles_x) % p.tiles_y) * kStemTH;
     const int n = t / (p.tiles_x * p.tiles_y);
 
-    if constexpr (kKind == 0) {
-      // ---- inc: stage the 3 x 10 x 18 fp32 source patch (zero outside the image) with coalesced loads, then every
-      // thread gathers its 27 taps from shared memory
-      // (the patch values of THIS tile were fetched into inc_raw one tile ahead, see load_inc_patch below)
+    // ---- inc: stage the 3 x 10 x 18 fp32 source patch (zero outside the image) with coalesced loads, then every
+    // thread gathers its 27 taps from shared memory
+    // (the patch values of THIS tile were fetched into inc_raw one tile ahead, see load_inc_patch below)
 #pragma unroll
-      for (int k = 0; k < kIncSteps; ++k) {
-        const int idx = tid + k * 128;
-        const int c = idx / (kIncPatchH * kIncPatchW), rem = idx - c * (kIncPatchH * kIncPatchW);
-        const int r = rem / kIncPatchW, xx = rem - r * kIncPatchW;
-        if (idx < kIncElems) sPatchF[(c * kIncPatchH + r) * kIncPatchPitch + xx] = inc_raw[k];
-      }
-      if (tid == 0) bulk_wait_group_read<0>();  // previous tile's TMA store has finished reading sO (= sA)
-      group_sync();
-      if (t + t_stride < p.total_tiles) load_inc_patch(t + t_stride);         // next tile's patch: in flight during
-                                                                              // the gather, the MMA and the epilogue
-      const float* pt = sPatchF + ty * kIncPatchPitch + tx;
-      float v[32];
+    for (int k = 0; k < kIncSteps; ++k) {
+      const int idx = tid + k * 128;
+      const int c = idx / (kIncPatchH * kIncPatchW), rem = idx - c * (kIncPatchH * kIncPatchW);
+      const int r = rem / kIncPatchW, xx = rem - r * kIncPatchW;
+      if (idx < kIncElems) sPatchF[(c * kIncPatchH + r) * kIncPatchPitch + xx] = inc_raw[k];
+    }
+    if (tid == 0) bulk_wait_group_read<0>();  // previous tile's TMA store has finished reading sO (= sA)
+    group_sync();
+    if (t + t_stride < p.total_tiles) load_inc_patch(t + t_stride);         // next tile's patch: in flight during
+                                                                            // the gather, the MMA and the epilogue
+    const float* pt = sPatchF + ty * kIncPatchPitch + tx;
+    float v[32];
 #pragma unroll
-      for (int i = 27; i < 32; ++i) v[i] = 0.0f;
+    for (int i = 27; i < 32; ++i) v[i] = 0.0f;
 #pragma unroll
-      for (int r = 0; r < 3; ++r)
+    for (int r = 0; r < 3; ++r)
 #pragma unroll
-        for (int sx = 0; sx < 3; ++sx)
+      for (int sx = 0; sx < 3; ++sx)
 #pragma unroll
-          for (int c = 0; c < 3; ++c)
-            v[(r * 3 + sx) * 3 + c] = pt[(c * kIncPatchH + r) * kIncPatchPitch + sx];
+        for (int c = 0; c < 3; ++c)
+          v[(r * 3 + sx) * 3 + c] = pt[(c * kIncPatchH + r) * kIncPatchPitch + sx];
 #pragma unroll
-      for (int g = 0; g < 4; ++g) {
-        uint4 o;
-        o.x = pack_bf16x2(v[g * 8 + 0], v[g * 8 + 1]);
-        o.y = pack_bf16x2(v[g * 8 + 2], v[g * 8 + 3]);
-        o.z = pack_bf16x2(v[g * 8 + 4], v[g * 8 + 5]);
-        o.w = pack_bf16x2(v[g * 8 + 6], v[g * 8 + 7]);
-        *reinterpret_cast<uint4*>(a_row + ((g ^ sw) << 4)) = o;
-      }
-    } else {
-      // ---- conv1: stage the transformed source patch (zero outside the image), then copy seven 22-element runs
-      const float sc[3] = {0.229f / 0.5f, 0.224f / 0.5f, 0.225f / 0.5f};
-      const float sh[3] = {(0.485f - 0.5f) / 0.5f, (0.456f - 0.5f) / 0.5f, (0.406f - 0.5f) / 0.5f};
-      // one source pixel (3 channels) per thread and step; all loads of a tile are issued before any is used
-      constexpr int kPix = kG1PatchW * kG1PatchH;
-      constexpr int kSteps = kG1Steps;   // source pixels of THIS tile were fetched one tile ahead (load_g1_patch)
-#pragma unroll
-      for (int k = 0; k < kSteps; ++k) {
-        const int idx = tid + k * 128;
-        const int r = idx / kG1PatchW, px = idx - r * kG1PatchW;
-        if (idx < kPix) {
-#pragma unroll
-          for (int c = 0; c < 3; ++c)  // zero padding is applied after the affine: out-of-image taps are exactly 0
-            sPatch[r * kG1PatchPitch + px * 3 + c] =
-                __float2bfloat16_rn(((g1_mask >> k) & 1u) ? g1_raw[k][c] * sc[c] + sh[c] : 0.0f);
-        }
-      }
-      if (tid == 0) bulk_wait_group_read<0>();  // previous tile's TMA store has finished reading sO (= sA)
-      group_sync();
-      if (t + t_stride < p.total_tiles) load_g1_patch(t + t_stride);         // next tile's source pixels in flight
-      uint32_t w[80];
-#pragma unroll
-      for (int r = 0; r < 7; ++r) {
-        const uint32_t* src =
-            reinterpret_cast<const uint32_t*>(sPatch + (2 * ty + r) * kG1PatchPitch + 6 * tx);
-#pragma unroll
-        for (int i = 0; i < 11; ++i) w[r * 11 + i] = src[i];
-      }
-      w[77] = w[78] = w[79] = 0u;
-#pragma unroll
-      for (int j = 0; j < 20; ++j) {
-        const uint4 o = make_uint4(w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
-        *reinterpret_cast<uint4*>(a_row + (j >> 3) * kABytesPerStage + (((j & 7) ^ sw) << 4)) = o;
-      }
+    for (int g = 0; g < 4; ++g) {
+      uint4 o;
+      o.x = pack_bf16x2(v[g * 8 + 0], v[g * 8 + 1]);
+      o.y = pack_bf16x2(v[g * 8 + 2], v[g * 8 + 3]);
+      o.z = pack_bf16x2(v[g * 8 + 4], v[g * 8 + 5]);
+      o.w = pack_bf16x2(v[g * 8 + 6], v[g * 8 + 7]);
+      *reinterpret_cast<uint4*>(a_row + ((g ^ sw) << 4)) = o;
     }
     fence_proxy_async_smem();  // generic-proxy writes of the A tile -> visible to the tensor core (async proxy)
     tc_fence_before();
@@ -277,14 +195,14 @@ __global__ void __launch_bounds__(128 * kGroups) stem_conv_kernel(const __grid_c
         if (p.pool) {
           // fused nn.MaxPool2d(2): pixel (tx, ty) = row ty*16 + tx; its 2x2 window lives in lanes ^1 (x) and ^16 (y)
           uint4 m = o;
-          m.x = stem_bf16x2_max(m.x, __shfl_xor_sync(0xffffffffu, m.x, 1));
-          m.y = stem_bf16x2_max(m.y, __shfl_xor_sync(0xffffffffu, m.y, 1));
-          m.z = stem_bf16x2_max(m.z, __shfl_xor_sync(0xffffffffu, m.z, 1));
-          m.w = stem_bf16x2_max(m.w, __shfl_xor_sync(0xffffffffu, m.w, 1));
-          m.x = stem_bf16x2_max(m.x, __shfl_xor_sync(0xffffffffu, m.x, 16));
-          m.y = stem_bf16x2_max(m.y, __shfl_xor_sync(0xffffffffu, m.y, 16));
-          m.z = stem_bf16x2_max(m.z, __shfl_xor_sync(0xffffffffu, m.z, 16));
-          m.w = stem_bf16x2_max(m.w, __shfl_xor_sync(0xffffffffu, m.w, 16));
+          m.x = bf16x2_max(m.x, __shfl_xor_sync(0xffffffffu, m.x, 1));
+          m.y = bf16x2_max(m.y, __shfl_xor_sync(0xffffffffu, m.y, 1));
+          m.z = bf16x2_max(m.z, __shfl_xor_sync(0xffffffffu, m.z, 1));
+          m.w = bf16x2_max(m.w, __shfl_xor_sync(0xffffffffu, m.w, 1));
+          m.x = bf16x2_max(m.x, __shfl_xor_sync(0xffffffffu, m.x, 16));
+          m.y = bf16x2_max(m.y, __shfl_xor_sync(0xffffffffu, m.y, 16));
+          m.z = bf16x2_max(m.z, __shfl_xor_sync(0xffffffffu, m.z, 16));
+          m.w = bf16x2_max(m.w, __shfl_xor_sync(0xffffffffu, m.w, 16));
           if (((tx | ty) & 1) == 0) {
             const int pr = (ty >> 1) * 8 + (tx >> 1);  // pooled pixel row of the 8 x 4 tile
             *reinterpret_cast<uint4*>(sPool + pr * 128 + ((((c0 >> 3) + g) ^ (pr & 7)) << 4)) = m;
@@ -308,56 +226,40 @@ __global__ void __launch_bounds__(128 * kGroups) stem_conv_kernel(const __grid_c
 }
 
 // ------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
 int stem_prepare(ug_engine* h, const ug_stem_desc* d, StemLaunch* L) {
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) return set_error(h, UG_ECUDA, "cuTensorMapEncodeTiled entry point unavailable");
-  if (d->kind != 0 && d->kind != 1) return set_error(h, UG_EINVAL, "stem: kind must be 0 (inc) or 1 (conv1)");
+  if (!get_encode_fn()) return set_error(h, UG_ECUDA, "cuTensorMapEncodeTiled entry point unavailable");
+  if (d->kind != 0) return set_error(h, UG_EINVAL, "stem: kind must be 0 (inc)");
   if (!d->w || !d->out || d->B <= 0 || d->H <= 0 || d->W <= 0) return set_error(h, UG_EINVAL, "stem: bad args");
-  if (d->kind == 0 && !d->in_f32) return set_error(h, UG_EINVAL, "stem(inc): fp32 NCHW input required");
-  if (d->kind == 1 && !d->in_f32 && !d->in_u8) return set_error(h, UG_EINVAL, "stem(conv1): no input");
-  if (d->kind == 1 && ((d->H | d->W) & 1)) return set_error(h, UG_EINVAL, "stem(conv1): even image size required");
+  if (!d->in_f32) return set_error(h, UG_EINVAL, "stem(inc): fp32 NCHW input required");
   if (d->out_cstride % 8 || d->out_cstride < 64 || (reinterpret_cast<uintptr_t>(d->out) & 15) ||
       (reinterpret_cast<uintptr_t>(d->w) & 15))
     return set_error(h, UG_EINVAL, "stem: out/w must be 16B aligned, channel stride a multiple of 8 (>= 64)");
-  const int OH = d->kind == 0 ? d->H : d->H / 2, OW = d->kind == 0 ? d->W : d->W / 2;
-  const int katoms = d->kind == 0 ? 1 : 3;
+  const int OH = d->H, OW = d->W;
   memset(L, 0, sizeof(*L));
-  L->kind = d->kind;
   StemParams& p = L->p;
-  p.in_f32 = d->in_f32; p.in_u8 = d->in_u8; p.scale = d->scale; p.bias = d->bias;
+  p.in_f32 = d->in_f32; p.scale = d->scale; p.bias = d->bias;
   p.B = d->B; p.H = d->H; p.W = d->W; p.OH = OH; p.OW = OW;
   p.tiles_x = (OW + kStemTW - 1) / kStemTW;
   p.tiles_y = (OH + kStemTH - 1) / kStemTH;
   p.total_tiles = p.tiles_x * p.tiles_y * d->B;
   p.pool = d->pool_out != nullptr;
-  if (p.pool && (d->kind != 0 || (d->H & 1) || (d->W & 1) || d->pool_cstride % 8 || d->pool_cstride < 64 ||
+  if (p.pool && ((d->H & 1) || (d->W & 1) || d->pool_cstride % 8 || d->pool_cstride < 64 ||
                  (reinterpret_cast<uintptr_t>(d->pool_out) & 15)))
-    return set_error(h, UG_EINVAL, "stem: fused max-pool needs kind 0 on an even image, 16B-aligned pooled output");
+    return set_error(h, UG_EINVAL, "stem: fused max-pool needs an even image, 16B-aligned pooled output");
   {
-    cuuint64_t dims[2] = {(cuuint64_t)katoms * 64, 64};
-    cuuint64_t strides[1] = {(cuuint64_t)katoms * 64 * 2};
+    cuuint64_t dims[2] = {64, 64};
+    cuuint64_t strides[1] = {64 * 2};
     cuuint32_t box[2] = {64, 64};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = encode(&L->tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(d->w), dims, strides, box, es,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(h, UG_ECUDA, "stem: weight tensor map encode failed (%d)", (int)r);
+    const int r = encode_bf16_sw128(&L->tmB, d->w, 2, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+    if (r) return set_error(h, UG_ECUDA, "stem: weight tensor map encode failed (%d)", r);
   }
   {
     cuuint64_t dims[4] = {64, (cuuint64_t)OW, (cuuint64_t)OH, (cuuint64_t)d->B};
     cuuint64_t strides[3] = {(cuuint64_t)d->out_cstride * 2, (cuuint64_t)OW * d->out_cstride * 2,
                              (cuuint64_t)OH * OW * d->out_cstride * 2};
     cuuint32_t box[4] = {64, (cuuint32_t)kStemTW, (cuuint32_t)kStemTH, 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    CUresult r = encode(&L->tmO, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, d->out, dims, strides, box, es,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(h, UG_ECUDA, "stem: output tensor map encode failed (%d)", (int)r);
+    const int r = encode_bf16_sw128(&L->tmO, d->out, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+    if (r) return set_error(h, UG_ECUDA, "stem: output tensor map encode failed (%d)", r);
   }
   if (p.pool) {
     const long long pcs = d->pool_cstride;
@@ -365,48 +267,27 @@ int stem_prepare(ug_engine* h, const ug_stem_desc* d, StemLaunch* L) {
     cuuint64_t strides[3] = {(cuuint64_t)(pcs * 2), (cuuint64_t)((OW / 2) * pcs * 2),
                              (cuuint64_t)((long long)(OH / 2) * (OW / 2) * pcs * 2)};
     cuuint32_t box[4] = {64, (cuuint32_t)(kStemTW / 2), (cuuint32_t)(kStemTH / 2), 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    CUresult r = encode(&L->tmP, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, d->pool_out, dims, strides, box, es,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(h, UG_ECUDA, "stem: pooled output tensor map encode failed (%d)", (int)r);
+    const int r = encode_bf16_sw128(&L->tmP, d->pool_out, 4, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+    if (r) return set_error(h, UG_ECUDA, "stem: pooled output tensor map encode failed (%d)", r);
   }
-  // One CTA per SM holding several warpgroups that share the weights: conv1 three (48 KB A tile each; measured 0.557 ->
-  // 0.435 ms per 256 images against two single-warpgroup CTAs per SM), inc six at 80 registers per thread (0.296 ->
-  // 0.263 ms per 128 images against five single-warpgroup CTAs per SM).  UG_STEM_GROUPS=1 / UG_INC_GROUPS=1: former shape.
-  static const int g1_groups = [] { const char* e = getenv("UG_STEM_GROUPS"); return e && atoi(e) == 1 ? 1 : 3; }();
-  static const int inc_groups = [] { const char* e = getenv("UG_INC_GROUPS"); return e && atoi(e) == 1 ? 1 : 6; }();
-  L->groups = d->kind == 0 ? inc_groups : g1_groups;
-  const int ctas_per_sm = d->kind == 0 ? (L->groups == 1 ? 7 : 1) : (L->groups == 1 ? 2 : 1);
-  L->grid = (unsigned)std::min<long long>((p.total_tiles + L->groups - 1) / L->groups, (long long)h->num_sms * ctas_per_sm);
-  const size_t patch = d->kind == 1 ? kG1PatchH * kG1PatchPitch * 2 : 3 * kIncPatchH * kIncPatchPitch * 4;
-  L->smem = 1024 + (size_t)katoms * 64 * 128 +
-            L->groups * ((size_t)katoms * kABytesPerStage + (p.pool ? kStemPoolBytes : 0) + (patch + 1023) / 1024 * 1024) +
-            2 * 64 * sizeof(float) + 8 * (1 + L->groups) + 16;
+  // one CTA per SM: its warpgroups share the weights (see the header comment)
+  L->grid = (unsigned)std::min<long long>((p.total_tiles + kStemGroups - 1) / kStemGroups, (long long)h->num_sms);
+  const size_t patch = 3 * kIncPatchH * kIncPatchPitch * 4;
+  L->smem = 1024 + (size_t)64 * 128 +
+            kStemGroups * ((size_t)kABytesPerStage + (p.pool ? kStemPoolBytes : 0) + (patch + 1023) / 1024 * 1024) +
+            2 * 64 * sizeof(float) + 8 * (1 + kStemGroups) + 16;
   return UG_OK;
 }
 
 int stem_launch(ug_engine* h, const StemLaunch* L, cudaStream_t s) {
   if (!h->attr_stem) {
-    cudaError_t e = cudaFuncSetAttribute((const void*)stem_conv_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         100 * 1024);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute((const void*)stem_conv_kernel<0, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               210 * 1024);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute((const void*)stem_conv_kernel<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               110 * 1024);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute((const void*)stem_conv_kernel<1, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               210 * 1024);
+    const cudaError_t e = cudaFuncSetAttribute((const void*)stem_conv_kernel<0, kStemGroups>,
+                                               cudaFuncAttributeMaxDynamicSharedMemorySize, 210 * 1024);
     if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(stem_conv_kernel)");
     h->attr_stem = true;
   }
-  cudaError_t le;
-  if (L->kind == 0 && L->groups == 6) le = launch_pdl(h, stem_conv_kernel<0, 6>, L->grid, 768, L->smem, s, L->tmB, L->tmO, L->tmP, L->p);
-  else if (L->kind == 0) le = launch_pdl(h, stem_conv_kernel<0, 1>, L->grid, 128, L->smem, s, L->tmB, L->tmO, L->tmP, L->p);
-  else if (L->groups == 1) le = launch_pdl(h, stem_conv_kernel<1, 1>, L->grid, 128, L->smem, s, L->tmB, L->tmO, L->tmP, L->p);
-  else le = launch_pdl(h, stem_conv_kernel<1, 3>, L->grid, 384, L->smem, s, L->tmB, L->tmO, L->tmP, L->p);
+  const cudaError_t le = launch_pdl(stem_conv_kernel<0, kStemGroups>, L->grid, 128 * kStemGroups, L->smem, s, L->tmB,
+                                    L->tmO, L->tmP, L->p);
   h->launches++;
   return check_cuda(h, le != cudaSuccess ? le : cudaGetLastError(), "stem_conv_kernel launch");
 }

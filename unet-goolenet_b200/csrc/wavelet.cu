@@ -252,8 +252,6 @@ __global__ void __launch_bounds__(256) wavelet_ragged_up_kernel(const unsigned c
                 e.H, e.W, (e.H + 1) / 2, (e.W + 1) / 2);
 }
 
-static inline int cdivw(long long a, long long b) { return (int)((a + b - 1) / b); }
-
 int launch_wavelet(ug_engine* h, const ug_wavelet_desc* d, cudaStream_t s) {
   if (!d->gray || !d->out_u8 || !d->workspace || d->B <= 0 || d->H < 2 || d->W < 2)
     return set_error(h, UG_EINVAL, "wavelet: bad args (H, W >= 2)");
@@ -264,10 +262,10 @@ int launch_wavelet(ug_engine* h, const ug_wavelet_desc* d, cudaStream_t s) {
   float* cA = reinterpret_cast<float*>(st + ((d->B + 3) / 4) * 4);
   float* hf = cA + (size_t)d->B * h2 * w2;
   const int HW = d->H * d->W;
-  const dim3 gfull(std::min(cdivw(HW, 256), 64), d->B);
-  wavelet_init_kernel<<<cdivw(d->B, 128), 128, 0, s>>>(st, d->B);
+  const dim3 gfull(std::min(ceil_div(HW, 256), 64), d->B);
+  wavelet_init_kernel<<<ceil_div(d->B, 128), 128, 0, s>>>(st, d->B);
   wavelet_gray_stats_kernel<<<gfull, 256, 0, s>>>(d->gray, st, HW);
-  wavelet_dwt_kernel<<<dim3(cdivw((long long)h2 * w2, 256), d->B), 256, 0, s>>>(d->gray, st, cA, hf, d->H, d->W, h2, w2);
+  wavelet_dwt_kernel<<<dim3(ceil_div((long long)h2 * w2, 256), d->B), 256, 0, s>>>(d->gray, st, cA, hf, d->H, d->W, h2, w2);
   wavelet_up_kernel<false><<<gfull, 256, 0, s>>>(d->gray, st, cA, hf, nullptr, d->H, d->W, h2, w2);
   wavelet_up_kernel<true><<<gfull, 256, 0, s>>>(d->gray, st, cA, hf, d->out_u8, d->H, d->W, h2, w2);
   h->launches += 5;
@@ -286,17 +284,17 @@ int launch_wavelet_ragged(ug_engine* h, const ug_wavelet_ragged_desc* d, cudaStr
   const WvRagged rg{d->index, d->status, d->capacity_px};
   // The table lives on the device, so the grid is sized from the capacity (a bound on the largest image) and every
   // kernel strides over its image; blocks past an image's extent do no work.
-  const dim3 grid(std::min(cdivw(d->capacity_px, 256), 64), d->B);
-  int rc = check_cuda(h, launch_pdl(h, wavelet_ragged_init_kernel, cdivw(d->B, 128), 128, 0, s, st, rg, d->B), "wavelet_ragged init");
+  const dim3 grid(std::min(ceil_div(d->capacity_px, 256), 64), d->B);
+  int rc = check_cuda(h, launch_pdl(wavelet_ragged_init_kernel, ceil_div(d->B, 128), 128, 0, s, st, rg, d->B), "wavelet_ragged init");
   if (rc == UG_OK)
-    rc = check_cuda(h, launch_pdl(h, wavelet_ragged_gray_stats_kernel, grid, 256, 0, s, d->gray, st, rg), "wavelet_ragged stats");
+    rc = check_cuda(h, launch_pdl(wavelet_ragged_gray_stats_kernel, grid, 256, 0, s, d->gray, st, rg), "wavelet_ragged stats");
   if (rc == UG_OK)
-    rc = check_cuda(h, launch_pdl(h, wavelet_ragged_dwt_kernel, grid, 256, 0, s, d->gray, st, cA, hf, rg), "wavelet_ragged dwt");
+    rc = check_cuda(h, launch_pdl(wavelet_ragged_dwt_kernel, grid, 256, 0, s, d->gray, st, cA, hf, rg), "wavelet_ragged dwt");
   if (rc == UG_OK)
-    rc = check_cuda(h, launch_pdl(h, wavelet_ragged_up_kernel<false>, grid, 256, 0, s, d->gray, st, cA, hf, nullptr, rg),
+    rc = check_cuda(h, launch_pdl(wavelet_ragged_up_kernel<false>, grid, 256, 0, s, d->gray, st, cA, hf, nullptr, rg),
                     "wavelet_ragged up");
   if (rc == UG_OK)
-    rc = check_cuda(h, launch_pdl(h, wavelet_ragged_up_kernel<true>, grid, 256, 0, s, d->gray, st, cA, hf, d->out_u8, rg),
+    rc = check_cuda(h, launch_pdl(wavelet_ragged_up_kernel<true>, grid, 256, 0, s, d->gray, st, cA, hf, d->out_u8, rg),
                     "wavelet_ragged up");
   h->launches += 5;
   return rc;

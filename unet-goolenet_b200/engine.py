@@ -139,7 +139,7 @@ _SINGLE_ENTRY = {OP_CONV: "ug_conv", OP_POOL: "ug_pool",
 EXPORTED_SYMBOLS = ["ug_version", "ug_create", "ug_destroy", "ug_last_error", "ug_launch_count",
                     *_SINGLE_ENTRY.values(), "ug_program_create", "ug_program_run", "ug_program_num_launches",
                     "ug_program_destroy", "ug_program_run_host", "ug_program_run_host_pipelined",
-                    "ug_program_run_timed", "ug_program_autotune", "ug_wavelet_workspace_bytes",
+                    "ug_program_run_timed", "ug_wavelet_workspace_bytes",
                     "ug_wavelet_ragged_workspace_bytes",
                     "ug_plan_load", "ug_plan_num_io", "ug_plan_io_name", "ug_plan_io", "ug_plan_device_bytes",
                     "ug_plan_program", "ug_plan_copy_in", "ug_plan_copy_out", "ug_plan_run", "ug_plan_destroy"]
@@ -183,7 +183,6 @@ def load_library():
     lib.ug_wavelet_workspace_bytes.restype = C.c_size_t
     lib.ug_wavelet_ragged_workspace_bytes.argtypes = [_i, _ll]
     lib.ug_wavelet_ragged_workspace_bytes.restype = C.c_size_t
-    lib.ug_program_autotune.argtypes = [_vp, _vp, _vp, C.POINTER(_i)]
     lib.ug_program_destroy.argtypes = [_vp, _vp]
     lib.ug_program_run_host.argtypes = [_vp, _vp, _vp, _i, _vp, _i, _vp]
     lib.ug_program_run_host_pipelined.argtypes = [_vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp]
@@ -229,14 +228,6 @@ class Program:
     def run(self, stream=None):
         s = stream if stream is not None else torch.cuda.current_stream().cuda_stream
         self.engine._check(self.engine.lib.ug_program_run(self.engine.handle, self.handle, s))
-
-    def autotune(self, stream=None):
-        """Time every auto-variant conv op with each kernel structure and keep the fastest (ug_program_autotune).
-        Overwrites the ops' output buffers; call before the first real run.  Returns the number of switched ops."""
-        s = stream if stream is not None else torch.cuda.current_stream().cuda_stream
-        n = _i(0)
-        self.engine._check(self.engine.lib.ug_program_autotune(self.engine.handle, self.handle, s, C.byref(n)))
-        return n.value
 
     def run_timed(self, stream=None):
         """Per-op device times in ms (event pair around every op; profiling aid, not the benchmark path)."""

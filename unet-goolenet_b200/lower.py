@@ -20,26 +20,6 @@ from . import pack
 from .util import ragged
 
 IMG = 224
-# UG_AUTOTUNE=1: measured kernel-variant choice at plan time (ug_program_autotune).  Off by default: on the B200 it
-# switched 52 of 133 conv ops but the step time stayed within run-to-run noise (9.69k vs 9.70k img/s), and the static
-# choice keeps results bit-identical from one process to the next.
-AUTOTUNE = os.environ.get("UG_AUTOTUNE", "0") == "1"
-# UG_FUSE_POOL=0 falls back to separate max-pool launches after the encoder convolutions (A/B measurements).
-FUSE_POOL = os.environ.get("UG_FUSE_POOL", "1") != "0"
-# UG_FUSE_STATS=<side>: fuse CoordAtt3's channel statistics into the conv1_e epilogue on maps up to <side> pixels.
-# Off by default: the extra epilogue work costs what the separate pass over e1 saves (same-box A/B: all maps fused
-# 10.01k vs 10.09k img/s, maps <= 56 fused 9.82k vs 9.88k).
-FUSE_STATS = int(os.environ.get("UG_FUSE_STATS", "0"))
-# UG_FUSE_REDUCE=0: run the two Inception reduce convolutions (branch2.0 / branch3.0, same input) as separate launches.
-# Same-box A/B: 9756 / 9721 img/s fused vs 9732 / 9742 separate (neutral); kept on, it removes 9 launches per batch.
-FUSE_REDUCE = os.environ.get("UG_FUSE_REDUCE", "1") != "0"
-# UG_FUSE_HEAD=0: keep Inception branch1 as its own 1x1 launch.  Default: ONE GEMM for the three 1x1 convolutions that
-# read the block input (branch1 | 3x3-reduce | 5x5-reduce; torchvision Inception.forward), branch1's columns stored
-# straight into the block's concat output and the two reduce results into a scratch tensor (ug_conv_desc.out2).
-FUSE_HEAD = os.environ.get("UG_FUSE_HEAD", "1") != "0" and FUSE_REDUCE
-# UG_CONV1_S2D=0: GoogLeNet conv1 (7x7 s2) on the thread-built im2col stem kernel.  Default: a space-to-depth pack of the
-# crop (ug_s2d_pack) followed by a regular TMA implicit GEMM with four row taps over overlapping 128-byte windows.
-CONV1_S2D = os.environ.get("UG_CONV1_S2D", "1") != "0"
 
 
 # Plans (program + activation workspace) kept per runner: a loader with ragged / varying batch sizes would otherwise
@@ -51,8 +31,6 @@ def _finish(engine, ops, ws, keepalive=()):
     """Compile `ops`.  The op descriptors hold raw device pointers only, so the program itself keeps every workspace
     tensor they point into alive (`keepalive` = every allocation the builder(s) made while emitting)."""
     ws["program"] = engine.program(ops, keepalive=list(keepalive))
-    if AUTOTUNE:
-        ws["tuned_ops"] = ws["program"].autotune()
     return ws
 
 
@@ -155,16 +133,19 @@ class _Builder:
         self.w = _map_tensors(self.w, view)
 
     # ---- weights -------------------------------------------------------------------------------
+    def fold(self, conv, bn, eps):
+        """Fold BatchNorm `bn`.* (eval) and the bias of conv `conv` into fp32 scale/bias."""
+        sd = self.sd
+        cb = _f32(sd[conv + ".bias"], self.dev) if (conv + ".bias") in sd else None
+        return pack.fold_bn(cb, _f32(sd[bn + ".weight"], self.dev), _f32(sd[bn + ".bias"], self.dev),
+                            _f32(sd[bn + ".running_mean"], self.dev), _f32(sd[bn + ".running_var"], self.dev), eps)
+
     def conv_bn(self, key, conv, bn, eps, bias_key=None):
         """Pack conv weight `conv`.weight and fold BatchNorm `bn`.* (eval) into fp32 scale/bias."""
         if key in self.w:
             return self.w[key]
-        sd = self.sd
-        wt = _f32(sd[conv + ".weight"], self.dev)
-        cb = _f32(sd[conv + ".bias"], self.dev) if (conv + ".bias") in sd else None
-        scale, bias = pack.fold_bn(cb, _f32(sd[bn + ".weight"], self.dev), _f32(sd[bn + ".bias"], self.dev),
-                                   _f32(sd[bn + ".running_mean"], self.dev), _f32(sd[bn + ".running_var"], self.dev),
-                                   eps)
+        wt = _f32(self.sd[conv + ".weight"], self.dev)
+        scale, bias = self.fold(conv, bn, eps)
         bn_tile = pack.choose_bn(wt.shape[0], r=wt.shape[2])
         self.w[key] = dict(w=pack.pack_conv_weight(wt, bn_tile), scale=scale, bias=bias, N=wt.shape[0],
                            Cin=wt.shape[1], R=wt.shape[2], BN=bn_tile)
@@ -188,7 +169,7 @@ class _Builder:
 
     # ---- ops -----------------------------------------------------------------------------------
     def conv(self, ops, wd, x, geom, out=None, act=E.ACT_RELU, mode=E.EPI_STORE, up=1, add=None, add_bstride=0,
-             gate=None, outc=None, pool_out=None, stats=None, out2=None, in_strides=None):
+             gate=None, outc=None, pool_out=None, out2=None, in_strides=None):
         B, H, W = geom
         d = E.ConvDesc()
         d.algo_k = wd.get("algo_k", wd["Cin"] * wd["R"] * wd["R"])   # true reduction length (for FLOP accounting)
@@ -216,8 +197,6 @@ class _Builder:
             d.gate = gate.data_ptr()
         if pool_out is not None:                                     # fused nn.MaxPool2d(2) side output
             d.pool_out, d.pool_cstride = pool_out.data_ptr(), pool_out.shape[-1]
-        if stats is not None:                                        # fused per-tile channel sums / maxima
-            d.stats_sum, d.stats_max, d.stats_tiles = stats[0].data_ptr(), stats[1].data_ptr(), stats[2]
         if out2 is not None:                                         # split 1x1 GEMM (Inception heads)
             d.out2, d.out2_cstride, d.n_split, d.n1 = out2.ptr, out2.cstride, wd["n_split"], wd["n1"]
         if outc is not None:
@@ -359,9 +338,7 @@ class UNetRunner(_Builder):
         wi = self.w["inc"]
         ops.append(E.StemDesc(0, ws["x_in"].data_ptr(), None, wi["w"].data_ptr(), wi["scale"].data_ptr(),
                               wi["bias"].data_ptr(), x1.data_ptr(), 64, B, IMG, IMG,
-                              pooled.data_ptr() if FUSE_POOL else None, 64))
-        if not FUSE_POOL:
-            ops.append(E.PoolDesc(x1.data_ptr(), 64, pooled.data_ptr(), 64, 64, B, IMG, IMG, IMG // 2, IMG // 2, 2, 2, 0))
+                              pooled.data_ptr(), 64))
         skips = [x1]
         size = IMG
         for blk, cout in (("down1", 128), ("down2", 256), ("down3", 512), ("down4", 512)):
@@ -370,10 +347,7 @@ class UNetRunner(_Builder):
             self.conv(ops, self.w[blk + ".0"], View(pooled), (B, half, half), View(t0))
             t1 = buf(B, half, half, cout)
             nxt = buf(B, half // 2, half // 2, cout) if blk != "down4" else None
-            self.conv(ops, self.w[blk + ".1"], View(t0), (B, half, half), View(t1), pool_out=nxt if FUSE_POOL else None)
-            if nxt is not None and not FUSE_POOL:
-                ops.append(E.PoolDesc(t1.data_ptr(), cout, nxt.data_ptr(), cout, cout, B, half, half, half // 2,
-                                      half // 2, 2, 2, 0))
+            self.conv(ops, self.w[blk + ".1"], View(t0), (B, half, half), View(t1), pool_out=nxt)
             pooled, size = nxt, half
             skips.append(t1)
             ws[blk] = t1
@@ -451,17 +425,10 @@ class UNetRunner(_Builder):
             self.conv(ops, self.w[blk + ".up"], View(prev), (B, psize, psize), View(cat, C, 0), act=E.ACT_NONE,
                       up=2)
             e1 = buf(B, size, size, C)
-            if size <= FUSE_STATS:
-                # AdaptiveAvg/MaxPool2d(1) of e1 (basicUnet.py:217-218), stage 1 fused into the conv epilogue: one
-                # partial per pixel tile (8 x TH pixels, TH = the conv kernel's tile height); ug_gate folds them
-                S = -(-size // 8) * -(-size // (-(-size // -(-size // 16))))
-                psum, pmax = buf(B, S, C, dtype=torch.float32), buf(B, S, C, dtype=torch.float32)
-                self.conv(ops, self.w[blk + ".conv1_e"], View(skip), geom, View(e1), stats=(psum, pmax, S))
-            else:
-                S = self.STATS_SPLITS
-                psum, pmax = buf(B, S, C, dtype=torch.float32), buf(B, S, C, dtype=torch.float32)
-                self.conv(ops, self.w[blk + ".conv1_e"], View(skip), geom, View(e1))
-                ops.append(E.ChanStatsDesc(e1.data_ptr(), C, C, B, size * size, S, psum.data_ptr(), pmax.data_ptr()))
+            S = self.STATS_SPLITS
+            psum, pmax = buf(B, S, C, dtype=torch.float32), buf(B, S, C, dtype=torch.float32)
+            self.conv(ops, self.w[blk + ".conv1_e"], View(skip), geom, View(e1))
+            ops.append(E.ChanStatsDesc(e1.data_ptr(), C, C, B, size * size, S, psum.data_ptr(), pmax.data_ptr()))
             gw = self.w[blk + ".gate"]
             g, ghid = buf(B, C, dtype=torch.float32), buf(B, C // 2, dtype=torch.float32)
             ops.append(E.GateDesc(psum.data_ptr(), pmax.data_ptr(), gw["w1"].data_ptr(), gw["b1"].data_ptr(),
@@ -571,43 +538,30 @@ class GoogLeNetRunner(_Builder):
 
     def _pack(self):
         sd, dev = self.sd, self.dev
-        # conv1 7x7 s2: GEMM weight [64][192], column r*22 + s*3 + c (each filter row padded 21 -> 22, see
-        # ug_stem_desc); 154 real columns
         wt = _f32(sd["conv1.conv.weight"], dev)                     # [64,3,7,7]
-        scale, bias = pack.fold_bn(None, _f32(sd["conv1.bn.weight"], dev), _f32(sd["conv1.bn.bias"], dev),
-                                   _f32(sd["conv1.bn.running_mean"], dev), _f32(sd["conv1.bn.running_var"], dev),
-                                   self.EPS)
-        gemm = torch.zeros(64, 7, 22)
-        gemm[:, :, :21] = wt.permute(0, 2, 3, 1).reshape(64, 7, 21)
-        self.w["conv1"] = dict(w=pack.pack_linear_weight(gemm.reshape(64, 154), 64), scale=scale, bias=bias, N=64,
-                               Cin=192, R=1, BN=64, algo_k=147)
+        scale, bias = self.fold("conv1.conv", "conv1.bn", self.EPS)
         self.w["conv1_s2d"] = dict(w=pack.pack_conv1_s2d(wt), scale=scale, bias=bias, N=64, Cin=64, R=4, S=1, pad=0,
                                    BN=64, algo_k=147)
         self.conv_bn("conv2", "conv2.conv", "conv2.bn", self.EPS)
         self.conv_bn("conv3", "conv3.conv", "conv3.bn", self.EPS)
         for name in _INCEPTION_CFG:
-            for br in ("branch1", "branch2.0", "branch2.1", "branch3.0", "branch3.1", "branch4.1"):
+            for br in ("branch2.1", "branch3.1", "branch4.1"):
                 self.conv_bn(f"{name}.{br}", f"{name}.{br}.conv", f"{name}.{br}.bn", self.EPS)
-            # the two 1x1 reduce convolutions read the same tensor: one GEMM with the output channels concatenated
-            # ([3x3-reduce | 5x5-reduce]); the 3x3 / 5x5 branches then read channel slices of its output
-            a, b = self.w[f"{name}.branch2.0"], self.w[f"{name}.branch3.0"]
-            wt = torch.cat([_f32(sd[f"{name}.branch2.0.conv.weight"], dev), _f32(sd[f"{name}.branch3.0.conv.weight"], dev)], 0)
-            bn_tile = pack.choose_bn(wt.shape[0])
-            self.w[f"{name}.reduce"] = dict(w=pack.pack_conv_weight(wt, bn_tile), scale=torch.cat([a["scale"], b["scale"]]),
-                                            bias=torch.cat([a["bias"], b["bias"]]), N=wt.shape[0], Cin=wt.shape[1], R=1,
-                                            BN=bn_tile)
-            # all three 1x1 heads of the block as one GEMM: [branch1 | zero rows up to a multiple of 64 | reduce]
-            h1 = self.w[f"{name}.branch1"]
-            n1 = h1["N"]
+            # the three 1x1 convolutions that read the block input (torchvision Inception.forward: branch1, 3x3-reduce,
+            # 5x5-reduce) as ONE GEMM [branch1 | zero rows up to a multiple of 64 | 3x3-reduce | 5x5-reduce]: branch1's
+            # columns go straight into the block's concat output, the two reduce results into a scratch tensor
+            # (ug_conv_desc.out2) whose channel slices the 3x3 / 5x5 branches read
+            heads = ("branch1", "branch2.0", "branch3.0")
+            w1, w2, w3 = (_f32(sd[f"{name}.{br}.conv.weight"], dev) for br in heads)
+            (s1, b1), (s2, b2), (s3, b3) = (self.fold(f"{name}.{br}.conv", f"{name}.{br}.bn", self.EPS) for br in heads)
+            n1 = w1.shape[0]
             n_split = pack.round_up(n1, 64)
-            w1 = _f32(sd[f"{name}.branch1.conv.weight"], dev)
             padw = torch.zeros((n_split - n1,) + tuple(w1.shape[1:]))
             padv = torch.zeros(n_split - n1)
             self.w[f"{name}.head"] = dict(
-                w=pack.pack_conv_weight(torch.cat([w1, padw, wt], 0), 128),
-                scale=torch.cat([h1["scale"], padv, a["scale"], b["scale"]]),
-                bias=torch.cat([h1["bias"], padv, a["bias"], b["bias"]]),
-                N=n_split + wt.shape[0], Cin=wt.shape[1], R=1, BN=128, n1=n1, n_split=n_split)
+                w=pack.pack_conv_weight(torch.cat([w1, padw, w2, w3], 0), 128),
+                scale=torch.cat([s1, padv, s2, s3]), bias=torch.cat([b1, padv, b2, b3]),
+                N=n_split + w2.shape[0] + w3.shape[0], Cin=w1.shape[1], R=1, BN=128, n1=n1, n_split=n_split)
         self.w["fc"] = (_f32(sd["fc.weight"], dev), _f32(sd["fc.bias"], dev))
         self.ncls = self.w["fc"][0].shape[0]
 
@@ -615,18 +569,13 @@ class GoogLeNetRunner(_Builder):
         """u8: [B,224,224,3] uint8 crops (HWC, channel order as the reference's roi_rgb), or f32: float NCHW."""
         buf = self.buf
         c1 = buf(B, 112, 112, 64)
-        if CONV1_S2D:
-            # conv1 7x7 s2 as a TMA implicit GEMM: space-to-depth pack of the crop (to_tensor + _transform_input folded,
-            # padding materialised), then four row taps over overlapping [4 px x 16 ch] windows (K = 4 x 64)
-            Q = IMG // 2 + 3
-            q = buf(B, Q, Q, 16)
-            ops.append(E.S2dDesc(E.ptr(u8), E.ptr(f32), q.data_ptr(), B, IMG))
-            self.conv(ops, self.w["conv1_s2d"], View(q, 64, 0, 16), (B, 112, 112), View(c1),
-                      in_strides=(Q * 16, Q * Q * 16))
-        else:                                                        # im2col built in smem (stem_conv.cu)
-            w1 = self.w["conv1"]
-            ops.append(E.StemDesc(1, E.ptr(f32), E.ptr(u8), w1["w"].data_ptr(), w1["scale"].data_ptr(),
-                                  w1["bias"].data_ptr(), c1.data_ptr(), 64, B, IMG, IMG))
+        # conv1 7x7 s2 as a TMA implicit GEMM: space-to-depth pack of the crop (to_tensor + _transform_input folded,
+        # padding materialised), then four row taps over overlapping [4 px x 16 ch] windows (K = 4 x 64)
+        Q = IMG // 2 + 3
+        q = buf(B, Q, Q, 16)
+        ops.append(E.S2dDesc(E.ptr(u8), E.ptr(f32), q.data_ptr(), B, IMG))
+        self.conv(ops, self.w["conv1_s2d"], View(q, 64, 0, 16), (B, 112, 112), View(c1),
+                  in_strides=(Q * 16, Q * Q * 16))
         p1 = buf(B, 56, 56, 64)
         ops.append(E.PoolDesc(c1.data_ptr(), 64, p1.data_ptr(), 64, 64, B, 112, 112, 56, 56, 3, 2, 0))
         c2 = buf(B, 56, 56, 64)
@@ -646,27 +595,12 @@ class GoogLeNetRunner(_Builder):
             out = buf(B, sp, sp, cout)                               # torch.cat([b1,b2,b3,b4],1) target
             flat = (1, 1, B * sp * sp)
             geom = (B, sp, sp)
-            xin = View(cur)
-            if FUSE_HEAD:
-                r23 = buf(B, sp, sp, c3r + c5r)
-                hw = dict(self.w[name + ".head"])
-                # (one tile per CTA below ~300 pixel tiles: whole 64-column n-tiles on either side of n_split)
-                hw["BN"] = 128 if B * sp * sp >= 296 * 128 else 64
-                self.conv(ops, hw, xin, flat, View(out, c1x1, 0), out2=View(r23))
-                r2, r3 = View(r23, c3r, 0), View(r23, c5r, c3r)
-            else:
-                self.conv(ops, self.w[name + ".branch1"], xin, flat, View(out, c1x1, 0))
-            if FUSE_HEAD:
-                pass                                                 # (r2 / r3 come from the fused head GEMM)
-            elif FUSE_REDUCE:
-                r23 = buf(B, sp, sp, c3r + c5r)
-                self.conv(ops, self.w[name + ".reduce"], xin, flat, View(r23))
-                r2, r3 = View(r23, c3r, 0), View(r23, c5r, c3r)
-            else:
-                t2, t3 = buf(B, sp, sp, c3r), buf(B, sp, sp, c5r)
-                self.conv(ops, self.w[name + ".branch2.0"], xin, flat, View(t2))
-                self.conv(ops, self.w[name + ".branch3.0"], xin, flat, View(t3))
-                r2, r3 = View(t2), View(t3)
+            r23 = buf(B, sp, sp, c3r + c5r)
+            hw = dict(self.w[name + ".head"])
+            # (one tile per CTA below ~300 pixel tiles: whole 64-column n-tiles on either side of n_split)
+            hw["BN"] = 128 if B * sp * sp >= 296 * 128 else 64
+            self.conv(ops, hw, View(cur), flat, View(out, c1x1, 0), out2=View(r23))
+            r2, r3 = View(r23, c3r, 0), View(r23, c5r, c3r)
             self.conv(ops, self.w[name + ".branch2.1"], r2, geom, View(out, c3x3, c1x1))
             self.conv(ops, self.w[name + ".branch3.1"], r3, geom, View(out, c5x5, c1x1 + c3x3))
             pl = buf(B, sp, sp, cin)

@@ -3,15 +3,7 @@
 BN fold (SURVEY Appendix B): scale = gamma / sqrt(var + eps); bias' = beta + (b_conv - mean) * scale.
 Packed conv weight: [Npad][R*S*Cin_pad] bf16, K index = (r*S + s)*Cin_pad + c (see ug_conv_desc).
 """
-import os
-
 import torch
-
-# UG_BN_FIT=0: always 128-wide n-tiles for N >= 128 (the last tile of N = 144 ... 320 layers is then mostly padding)
-BN_FIT = os.environ.get("UG_BN_FIT", "1") != "0"
-# UG_BN_FIT3=1: single n-tiles of 144 ... 240 columns for 3x3 layers as well.  Supported by the kernel (tests) but measured
-# slower (GoogLeNet stage 2.358 -> 2.400 ms: one accumulator per issuer and a 3-4 slot weight ring), hence off.
-BN_FIT3 = os.environ.get("UG_BN_FIT3", "0") == "1"
 
 
 def round_up(x, m):
@@ -29,12 +21,11 @@ def choose_bn(n_out, convt_cout=None, r=1):
         return 256        # wide linear layers (qkv, FFN): persistent kernel with 256-wide n-tiles (measured)
     if n_out <= 128:
         return round_up(n_out, 16)
-    if n_out % 128 == 0 or not BN_FIT:
+    if n_out % 128 == 0 or r != 1:
+        # 3x3 layers keep 128-wide n-tiles: one fitted tile of 144 ... 240 columns (supported by the kernel, see
+        # ug_conv_desc.BN) measured slower (GoogLeNet stage 2.358 -> 2.400 ms: one accumulator per issuer and a 3-4
+        # slot weight ring)
         return 128
-    if r != 1:
-        # the 3x3 multi-issuer kernel stores 64-column boxes, so its n-tiles must be multiples of 64 when there are
-        # several of them (N = 288, 320 stay at 128); up to 256 columns fit ONE tile (GoogLeNet N = 192, 208, 224)
-        return round_up(n_out, 16) if (n_out < 256 and BN_FIT3) else 128
     # 1x1 layers whose width is not a multiple of 128 (GoogLeNet: 136 ... 240): pick the tile width that minimises
     # n_tiles * (MMA issue interval of an M=128 x BN MMA); the single-issuer GEMM kernels issue one MMA per ~110 cycles
     # up to N = 220, then N/2 (profiles/r01_mma_*.txt), BN <= 256.  Ties go to the least padding.
