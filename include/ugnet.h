@@ -8,7 +8,9 @@
  *   GoogLeNetClassifier.forward / torchvision GoogLeNet (分类/test.py:64-73)
  *   inference_all                                      (分类/test.py:74-96, 分割/predict.py:11-51)
  * The Python shells in unet-goolenet_b200/ keep those names and lower each forward into a list of the ops
- * declared here (a "program"), which the engine executes on one CUDA stream.  Every entry point:
+ * declared here (a "program"), which the engine executes on one CUDA stream.  Grad-CAM of the classifier at inception5b
+ * (pytorch-grad-cam's GradCAM on model.googlenet.inception5b) is one more op, ug_cam, which programs built with
+ * cam=True append after the head.  Every entry point:
  *   - takes raw device pointers and explicit shapes, never owns caller memory, never throws;
  *   - returns UG_OK (0) or a negative UG_E* code; the message is available via ug_last_error();
  *   - is asynchronous on the given stream (cudaStream_t passed as void*), except *_host helpers;
@@ -286,6 +288,31 @@ typedef struct ug_head_desc {
   int B, HW, C, ncls;
 } ug_head_desc;
 
+/* Grad-CAM at GoogLeNet's inception5b (pytorch-grad-cam's GradCAM(model, target_layers=[model.googlenet.inception5b])).
+ * torchvision's GoogLeNet ends in avgpool(h x w) -> flatten -> dropout (identity in eval) -> fc, so the gradient of
+ * logit c with respect to feat[y][x][k] is W[c][k] / (h*w) at every position: the Grad-CAM channel weights need no
+ * backward pass.  Per image i, one launch for the whole batch:
+ *   c = cls ? cls[i] : the first argmax of logits[i] (torch.argmax, 分类/test.py:86);
+ *   cam[i][y][x] = max(0, sum_k (W[c][k] / (h*w)) * feat[i][y*w+x][k])                              (fp32);
+ *   v = cam[i] - min(cam[i]);  v = v / (1e-7f + max(v))             (pytorch-grad-cam scale_cam_image, fp32);
+ *   cam_map[i] = 0 outside the box {x0,y0,x1,y1} (end-exclusive, ug_bbox output; NULL = the whole SxS frame), and
+ *                cv2.resize(v, (x1-x0, y1-y0), INTER_LINEAR) placed at (x0, y0) inside it (bit-exact against cv2 4.13).
+ * cls and boxes may come from outside the library (a plan image's host): an entry whose class is outside [0, ncls) or
+ * whose box is not 0 <= x0 < x1 <= S, 0 <= y0 < y1 <= S is rejected: cam[i] and cam_map[i] are zero, status[i] = 1
+ * (0 otherwise; status is optional), and nothing is read through that entry.  feat must be 16-byte aligned and C a
+ * multiple of 8; h, w <= 32, C <= 2048, S <= 1024. */
+typedef struct ug_cam_desc {
+  const void* feat;      /* bf16 NHWC [B][h*w][C]: the GoogLeNet inception5b output (h = w = 7, C = 1024) */
+  const float* fc_w;     /* fp32 [ncls][C] (the head's weight, unfolded) */
+  const float* logits;   /* fp32 [B][ncls]: class = first argmax (torch.argmax, test.py:86), used when cls is NULL */
+  const int* cls;        /* optional int32 [B]: explicit target class per image */
+  const int* boxes;      /* optional int32 [B][4] {x0,y0,x1,y1} (ug_bbox output, end-exclusive); NULL = the whole SxS frame */
+  int* status;           /* optional int32 [B]: 1 = entry rejected (class or box out of range), else 0 */
+  float* cam;            /* fp32 [B][h][w]: the Grad-CAM map, ReLU(sum_k W[c][k]/(h*w) * feat[..][k]) */
+  float* cam_map;        /* fp32 [B][S][S]: the map normalised and resized into the box, zero outside it */
+  int B, h, w, C, ncls, S;
+} ug_cam_desc;
+
 enum {
   UG_OP_CONV = 1,
   /* 2 and 10 were the stand-alone im2col packs of round 1 (replaced by UG_OP_STEM); the numbers stay retired */
@@ -302,7 +329,8 @@ enum {
   UG_OP_WAVELET = 14,
   UG_OP_S2D = 15,
   UG_OP_RESIZE_RAGGED = 16,
-  UG_OP_WAVELET_RAGGED = 17
+  UG_OP_WAVELET_RAGGED = 17,
+  UG_OP_CAM = 18
 };
 
 typedef struct ug_op {
@@ -324,6 +352,7 @@ typedef struct ug_op {
     ug_s2d_desc s2d;
     ug_resize_ragged_desc resize_ragged; /* both smaller than ug_conv_desc: sizeof(ug_op) is unchanged */
     ug_wavelet_ragged_desc wavelet_ragged;
+    ug_cam_desc cam; /* smaller than ug_conv_desc as well */
   } u;
 } ug_op;
 
@@ -350,6 +379,7 @@ int ug_wavelet(ug_handle h, const ug_wavelet_desc* d, void* stream);
 int ug_s2d_pack(ug_handle h, const ug_s2d_desc* d, void* stream);
 int ug_resize_ragged(ug_handle h, const ug_resize_ragged_desc* d, void* stream);
 int ug_wavelet_ragged(ug_handle h, const ug_wavelet_ragged_desc* d, void* stream);
+int ug_cam(ug_handle h, const ug_cam_desc* d, void* stream);
 size_t ug_wavelet_workspace_bytes(int B, int H, int W);
 size_t ug_wavelet_ragged_workspace_bytes(int B, long long capacity_px);
 
@@ -394,7 +424,9 @@ int ug_program_run_host_pipelined(ug_handle h, ug_program p, const ug_copy* h2d,
  * front-end), "logits" f32 [B,1,224,224], "mask" u8 [B,224,224], "boxes" i32 [B,4], "u8" u8 [B,224,224,3] (the ROI
  * crops), "cls_logits" f32 [B,6].  A ragged plan (export_plan(B, source="ragged", capacity=P)) takes packed sources
  * instead: "src_u8" u8 [P*3] (images back to back, HWC), "src_index" ug_ragged_image [B] and reports "src_status"
- * i32 [B] (1 = the table entry was rejected and the image's outputs are those of a zero input). */
+ * i32 [B] (1 = the table entry was rejected and the image's outputs are those of a zero input).  A plan exported with
+ * cam=True (export_plan(B, ..., cam=True)) also reports the Grad-CAM of each image's predicted class (ug_cam_desc):
+ * "cam" f32 [B,7,7] and "cam_map" f32 [B,224,224] (the map in the UNet input frame, inside the ROI box). */
 typedef struct ug_plan_s* ug_plan;
 /* Parses the image (host memory, may be freed afterwards), allocates ONE device arena for every buffer of the plan
  * (ug_plan_device_bytes), uploads the constants, relocates the op list and prepares the program. */

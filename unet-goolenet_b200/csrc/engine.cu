@@ -54,6 +54,7 @@ static int run_simple(ug_engine* h, const ug_op* op, cudaStream_t s) {
     case UG_OP_S2D: return launch_s2d_pack(h, &op->u.s2d, s);
     case UG_OP_RESIZE_RAGGED: return launch_resize_ragged(h, &op->u.resize_ragged, s);
     case UG_OP_WAVELET_RAGGED: return launch_wavelet_ragged(h, &op->u.wavelet_ragged, s);
+    case UG_OP_CAM: return launch_cam(h, &op->u.cam, s);
     default: return set_error(h, UG_EINVAL, "unknown op kind %d", op->kind);
   }
 }
@@ -137,6 +138,7 @@ UG_SIMPLE_ENTRY(ug_wavelet, ug_wavelet_desc, launch_wavelet)
 UG_SIMPLE_ENTRY(ug_s2d_pack, ug_s2d_desc, launch_s2d_pack)
 UG_SIMPLE_ENTRY(ug_resize_ragged, ug_resize_ragged_desc, launch_resize_ragged)
 UG_SIMPLE_ENTRY(ug_wavelet_ragged, ug_wavelet_ragged_desc, launch_wavelet_ragged)
+UG_SIMPLE_ENTRY(ug_cam, ug_cam_desc, launch_cam)
 
 int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out) {
   if (!h || !ops || n_ops <= 0 || !out) return UG_EINVAL;
@@ -164,7 +166,7 @@ int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out)
         delete p;
         return rc;
       }
-    } else if (po.kind < UG_OP_CONV || po.kind > UG_OP_WAVELET_RAGGED) {
+    } else if (po.kind < UG_OP_CONV || po.kind > UG_OP_CAM) {
       delete p;
       return set_error(h, UG_EINVAL, "op %d: unknown kind %d", i, po.kind);
     }

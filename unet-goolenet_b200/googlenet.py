@@ -74,3 +74,13 @@ class GoogLeNetClassifier(nn.Module):
         if self.training:
             raise RuntimeError("the ugnet engine is inference-only: call model.eval() (test.py:75)")
         return self.runner().forward(x)
+
+    def grad_cam(self, x, classes=None):
+        """Grad-CAM at `googlenet.inception5b`, the engine form of pytorch-grad-cam's
+        `GradCAM(model, target_layers=[model.googlenet.inception5b])(x, targets)` followed by its scale_cam_image:
+        x float [B,3,224,224] in [0,1] -> (cam_map f32 [B,224,224] in [0,1], cam f32 [B,7,7]), both in the crop frame.
+        classes: int [B] target classes, or None for each image's predicted class (argmax of the logits).
+        GoogLeNet's head is avgpool -> fc, so the Grad-CAM weights are fc.weight[c] / 49 and no backward pass runs."""
+        if self.training:
+            raise RuntimeError("the ugnet engine is inference-only: call model.eval() (test.py:75)")
+        return self.runner().grad_cam(x, classes)

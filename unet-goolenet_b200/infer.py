@@ -55,7 +55,7 @@ def inference_all_seg(model, test_loader, device, save_dir=None):
 
 
 @torch.no_grad()
-def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256):
+def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256, cam_dir=None):
     """The whole of 分类/test.py:122-134 + :74-96 on the device for a batch of grayscale images:
     cv2.imread(path, 0) output (uint8 [H, W]) -> wavelet_enhance -> resize 224 + to_tensor -> UNet -> mask -> bbox ->
     ROI crop/resize -> GoogLeNet -> argmax; returns the sorted "<name> <class>" records (and writes result.txt).
@@ -64,31 +64,46 @@ def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256
     list of uint8 [H, W] images of any sizes (2 <= H, W <= 8*224), as the reference reads a directory.  A list runs as
     ragged batches (util/ragged.py): per chunk of the pipeline, one copy of the packed gray bytes and one of the table,
     the wavelet step writing its RGB output straight into the plan's source buffer, then the program; batch_size is
-    not used (the pipeline's own chunking applies)."""
+    not used (the pipeline's own chunking applies).
+
+    cam_dir: also write, per image, `cam_dir/<name without extension>.png`: the Grad-CAM map of the predicted class at
+    GoogLeNet's inception5b in the 224x224 UNet input frame (inside the ROI box, 0 outside) as a grayscale PNG of
+    (cam_map * 255).astype(uint8), truncated as pytorch-grad-cam's show_cam_on_image does."""
     from .util.wavelet import wavelet_enhance_batch
     runner = getattr(pipeline, "runner", pipeline)
     if isinstance(gray_images, (list, tuple)):
-        records = _grade_ragged(runner, gray_images, filenames)
+        records = _grade_ragged(runner, gray_images, filenames, cam_dir)
         return _write_records(records, save_dir)
     g = torch.as_tensor(np.ascontiguousarray(gray_images) if isinstance(gray_images, np.ndarray) else gray_images)
     records = []
     for s in range(0, g.shape[0], batch_size):
         rgb = wavelet_enhance_batch(g[s:s + batch_size].to(runner.dev))      # [B,H,W,3] uint8, test.py:128-129
-        _, _, cls = runner(rgb)                                              # test.py:130-131 and :82-84
-        pred = torch.argmax(torch.softmax(cls, dim=1), dim=1).cpu().numpy()  # test.py:86
+        out = runner(rgb, return_cam=cam_dir is not None)                   # test.py:130-131 and :82-84
+        pred = torch.argmax(torch.softmax(out[2], dim=1), dim=1).cpu().numpy()  # test.py:86
         for i, name in enumerate(filenames[s:s + batch_size]):
             records.append(f"{name.replace('.png', '')} {int(pred[i])}")
+        if cam_dir is not None:
+            _write_cams(out[3], filenames[s:s + batch_size], cam_dir)
     return _write_records(records, save_dir)
 
 
-def _grade_ragged(runner, gray_images, filenames):
+def _write_cams(cam_map, names, cam_dir):
+    """Grayscale PNGs (cam_map * 255).astype(uint8), one per image, named after the image."""
+    from PIL import Image
+    os.makedirs(cam_dir, exist_ok=True)
+    u8 = (cam_map.cpu().numpy() * np.float32(255)).astype(np.uint8)
+    for m, name in zip(u8, names):
+        Image.fromarray(m, "L").save(os.path.join(cam_dir, os.path.splitext(os.path.basename(name))[0] + ".png"))
+
+
+def _grade_ragged(runner, gray_images, filenames, cam_dir=None):
     from .util import ragged
     from .util.wavelet import wavelet_ragged_into
     packed = ragged.pack(gray_images, 1, min_side=ragged.WAVELET_MIN_SIDE, max_side=ragged.MAX_RATIO * 224)
     records = []
     for s, c in runner._chunks(len(gray_images)):
         part = ragged.chunk(packed, s, s + c)
-        ws = runner.plan(c, source="ragged", capacity=part.n_px)
+        ws = runner.plan(c, source="ragged", capacity=part.n_px, cam=cam_dir is not None)
         gray = part.data.to(runner.dev, non_blocking=True)
         ws["src_index"].copy_(ragged.table_tensor(part.table))
         wavelet_ragged_into(gray, ws["src_index"], ws["src_u8"], c)         # test.py:128-129, into the plan's input
@@ -96,6 +111,8 @@ def _grade_ragged(runner, gray_images, filenames):
         pred = torch.argmax(torch.softmax(ws["cls_logits"], dim=1), dim=1).cpu().numpy()  # test.py:86
         for i, name in enumerate(filenames[s:s + c]):
             records.append(f"{name.replace('.png', '')} {int(pred[i])}")
+        if cam_dir is not None:
+            _write_cams(ws["cam_map"], filenames[s:s + c], cam_dir)
     return records
 
 

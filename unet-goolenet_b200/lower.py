@@ -6,6 +6,7 @@ lays out the NHWC bf16 activation workspace in HBM and emits the op descriptors 
   UNetTaskAligWeight.forward (basicUnet.py:406-437)      -> UNetRunner._emit_unet
   roi.py:22-49 (threshold, bbox, crop, quantise, resize) -> fused into the UNet tail + bbox/cropresize ops
   GoogLeNetClassifier.forward (test.py:64-73)            -> GoogLeNetRunner._emit_googlenet
+  Grad-CAM at inception5b (GoogLeNetClassifier.grad_cam) -> GoogLeNetRunner._emit_cam (programs built with cam=True)
   whole two-stage path                                   -> PipelineRunner
 
 Dead compute of the reference forward is skipped: the `x` output of the bottleneck (attention1, the first
@@ -612,7 +613,19 @@ class GoogLeNetRunner(_Builder):
         ops.append(E.HeadDesc(cur.data_ptr(), self.w["fc"][0].data_ptr(), self.w["fc"][1].data_ptr(),
                               ws["cls_logits"].data_ptr(), B, 49, 1024, self.ncls))
 
-    def plan(self, B, kind="f32"):
+    def _emit_cam(self, B, ws, ops, boxes=None):
+        """Grad-CAM of the predicted class at inception5b (ug_cam_desc), appended after the head: ws["cam"] f32 [B,7,7]
+        and ws["cam_map"] f32 [B,224,224], the map normalised and resized into `boxes` (int32 [B,4] of the 224x224
+        frame) or over the whole frame.  Both are fresh per call (outputs, never shared with another plan)."""
+        feat = ws["inception5b"]
+        ws["cam"] = self.buf(B, 7, 7, dtype=torch.float32)
+        ws["cam_map"] = self.buf(B, IMG, IMG, dtype=torch.float32)
+        ops.append(E.CamDesc(feat.data_ptr(), self.w["fc"][0].data_ptr(), ws["cls_logits"].data_ptr(), None,
+                             E.ptr(boxes), None, ws["cam"].data_ptr(), ws["cam_map"].data_ptr(), B, 7, 7,
+                             feat.shape[-1], self.ncls, IMG))
+
+    def plan(self, B, kind="f32", cam=False):
+        """Program for B crops (kind "u8": uint8 HWC, "f32": float NCHW); cam=True appends the Grad-CAM op."""
         def build():
             ws, ops = {}, []
             allocs = self.begin()
@@ -622,8 +635,10 @@ class GoogLeNetRunner(_Builder):
             else:
                 ws["in"] = self.buf(B, 3, IMG, IMG, dtype=torch.float32)
                 self._emit_googlenet(B, ws, ops, f32=ws["in"])
+            if cam:
+                self._emit_cam(B, ws, ops)
             return _finish(self.engine, ops, ws, allocs)
-        return self.plans.get_or_build((B, kind), build)
+        return self.plans.get_or_build((B, kind, "cam") if cam else (B, kind), build)
 
     def _run(self, x, kind):
         if x.device.type != "cuda":
@@ -636,6 +651,35 @@ class GoogLeNetRunner(_Builder):
             ws["program"].run()
             outs.append(ws["cls_logits"].clone())
         return torch.cat(outs) if len(outs) > 1 else outs[0]
+
+    @torch.no_grad()
+    def grad_cam(self, x, classes=None):
+        """x: float [B,3,224,224] in [0,1] -> (cam_map f32 [B,224,224], cam f32 [B,7,7]): Grad-CAM at inception5b in
+        the crop frame, for `classes` (int [B]) or, when None, the predicted class of each image."""
+        if x.device.type != "cuda":
+            raise RuntimeError("ugnet: input must be a CUDA tensor (no CPU path)")
+        if x.dim() != 4 or x.shape[1] != 3 or x.shape[2] != IMG or x.shape[3] != IMG:
+            raise ValueError(f"expected [B,3,{IMG},{IMG}] input, got {tuple(x.shape)}")
+        if classes is not None:
+            classes = torch.as_tensor(classes, device=x.device).to(torch.int32).reshape(-1)
+            if classes.numel() != x.shape[0]:
+                raise ValueError(f"expected {x.shape[0]} classes, got {classes.numel()}")
+            if bool(((classes < 0) | (classes >= self.ncls)).any()):
+                raise ValueError(f"classes must lie in [0, {self.ncls})")
+        maps, cams = [], []
+        for s in range(0, x.shape[0], self.max_batch):
+            xb = x[s:s + self.max_batch]
+            ws = self.plan(xb.shape[0], "f32", cam=True)
+            ws["in"].copy_(xb)
+            ws["program"].run()
+            if classes is not None:                              # the same op again, with explicit targets
+                d = E.CamDesc.from_buffer_copy(ws["program"].descs[-1])
+                cls = classes[s:s + xb.shape[0]].contiguous()
+                d.cls = cls.data_ptr()
+                self.engine.run_op(d)
+            maps.append(ws["cam_map"].clone())
+            cams.append(ws["cam"].clone())
+        return torch.cat(maps), torch.cat(cams)
 
     @torch.no_grad()
     def forward_u8(self, u8):
@@ -680,7 +724,7 @@ class PipelineRunner:
         for b in [m for m in self._gpools if m not in liveb]:
             del self._gpools[b]
 
-    def plan(self, B, source=None, slot=0, capacity=None):
+    def plan(self, B, source=None, slot=0, capacity=None, cam=False):
         """Program for a batch of B images; B must be <= micro_batch or a multiple of it.  With `source` =
         (Hs, Ws) the program starts with the device front-end (PIL-exact resize of uint8 HWC sources + to_tensor,
         util/data_utils.py) writing the UNet input, and `ws["src_u8"]` is the program's input buffer.
@@ -689,12 +733,16 @@ class PipelineRunner:
         `ws["src_index"]` their table (util/ragged.py); `ws["src_status"]` receives 1 for a rejected table entry.
         `slot` selects one of several programs of the same shape with their OWN input / output buffers (x_in, src_u8,
         logits, mask, boxes, u8) over the SAME activation workspaces: a host-fed serving loop alternates slots so that
-        the H2D copy of step i+1 lands in place while step i computes (Program.run_host_pipelined(direct=True))."""
+        the H2D copy of step i+1 lands in place while step i computes (Program.run_host_pipelined(direct=True)).
+        cam=True appends the Grad-CAM op (GoogLeNetRunner._emit_cam) after the classifier head: `ws["cam"]` f32
+        [B,7,7] and `ws["cam_map"]` f32 [B,224,224], the map placed in each image's ROI box of the UNet input frame."""
         if source == "ragged":
             capacity = ragged.capacity(capacity or 0)
             key = (B, slot, "ragged", capacity)
         else:
             key = (B, slot) if source is None else (B, slot) + tuple(source)
+        if cam:
+            key += ("cam",)
 
         def build():
             mb = min(B, self.micro_batch)
@@ -732,18 +780,21 @@ class PipelineRunner:
                 ws.setdefault("sub", []).append(sub)
             with self.gnet.sharing(gpool):
                 self.gnet._emit_googlenet(B, ws, ops, u8=ws["u8"])
+            if cam:
+                self.gnet._emit_cam(B, ws, ops, boxes=ws["boxes"])
             return _finish(self.engine, ops, ws, ua + ga + [v for v in ws.values() if isinstance(v, torch.Tensor)])
         return self.plans.get_or_build(key, build)
 
-    def export_plan(self, B, source=None, capacity=None):
+    def export_plan(self, B, source=None, capacity=None, cam=False):
         """The whole two-stage program for a batch of B images as a relocatable plan image (bytes): op list, device
         memory layout, BN-folded packed weights of both networks.  A host in any language runs it through the C ABI
         alone (ug_plan_load / ug_plan_copy_in / ug_plan_run / ug_plan_copy_out, include/ugnet.h; examples/run_plan.c).
-        source / capacity as for plan(); a ragged plan's inputs are "src_u8" and "src_index"."""
-        ws = self.plan(B, source=source, capacity=capacity)
+        source / capacity / cam as for plan(); a ragged plan's inputs are "src_u8" and "src_index", a cam plan also
+        reports "cam" and "cam_map"."""
+        ws = self.plan(B, source=source, capacity=capacity, cam=cam)
         prog = ws["program"]
         io = {k: ws[k] for k in ("x_in", "src_u8", "src_index", "src_status", "logits", "mask", "boxes", "u8",
-                                 "cls_logits") if k in ws}
+                                 "cls_logits", "cam", "cam_map") if k in ws}
         tensors = list(prog.keepalive) + list(io.values()) + [(self.unet.w_blob, True), (self.gnet.w_blob, True)]
         return E.export_plan(prog.descs, io, tensors)
 
@@ -758,21 +809,23 @@ class PipelineRunner:
             out.append((s, n - s))
         return out
 
-    def feed_ragged(self, part):
+    def feed_ragged(self, part, cam=False):
         """The ragged plan for one chunk (a ragged.Packed of HWC images, at most one plan's batch) with its packed
         sources and table copied in (one copy each)."""
-        ws = self.plan(len(part.table), source="ragged", capacity=part.n_px)
+        ws = self.plan(len(part.table), source="ragged", capacity=part.n_px, cam=cam)
         ws["src_u8"][:part.data.numel()].copy_(part.data, non_blocking=True)
         ws["src_index"].copy_(ragged.table_tensor(part.table))
         return ws
 
     @torch.no_grad()
-    def __call__(self, imgs, return_logits=False):
+    def __call__(self, imgs, return_logits=False, return_cam=False):
         """imgs: float [B,3,224,224] CUDA, or uint8 [B,Hs,Ws,3] CUDA source images of any size (resized on the
         device exactly as the reference's PIL transform does), or a list of uint8 [H,W,3] images of different sizes
         (CUDA tensors or numpy arrays, sides up to 8*224; one ragged batch, util/ragged.py) ->
-        (masks u8 [B,224,224], boxes i32 [B,4], cls_logits f32 [B,6])."""
-        masks, boxes, cls, seg = [], [], [], []
+        (masks u8 [B,224,224], boxes i32 [B,4], cls_logits f32 [B,6]), then the segmentation logits f32 [B,1,224,224]
+        if return_logits, then the Grad-CAM map of the predicted class f32 [B,224,224] (in [0,1] inside the ROI box,
+        0 outside; see plan(cam=True)) if return_cam."""
+        masks, boxes, cls, seg, cams = [], [], [], [], []
         packed = None
         if isinstance(imgs, (list, tuple)):
             packed = ragged.pack(imgs, 3, max_side=ragged.MAX_RATIO * IMG)
@@ -783,12 +836,13 @@ class PipelineRunner:
             raise ValueError(f"uint8 input must be HWC [B,H,W,3], got {tuple(imgs.shape)}")
         for s, c in self._chunks(n):
             if packed is not None:
-                ws = self.feed_ragged(ragged.chunk(packed, s, s + c))
+                part = ragged.chunk(packed, s, s + c)
+                ws = self.feed_ragged(part, cam=True) if return_cam else self.feed_ragged(part)
             elif from_u8:
-                ws = self.plan(c, source=(imgs.shape[1], imgs.shape[2]))
+                ws = self.plan(c, source=(imgs.shape[1], imgs.shape[2]), cam=return_cam)
                 ws["src_u8"].copy_(imgs[s:s + c])
             else:
-                ws = self.plan(c)
+                ws = self.plan(c, cam=return_cam)
                 ws["x_in"].copy_(imgs[s:s + c])
             ws["program"].run()
             masks.append(ws["mask"].clone())
@@ -796,5 +850,9 @@ class PipelineRunner:
             cls.append(ws["cls_logits"].clone())
             if return_logits:
                 seg.append(ws["logits"].clone())
+            if return_cam:
+                cams.append(ws["cam_map"].clone())
         out = (torch.cat(masks), torch.cat(boxes), torch.cat(cls))
-        return out + (torch.cat(seg),) if return_logits else out
+        if return_logits:
+            out += (torch.cat(seg),)
+        return out + (torch.cat(cams),) if return_cam else out
