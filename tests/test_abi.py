@@ -76,3 +76,36 @@ def test_product_package_never_touches_the_oracle_or_the_reference():
                 if re.search(pat, src, flags=re.M):
                     bad.append((rel, pat))
     assert not bad, bad
+
+
+def _dev_header_functions():
+    src = open(os.path.join(ROOT, "include", "ugnet_dev.h")).read()
+    src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
+    return sorted(set(re.findall(r"\b(ug_[a-z0-9_]+)\s*\(", src)))
+
+
+def test_dev_library_keeps_its_hooks_out_of_the_product_library():
+    lib, dev = E.load_library(), ctypes.CDLL(E.DEV_LIB_PATH)
+    assert sorted(E.DEV_SYMBOLS) == _dev_header_functions()
+    for name in E.DEV_SYMBOLS:
+        assert hasattr(dev, name), f"{name} declared in ugnet_dev.h but not exported by libugnet_dev.so"
+        assert not hasattr(lib, name), f"{name} leaked into the product library"
+    assert dev.ug_conv_launch_info(None, None, None) != 0
+
+
+def test_conv_instance_tables():
+    """ug_conv_instances (host only): 3 activations for each GEMM kernel, the multi kernel's table (both kinds, told
+    apart by `pair`, no row listed twice), the pair kernel's 3 epilogues."""
+    dev = ctypes.CDLL(E.DEV_LIB_PATH)
+    row = ctypes.c_int * 6
+    tables = []
+    for k in range(5):
+        n = dev.ug_conv_instances(k, None, 0)
+        rows = (row * n)()
+        assert dev.ug_conv_instances(k, rows, n) == n
+        tables.append([tuple(r) for r in rows])
+    assert dev.ug_conv_instances(5, None, 0) < 0
+    assert tables[0] == tables[1] == [(a, -1, -1, -1, -1, -1) for a in (E.ACT_NONE, E.ACT_RELU, E.ACT_GELU)]
+    assert tables[2] == tables[3] and len(set(tables[2])) == len(tables[2])
+    assert any(t[5] for t in tables[2]) and not all(t[5] for t in tables[2])
+    assert [t[2] for t in tables[4]] == [E.EPI_STORE, E.EPI_OUTC, E.EPI_GATE]

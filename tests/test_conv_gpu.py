@@ -138,10 +138,10 @@ CASES = [
     dict(B=1, H=1, W=392, Cin=512, N=512, R=1, mode=1, act=0),     # linear + residual
     dict(B=2, H=28, W=28, Cin=512, N=512, R=3, mode=2),            # CoordAtt3 gate combine
     dict(B=2, H=32, W=48, Cin=64, N=64, R=3, mode=3),              # fused outc + threshold
-    dict(B=1, H=16, W=16, Cin=64, N=64, R=3, tile=(16, 8, 1), stages=2),
-    dict(B=1, H=16, W=16, Cin=128, N=256, R=3, bn=256, stages=3),  # BN=256
-    dict(B=4, H=56, W=56, Cin=128, N=512, R=3, bn=256),            # BN=256, single staging buffer, many tiles
-    dict(B=8, H=28, W=28, Cin=64, N=64, R=3, mode=2, variant=2),   # persistent: gate combine, several tiles per CTA
+    dict(B=1, H=16, W=16, Cin=64, N=64, R=3, tile=(16, 8, 1), stages=2),  # multi-issuer kernel: tile / stages not used
+    dict(B=1, H=16, W=16, Cin=128, N=256, R=3, bn=256, stages=3),  # packed for BN=256, runs as CTA pairs with BN=128
+    dict(B=4, H=56, W=56, Cin=128, N=512, R=3, bn=256),            # packed for BN=256; CTA pairs, BN=128, two rounds
+    dict(B=8, H=28, W=28, Cin=64, N=64, R=3, mode=2, variant=2),   # persistent: gate combine, 28x4 tiles
     dict(B=3, H=14, W=14, Cin=256, N=208, R=3, out_extra=48, out_off=16, variant=2),   # persistent: ragged n-tile
     dict(B=1, H=224, W=224, Cin=64, N=64, R=3, variant=2),        # persistent: 392 tiles over 148 CTAs
     dict(B=2, H=32, W=48, Cin=64, N=64, R=3, mode=3, variant=2),   # persistent: fused outc
@@ -149,12 +149,12 @@ CASES = [
     dict(B=1, H=1, W=392, Cin=512, N=2048, R=1, act=2, variant=2),  # persistent: GELU
     # 3x3 multi-issuer kernel (one CTA per SM, two MMA issuers sharing the weights)
     dict(B=1, H=224, W=224, Cin=64, N=64, R=3, variant=5),        # weights resident, 392 tiles over 148 CTAs
-    dict(B=3, H=28, W=28, Cin=128, N=192, R=3, bn=192, variant=5, out_extra=64, out_off=32),  # one 192-wide n-tile
-    dict(B=2, H=14, W=14, Cin=96, N=208, R=3, bn=208, variant=5),   # one 208-wide n-tile (last store box clipped at N)
+    dict(B=3, H=28, W=28, Cin=128, N=192, R=3, bn=192, variant=5, out_extra=64, out_off=32),  # strips, BN=128: ragged 2nd n-tile
+    dict(B=2, H=14, W=14, Cin=96, N=208, R=3, bn=208, variant=5),   # BN=128: second n-tile 80 wide (store box clipped at N)
     dict(B=2, H=56, W=56, Cin=64, N=192, R=3, bn=192),              # auto -> multi-issuer with the fitted n-tile
     dict(B=3, H=16, W=8, Cin=64, N=64, R=3, variant=5),           # odd tile count: the second issuer idles once
     dict(B=2, H=28, W=28, Cin=128, N=256, R=3, variant=5),        # streamed weights, two n-tiles
-    dict(B=1, H=24, W=8, Cin=128, N=256, R=3, variant=5),         # streamed weights + odd tile count
+    dict(B=1, H=24, W=8, Cin=128, N=256, R=3, variant=5),         # streamed weights, 12-row tiles, one tile group per n-tile
     dict(B=2, H=56, W=56, Cin=256, N=128, R=3, mode=2, variant=5),   # gate combine
     dict(B=2, H=32, W=48, Cin=64, N=64, R=3, mode=3, variant=5),  # fused outc (no staging buffers)
     dict(B=2, H=14, W=14, Cin=24, N=64, R=3, in_extra=40, in_off=16, variant=5),
@@ -181,7 +181,7 @@ CASES = [
     dict(B=2, H=30, W=44, Cin=64, N=64, R=3, mode=2, variant=5),      # ragged tiles in both directions
     dict(B=5, H=16, W=8, Cin=64, N=64, R=3, mode=2, variant=5),       # odd tile count: one stream idles in the last round
     dict(B=37, H=32, W=32, Cin=64, N=64, R=3, mode=2, variant=5),     # many rounds per CTA: staging-buffer hand-over
-    # fused 2x2 max-pool side output (DownBlock): exact tiles, ragged width (28 = 3.5 tiles), streamed and resident weights
+    # fused 2x2 max-pool side output (DownBlock): CTA pairs on tiles and on strips, multi-issuer tiles with resident weights
     dict(B=2, H=112, W=112, Cin=128, N=128, R=3, pool=True),
     dict(B=3, H=28, W=28, Cin=256, N=512, R=3, pool=True, out_extra=64, out_off=32),
     dict(B=2, H=56, W=56, Cin=64, N=64, R=3, pool=True),
@@ -196,7 +196,7 @@ CASES = [
     dict(B=2, H=14, W=14, Cin=512, N=2048, R=1, up=2, act=0, variant=5),      # ConvTranspose 2x2 s2 (512 -> 512)
     dict(B=1, H=112, W=112, Cin=64, N=256, R=1, up=2, act=0, out_extra=64, variant=5),  # ConvT into a concat buffer
     dict(B=3, H=28, W=28, Cin=256, N=1024, R=1, up=2, act=0, out_extra=256, variant=5),  # ConvT, odd tile count
-    dict(B=70, H=14, W=14, Cin=480, N=192, R=1, variant=5),                   # several rounds, ragged channel chunk
+    dict(B=70, H=14, W=14, Cin=480, N=192, R=1, variant=5),                   # 140 tile groups, ragged channel chunk
     # CTA-pair kernel (conv_pair.cu, tcgen05.mma.cta_group::2): 3x3 ReLU layers with <= 64 output channels
     dict(B=1, H=224, W=224, Cin=64, N=64, R=3, variant=6),            # 448 tiles = 112 quads over 74 pairs
     dict(B=2, H=224, W=224, Cin=128, N=64, R=3, variant=6),           # two k-chunks (nConvs.0 of the last UpBlock)
@@ -205,14 +205,14 @@ CASES = [
     dict(B=2, H=32, W=48, Cin=64, N=64, R=3, mode=3, variant=6),      # fused outc + sigmoid + threshold
     dict(B=3, H=224, W=224, Cin=64, N=64, R=3, mode=3, variant=6),
     dict(B=2, H=56, W=56, Cin=64, N=64, R=3, pool=True, variant=6),   # fused 2x2 max-pool side output
-    dict(B=37, H=32, W=32, Cin=24, N=48, R=3, variant=6),             # many rounds per pair; ragged channels both sides
+    dict(B=37, H=32, W=32, Cin=24, N=48, R=3, variant=6),             # 74 tile groups; ragged channels both sides
     dict(B=2, H=112, W=112, Cin=192, N=64, R=3, variant=6),           # three k-chunks: one tile stream per CTA, 3 stages
     dict(B=3, H=112, W=112, Cin=256, N=64, R=3, variant=6),           # up2.nConvs.0: one stream, 2 stages, 144 KB of weights
-    dict(B=5, H=24, W=8, Cin=256, N=64, R=3, mode=3, variant=6),      # one stream + fused outc, odd tile count
+    dict(B=5, H=24, W=8, Cin=256, N=64, R=3, mode=3, variant=6),      # 12-row tiles leave room for two streams; 2 tiles past the end
     dict(B=2, H=224, W=224, Cin=64, N=64, R=3, mode=2, variant=6, in_extra=64, out_extra=64, out_off=64),   # up1.cca.conv2_e layout
     dict(B=2, H=30, W=44, Cin=64, N=64, R=3, mode=2, variant=6),      # GATE, ragged tiles in both directions
     dict(B=5, H=16, W=8, Cin=128, N=64, R=3, mode=2, variant=6),      # GATE, odd tile count (tiles past the end)
-    dict(B=37, H=32, W=32, Cin=64, N=48, R=3, mode=2, variant=6),     # GATE, many rounds: staging-buffer hand-over; N < 64
+    dict(B=37, H=32, W=32, Cin=64, N=48, R=3, mode=2, variant=6),     # GATE, 74 tile groups: staging-buffer hand-over; N < 64
     # CTA pairs on the multi-issuer kernel (variant 7): 128-column n-tiles, each CTA streams half of every weight tile
     dict(B=2, H=112, W=112, Cin=128, N=128, R=3, variant=7),          # 8-pixel-wide tiles, TH = 16, streamed weights
     dict(B=3, H=56, W=56, Cin=256, N=256, R=3, variant=7),            # two n-tiles
@@ -220,12 +220,12 @@ CASES = [
     dict(B=5, H=28, W=28, Cin=1024, N=256, R=3, variant=7),           # 16 k-chunks, odd tile count (tiles past the end)
     dict(B=2, H=112, W=112, Cin=64, N=128, R=3, variant=7, pool=True),   # resident weight halves + fused 2x2 max-pool
     dict(B=3, H=28, W=28, Cin=256, N=512, R=3, pool=True, out_extra=64, out_off=32, variant=7),   # strips + pool from the staged tile
-    dict(B=2, H=56, W=56, Cin=256, N=128, R=3, mode=2, variant=7),    # CoordAtt3 combine (register-prefetched residual)
+    dict(B=2, H=56, W=56, Cin=256, N=128, R=3, mode=2, variant=7),    # CoordAtt3 combine (TMA-loaded residual sub-tiles)
     dict(B=3, H=28, W=28, Cin=512, N=512, R=3, mode=2, variant=7),    # combine on strips, four n-tiles
     dict(B=5, H=14, W=14, Cin=512, N=512, R=3, variant=7),            # 14x14: two tiles per image, 10 tiles = 3 groups
-    dict(B=37, H=30, W=20, Cin=128, N=128, R=3, variant=7, in_extra=64, in_off=64),   # ragged both ways, many rounds
+    dict(B=37, H=30, W=20, Cin=128, N=128, R=3, variant=7, in_extra=64, in_off=64),   # ragged both ways, tiles past the end
     dict(B=2, H=112, W=112, Cin=128, N=128, R=3, mode=2, variant=7),  # combine, residual sub-tiles by TMA (two per tile)
-    dict(B=37, H=20, W=16, Cin=128, N=256, R=3, mode=2, variant=7),   # combine: many rounds (staging-buffer hand-over), ragged tiles
+    dict(B=37, H=20, W=16, Cin=128, N=256, R=3, mode=2, variant=7),   # combine on strips (16x7), ragged last strip
     dict(B=5, H=14, W=14, Cin=256, N=192, R=3, bn=128, mode=2, variant=7),   # combine with a ragged last n-tile (one sub-tile)
     dict(B=3, H=56, W=56, Cin=64, N=192, R=3, bn=128, variant=7),     # GoogLeNet conv3: ragged second n-tile (64 of 128 columns)
     dict(B=5, H=14, W=14, Cin=160, N=320, R=3, variant=7),            # three n-tiles, last one half full; ragged k-chunk

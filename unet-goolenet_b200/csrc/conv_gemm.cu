@@ -739,6 +739,8 @@ int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   p.tma_store = tma_store; p.obufs = obufs; p.npad = npad; p.stage_copy = stage_copy;
   p.out2 = d->out2; p.out2_cstride = d->out2_cstride; p.n_split = split ? d->n_split : 0; p.n1 = d->n1;
   L->kernel = persistent ? ConvKernel::Persistent : ConvKernel::OneTile;
+  L->instance = d->act;   // conv_gemm_kernel / conv_gemm_persistent_kernel<UG_ACT_NONE, RELU, GELU>
+  L->item_tiles = 1;
   L->block = kThreads;
   if (persistent) {
     int tcols = 32;

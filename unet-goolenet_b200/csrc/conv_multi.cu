@@ -809,30 +809,14 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
 // ------------------------------------------------------------------------------------------ host side
 void choose_tile(int B, int H, int W, int* TW, int* TH, int* TN);  // conv_gemm.cu
 
-// The instantiated (activation, taps, epilogue mode, K-split, TMA residual, CTA pair) combinations; conv_multi_prepare
-// admits exactly these.
+// The instantiated (activation, taps, epilogue mode, K-split, TMA residual, CTA pair) combinations (UG_MULTI_INSTANCES,
+// engine.h); conv_multi_prepare admits exactly these.
 struct MultiInstance {
   int act, taps, mode, ks, rt, pair;
   MultiKernelFn fn;
 };
 #define UG_MULTI_CASE(A, T, M, K, RT, P) {A, T, M, K, RT, P, conv_multi_kernel<A, T, M, K, RT, P>},
-static const MultiInstance kMultiInstances[] = {
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_STORE, 1, 0, 0)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_STORE, 2, 0, 0)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_ADD, 1, 0, 0)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 1, 0, 0)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 2, 0, 0)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 2, 1, 0)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_OUTC, 1, 0, 0)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_OUTC, 2, 0, 0)
-    UG_MULTI_CASE(UG_ACT_NONE, 1, UG_EPI_STORE, 1, 0, 0)
-    UG_MULTI_CASE(UG_ACT_RELU, 1, UG_EPI_STORE, 1, 0, 0)
-    UG_MULTI_CASE(UG_ACT_GELU, 1, UG_EPI_STORE, 1, 0, 0)
-    UG_MULTI_CASE(UG_ACT_NONE, 1, UG_EPI_ADD, 1, 0, 0)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_STORE, 1, 0, 1)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 1, 0, 1)
-    UG_MULTI_CASE(UG_ACT_RELU, 9, UG_EPI_GATE, 1, 1, 1)
-};
+static const MultiInstance kMultiInstances[] = {UG_MULTI_INSTANCES(UG_MULTI_CASE)};
 #undef UG_MULTI_CASE
 
 // Fills L for the multi-issuer kernel: 3x3 pad-1 convolutions (halo tiles) and 1x1 convolutions / linear layers /
@@ -1015,8 +999,14 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
   hp.debug = d->stages >= 100 ? d->stages - 100 : 0;  // profiling ablations (scripts/conv_prof.py)
   L->kernel = pair ? ConvKernel::MultiPair : ConvKernel::Multi;
   L->multi_fn = nullptr;
-  for (const MultiInstance& k : kMultiInstances)
-    if (k.act == d->act && k.taps == taps && k.mode == d->mode && k.ks == ks && k.rt == rt && k.pair == pair) L->multi_fn = k.fn;
+  for (int i = 0; i < (int)(sizeof(kMultiInstances) / sizeof(kMultiInstances[0])); ++i) {
+    const MultiInstance& k = kMultiInstances[i];
+    if (k.act == d->act && k.taps == taps && k.mode == d->mode && k.ks == ks && k.rt == rt && k.pair == pair) {
+      L->multi_fn = k.fn;
+      L->instance = i;
+    }
+  }
+  L->item_tiles = kMI * (pair ? 2 : 1);
   if (!L->multi_fn) return set_error(h, UG_EUNSUPPORTED, "conv(multi): no kernel instantiated for this layer");
   L->block = kMultiThreads(ks, rt && pair);
 

@@ -386,6 +386,15 @@ __global__ void __launch_bounds__(kPThreads, 1) conv_pair_kernel(const __grid_co
 
 // ------------------------------------------------------------------------------------------ host side
 
+// The instantiated (epilogue mode, TMA residual) forms (UG_PAIR_INSTANCES, engine.h).
+struct PairInstance {
+  int mode, rt;
+  PairKernelFn fn;
+};
+#define UG_PAIR_CASE(M, RT) {M, RT, conv_pair_kernel<M, RT>},
+static const PairInstance kPairInstances[] = {UG_PAIR_INSTANCES(UG_PAIR_CASE)};
+#undef UG_PAIR_CASE
+
 // Fills L for the CTA-pair kernel.  UG_EUNSUPPORTED when the layer is not one it takes (the caller falls back to
 // conv_multi_prepare): 3x3 pad 1, ReLU, <= 64 output channels in one 64-column n-tile, STORE (optionally with the fused
 // 2x2 pool), OUTC or GATE epilogue, weights resident at 36 KB per 64 input channels per CTA, an even number of SMs.
@@ -453,9 +462,13 @@ int conv_pair_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   hp.d_tx = make_fastdiv(p.tiles_x);
   hp.d_ty = make_fastdiv(p.tiles_y);
   L->kernel = ConvKernel::Pair;
-  L->pair_fn = d->mode == UG_EPI_OUTC ? conv_pair_kernel<UG_EPI_OUTC, 0>
-               : gate                 ? conv_pair_kernel<UG_EPI_GATE, 1>
-                                      : conv_pair_kernel<UG_EPI_STORE, 0>;
+  L->pair_fn = nullptr;
+  for (int i = 0; i < (int)(sizeof(kPairInstances) / sizeof(kPairInstances[0])); ++i)
+    if (kPairInstances[i].mode == d->mode) {
+      L->pair_fn = kPairInstances[i].fn;
+      L->instance = i;
+    }
+  L->item_tiles = 2 * streams;
   L->block = kPThreads;
 
   {
@@ -524,8 +537,8 @@ int max_cluster_pairs(ug_engine* h) {
 
 int conv_pair_launch(ug_engine* h, const ConvLaunch* L, cudaStream_t s) {
   if (!h->attr_pair) {
-    for (PairKernelFn fn : {conv_pair_kernel<UG_EPI_STORE, 0>, conv_pair_kernel<UG_EPI_OUTC, 0>, conv_pair_kernel<UG_EPI_GATE, 1>}) {
-      const cudaError_t e = cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    for (const PairInstance& k : kPairInstances) {
+      const cudaError_t e = cudaFuncSetAttribute((const void*)k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
       if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(conv_pair_kernel)");
     }
     h->attr_pair = true;

@@ -145,6 +145,27 @@ enum class ConvKernel {
 typedef void (*MultiKernelFn)(CUtensorMap, CUtensorMap, StoreMaps, ConvKParams, MultiParams);
 typedef void (*PairKernelFn)(CUtensorMap, CUtensorMap, PairMaps, ConvKParams, PairParams);
 
+// The instantiated conv_multi_kernel<activation, taps, epilogue mode, K-split, TMA residual, CTA pair> combinations and
+// conv_pair_kernel<epilogue mode, TMA residual> forms, in table order: conv_multi.cu / conv_pair.cu build their kernel
+// tables from these lists (prepare admits exactly these), and the launch-plan query of libugnet_dev.so enumerates them.
+#define UG_MULTI_INSTANCES(X)                   \
+  X(UG_ACT_RELU, 9, UG_EPI_STORE, 1, 0, 0)      \
+  X(UG_ACT_RELU, 9, UG_EPI_STORE, 2, 0, 0)      \
+  X(UG_ACT_RELU, 9, UG_EPI_ADD, 1, 0, 0)        \
+  X(UG_ACT_RELU, 9, UG_EPI_GATE, 1, 0, 0)       \
+  X(UG_ACT_RELU, 9, UG_EPI_GATE, 2, 0, 0)       \
+  X(UG_ACT_RELU, 9, UG_EPI_GATE, 2, 1, 0)       \
+  X(UG_ACT_RELU, 9, UG_EPI_OUTC, 1, 0, 0)       \
+  X(UG_ACT_RELU, 9, UG_EPI_OUTC, 2, 0, 0)       \
+  X(UG_ACT_NONE, 1, UG_EPI_STORE, 1, 0, 0)      \
+  X(UG_ACT_RELU, 1, UG_EPI_STORE, 1, 0, 0)      \
+  X(UG_ACT_GELU, 1, UG_EPI_STORE, 1, 0, 0)      \
+  X(UG_ACT_NONE, 1, UG_EPI_ADD, 1, 0, 0)        \
+  X(UG_ACT_RELU, 9, UG_EPI_STORE, 1, 0, 1)      \
+  X(UG_ACT_RELU, 9, UG_EPI_GATE, 1, 0, 1)       \
+  X(UG_ACT_RELU, 9, UG_EPI_GATE, 1, 1, 1)
+#define UG_PAIR_INSTANCES(X) X(UG_EPI_STORE, 0) X(UG_EPI_OUTC, 0) X(UG_EPI_GATE, 1)
+
 // A fully prepared launch of one of the conv kernels: the prepare functions fill the kernel's parameter blocks and
 // tensor maps, the launch functions only launch.
 struct ConvLaunch {
@@ -160,6 +181,8 @@ struct ConvLaunch {
   ConvKernel kernel;
   MultiKernelFn multi_fn;        // the conv_multi_kernel instantiation (activation, taps, epilogue, K-split, ...)
   PairKernelFn pair_fn;          // the conv_pair_kernel instantiation (epilogue)
+  int instance;                  // row of UG_MULTI_INSTANCES (Multi, MultiPair) / UG_PAIR_INSTANCES (Pair); 0 otherwise
+  int item_tiles;                // pixel tiles per work item: kMI (Multi), 2 kMI (MultiPair), 2 streams (Pair), 1 (GEMM)
   dim3 grid;
   unsigned block;
   size_t smem;
