@@ -10,7 +10,8 @@
  * The Python shells in unet-goolenet_b200/ keep those names and lower each forward into a list of the ops
  * declared here (a "program"), which the engine executes on one CUDA stream.  Grad-CAM of the classifier at inception5b
  * (pytorch-grad-cam's GradCAM on model.googlenet.inception5b) is one more op, ug_cam, which programs built with
- * cam=True append after the head.  Every entry point:
+ * cam=True append after the head; ug_source_frame, which programs built with source_frame=True append last, carries the
+ * mask, the box and the map to each source image's own size.  Every entry point:
  *   - takes raw device pointers and explicit shapes, never owns caller memory, never throws;
  *   - returns UG_OK (0) or a negative UG_E* code; the message is available via ug_last_error();
  *   - is asynchronous on the given stream (cudaStream_t passed as void*), except *_host helpers;
@@ -313,6 +314,35 @@ typedef struct ug_cam_desc {
   int B, h, w, C, ncls, S;
 } ug_cam_desc;
 
+/* Source-frame outputs of a pipeline program: each image's mask, ROI box and Grad-CAM map at the image's own size H x W
+ * instead of the S x S UNet input frame (S = 224), as a user draws them on the image they read.  Image i is H x W =
+ * index[i].H x index[i].W at pixel offset index[i].px_offset (a ragged batch) or Hs x Ws at pixel offset i*Hs*Ws
+ * (index NULL).  Per image, one launch for the whole batch:
+ *   L = cv2.resize(logits[i], (W, H), INTER_LINEAR) in fp32 (cv2 4.13's scale = in / out, bit-exact);
+ *   mask[px + y*W + x] = 1.0f / (1.0f + expf(-L[y][x])) > 0.5f   (the fp32 threshold of the UNet's outc epilogue);
+ *   src_boxes[i] = {floor(x0*W/S), floor(y0*H/S), ceil(x1*W/S), ceil(y1*H/S)} for boxes[i] = {x0,y0,x1,y1} (64-bit
+ *                  integers): the smallest source-pixel box covering the S-frame box;
+ *   with cam: v = cam[i] - min(cam[i]);  v = v / (1e-7f + max(v)) (as ug_cam), and cam_map = cv2.resize(v, (X1-X0,
+ *             Y1-Y0), INTER_LINEAR) placed at (X0, Y0) of the source box, zero outside it.
+ * When H = W = S the outputs equal the S-frame ones bit for bit (mask, boxes, and ug_cam's cam_map).  The table and the
+ * boxes may come from outside the library (a plan image's host): an entry with a negative offset, a side outside
+ * [1, 8*S], an extent past capacity_px, or a box that is not 0 <= x0 < x1 <= S, 0 <= y0 < y1 <= S is rejected: nothing
+ * is read or written through it, src_boxes[i] = {0,0,0,0} and status[i] = 1 (0 otherwise; status is optional).  The
+ * launch geometry depends on B, S and Hs only, never on the table.  logits must be 16-byte aligned, S a multiple of 4
+ * and at most 256, h, w <= 32. */
+typedef struct ug_source_frame_desc {
+  const float* logits;             /* fp32 [B][S][S]: the UNet's segmentation logits (outc output) */
+  const int* boxes;                /* int32 [B][4] {x0,y0,x1,y1}, end-exclusive (ug_bbox output) */
+  const float* cam;                /* optional fp32 [B][h][w]: ug_cam's raw map; NULL = no CAM map */
+  const ug_ragged_image* index;    /* optional device table [B]; NULL = every image is Hs x Ws */
+  int* status;                     /* optional int32 [B]: 1 = entry rejected, else 0 */
+  unsigned char* mask;             /* u8: image i at mask + px_offset (ragged) or mask + i*Hs*Ws, H*W bytes */
+  int* src_boxes;                  /* int32 [B][4]: the box in source pixels, end-exclusive */
+  float* cam_map;                  /* fp32, placed like mask; required iff cam is set */
+  long long capacity_px;           /* ragged: pixels of mask (and cam_map); unused when index is NULL */
+  int B, S, Hs, Ws, h, w;
+} ug_source_frame_desc;
+
 enum {
   UG_OP_CONV = 1,
   /* 2 and 10 were the stand-alone im2col packs of round 1 (replaced by UG_OP_STEM); the numbers stay retired */
@@ -330,7 +360,8 @@ enum {
   UG_OP_S2D = 15,
   UG_OP_RESIZE_RAGGED = 16,
   UG_OP_WAVELET_RAGGED = 17,
-  UG_OP_CAM = 18
+  UG_OP_CAM = 18,
+  UG_OP_SOURCE_FRAME = 19
 };
 
 typedef struct ug_op {
@@ -353,6 +384,7 @@ typedef struct ug_op {
     ug_resize_ragged_desc resize_ragged; /* both smaller than ug_conv_desc: sizeof(ug_op) is unchanged */
     ug_wavelet_ragged_desc wavelet_ragged;
     ug_cam_desc cam; /* smaller than ug_conv_desc as well */
+    ug_source_frame_desc source_frame; /* and so is this one */
   } u;
 } ug_op;
 
@@ -380,6 +412,7 @@ int ug_s2d_pack(ug_handle h, const ug_s2d_desc* d, void* stream);
 int ug_resize_ragged(ug_handle h, const ug_resize_ragged_desc* d, void* stream);
 int ug_wavelet_ragged(ug_handle h, const ug_wavelet_ragged_desc* d, void* stream);
 int ug_cam(ug_handle h, const ug_cam_desc* d, void* stream);
+int ug_source_frame(ug_handle h, const ug_source_frame_desc* d, void* stream);
 size_t ug_wavelet_workspace_bytes(int B, int H, int W);
 size_t ug_wavelet_ragged_workspace_bytes(int B, long long capacity_px);
 
@@ -426,7 +459,10 @@ int ug_program_run_host_pipelined(ug_handle h, ug_program p, const ug_copy* h2d,
  * instead: "src_u8" u8 [P*3] (images back to back, HWC), "src_index" ug_ragged_image [B] and reports "src_status"
  * i32 [B] (1 = the table entry was rejected and the image's outputs are those of a zero input).  A plan exported with
  * cam=True (export_plan(B, ..., cam=True)) also reports the Grad-CAM of each image's predicted class (ug_cam_desc):
- * "cam" f32 [B,7,7] and "cam_map" f32 [B,224,224] (the map in the UNet input frame, inside the ROI box). */
+ * "cam" f32 [B,7,7] and "cam_map" f32 [B,224,224] (the map in the UNet input frame, inside the ROI box).  A plan
+ * exported with source_frame=True (a plan with a uint8 or ragged source) also reports the outputs at each image's own
+ * size (ug_source_frame_desc): "src_mask" u8 [B,Hs,Ws] (ragged: [P], image i at px_offset), "src_boxes" i32 [B,4]
+ * and, with cam=True, "src_cam_map" f32 [B,Hs,Ws] (ragged: [P]). */
 typedef struct ug_plan_s* ug_plan;
 /* Parses the image (host memory, may be freed afterwards), allocates ONE device arena for every buffer of the plan
  * (ug_plan_device_bytes), uploads the constants, relocates the op list and prepares the program. */

@@ -7,6 +7,7 @@
 // cam_map write (S*S*4 bytes per image), so the recomputation costs L2 reads only.
 #include <cfloat>
 #include <cstdint>
+#include "cam_scale.cuh"
 #include "common.cuh"
 #include "cv_resize.cuh"
 #include "engine.h"
@@ -101,23 +102,8 @@ __global__ void __launch_bounds__(kCamThreads) cam_kernel(ug_cam_desc d) {
   }
   __syncthreads();
 
-  // scale_cam_image: v = cam - min(cam); v = v / (1e-7f + max(v))   (fp32; min / max are exact in any order)
-  if (warp == 0) {
-    float mn = FLT_MAX;
-    for (int p = lane; p < hw; p += 32) mn = fminf(mn, v[p]);
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
-    float mx = 0.0f;
-    for (int p = lane; p < hw; p += 32) mx = fmaxf(mx, __fsub_rn(v[p], mn));
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-    const float den = __fadd_rn(1e-7f, mx);
-    for (int p = lane; p < hw; p += 32) {
-      const float cam = v[p];
-      if (blockIdx.y == 0) d.cam[(long long)i * hw + p] = cam;
-      v[p] = __fdiv_rn(__fsub_rn(cam, mn), den);
-    }
-  }
+  // scale_cam_image (band 0 also stores the raw cam)
+  if (warp == 0) cam_scale_warp(v, hw, lane, blockIdx.y == 0 ? d.cam + (long long)i * hw : nullptr);
   __syncthreads();
 
   // this band of cam_map: cv2.resize(v, (bw, bh), INTER_LINEAR) at (x0, y0), zero elsewhere

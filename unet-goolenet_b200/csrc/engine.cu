@@ -55,6 +55,7 @@ static int run_simple(ug_engine* h, const ug_op* op, cudaStream_t s) {
     case UG_OP_RESIZE_RAGGED: return launch_resize_ragged(h, &op->u.resize_ragged, s);
     case UG_OP_WAVELET_RAGGED: return launch_wavelet_ragged(h, &op->u.wavelet_ragged, s);
     case UG_OP_CAM: return launch_cam(h, &op->u.cam, s);
+    case UG_OP_SOURCE_FRAME: return launch_source_frame(h, &op->u.source_frame, s);
     default: return set_error(h, UG_EINVAL, "unknown op kind %d", op->kind);
   }
 }
@@ -139,6 +140,7 @@ UG_SIMPLE_ENTRY(ug_s2d_pack, ug_s2d_desc, launch_s2d_pack)
 UG_SIMPLE_ENTRY(ug_resize_ragged, ug_resize_ragged_desc, launch_resize_ragged)
 UG_SIMPLE_ENTRY(ug_wavelet_ragged, ug_wavelet_ragged_desc, launch_wavelet_ragged)
 UG_SIMPLE_ENTRY(ug_cam, ug_cam_desc, launch_cam)
+UG_SIMPLE_ENTRY(ug_source_frame, ug_source_frame_desc, launch_source_frame)
 
 int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out) {
   if (!h || !ops || n_ops <= 0 || !out) return UG_EINVAL;
@@ -166,7 +168,7 @@ int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out)
         delete p;
         return rc;
       }
-    } else if (po.kind < UG_OP_CONV || po.kind > UG_OP_CAM) {
+    } else if (po.kind < UG_OP_CONV || po.kind > UG_OP_SOURCE_FRAME) {
       delete p;
       return set_error(h, UG_EINVAL, "op %d: unknown kind %d", i, po.kind);
     }

@@ -299,5 +299,6 @@ int launch_s2d_pack(ug_engine* h, const ug_s2d_desc* d, cudaStream_t s);
 int launch_resize_ragged(ug_engine* h, const ug_resize_ragged_desc* d, cudaStream_t s);
 int launch_wavelet_ragged(ug_engine* h, const ug_wavelet_ragged_desc* d, cudaStream_t s);
 int launch_cam(ug_engine* h, const ug_cam_desc* d, cudaStream_t s);
+int launch_source_frame(ug_engine* h, const ug_source_frame_desc* d, cudaStream_t s);
 
 }  // namespace ug

@@ -7,12 +7,14 @@ lays out the NHWC bf16 activation workspace in HBM and emits the op descriptors 
   roi.py:22-49 (threshold, bbox, crop, quantise, resize) -> fused into the UNet tail + bbox/cropresize ops
   GoogLeNetClassifier.forward (test.py:64-73)            -> GoogLeNetRunner._emit_googlenet
   Grad-CAM at inception5b (GoogLeNetClassifier.grad_cam) -> GoogLeNetRunner._emit_cam (programs built with cam=True)
+  outputs at each source image's own size               -> PipelineRunner._emit_source_frame (source_frame=True)
   whole two-stage path                                   -> PipelineRunner
 
 Dead compute of the reference forward is skipped: the `x` output of the bottleneck (attention1, the first
 cross_attention_cl call, x_mlp_norm, x_feed) feeds only a discarded result (basicUnet.py:418).
 """
 import os
+from typing import NamedTuple, Optional
 
 import torch
 
@@ -21,6 +23,15 @@ from . import pack
 from .util import ragged
 
 IMG = 224
+
+
+class SourceFrame(NamedTuple):
+    """Per-image outputs at each source image's own size H x W (PipelineRunner.__call__(..., return_source=True)):
+    masks u8 [B,H,W] (a list of [H_i,W_i] for a list of images), boxes i32 [B,4] (x0,y0,x1,y1 in source pixels,
+    end-exclusive) and the Grad-CAM maps f32 placed like the masks, or None without return_cam."""
+    masks: object
+    boxes: torch.Tensor
+    cam_maps: Optional[object]
 
 
 # Plans (program + activation workspace) kept per runner: a loader with ragged / varying batch sizes would otherwise
@@ -724,7 +735,7 @@ class PipelineRunner:
         for b in [m for m in self._gpools if m not in liveb]:
             del self._gpools[b]
 
-    def plan(self, B, source=None, slot=0, capacity=None, cam=False):
+    def plan(self, B, source=None, slot=0, capacity=None, cam=False, source_frame=False):
         """Program for a batch of B images; B must be <= micro_batch or a multiple of it.  With `source` =
         (Hs, Ws) the program starts with the device front-end (PIL-exact resize of uint8 HWC sources + to_tensor,
         util/data_utils.py) writing the UNet input, and `ws["src_u8"]` is the program's input buffer.
@@ -735,7 +746,11 @@ class PipelineRunner:
         logits, mask, boxes, u8) over the SAME activation workspaces: a host-fed serving loop alternates slots so that
         the H2D copy of step i+1 lands in place while step i computes (Program.run_host_pipelined(direct=True)).
         cam=True appends the Grad-CAM op (GoogLeNetRunner._emit_cam) after the classifier head: `ws["cam"]` f32
-        [B,7,7] and `ws["cam_map"]` f32 [B,224,224], the map placed in each image's ROI box of the UNet input frame."""
+        [B,7,7] and `ws["cam_map"]` f32 [B,224,224], the map placed in each image's ROI box of the UNet input frame.
+        source_frame=True appends, last, the op that carries the outputs to each source image's own size
+        (_emit_source_frame); it needs a `source`."""
+        if source_frame and source is None:
+            raise ValueError("source_frame=True needs uint8 or ragged sources: float input has no source frame")
         if source == "ragged":
             capacity = ragged.capacity(capacity or 0)
             key = (B, slot, "ragged", capacity)
@@ -743,6 +758,8 @@ class PipelineRunner:
             key = (B, slot) if source is None else (B, slot) + tuple(source)
         if cam:
             key += ("cam",)
+        if source_frame:
+            key += ("source_frame",)
 
         def build():
             mb = min(B, self.micro_batch)
@@ -782,19 +799,40 @@ class PipelineRunner:
                 self.gnet._emit_googlenet(B, ws, ops, u8=ws["u8"])
             if cam:
                 self.gnet._emit_cam(B, ws, ops, boxes=ws["boxes"])
+            if source_frame:
+                self._emit_source_frame(B, source, capacity, ws, ops)
             return _finish(self.engine, ops, ws, ua + ga + [v for v in ws.values() if isinstance(v, torch.Tensor)])
         return self.plans.get_or_build(key, build)
 
-    def export_plan(self, B, source=None, capacity=None, cam=False):
+    def _emit_source_frame(self, B, source, capacity, ws, ops):
+        """ug_source_frame_desc over the plan's logits, boxes and (cam plans) raw cam: ws["src_mask"] u8 and
+        ws["src_cam_map"] f32, each [capacity] (ragged: image i at its px_offset) or [B,Hs,Ws], and ws["src_boxes"] i32
+        [B,4].  The front-end op already reports rejected table entries in src_status, so status is not written."""
+        dev = self.dev
+        ragged_src = source == "ragged"
+        shape = (capacity,) if ragged_src else (B, source[0], source[1])
+        ws["src_mask"] = torch.empty(shape, device=dev, dtype=torch.uint8)
+        ws["src_boxes"] = torch.empty((B, 4), device=dev, dtype=torch.int32)
+        if "cam" in ws:
+            ws["src_cam_map"] = torch.empty(shape, device=dev, dtype=torch.float32)
+        Hs, Ws = (0, 0) if ragged_src else source
+        ops.append(E.SourceFrameDesc(ws["logits"].data_ptr(), ws["boxes"].data_ptr(), E.ptr(ws.get("cam")),
+                                     ws["src_index"].data_ptr() if ragged_src else None, None,
+                                     ws["src_mask"].data_ptr(), ws["src_boxes"].data_ptr(),
+                                     E.ptr(ws.get("src_cam_map")), capacity if ragged_src else 0, B, IMG, Hs, Ws,
+                                     7 if "cam" in ws else 0, 7 if "cam" in ws else 0))
+
+    def export_plan(self, B, source=None, capacity=None, cam=False, source_frame=False):
         """The whole two-stage program for a batch of B images as a relocatable plan image (bytes): op list, device
         memory layout, BN-folded packed weights of both networks.  A host in any language runs it through the C ABI
         alone (ug_plan_load / ug_plan_copy_in / ug_plan_run / ug_plan_copy_out, include/ugnet.h; examples/run_plan.c).
-        source / capacity / cam as for plan(); a ragged plan's inputs are "src_u8" and "src_index", a cam plan also
-        reports "cam" and "cam_map"."""
-        ws = self.plan(B, source=source, capacity=capacity, cam=cam)
+        source / capacity / cam / source_frame as for plan(); a ragged plan's inputs are "src_u8" and "src_index", a cam
+        plan also reports "cam" and "cam_map", a source_frame plan "src_mask", "src_boxes" and (with cam)
+        "src_cam_map"."""
+        ws = self.plan(B, source=source, capacity=capacity, cam=cam, source_frame=source_frame)
         prog = ws["program"]
         io = {k: ws[k] for k in ("x_in", "src_u8", "src_index", "src_status", "logits", "mask", "boxes", "u8",
-                                 "cls_logits", "cam", "cam_map") if k in ws}
+                                 "cls_logits", "cam", "cam_map", "src_mask", "src_boxes", "src_cam_map") if k in ws}
         tensors = list(prog.keepalive) + list(io.values()) + [(self.unet.w_blob, True), (self.gnet.w_blob, True)]
         return E.export_plan(prog.descs, io, tensors)
 
@@ -809,23 +847,26 @@ class PipelineRunner:
             out.append((s, n - s))
         return out
 
-    def feed_ragged(self, part, cam=False):
+    def feed_ragged(self, part, cam=False, source_frame=False):
         """The ragged plan for one chunk (a ragged.Packed of HWC images, at most one plan's batch) with its packed
         sources and table copied in (one copy each)."""
-        ws = self.plan(len(part.table), source="ragged", capacity=part.n_px, cam=cam)
+        ws = self.plan(len(part.table), source="ragged", capacity=part.n_px, cam=cam, source_frame=source_frame)
         ws["src_u8"][:part.data.numel()].copy_(part.data, non_blocking=True)
         ws["src_index"].copy_(ragged.table_tensor(part.table))
         return ws
 
     @torch.no_grad()
-    def __call__(self, imgs, return_logits=False, return_cam=False):
+    def __call__(self, imgs, return_logits=False, return_cam=False, return_source=False):
         """imgs: float [B,3,224,224] CUDA, or uint8 [B,Hs,Ws,3] CUDA source images of any size (resized on the
         device exactly as the reference's PIL transform does), or a list of uint8 [H,W,3] images of different sizes
         (CUDA tensors or numpy arrays, sides up to 8*224; one ragged batch, util/ragged.py) ->
         (masks u8 [B,224,224], boxes i32 [B,4], cls_logits f32 [B,6]), then the segmentation logits f32 [B,1,224,224]
         if return_logits, then the Grad-CAM map of the predicted class f32 [B,224,224] (in [0,1] inside the ROI box,
-        0 outside; see plan(cam=True)) if return_cam."""
+        0 outside; see plan(cam=True)) if return_cam, then a SourceFrame of the mask, box and (with return_cam) map at
+        each source image's own size if return_source (uint8 sources only: tensors [B,Hs,Ws] for a uint8 batch, lists of
+        [H_i,W_i] tensors for a list; see plan(source_frame=True))."""
         masks, boxes, cls, seg, cams = [], [], [], [], []
+        src_masks, src_boxes, src_cams = [], [], []
         packed = None
         if isinstance(imgs, (list, tuple)):
             packed = ragged.pack(imgs, 3, max_side=ragged.MAX_RATIO * IMG)
@@ -834,12 +875,15 @@ class PipelineRunner:
             n, from_u8 = imgs.shape[0], imgs.dtype == torch.uint8
         if from_u8 and (imgs.dim() != 4 or imgs.shape[3] != 3):
             raise ValueError(f"uint8 input must be HWC [B,H,W,3], got {tuple(imgs.shape)}")
+        if return_source and packed is None and not from_u8:
+            raise ValueError("return_source=True needs uint8 sources: float [B,3,224,224] input has no source frame")
         for s, c in self._chunks(n):
             if packed is not None:
                 part = ragged.chunk(packed, s, s + c)
-                ws = self.feed_ragged(part, cam=True) if return_cam else self.feed_ragged(part)
+                kw = {k: True for k, on in (("cam", return_cam), ("source_frame", return_source)) if on}
+                ws = self.feed_ragged(part, **kw)
             elif from_u8:
-                ws = self.plan(c, source=(imgs.shape[1], imgs.shape[2]), cam=return_cam)
+                ws = self.plan(c, source=(imgs.shape[1], imgs.shape[2]), cam=return_cam, source_frame=return_source)
                 ws["src_u8"].copy_(imgs[s:s + c])
             else:
                 ws = self.plan(c, cam=return_cam)
@@ -852,7 +896,24 @@ class PipelineRunner:
                 seg.append(ws["logits"].clone())
             if return_cam:
                 cams.append(ws["cam_map"].clone())
+            if return_source:
+                src_boxes.append(ws["src_boxes"].clone())
+                if packed is not None:     # copy the chunk's extent once, then per-image views of the copy
+                    src_masks += ragged.unpack(ws["src_mask"][:part.n_px].clone(), part.table, 1)
+                    if return_cam:
+                        src_cams += ragged.unpack(ws["src_cam_map"][:part.n_px].clone(), part.table, 1)
+                else:
+                    src_masks.append(ws["src_mask"].clone())
+                    if return_cam:
+                        src_cams.append(ws["src_cam_map"].clone())
         out = (torch.cat(masks), torch.cat(boxes), torch.cat(cls))
         if return_logits:
             out += (torch.cat(seg),)
-        return out + (torch.cat(cams),) if return_cam else out
+        if return_cam:
+            out += (torch.cat(cams),)
+        if return_source:
+            if packed is None:
+                src_masks = torch.cat(src_masks)
+                src_cams = torch.cat(src_cams) if return_cam else None
+            out += (SourceFrame(src_masks, torch.cat(src_boxes), src_cams if return_cam else None),)
+        return out
