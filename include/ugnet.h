@@ -107,7 +107,8 @@ typedef struct ug_conv_desc {
 } ug_conv_desc;
 
 /* Max pooling on NHWC bf16 with -inf padding (nn.MaxPool2d(2), basicUnet.py:47; torchvision GoogLeNet
- * maxpool1-4 and Inception branch4 with ceil_mode=True: caller passes the ceil-mode OH/OW). */
+ * maxpool1-4 and Inception branch4 with ceil_mode=True: caller passes the ceil-mode OH/OW).  C and both channel
+ * strides are multiples of 8 and in / out are 16-byte aligned (8-channel vector accesses). */
 typedef struct ug_pool_desc {
   const void* in;
   int in_cstride;
@@ -116,7 +117,8 @@ typedef struct ug_pool_desc {
   int C, B, H, W, OH, OW, k, stride, pad;
 } ug_pool_desc;
 
-/* nn.LayerNorm(C) over the last dim of [M][C] bf16 tokens (tasks.py:161-164), fp32 statistics. */
+/* nn.LayerNorm(C) over the last dim of [M][C] bf16 tokens (tasks.py:161-164), fp32 statistics.  C is 256, 512, 768
+ * or 1024; in / out / gamma / beta are 16-byte aligned. */
 typedef struct ug_layernorm_desc {
   const void* in;
   void* out;
@@ -127,7 +129,8 @@ typedef struct ug_layernorm_desc {
 } ug_layernorm_desc;
 
 /* softmax(q k^T * scale) v per (image, head), dim_head = 64 (tasks.py:132-147 and :73-96).
- * q/k/v rows are tokens (b*S + i) with the given row strides (elements); head h uses columns [64h,64h+64). */
+ * q/k/v rows are tokens (b*S + i) with the given row strides (elements); head h uses columns [64h,64h+64).  Every row
+ * stride is a multiple of 8 and at least 64*heads; k and v are 16-byte aligned, q and out 4-byte aligned. */
 typedef struct ug_attn_desc {
   const void* q;
   const void* k;
@@ -142,7 +145,8 @@ typedef struct ug_attn_desc {
 
 /* AdaptiveAvgPool2d(1)/AdaptiveMaxPool2d(1) of an NHWC bf16 map (basicUnet.py:217-218), stage 1: each of
  * `splits` blocks per image reduces a contiguous pixel range to fp32 partial sums / maxima
- * psum,pmax: [B][splits][C].  Deterministic (no atomics); stage 2 lives in the gate op. */
+ * psum,pmax: [B][splits][C].  Deterministic (no atomics); stage 2 lives in the gate op.  C = 8*2^k <= 512,
+ * in_cstride a multiple of 8, in 16-byte aligned. */
 typedef struct ug_chanstats_desc {
   const void* in;
   int in_cstride, C, B, HW, splits;
@@ -280,7 +284,8 @@ typedef struct ug_wavelet_ragged_desc {
   int B;
 } ug_wavelet_ragged_desc;
 
-/* AdaptiveAvgPool2d(1) + Linear(C, ncls): in NHWC bf16 [B][HW][C], w fp32 [ncls][C], logits fp32 [B][ncls]. */
+/* AdaptiveAvgPool2d(1) + Linear(C, ncls): in NHWC bf16 [B][HW][C], w fp32 [ncls][C], logits fp32 [B][ncls].  C is
+ * even and at most 1024, in is 4-byte aligned (read as bf16 pairs). */
 typedef struct ug_head_desc {
   const void* in;
   const float* w;

@@ -2,9 +2,10 @@
  *
  * libugnet_dev.so links the same objects as libugnet.so plus csrc/dev_hooks.cu and csrc/microbench.cu; it exists so
  * that scripts/conv_prof.py and scripts/mma_bench*.py can read per-role cycle counters and run tcgen05 issue-rate
- * micro-benchmarks, and tests/test_conv_coverage_gpu.py can ask which kernel and configuration a conv descriptor
- * selects, without those entry points shipping in the product library.  Load it with UG_DEV_LIB=1
- * (unet-goolenet_b200/engine.py); handles are not interchangeable between the two libraries. */
+ * micro-benchmarks, and tests/test_conv_coverage_gpu.py / tests/test_memops_coverage_gpu.py can ask which kernel and
+ * configuration a conv, memory-bound or stem descriptor selects, without those entry points shipping in the product
+ * library.  Load it with UG_DEV_LIB=1 (unet-goolenet_b200/engine.py); handles are not interchangeable between the two
+ * libraries. */
 #ifndef UGNET_DEV_H_
 #define UGNET_DEV_H_
 #include "ugnet.h"
@@ -81,6 +82,37 @@ typedef struct ug_conv_launch_info {
 /* Runs the conv's plan-time preparation (validation, kernel and configuration choice) and copies the plan out.  Launches
  * nothing and allocates no device memory.  Returns what ug_conv would return for a rejected descriptor. */
 int ug_conv_launch_info(ug_handle h, const ug_conv_desc* d, ug_conv_launch_info_t* out);
+
+/* Kernels of the memory-bound ops (csrc/mem_kernels.cu) and of the stem (csrc/stem_conv.cu). */
+enum {
+  UG_MEMOP_KERNEL_POOL = 0,              /* pool_kernel: any window */
+  UG_MEMOP_KERNEL_POOL_3X3S1 = 1,        /* pool3x3s1_kernel: sliding rows */
+  UG_MEMOP_KERNEL_POOL_3X3S1_BLOCK = 2,  /* pool3x3s1_block_kernel: 2x2 output blocks (H*W >= 196) */
+  UG_MEMOP_KERNEL_POOL_3X3S2 = 3,        /* pool3x3s2_kernel: 2x2 output blocks */
+  UG_MEMOP_KERNEL_LAYERNORM = 4,         /* layernorm_kernel<variant> */
+  UG_MEMOP_KERNEL_ATTENTION = 5,         /* attention_mma_kernel */
+  UG_MEMOP_KERNEL_CHANSTATS = 6,         /* chanstats_kernel */
+  UG_MEMOP_KERNEL_GATE = 7,              /* gate_hidden_kernel + gate_out_kernel, same grid */
+  UG_MEMOP_KERNEL_BBOX = 8,              /* bbox_kernel */
+  UG_MEMOP_KERNEL_CROPRESIZE = 9,        /* resize_u8_kernel<variant> (1 = crop mode) */
+  UG_MEMOP_KERNEL_S2D = 10,              /* s2d_pack_kernel */
+  UG_MEMOP_KERNEL_HEAD = 11,             /* head_kernel */
+  UG_MEMOP_KERNEL_STEM = 12              /* stem_conv_kernel (UNet inc) */
+};
+
+/* The launch that the single-op entry point would make for a memory-bound or stem op. */
+typedef struct ug_memop_launch_info {
+  int kernel;                  /* UG_MEMOP_KERNEL_* */
+  int variant;                 /* layernorm: the template argument C / 256; cropresize: the resize mode; -1 otherwise */
+  int grid_x, grid_y, block;   /* CTAs and threads per CTA */
+  int launches;                /* kernels launched (gate: 2 with the same grid) */
+  long long smem;              /* dynamic shared memory per CTA */
+} ug_memop_launch_info_t;
+
+/* Runs the op's validation and launch decision (the same host function its launcher calls) for op->kind in {POOL,
+ * LAYERNORM, ATTN, CHANSTATS, GATE, BBOX, CROPRESIZE, HEAD, S2D, STEM} and copies the launch out.  Launches nothing.
+ * Returns what the op's entry point would return for a rejected descriptor (UG_EINVAL for any other kind). */
+int ug_memop_launch_info(ug_handle h, const ug_op* op, ug_memop_launch_info_t* out);
 
 #ifdef __cplusplus
 }

@@ -14,11 +14,15 @@ def _gen(seed=0):
     return torch.Generator(device="cuda").manual_seed(seed)
 
 
-@pytest.mark.parametrize("k,stride,pad,H,W", [(2, 2, 0, 28, 28), (3, 2, 0, 112, 112), (3, 2, 0, 56, 56),
-                                              (3, 1, 1, 14, 14), (2, 2, 0, 14, 14), (3, 2, 0, 13, 15),
-                                              (3, 1, 1, 28, 28), (3, 1, 1, 7, 7), (3, 1, 1, 1, 5), (3, 1, 1, 9, 1),
-                                              (3, 2, 0, 28, 28), (3, 2, 0, 14, 14), (3, 2, 0, 8, 9), (3, 2, 0, 3, 3),
-                                              (3, 2, 1, 14, 14)])
+# (k, stride, pad, H, W); also rows of tests/test_memops_coverage_gpu.py
+POOL_CASES = [(2, 2, 0, 28, 28), (3, 2, 0, 112, 112), (3, 2, 0, 56, 56), (3, 1, 1, 14, 14), (2, 2, 0, 14, 14),
+              (3, 2, 0, 13, 15), (3, 1, 1, 28, 28), (3, 1, 1, 7, 7), (3, 1, 1, 1, 5), (3, 1, 1, 9, 1), (3, 2, 0, 28, 28),
+              (3, 2, 0, 14, 14), (3, 2, 0, 8, 9), (3, 2, 0, 3, 3), (3, 2, 1, 14, 14)]
+ATTN_CASES = [(196, 0), (50, 0), (208, 0), (1, 0), (17, 0)]                        # (S, variant)
+CHANSTATS_CASES = [(64, 224 * 224), (128, 112 * 112), (256, 56 * 56), (512, 28 * 28)]   # (C, HW)
+
+
+@pytest.mark.parametrize("k,stride,pad,H,W", POOL_CASES)
 def test_pool(engine, k, stride, pad, H, W):
     from ugnet_b200 import engine as E
     g = _gen(2)
@@ -60,7 +64,7 @@ def test_attention_rejects_long_sequences(engine):
         engine.run_op(d)
 
 
-@pytest.mark.parametrize("S,variant", [(196, 0), (50, 0), (208, 0), (1, 0), (17, 0)])
+@pytest.mark.parametrize("S,variant", ATTN_CASES)
 def test_attention(engine, S, variant):
     from ugnet_b200 import engine as E
     g = _gen(4)
@@ -79,7 +83,7 @@ def test_attention(engine, S, variant):
     assert ((out.float() - ref).abs() <= 2.0 ** -7 * ref.abs() + 4e-3).all()
 
 
-@pytest.mark.parametrize("C,HW", [(64, 224 * 224), (128, 112 * 112), (256, 56 * 56), (512, 28 * 28)])
+@pytest.mark.parametrize("C,HW", CHANSTATS_CASES)
 def test_chanstats_gate(engine, C, HW):
     from ugnet_b200 import engine as E
     g = _gen(5)

@@ -20,8 +20,13 @@ def _check(got, ref):
                            f"{(got - ref).abs().max().item():.4f}, first at {bad.nonzero()[0].tolist()}")
 
 
+# (B, H, W, extra output channels); also rows of tests/test_memops_coverage_gpu.py
+STEM_CASES = [(1, 224, 224, 0), (3, 224, 224, 64), (2, 40, 56, 0), (70, 32, 48, 0)]
+S2D_CASES = [(1, 224, "u8"), (5, 224, "u8"), (2, 224, "f32"), (3, 64, "u8"), (40, 32, "f32")]   # (B, S, source)
+
+
 @pytest.mark.parametrize("pool", [False, True])
-@pytest.mark.parametrize("B,H,W,extra", [(1, 224, 224, 0), (3, 224, 224, 64), (2, 40, 56, 0), (70, 32, 48, 0)])
+@pytest.mark.parametrize("B,H,W,extra", STEM_CASES)
 def test_stem_inc(engine, B, H, W, extra, pool):
     from ugnet_b200 import engine as E
     from ugnet_b200 import pack
@@ -48,7 +53,7 @@ def test_stem_inc(engine, B, H, W, extra, pool):
         assert (out[..., 64:] == 7.0).all()
 
 
-@pytest.mark.parametrize("B,S,src", [(1, 224, "u8"), (5, 224, "u8"), (2, 224, "f32"), (3, 64, "u8"), (40, 32, "f32")])
+@pytest.mark.parametrize("B,S,src", S2D_CASES)
 def test_conv1_space_to_depth(engine, B, S, src):
     """GoogLeNet conv1 as ug_s2d_pack + a four-row-tap implicit GEMM over overlapping TMA windows (ug_conv_desc.in_rstride)
     against F.conv2d(7x7, stride 2, padding 3) on the transformed image; the packed tensor itself is checked exactly."""

@@ -1,5 +1,5 @@
 // Development hooks (libugnet_dev.so only; declared in include/ugnet_dev.h): per-role cycle counters of the conv
-// kernels and the conv launch-plan query.  Not part of the product library.
+// kernels and the launch-plan queries of the conv and memory-bound ops.  Not part of the product library.
 #include <algorithm>
 #include <cstring>
 #include <vector>
@@ -139,6 +139,53 @@ int ug_conv_launch_info(ug_handle h, const ug_conv_desc* d, ug_conv_launch_info_
   o.last_round_items = o.items - (long long)(o.rounds - 1) * o.units;
   o.tiles_past_end = (o.items / p.n_tiles) * L.item_tiles - p.m_tiles;
   if (L.kernel == ConvKernel::OneTile || L.kernel == ConvKernel::Persistent) o.tiles_past_end = 0;
+  return UG_OK;
+}
+
+static_assert((int)MemKernel::Pool == UG_MEMOP_KERNEL_POOL && (int)MemKernel::LayerNorm == UG_MEMOP_KERNEL_LAYERNORM &&
+                  (int)MemKernel::CropResize == UG_MEMOP_KERNEL_CROPRESIZE && (int)MemKernel::Head == UG_MEMOP_KERNEL_HEAD,
+              "MemKernel and UG_MEMOP_KERNEL_* must list the kernels in the same order");
+
+int ug_memop_launch_info(ug_handle h, const ug_op* op, ug_memop_launch_info_t* out) {
+  if (!h || !op || !out) return UG_EINVAL;
+  DeviceGuard guard(h);
+  ug_memop_launch_info_t& o = *out;
+  memset(&o, 0, sizeof(o));
+  o.launches = 1;
+  if (op->kind == UG_OP_STEM) {
+    StemLaunch L;
+    const int rc = stem_prepare(h, &op->u.stem, &L);
+    if (rc != UG_OK) return rc;
+    o.kernel = UG_MEMOP_KERNEL_STEM;
+    o.variant = -1;
+    o.grid_x = (int)L.grid;
+    o.grid_y = 1;
+    o.block = (int)L.block;
+    o.smem = (long long)L.smem;
+    return UG_OK;
+  }
+  MemLaunch L;
+  int rc;
+  switch (op->kind) {
+    case UG_OP_POOL: rc = plan_pool(h, &op->u.pool, &L); break;
+    case UG_OP_LAYERNORM: rc = plan_layernorm(h, &op->u.ln, &L); break;
+    case UG_OP_ATTN: rc = plan_attention(h, &op->u.attn, &L); break;
+    case UG_OP_CHANSTATS: rc = plan_chanstats(h, &op->u.stats, &L); break;
+    case UG_OP_GATE: rc = plan_gate(h, &op->u.gate, &L); break;
+    case UG_OP_BBOX: rc = plan_bbox(h, &op->u.bbox, &L); break;
+    case UG_OP_CROPRESIZE: rc = plan_cropresize(h, &op->u.crop, &L); break;
+    case UG_OP_HEAD: rc = plan_head(h, &op->u.head, &L); break;
+    case UG_OP_S2D: rc = plan_s2d_pack(h, &op->u.s2d, &L); break;
+    default: return set_error(h, UG_EINVAL, "memop_launch_info: op kind %d is not a memory-bound op", op->kind);
+  }
+  if (rc != UG_OK) return rc;
+  o.kernel = (int)L.kernel;
+  o.variant = L.variant;
+  o.grid_x = (int)L.grid.x;
+  o.grid_y = (int)L.grid.y;
+  o.block = (int)L.block;
+  o.smem = (long long)L.smem;
+  if (L.kernel == MemKernel::Gate) o.launches = 2;
   return UG_OK;
 }
 

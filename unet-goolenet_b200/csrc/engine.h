@@ -204,7 +204,7 @@ struct StemLaunch {
   alignas(64) CUtensorMap tmO;
   alignas(64) CUtensorMap tmP;  // pooled output (pool_out)
   StemParams p;
-  unsigned grid;
+  unsigned grid, block;
   size_t smem;
 };
 
@@ -284,6 +284,42 @@ inline cudaError_t launch_pairs(ug_engine* h, void (*kernel)(KArgs...), unsigned
 
 int stem_prepare(ug_engine* h, const ug_stem_desc* d, StemLaunch* out);
 int stem_launch(ug_engine* h, const StemLaunch* l, cudaStream_t s);
+
+// Which kernel a memory-bound op of csrc/mem_kernels.cu launches (same order as UG_MEMOP_KERNEL_* of ugnet_dev.h).
+enum class MemKernel {
+  Pool,            // pool_kernel: any window
+  Pool3x3s1,       // pool3x3s1_kernel: sliding rows (maps under 196 pixels)
+  Pool3x3s1Block,  // pool3x3s1_block_kernel: 2x2 output blocks
+  Pool3x3s2,       // pool3x3s2_kernel: 2x2 output blocks, ceil mode
+  LayerNorm,       // layernorm_kernel<C / 256>
+  Attention,       // attention_mma_kernel
+  ChanStats,       // chanstats_kernel
+  Gate,            // gate_hidden_kernel + gate_out_kernel (two launches, same grid)
+  BBox,            // bbox_kernel
+  CropResize,      // resize_u8_kernel<kCrop>
+  S2d,             // s2d_pack_kernel
+  Head,            // head_kernel
+};
+
+// The launch of a memory-bound op: validation and every dispatch rule live in the op's plan_* function, which both the
+// launcher and the launch-plan query of libugnet_dev.so (ug_memop_launch_info) call.
+struct MemLaunch {
+  MemKernel kernel;
+  int variant;       // layernorm_kernel<kNV>: kNV; resize_u8_kernel<kMode>: kMode; -1 otherwise
+  dim3 grid;
+  unsigned block;
+  size_t smem;       // dynamic shared memory
+  int max_rows;      // resize_u8_kernel: source rows staged per block
+};
+int plan_pool(ug_engine* h, const ug_pool_desc* d, MemLaunch* L);
+int plan_layernorm(ug_engine* h, const ug_layernorm_desc* d, MemLaunch* L);
+int plan_attention(ug_engine* h, const ug_attn_desc* d, MemLaunch* L);
+int plan_chanstats(ug_engine* h, const ug_chanstats_desc* d, MemLaunch* L);
+int plan_gate(ug_engine* h, const ug_gate_desc* d, MemLaunch* L);
+int plan_bbox(ug_engine* h, const ug_bbox_desc* d, MemLaunch* L);
+int plan_cropresize(ug_engine* h, const ug_cropresize_desc* d, MemLaunch* L);
+int plan_s2d_pack(ug_engine* h, const ug_s2d_desc* d, MemLaunch* L);
+int plan_head(ug_engine* h, const ug_head_desc* d, MemLaunch* L);
 
 int launch_pool(ug_engine* h, const ug_pool_desc* d, cudaStream_t s);
 int launch_layernorm(ug_engine* h, const ug_layernorm_desc* d, cudaStream_t s);

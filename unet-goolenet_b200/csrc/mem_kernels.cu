@@ -201,39 +201,52 @@ __global__ void __launch_bounds__(256) pool3x3s1_block_kernel(const __nv_bfloat1
     }
 }
 
-int launch_pool(ug_engine* h, const ug_pool_desc* d, cudaStream_t s) {
+static bool misaligned(const void* p, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(p) & (bytes - 1)) != 0; }
+
+static void plan_grid(MemLaunch* L, MemKernel k, dim3 grid, unsigned block, int variant = -1, size_t smem = 0) {
+  L->kernel = k;
+  L->variant = variant;
+  L->grid = grid;
+  L->block = block;
+  L->smem = smem;
+  L->max_rows = 0;
+}
+
+int plan_pool(ug_engine* h, const ug_pool_desc* d, MemLaunch* L) {
   if (!d->in || !d->out || d->C % 8 || d->in_cstride % 8 || d->out_cstride % 8 || d->k <= 0 || d->stride <= 0)
     return set_error(h, UG_EINVAL, "pool: bad args (C and strides must be multiples of 8)");
+  if (misaligned(d->in, 16) || misaligned(d->out, 16))
+    return set_error(h, UG_EINVAL, "pool: in / out must be 16-byte aligned");
   if ((d->OH - 1) * d->stride - d->pad >= d->H || (d->OW - 1) * d->stride - d->pad >= d->W)
     return set_error(h, UG_EINVAL, "pool: last window starts outside the input");
   // Block forms for 3x3 windows (profiles/r02_pool_s2.txt, against the generic kernel for stride 2 and sliding rows for
   // stride 1): maxpool1 0.1505 -> 0.107 ms per 256 images (4.8 TB/s of DRAM traffic), maxpool2 0.118 ->
   // 0.086, the branch-4 pools on 28x28 / 14x14 maps 0.074 / 0.042 -> 0.058 / 0.033; the 7x7 maps stay on sliding rows
   // (0.015 against 0.0195 ms).
-  if (d->k == 3 && d->stride == 1 && d->pad == 1 && d->OH == d->H && d->OW == d->W && d->H * d->W >= 196) {
-    const long long total = (long long)d->B * ((d->H + 1) / 2) * ((d->W + 1) / 2) * (d->C / 8);
-    launch_pdl(pool3x3s1_block_kernel, ceil_div(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
-                                                         reinterpret_cast<__nv_bfloat16*>(d->out), *d);
-    h->launches++;
-    return check_cuda(h, cudaGetLastError(), "pool3x3s1 launch");
+  const long long cg = d->C / 8;
+  if (d->k == 3 && d->stride == 1 && d->pad == 1 && d->OH == d->H && d->OW == d->W && d->H * d->W >= 196)
+    plan_grid(L, MemKernel::Pool3x3s1Block, ceil_div((long long)d->B * ((d->H + 1) / 2) * ((d->W + 1) / 2) * cg, 256), 256);
+  else if (d->k == 3 && d->stride == 1 && d->pad == 1 && d->OH == d->H && d->OW == d->W)
+    plan_grid(L, MemKernel::Pool3x3s1, ceil_div((long long)d->B * d->H * cg, 256), 256);
+  else if (d->k == 3 && d->stride == 2 && d->pad == 0 && 2 * (d->OH - 1) < d->H && 2 * (d->OW - 1) < d->W)
+    plan_grid(L, MemKernel::Pool3x3s2, ceil_div((long long)d->B * ((d->OH + 1) / 2) * ((d->OW + 1) / 2) * cg, 256), 256);
+  else
+    plan_grid(L, MemKernel::Pool, ceil_div((long long)d->B * d->OH * d->OW * cg, 256), 256);
+  return UG_OK;
+}
+
+int launch_pool(ug_engine* h, const ug_pool_desc* d, cudaStream_t s) {
+  MemLaunch L;
+  const int rc = plan_pool(h, d, &L);
+  if (rc != UG_OK) return rc;
+  const __nv_bfloat16* in = reinterpret_cast<const __nv_bfloat16*>(d->in);
+  __nv_bfloat16* out = reinterpret_cast<__nv_bfloat16*>(d->out);
+  switch (L.kernel) {
+    case MemKernel::Pool3x3s1Block: launch_pdl(pool3x3s1_block_kernel, L.grid, L.block, 0, s, in, out, *d); break;
+    case MemKernel::Pool3x3s1: launch_pdl(pool3x3s1_kernel, L.grid, L.block, 0, s, in, out, *d); break;
+    case MemKernel::Pool3x3s2: launch_pdl(pool3x3s2_kernel, L.grid, L.block, 0, s, in, out, *d); break;
+    default: launch_pdl(pool_kernel, L.grid, L.block, 0, s, in, out, *d); break;
   }
-  if (d->k == 3 && d->stride == 1 && d->pad == 1 && d->OH == d->H && d->OW == d->W) {
-    const long long total = (long long)d->B * d->H * (d->C / 8);
-    launch_pdl(pool3x3s1_kernel, ceil_div(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
-                                                   reinterpret_cast<__nv_bfloat16*>(d->out), *d);
-    h->launches++;
-    return check_cuda(h, cudaGetLastError(), "pool3x3s1 launch");
-  }
-  if (d->k == 3 && d->stride == 2 && d->pad == 0 && 2 * (d->OH - 1) < d->H && 2 * (d->OW - 1) < d->W) {
-    const long long total = (long long)d->B * ((d->OH + 1) / 2) * ((d->OW + 1) / 2) * (d->C / 8);
-    launch_pdl(pool3x3s2_kernel, ceil_div(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
-                                                   reinterpret_cast<__nv_bfloat16*>(d->out), *d);
-    h->launches++;
-    return check_cuda(h, cudaGetLastError(), "pool3x3s2 launch");
-  }
-  const long long total = (long long)d->B * d->OH * d->OW * (d->C / 8);
-  launch_pdl(pool_kernel, ceil_div(total, 256), 256, 0, s, reinterpret_cast<const __nv_bfloat16*>(d->in),
-                                            reinterpret_cast<__nv_bfloat16*>(d->out), *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "pool launch");
 }
@@ -318,21 +331,27 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
   }
 }
 
-int launch_layernorm(ug_engine* h, const ug_layernorm_desc* d, cudaStream_t s) {
+int plan_layernorm(ug_engine* h, const ug_layernorm_desc* d, MemLaunch* L) {
   if (!d->in || !d->out || !d->gamma || !d->beta || d->M <= 0 || d->C % 256 || d->C > 1024 || d->C <= 0)
     return set_error(h, UG_EINVAL, "layernorm: C must be a multiple of 256 up to 1024");
-  if ((reinterpret_cast<uintptr_t>(d->gamma) & 15) || (reinterpret_cast<uintptr_t>(d->beta) & 15) ||
-      (reinterpret_cast<uintptr_t>(d->in) & 15) || (reinterpret_cast<uintptr_t>(d->out) & 15))
+  if (misaligned(d->gamma, 16) || misaligned(d->beta, 16) || misaligned(d->in, 16) || misaligned(d->out, 16))
     return set_error(h, UG_EINVAL, "layernorm: in / out / gamma / beta must be 16-byte aligned");
   const long long warps = ((long long)d->M + kLnTok - 1) / kLnTok;
-  const dim3 grid(ceil_div(warps * 32, 256));
+  plan_grid(L, MemKernel::LayerNorm, ceil_div(warps * 32, 256), 256, d->C / 256);
+  return UG_OK;
+}
+
+int launch_layernorm(ug_engine* h, const ug_layernorm_desc* d, cudaStream_t s) {
+  MemLaunch L;
+  const int rc = plan_layernorm(h, d, &L);
+  if (rc != UG_OK) return rc;
   const __nv_bfloat16* in = reinterpret_cast<const __nv_bfloat16*>(d->in);
   __nv_bfloat16* out = reinterpret_cast<__nv_bfloat16*>(d->out);
-  switch (d->C / 256) {
-    case 1: launch_pdl(layernorm_kernel<1>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
-    case 2: launch_pdl(layernorm_kernel<2>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
-    case 3: launch_pdl(layernorm_kernel<3>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
-    default: launch_pdl(layernorm_kernel<4>, grid, 256, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
+  switch (L.variant) {
+    case 1: launch_pdl(layernorm_kernel<1>, L.grid, L.block, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
+    case 2: launch_pdl(layernorm_kernel<2>, L.grid, L.block, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
+    case 3: launch_pdl(layernorm_kernel<3>, L.grid, L.block, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
+    default: launch_pdl(layernorm_kernel<4>, L.grid, L.block, 0, s, in, out, d->gamma, d->beta, d->M, d->C, d->eps); break;
   }
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "layernorm launch");
@@ -475,19 +494,33 @@ __global__ void __launch_bounds__(128, 3) attention_mma_kernel(ug_attn_desc d) {
   }
 }
 
-int launch_attention(ug_engine* h, const ug_attn_desc* d, cudaStream_t s) {
+int plan_attention(ug_engine* h, const ug_attn_desc* d, MemLaunch* L) {
   if (!d->q || !d->k || !d->v || !d->out || d->S <= 0 || d->heads <= 0 || d->B <= 0 || d->variant != 0)
     return set_error(h, UG_EINVAL, "attention: bad args");
   if (d->S > kAttnSP) return set_error(h, UG_EUNSUPPORTED, "attention: S <= %d tokens (the 14x14 bottleneck has 196)", kAttnSP);
   if (d->q_stride % 8 || d->k_stride % 8 || d->v_stride % 8 || d->out_stride % 8)
     return set_error(h, UG_EINVAL, "attention: row strides must be multiples of 8");
+  const long long cols = 64LL * d->heads;
+  if (cols > d->q_stride || cols > d->k_stride || cols > d->v_stride || cols > d->out_stride)
+    return set_error(h, UG_EINVAL, "attention: 64 * heads = %lld columns must fit in every row stride", cols);
+  // K and V rows are staged with 16-byte cp.async, q is read and out written as bf16 pairs
+  if (misaligned(d->k, 16) || misaligned(d->v, 16) || misaligned(d->q, 4) || misaligned(d->out, 4))
+    return set_error(h, UG_EINVAL, "attention: k / v must be 16-byte aligned, q / out 4-byte aligned");
+  plan_grid(L, MemKernel::Attention, d->B * d->heads, 128, -1,
+            (size_t)(kAttnSP * kAttnKPitch + kAttnSP * kAttnVPitch) * sizeof(__nv_bfloat16));
+  return UG_OK;
+}
+
+int launch_attention(ug_engine* h, const ug_attn_desc* d, cudaStream_t s) {
+  MemLaunch L;
+  const int rc = plan_attention(h, d, &L);
+  if (rc != UG_OK) return rc;
   if (!h->attr_attn) {
     const cudaError_t e = cudaFuncSetAttribute(attention_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
     if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(attention_mma_kernel)");
     h->attr_attn = true;
   }
-  const size_t smem = (size_t)(kAttnSP * kAttnKPitch + kAttnSP * kAttnVPitch) * sizeof(__nv_bfloat16);
-  launch_pdl(attention_mma_kernel, d->B * d->heads, 128, smem, s, *d);
+  launch_pdl(attention_mma_kernel, L.grid, L.block, L.smem, s, *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "attention launch");
 }
@@ -547,11 +580,20 @@ __global__ void __launch_bounds__(256) chanstats_kernel(ug_chanstats_desc d) {
   }
 }
 
-int launch_chanstats(ug_engine* h, const ug_chanstats_desc* d, cudaStream_t s) {
+int plan_chanstats(ug_engine* h, const ug_chanstats_desc* d, MemLaunch* L) {
   if (!d->in || !d->psum || !d->pmax || d->C % 8 || d->C > 512 || d->C < 8 || (256 % (d->C / 8)) || d->splits <= 0 ||
       d->in_cstride % 8)
     return set_error(h, UG_EINVAL, "chanstats: C must be 8*2^k <= 512");
-  launch_pdl(chanstats_kernel, dim3(d->splits, d->B), 256, 0, s, *d);
+  if (misaligned(d->in, 16)) return set_error(h, UG_EINVAL, "chanstats: in must be 16-byte aligned");
+  plan_grid(L, MemKernel::ChanStats, dim3(d->splits, d->B), 256);
+  return UG_OK;
+}
+
+int launch_chanstats(ug_engine* h, const ug_chanstats_desc* d, cudaStream_t s) {
+  MemLaunch L;
+  const int rc = plan_chanstats(h, d, &L);
+  if (rc != UG_OK) return rc;
+  launch_pdl(chanstats_kernel, L.grid, L.block, 0, s, *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "chanstats launch");
 }
@@ -616,12 +658,20 @@ __global__ void __launch_bounds__(256) gate_out_kernel(ug_gate_desc d, const flo
   }
 }
 
-int launch_gate(ug_engine* h, const ug_gate_desc* d, cudaStream_t s) {
+int plan_gate(ug_engine* h, const ug_gate_desc* d, MemLaunch* L) {
   if (!d->psum || !d->pmax || !d->w1 || !d->w2 || !d->w3 || !d->b1 || !d->b2 || !d->b3 || !d->g || !d->hid ||
       d->C > 512 || d->C % 2 || d->HW <= 0 || d->splits <= 0)
     return set_error(h, UG_EINVAL, "gate: bad args (C <= 512, hid scratch required)");
-  launch_pdl(gate_hidden_kernel, dim3(kGateSplit, d->B), 256, 0, s, *d, d->hid);
-  launch_pdl(gate_out_kernel, dim3(kGateSplit, d->B), 256, 0, s, *d, d->hid);
+  plan_grid(L, MemKernel::Gate, dim3(kGateSplit, d->B), 256);
+  return UG_OK;
+}
+
+int launch_gate(ug_engine* h, const ug_gate_desc* d, cudaStream_t s) {
+  MemLaunch L;
+  const int rc = plan_gate(h, d, &L);
+  if (rc != UG_OK) return rc;
+  launch_pdl(gate_hidden_kernel, L.grid, L.block, 0, s, *d, d->hid);
+  launch_pdl(gate_out_kernel, L.grid, L.block, 0, s, *d, d->hid);
   h->launches += 2;
   return check_cuda(h, cudaGetLastError(), "gate launch");
 }
@@ -696,9 +746,17 @@ __global__ void __launch_bounds__(1024) bbox_kernel(const unsigned char* __restr
   }
 }
 
-int launch_bbox(ug_engine* h, const ug_bbox_desc* d, cudaStream_t s) {
+int plan_bbox(ug_engine* h, const ug_bbox_desc* d, MemLaunch* L) {
   if (!d->mask || !d->boxes || d->B <= 0 || d->H <= 0 || d->W <= 0) return set_error(h, UG_EINVAL, "bbox: bad args");
-  launch_pdl(bbox_kernel, d->B, 1024, 0, s, d->mask, d->boxes, d->H, d->W, d->padding);
+  plan_grid(L, MemKernel::BBox, d->B, 1024);
+  return UG_OK;
+}
+
+int launch_bbox(ug_engine* h, const ug_bbox_desc* d, cudaStream_t s) {
+  MemLaunch L;
+  const int rc = plan_bbox(h, d, &L);
+  if (rc != UG_OK) return rc;
+  launch_pdl(bbox_kernel, L.grid, L.block, 0, s, d->mask, d->boxes, d->H, d->W, d->padding);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "bbox launch");
 }
@@ -925,23 +983,32 @@ int launch_resize_ragged(ug_engine* h, const ug_resize_ragged_desc* d, cudaStrea
 // ROI stage (roi.py:39-44 + data_utils.py:102,146-147): the same two-pass kernel reading the box of the float image.
 // Crops are at most HxW with S >= both sides in the pipeline (224 -> 224: up-sampling, <= 3 taps), but any ratio up
 // to 8x is handled.
-int launch_cropresize(ug_engine* h, const ug_cropresize_desc* d, cudaStream_t s) {
+int plan_cropresize(ug_engine* h, const ug_cropresize_desc* d, MemLaunch* L) {
   if (!d->img || !d->boxes || !d->out_u8 || d->S <= 0 || d->S > 512 || d->B <= 0 || d->H <= 0 || d->W <= 0)
     return set_error(h, UG_EINVAL, "cropresize: bad args (S <= 512)");
   const double sc = std::max(std::max((double)d->H / d->S, (double)d->W / d->S), 1.0);
   if (2 * (int)ceil(sc) + 1 > kRsMaxTaps) return set_error(h, UG_EUNSUPPORTED, "cropresize: image more than 8x the output");
   const int max_rows = std::min(d->H, (int)ceil((kRsRows - 1) * sc + 2.0 * sc + 3.0));
   const size_t smem = (size_t)(d->S + kRsRows) * sizeof(RsCoef) + (size_t)max_rows * d->S * 3;
-  if (smem > h->attr_crop) {
-    if (smem > 200 * 1024) return set_error(h, UG_EUNSUPPORTED, "cropresize: shared memory request %zu too large", smem);
-    cudaError_t e = cudaFuncSetAttribute((const void*)resize_u8_kernel<kCrop>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (smem > 200 * 1024) return set_error(h, UG_EUNSUPPORTED, "cropresize: shared memory request %zu too large", smem);
+  plan_grid(L, MemKernel::CropResize, dim3(ceil_div(d->S, kRsRows), d->B), 256, kCrop, smem);
+  L->max_rows = max_rows;
+  return UG_OK;
+}
+
+int launch_cropresize(ug_engine* h, const ug_cropresize_desc* d, cudaStream_t s) {
+  MemLaunch L;
+  const int rc = plan_cropresize(h, d, &L);
+  if (rc != UG_OK) return rc;
+  if (L.smem > h->attr_crop) {
+    cudaError_t e = cudaFuncSetAttribute((const void*)resize_u8_kernel<kCrop>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.smem);
     if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(resize_u8_kernel<crop>)");
-    h->attr_crop = smem;
+    h->attr_crop = L.smem;
   }
   ug_resize_desc r;
   r.src = nullptr; r.out_f32 = nullptr; r.out_u8 = d->out_u8; r.B = d->B; r.Hs = d->H; r.Ws = d->W; r.S = d->S;
-  launch_pdl(resize_u8_kernel<kCrop>, dim3(ceil_div(d->S, kRsRows), d->B), 256, smem, s, r, max_rows, d->img, d->boxes,
-             d->H, d->W, RaggedSrc{});
+  launch_pdl(resize_u8_kernel<kCrop>, L.grid, L.block, L.smem, s, r, L.max_rows, d->img, d->boxes, d->H, d->W,
+             RaggedSrc{});
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "cropresize launch");
 }
@@ -960,9 +1027,11 @@ __global__ void __launch_bounds__(256) s2d_pack_kernel(ug_s2d_desc d) {
   const int X = (int)(t % Q);
   const int Y = (int)((t / Q) % Q);
   const int n = (int)(t / ((long long)Q * Q));
-  // torchvision GoogLeNet._transform_input: x_c * (std_c / 0.5) + (mean_c - 0.5) / 0.5
-  const float sc[3] = {0.229f / 0.5f, 0.224f / 0.5f, 0.225f / 0.5f};
-  const float sh[3] = {(0.485f - 0.5f) / 0.5f, (0.456f - 0.5f) / 0.5f, (0.406f - 0.5f) / 0.5f};
+  // torchvision GoogLeNet._transform_input: x_c * (std_c / 0.5) + (mean_c - 0.5) / 0.5, the constants evaluated in
+  // double and rounded once, as torch applies those Python scalars to a float tensor (evaluated from the float-rounded
+  // means, the shifts of channels 0 and 2 were 15 and 2 float ulps off)
+  const float sc[3] = {(float)(0.229 / 0.5), (float)(0.224 / 0.5), (float)(0.225 / 0.5)};
+  const float sh[3] = {(float)((0.485 - 0.5) / 0.5), (float)((0.456 - 0.5) / 0.5), (float)((0.406 - 0.5) / 0.5)};
   float v[16];
 #pragma unroll
   for (int i = 0; i < 16; ++i) v[i] = 0.0f;
@@ -995,12 +1064,19 @@ __global__ void __launch_bounds__(256) s2d_pack_kernel(ug_s2d_desc d) {
   out[1] = o1;
 }
 
-int launch_s2d_pack(ug_engine* h, const ug_s2d_desc* d, cudaStream_t s) {
-  if ((!d->in_u8 && !d->in_f32) || !d->out || d->B <= 0 || d->S <= 0 || (d->S & 1) || (reinterpret_cast<uintptr_t>(d->out) & 15))
+int plan_s2d_pack(ug_engine* h, const ug_s2d_desc* d, MemLaunch* L) {
+  if ((!d->in_u8 && !d->in_f32) || !d->out || d->B <= 0 || d->S <= 0 || (d->S & 1) || misaligned(d->out, 16))
     return set_error(h, UG_EINVAL, "s2d_pack: bad args (even image side, 16-byte aligned output)");
   const int Q = d->S / 2 + 3;
-  const long long total = (long long)d->B * Q * Q;
-  launch_pdl(s2d_pack_kernel, ceil_div(total, 256), 256, 0, s, *d);
+  plan_grid(L, MemKernel::S2d, ceil_div((long long)d->B * Q * Q, 256), 256);
+  return UG_OK;
+}
+
+int launch_s2d_pack(ug_engine* h, const ug_s2d_desc* d, cudaStream_t s) {
+  MemLaunch L;
+  const int rc = plan_s2d_pack(h, d, &L);
+  if (rc != UG_OK) return rc;
+  launch_pdl(s2d_pack_kernel, L.grid, L.block, 0, s, *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "s2d_pack launch");
 }
@@ -1034,10 +1110,19 @@ __global__ void __launch_bounds__(256) head_kernel(ug_head_desc d) {
   }
 }
 
-int launch_head(ug_engine* h, const ug_head_desc* d, cudaStream_t s) {
+int plan_head(ug_engine* h, const ug_head_desc* d, MemLaunch* L) {
   if (!d->in || !d->w || !d->b || !d->logits || d->C > 1024 || d->C % 2 || d->HW <= 0 || d->ncls <= 0)
     return set_error(h, UG_EINVAL, "head: bad args (C <= 1024)");
-  launch_pdl(head_kernel, d->B, 256, 0, s, *d);
+  if (misaligned(d->in, 4)) return set_error(h, UG_EINVAL, "head: in must be 4-byte aligned (read as bf16 pairs)");
+  plan_grid(L, MemKernel::Head, d->B, 256);
+  return UG_OK;
+}
+
+int launch_head(ug_engine* h, const ug_head_desc* d, cudaStream_t s) {
+  MemLaunch L;
+  const int rc = plan_head(h, d, &L);
+  if (rc != UG_OK) return rc;
+  launch_pdl(head_kernel, L.grid, L.block, 0, s, *d);
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "head launch");
 }

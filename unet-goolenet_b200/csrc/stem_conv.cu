@@ -272,6 +272,7 @@ int stem_prepare(ug_engine* h, const ug_stem_desc* d, StemLaunch* L) {
   }
   // one CTA per SM: its warpgroups share the weights (see the header comment)
   L->grid = (unsigned)std::min<long long>((p.total_tiles + kStemGroups - 1) / kStemGroups, (long long)h->num_sms);
+  L->block = 128 * kStemGroups;
   const size_t patch = 3 * kIncPatchH * kIncPatchPitch * 4;
   L->smem = 1024 + (size_t)64 * 128 +
             kStemGroups * ((size_t)kABytesPerStage + (p.pool ? kStemPoolBytes : 0) + (patch + 1023) / 1024 * 1024) +
@@ -286,7 +287,7 @@ int stem_launch(ug_engine* h, const StemLaunch* L, cudaStream_t s) {
     if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(stem_conv_kernel)");
     h->attr_stem = true;
   }
-  const cudaError_t le = launch_pdl(stem_conv_kernel<0, kStemGroups>, L->grid, 128 * kStemGroups, L->smem, s, L->tmB,
+  const cudaError_t le = launch_pdl(stem_conv_kernel<0, kStemGroups>, L->grid, L->block, L->smem, s, L->tmB,
                                     L->tmO, L->tmP, L->p);
   h->launches++;
   return check_cuda(h, le != cudaSuccess ? le : cudaGetLastError(), "stem_conv_kernel launch");

@@ -159,7 +159,7 @@ EXPORTED_SYMBOLS = ["ug_version", "ug_create", "ug_destroy", "ug_last_error", "u
                     "ug_plan_load", "ug_plan_num_io", "ug_plan_io_name", "ug_plan_io", "ug_plan_device_bytes",
                     "ug_plan_program", "ug_plan_copy_in", "ug_plan_copy_out", "ug_plan_run", "ug_plan_destroy"]
 DEV_SYMBOLS = ["ug_conv_profile", "ug_conv_profile16", "ug_mma_microbench", "ug_mma_microbench2",
-               "ug_mma_microbench_pair", "ug_conv_launch_info", "ug_conv_instances"]
+               "ug_mma_microbench_pair", "ug_conv_launch_info", "ug_conv_instances", "ug_memop_launch_info"]
 
 _lib = None
 
