@@ -103,7 +103,8 @@ typedef struct ug_conv_desc {
                                  weight rows; 3x3 ReLU layers with N <= 64, STORE / OUTC / GATE epilogues);
                                  7 = the multi-issuer kernel in CTA-pair mode (3x3 ReLU layers with 128-column
                                  n-tiles, STORE / GATE epilogues; each CTA streams half of every weight tile).
-                                 0 picks by the measured static rule of csrc/conv_gemm.cu (conv_prepare) */
+                                 0 picks by the measured static rule of csrc/conv_gemm.cu (conv_prepare).
+                                 Any other value is rejected with UG_EINVAL */
 } ug_conv_desc;
 
 /* Max pooling on NHWC bf16 with -inf padding (nn.MaxPool2d(2), basicUnet.py:47; torchvision GoogLeNet

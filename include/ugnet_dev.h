@@ -1,11 +1,10 @@
 /* ugnet_dev.h — development hooks of libugnet_dev.so (NOT part of the product ABI in ugnet.h).
  *
  * libugnet_dev.so links the same objects as libugnet.so plus csrc/dev_hooks.cu and csrc/microbench.cu; it exists so
- * that scripts/conv_prof.py and scripts/mma_bench*.py can read per-role cycle counters and run tcgen05 issue-rate
- * micro-benchmarks, and tests/test_conv_coverage_gpu.py / tests/test_memops_coverage_gpu.py can ask which kernel and
- * configuration a conv, memory-bound or stem descriptor selects, without those entry points shipping in the product
- * library.  Load it with UG_DEV_LIB=1 (unet-goolenet_b200/engine.py); handles are not interchangeable between the two
- * libraries. */
+ * that scripts/mma_bench*.py can run tcgen05 issue-rate micro-benchmarks, and tests/test_conv_coverage_gpu.py /
+ * tests/test_memops_coverage_gpu.py can ask which kernel and configuration a conv, memory-bound or stem descriptor
+ * selects, without those entry points shipping in the product library.  Load it with UG_DEV_LIB=1
+ * (unet-goolenet_b200/engine.py); handles are not interchangeable between the two libraries. */
 #ifndef UGNET_DEV_H_
 #define UGNET_DEV_H_
 #include "ugnet.h"
@@ -14,14 +13,6 @@
 extern "C" {
 #endif
 
-/* Persistent conv kernel (variant 2), averaged over CTAs: {producer wait-for-free-slot, producer total, MMA
- * wait-for-data, MMA wait-for-accumulator, epilogue wait-for-accumulator, epilogue wait-for-staging, epilogue math,
- * epilogue store} in SM cycles, out[8] = number of CTAs, out[9] = tiles per CTA.  Synchronizes the stream. */
-int ug_conv_profile(ug_handle h, const ug_conv_desc* d, void* stream, double* out10);
-/* Multi-issuer kernel (variant 5), averages over CTAs: out[0..3] = producer {wait activation slot, wait weight slot,
- * total cycles, total ns}; out[4..7] / out[8..11] = issuer 0 / 1 {wait activations, wait weights, wait accumulator,
- * total cycles}; out[12..15] = epilogue group 0 {wait accumulator, wait staging, total cycles, tiles}. */
-int ug_conv_profile16(ug_handle h, const ug_conv_desc* d, void* stream, double* out16);
 /* Average SM cycles per tcgen05.mma (M=128, N, K=16) with n_acc interleaved TMEM accumulators and ctas_per_sm
  * co-resident CTAs. */
 int ug_mma_microbench(ug_handle h, int N, int n_acc, int iters, int ctas_per_sm, int distinct_ab,

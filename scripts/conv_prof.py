@@ -1,9 +1,8 @@
-"""Sweep the conv kernel over the hot layer shapes at batch 64: time per config + per-role cycle counters."""
+"""Sweep the conv kernel over the hot layer shapes at batch 64: time per config (CUDA events)."""
 import json
 import sys
 import os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-os.environ.setdefault("UG_DEV_LIB", "1")   # profiling hooks live in libugnet_dev.so (include/ugnet_dev.h)
 import torch
 import ugnet_b200  # noqa
 from ugnet_b200 import engine as E, pack
@@ -12,7 +11,7 @@ eng = E.Engine.get(0)
 g = torch.Generator(device="cuda").manual_seed(0)
 
 
-def make(B, H, W, Cin, N, R, mode=0, bn=None, stages=0, variant=0, tile=None, up=1, act=1):
+def make(B, H, W, Cin, N, R, mode=0, bn=None, variant=0, tile=None, up=1, act=1):
     x = torch.randn((B, H, W, Cin), generator=g, device="cuda").to(torch.bfloat16)
     wt = torch.randn((N, Cin, R, R), generator=g, device="cuda") * (Cin * R * R) ** -0.5
     BN = bn or (pack.choose_bn(N, N // 4) if up == 2 else pack.choose_bn(N))
@@ -23,7 +22,7 @@ def make(B, H, W, Cin, N, R, mode=0, bn=None, stages=0, variant=0, tile=None, up
     d.inp = x.data_ptr(); d.in_cstride = Cin; d.Cin = Cin; d.B, d.H, d.W = B, H, W
     d.R = d.S = R; d.pad = (R - 1) // 2; d.w = wp.data_ptr(); d.N = N
     d.scale = scale.data_ptr(); d.bias = bias.data_ptr(); d.act = act; d.mode = mode
-    d.out = out.data_ptr(); d.out_cstride = N // (up * up); d.up = up; d.BN = BN; d.stages = stages; d.variant = variant
+    d.out = out.data_ptr(); d.out_cstride = N // (up * up); d.up = up; d.BN = BN; d.variant = variant
     if up == 2:
         d.convt_cout = N // 4; d.act = 0
     if tile: d.TW, d.TH, d.TN = tile
@@ -85,10 +84,6 @@ if os.environ.get("UG_CONFIGS") == "gate128":  # CoordAtt3 combine on 128-column
     CONFIGS = [dict(variant=5, mode=2), dict(variant=7, mode=2), dict(variant=7)]
 if os.environ.get("UG_CONFIGS") == "pair128":  # 128-column n-tiles: multi-issuer kernel with / without CTA pairs
     CONFIGS = [dict(variant=5), dict(variant=7), dict(variant=5, mode=2), dict(variant=7, mode=2)]
-if os.environ.get("UG_ABLATE"):
-    CONFIGS = [dict(variant=5, stages=108), dict(variant=5, stages=108, mode=2)]
-if os.environ.get("UG_ABLATE") == "resid":    # GATE epilogue with / without its residual loads (results wrong without)
-    CONFIGS = [dict(variant=5, mode=2), dict(variant=5, mode=2, stages=116)]
 for shp in SHAPES:
     B, H, W, Cin, N, R = shp
     fl = 2.0 * B * H * W * N * Cin * max(R, 1) ** 2
@@ -107,14 +102,6 @@ for shp in SHAPES:
         try:
             d, keep = make(*shp, **cfg)
             ms = timeit(d)
-            line = f"{shp} {cfg}: {ms:.3f} ms {fl / ms / 1e9:.0f} TF/s"
-            if cfg.get("variant", 0) == 2:
-                pr = eng.conv_profile(d)
-                line += " | " + " ".join(f"{k}={v:.0f}" for k, v in pr.items())
-            if cfg.get("variant", 0) in (5, 7) and cfg.get("mode", 0) == 0:
-                pr = eng.conv_profile16(d)
-                line += f" | clk {pr['prod_cycles'] / max(pr['prod_ns'], 1):.3f} GHz " + " ".join(
-                    f"{k}={v:.0f}" for k, v in pr.items())
-            print(line, flush=True)
+            print(f"{shp} {cfg}: {ms:.3f} ms {fl / ms / 1e9:.0f} TF/s", flush=True)
         except Exception as ex:
             print(shp, cfg, "ERR", ex, flush=True)

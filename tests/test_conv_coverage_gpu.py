@@ -256,6 +256,16 @@ COVER_CASES = [
     dict(B=3, H=16, W=8, Cin=64, N=64, R=3, mode=GATE, variant=6, expect=("pair", ("mode", GATE))),
     dict(B=4, H=16, W=8, Cin=128, N=64, R=3, mode=GATE, variant=6, expect=("pair", ("mode", GATE))),
 ]
+# the multi-issuer kernel does not read `stages`, whatever its value: large values on a K-split STORE layer, the
+# register-prefetched GATE layer of the first row, a TMA-residual GATE layer (24 images: three rounds per CTA) and a
+# pair-mode layer
+for _st in (101, 102, 104, 116):
+    COVER_CASES += [
+        dict(B=24, H=56, W=56, Cin=64, N=64, R=3, variant=5, stages=_st, expect=_ms(RELU, 9, STORE, 2)),
+        dict(B=24, H=56, W=56, Cin=128, N=64, R=3, mode=GATE, variant=5, stages=_st, expect=_ms(RELU, 9, GATE, 2)),
+        dict(B=24, H=56, W=56, Cin=64, N=64, R=3, mode=GATE, variant=5, stages=_st, expect=_ms(RELU, 9, GATE, 2, 1)),
+        dict(B=2, H=56, W=56, Cin=128, N=128, R=3, variant=7, stages=_st, expect=_ms(RELU, 9, STORE, 1, 0, 1)),
+    ]
 # one-tile and persistent GEMM kernels: every activation x every epilogue prepare accepts, and TN > 1
 for _v, _k in ((1, "onetile"), (2, "persistent")):
     for _a in (NONE, RELU, GELU):
@@ -336,6 +346,12 @@ UNREACHABLE = [
     ("multi_pair: ConvTranspose", dict(B=2, H=14, W=14, Cin=512, N=2048, R=1, up=2, act=0, variant=7),
      "conv(multi, pairs): 3x3 layers with 128-column n-tiles"),
 ]
+# ... descriptors with a variant outside {0, 1, 2, 5, 6, 7}, which ug_conv rejects with UG_EINVAL as well (row taps
+# too, whose branch of prepare would otherwise accept any variant but 1 and 2) ...
+REJECTED = [(f"variant {v}", dict(B=2, H=56, W=56, Cin=64, N=64, R=3, variant=v), f"conv: unknown variant {v}")
+            for v in (3, 4, 8)]
+REJECTED.append(("row taps, variant 3", dict(B=2, H=56, W=56, Cin=64, N=64, R=4, rowtap=True, variant=3),
+                 "conv: unknown variant 3"))
 # ... or the kernel prepare runs instead: every row-tap layer goes to the single-CTA multi kernel, whatever the variant
 ROUTED = [
     ("multi_pair: row taps", dict(B=2, H=56, W=56, Cin=64, N=128, R=4, rowtap=True, variant=7), "multi"),
@@ -463,7 +479,8 @@ def test_conv_case(engine, query, src, case):
 # ------------------------------------------------------------------------------------------------ coverage
 def test_coverage(engine, query):
     """Every instantiation of ug_conv_instances and every configuration class is run by some case; the classes listed
-    as unreachable are rejected (or routed elsewhere) by prepare as stated."""
+    as unreachable are rejected (or routed elsewhere) by prepare as stated, and an unknown variant is rejected with
+    UG_EINVAL by the launch-plan query and by ug_conv, which writes nothing."""
     insts = {k: [] for k in all_instances(query)}
     classes = {k: [] for k in CLASSES}
     lines = []
@@ -485,6 +502,15 @@ def test_coverage(engine, query):
         with pytest.raises(RuntimeError) as ex:
             query.info(build(case).desc)
         assert err in str(ex.value), f"{name}: prepare says {ex.value}"
+    for name, case, err in REJECTED:
+        b = build(case)
+        before = [t.clone() for t in b.tensors]
+        with pytest.raises(RuntimeError, match=f"rc -1: {err}"):
+            query.info(b.desc)
+        with pytest.raises(RuntimeError, match=f"ugnet error -1: {err}"):
+            engine.run_op(b.desc)
+        torch.cuda.synchronize()
+        assert all(torch.equal(t, t0) for t, t0 in zip(b.tensors, before)), f"{name}: a rejected descriptor wrote"
     for name, case, kernel in ROUTED:
         assert query.info(build(case).desc)["kernel"] == kernel, name
     missing_i = [k for k, v in insts.items() if not v]

@@ -270,8 +270,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_persistent_kernel(const
     int stage = 0;
     uint32_t phase = 0;
     const uint32_t tx_bytes = p.a_bytes + p.b_bytes;
-    long long w_empty = 0;
-    const long long t_start = clock64();
     for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
       // (m-major order: the n-tiles of a pixel tile run on neighbouring CTAs at the same time and share its HBM read)
       const int mt = p.m_major ? t / p.n_tiles : t % p.m_tiles, nt = p.m_major ? t % p.n_tiles : t / p.m_tiles;
@@ -282,9 +280,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_persistent_kernel(const
       for (int tap = 0; tap < p.R * p.S; ++tap) {
         const int r = tap / p.S, s = tap % p.S;
         for (int kc = 0; kc < p.kchunks; ++kc, ++it) {
-          const long long tw0 = p.prof ? clock64() : 0;
           mbar_wait(&empty[stage], phase ^ 1);
-          if (p.prof) w_empty += clock64() - tw0;
           if (elect_one_sync()) {
             mbar_arrive_expect_tx(&full[stage], tx_bytes);
             tma_load_4d(sA + stage * kABytesPerStage, &tmA, &full[stage], kc * 64, x0 + s - p.pad, y0 + r - p.pad, n0);
@@ -298,26 +294,17 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_persistent_kernel(const
         }
       }
     }
-    if (p.prof && lane == 0) {
-      p.prof[blockIdx.x * 8 + 0] = w_empty;
-      p.prof[blockIdx.x * 8 + 1] = clock64() - t_start;
-    }
   } else if (warp == kMmaWarp) {
     // ------------------------------------------------------------------ MMA issuer (whole warp, elected lane issues)
     const uint32_t idesc = umma_idesc_bf16(128, p.BN);
     int stage = 0, acc = 0;
     uint32_t phase = 0, acc_phase = 0;
-    long long w_full = 0, w_acc = 0;
     for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
-      long long tw0 = p.prof ? clock64() : 0;
       mbar_wait(&acc_empty[acc], acc_phase ^ 1);  // epilogue has drained this accumulator
-      if (p.prof) w_acc += clock64() - tw0;
       tc_fence_after();
       const uint32_t d_tmem = tmem_base + acc * p.BN;
       for (int it = 0; it < p.num_k; ++it) {
-        tw0 = p.prof ? clock64() : 0;
         mbar_wait(&full[stage], phase);
-        if (p.prof) w_full += clock64() - tw0;
         tc_fence_after();
         const uint64_t ad = umma_desc_sw128(smem_u32(sA + stage * kABytesPerStage));
         const uint64_t bd = umma_desc_sw128(smem_u32(sB + stage * b_stage_bytes));
@@ -341,16 +328,11 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_persistent_kernel(const
         acc_phase ^= 1;
       }
     }
-    if (p.prof && lane == 0) {
-      p.prof[blockIdx.x * 8 + 2] = w_full;
-      p.prof[blockIdx.x * 8 + 3] = w_acc;
-    }
   } else {
     // ------------------------------------------------------------------ epilogue (4 warps, 1 pixel / thread)
     const int q = warp & 3;
     const int row = q * 32 + lane;
     const int etid = threadIdx.x;  // 0..127
-    long long w_accfull = 0, w_obuf = 0, t_proc = 0, t_store = 0;
     const int tx = row % p.TW;
     const int trest = row / p.TW;
     const int ty = trest % p.TH;
@@ -385,9 +367,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_persistent_kernel(const
       const float* gate_row = p.gate + (long long)n * p.N + ncol0;
       uint8_t* so_row = sO + obuf * obuf_bytes + row * 128;
 
-      long long tw0 = p.prof ? clock64() : 0;
       mbar_wait(&acc_full[acc], acc_phase);
-      if (p.prof) { const long long c = clock64(); w_accfull += c - tw0; tw0 = c; }
       tc_fence_after();
       if (p.tma_store) {
         // the TMA store that last read this staging buffer must have finished reading it
@@ -397,7 +377,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_persistent_kernel(const
         }
         named_bar_sync(1, 128);
       }
-      if (p.prof) { const long long c = clock64(); w_obuf += c - tw0; tw0 = c; }
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * p.BN;
       float dot = 0.0f;
       const int ncols = min(p.BN, p.N - ncol0);  // valid columns of this n-tile (multiple of 8)
@@ -439,7 +418,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_persistent_kernel(const
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&acc_empty[acc]);
-      if (p.prof) { const long long c = clock64(); t_proc += c - tw0; tw0 = c; }
       if (++acc == p.acc_stages) {
         acc = 0;
         acc_phase ^= 1;
@@ -489,15 +467,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_persistent_kernel(const
         }
         obuf ^= 1;  // two staging buffers: the barrier of the next tile orders reuse
       }
-      if (p.prof) t_store += clock64() - tw0;
     }
     if (p.tma_store && etid == 0) bulk_wait_group_all();
-    if (p.prof && etid == 0) {
-      p.prof[blockIdx.x * 8 + 4] = w_accfull;
-      p.prof[blockIdx.x * 8 + 5] = w_obuf;
-      p.prof[blockIdx.x * 8 + 6] = t_proc;
-      p.prof[blockIdx.x * 8 + 7] = t_store;
-    }
   }
 
   tc_fence_before();
@@ -557,6 +528,8 @@ int conv_prepare(ug_engine* h, const ug_conv_desc* d, ConvLaunch* L) {
   if (d->B <= 0 || d->H <= 0 || d->W <= 0 || d->Cin <= 0 || d->N <= 0)
     return set_error(h, UG_EINVAL, "conv: non-positive shape");
   if (d->act < UG_ACT_NONE || d->act > UG_ACT_GELU) return set_error(h, UG_EINVAL, "conv: unknown activation");
+  if (!(d->variant == 0 || d->variant == 1 || d->variant == 2 || (d->variant >= 5 && d->variant <= 7)))
+    return set_error(h, UG_EINVAL, "conv: unknown variant %d (0, 1, 2, 5, 6 or 7)", d->variant);
   const bool rowtaps = d->R > 1 && d->S == 1 && d->pad == 0 && d->up != 2 && d->Cin <= 64;   // ug_conv_desc.in_rstride
   if (!rowtaps && (d->R <= 0 || d->S <= 0 || 2 * d->pad != d->R - 1 || d->R != d->S))
     return set_error(h, UG_EINVAL, "conv: only square stride-1 'same' filters (2*pad == R-1) or R x 1 row taps are supported");

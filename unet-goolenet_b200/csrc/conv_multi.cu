@@ -236,10 +236,6 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
     int as[kMI] = {0, 0};
     uint32_t aph[kMI] = {0, 0};
     const uint32_t a_tx = kTaps == 9 ? (uint32_t)(hp.pitch * (hp.TH + 2) * 128) : p.a_bytes;
-    long long w_a = 0;
-    const long long t_start = clock64();
-    unsigned long long ns0 = 0;
-    if (p.prof) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(ns0));
     for (int s = cta0; s < total_super; s += ncta) {
       int nt, ms;
       decode(s, nt, ms);
@@ -259,15 +255,11 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
           if (kTaps == 1 && hp.rowtaps == 2 && kc > 0) continue;   // row halo: the tile's single box was loaded at kc == 0
           const int x0 = cx[i], y0 = cy[i], n = cn[i];
           const int slot = i * hp.sa + as[i];
-          const long long tw0 = p.prof ? clock64() : 0;
           mbar_wait(&a_empty[slot], aph[i] ^ 1);
-          if (p.prof) w_a += clock64() - tw0;
           if (elect_one_sync()) {
             if constexpr (kPair) {   // the leader's barrier collects the bytes of both CTAs' loads
               if (rank == 0) mbar_arrive_expect_tx(&a_full[slot], 2 * a_tx);
               tma_load_4d_pair(sA + slot * hp.a_stage_bytes, &tmA, leader_addr(&a_full[slot]), kc * 64, x0 - 1, y0 - 1, n);
-            } else if ((hp.debug & 4) && s >= (int)gridDim.x * 2) {
-              mbar_arrive(&a_full[slot]);
             } else {
               mbar_arrive_expect_tx(&a_full[slot], a_tx);
               if (kTaps == 9) tma_load_4d(sA + slot * hp.a_stage_bytes, &tmA, &a_full[slot], kc * 64, x0 - 1, y0 - 1, n);
@@ -283,17 +275,9 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
         }
       }
     }
-    if (p.prof && lane == 0) {
-      unsigned long long ns1;
-      asm volatile("mov.u64 %0, %globaltimer;" : "=l"(ns1));
-      p.prof[blockIdx.x * 16 + 0] = w_a;
-      p.prof[blockIdx.x * 16 + 2] = clock64() - t_start;
-      p.prof[blockIdx.x * 16 + 3] = (long long)(ns1 - ns0);
-    }
   } else if (warp == kMAllocWarp) {
     // ------------------------------------------------------------------ weight producer (its own warp: a full weight
     // ring must not delay the activation loads of the next chunk, and vice versa)
-    long long w_b = 0;
     if (hp.b_resident) {
       if (elect_one_sync()) {
         if constexpr (kPair) {
@@ -321,10 +305,12 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
         int nt, ms_unused;
         decode(s, nt, ms_unused);
         for (int kc = 0; kc < p.kchunks; ++kc) {
+          // (CTA pairs: rolled.  Fully unrolled, the pair forms grow by ~430 SASS instructions, and this warp shares its
+          // SMSP's 6 KB L0 instruction cache with two epilogue warps, DESIGN.md §3.1.  The single-CTA forms were
+          // measured fully unrolled.)
+#pragma unroll (kPair ? 1 : kTaps)
           for (int tap = 0; tap < kTaps; ++tap) {
-            const long long tw0 = p.prof ? clock64() : 0;
             mbar_wait(&b_empty[bs], bph ^ 1);
-            if (p.prof) w_b += clock64() - tw0;
             if (elect_one_sync()) {
               if constexpr (kPair) {
                 if (rank == 0) mbar_arrive_expect_tx(&b_full[bs], (uint32_t)(2 * b_tile_bytes));
@@ -344,7 +330,6 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
         }
       }
     }
-    if (p.prof && lane == 0) p.prof[blockIdx.x * 16 + 1] = w_b;
   } else if ((kRT && kPair) && warp == kResidWarp) {
     resid_loop();   // (this warp executed pdl_wait above)
   } else if (warp >= kMIssuerWarp0 && rank != 0) {
@@ -357,8 +342,6 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
     const uint32_t idesc = umma_idesc_bf16(kPair ? 256 : 128, p.BN);
     int as = 0, bs = 0, acc = 0;
     uint32_t aph = 0, bph = 0, acc_phase = 0;
-    long long w_af = 0, w_bf = 0, w_acc = 0;
-    const long long t_start = clock64();
     if (hp.b_resident) {
       mbar_wait(&b_full[0], 0);
       tc_fence_after();
@@ -370,9 +353,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
       const bool valid = tile_live(tile_of(ms, i));
       uint32_t d_tmem = 0;
       if (valid) {
-        const long long tw0 = p.prof ? clock64() : 0;
         mbar_wait(&acc_empty[i * p.acc_stages + acc], acc_phase ^ 1);
-        if (p.prof) w_acc += clock64() - tw0;
         tc_fence_after();
         d_tmem = tmem_base + ((i * p.acc_stages + acc) * kKS + h) * p.BN;
       }
@@ -381,9 +362,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
         const bool row_halo = kTaps == 1 && hp.rowtaps == 2;
         if (valid) {
           if (!(row_halo && kc > 0)) {
-            const long long tw0 = p.prof ? clock64() : 0;
             mbar_wait(&a_full[i * hp.sa + as], aph);
-            if (p.prof) w_af += clock64() - tw0;
             tc_fence_after();
           }
           ad0 = kTaps == 9 ? umma_desc_sw128_sbo(smem_u32(sA + (i * hp.sa + as) * hp.a_stage_bytes), hp.sbo)
@@ -399,9 +378,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
           if (hp.b_resident) {
             b_addr = sB_u32 + (kc * kTaps + tap) * b_tile_bytes;
           } else if (mine) {
-            const long long tw0 = p.prof ? clock64() : 0;
             mbar_wait(&b_full[bs], bph);
-            if (p.prof) w_bf += clock64() - tw0;
             tc_fence_after();
             b_addr = sB_u32 + bs * b_tile_bytes;
           }
@@ -450,12 +427,6 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
         }
       }
     }
-    if (p.prof && lane == 0 && h == 0 && !((hp.debug & 8) && i == 1)) {
-      p.prof[blockIdx.x * 16 + 4 + i * 4 + 0] = w_af;
-      p.prof[blockIdx.x * 16 + 4 + i * 4 + 1] = w_bf;
-      p.prof[blockIdx.x * 16 + 4 + i * 4 + 2] = w_acc;
-      p.prof[blockIdx.x * 16 + 4 + i * 4 + 3] = clock64() - t_start;
-    }
   } else if (warp < 4 * kMI) {
     // ------------------------------------------------------------------ epilogue (4 warps per issuer)
     const int i = warp >> 2;
@@ -474,8 +445,6 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
     uint8_t* sOi = sO + i * p.obufs * obuf_bytes;
     int acc = 0, obuf = 0;
     uint32_t acc_phase = 0;
-    long long e_wacc = 0, e_wobuf = 0, e_tiles = 0, e_loop = 0, e_tail = 0;
-    const long long e_start = clock64();
 
     // Residual (ADD / GATE) rows: 16-byte pieces of this thread's own pixel row, prefetched into registers ONE
     // SUB-TILE AHEAD (right after the chunk loop of the previous sub-tile, whose residual registers are dead by
@@ -497,7 +466,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
                                 ((long long)y2 * p.W + x2) * p.add_cstride + col2;
 #pragma unroll
       for (int g = 0; g < 8; ++g)
-        addv[g] = (v2 && col2 + g * 8 < p.N && !(hp.debug & 16)) ? __ldg(reinterpret_cast<const uint4*>(ar + g * 8)) : make_uint4(0, 0, 0, 0);
+        addv[g] = (v2 && col2 + g * 8 < p.N) ? __ldg(reinterpret_cast<const uint4*>(ar + g * 8)) : make_uint4(0, 0, 0, 0);
     };
     if (has_add) {
       int s0 = cta0;
@@ -511,7 +480,6 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
       decode(s, nt, ms);
       const int mt = tile_of(ms, i);
       if (!tile_live(mt)) continue;
-      ++e_tiles;
       const int t1 = hp.d_tx.div(mt), t2 = hp.d_ty.div(t1);
       const int x0 = (mt - t1 * p.tiles_x) * p.TW;
       const int y0 = (t1 - t2 * p.tiles_y) * p.TH;
@@ -523,9 +491,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
       const float* gate_row = p.gate + (long long)n * p.N + ncol0;
       const int ncols = min(p.BN, p.N - ncol0);
       if (kMode == UG_EPI_GATE && etid < ncols && n < p.B) sGate[i * 128 + etid] = 1.0f + __ldg(gate_row + etid);
-      long long tw0 = p.prof ? clock64() : 0;
       mbar_wait(&acc_full[i * p.acc_stages + acc], acc_phase);
-      if (p.prof) e_wacc += clock64() - tw0;
       tc_fence_after();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + (i * p.acc_stages + acc) * kKS * p.BN;
       float dot = 0.0f;
@@ -533,22 +499,12 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
       uint32_t v[16];
       uint32_t v2[kKS == 2 ? 16 : 1];   // partial sums of the second K-half
       __syncwarp();
-      if (hp.debug & 1) {
-#pragma unroll
-        for (int j = 0; j < 16; ++j) v[j] = 0u;
-        if (kKS == 2) {
-#pragma unroll
-          for (int j = 0; j < (kKS == 2 ? 16 : 1); ++j) v2[j] = 0u;
-        }
-      } else {
-        tmem_ld16(taddr, v);
-        if constexpr (kKS == 2) tmem_ld16(taddr + p.BN, reinterpret_cast<uint32_t(&)[16]>(v2));
-      }
+      tmem_ld16(taddr, v);
+      if constexpr (kKS == 2) tmem_ld16(taddr + p.BN, reinterpret_cast<uint32_t(&)[16]>(v2));
       for (int sub = 0; sub * 64 < ncols; ++sub) {
         if (p.tma_store) {
           // staging buffer `obuf` must no longer be read by the TMA store issued obufs sub-tiles ago
           // (the barrier also publishes sGate of this tile)
-          tw0 = p.prof ? clock64() : 0;
           if constexpr (smem_add) {
             // the store of the previous sub-tile (other buffer) has finished reading: hand that buffer to the residual
             // producer for the NEXT sub-tile, then wait for this sub-tile's residual (loaded one sub-tile ago)
@@ -563,14 +519,12 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
             else bulk_wait_group_read<0>();
           }
           named_bar_sync(1 + i, 128);
-          if (p.prof) e_wobuf += clock64() - tw0;
         }
         uint8_t* so_row = sOi + obuf * obuf_bytes + srow * 128;
         // the chunk loop is not unrolled (kEpiUnroll): the epilogue warps of an SMSP share its 6 KB L0 instruction
         // cache with an MMA issuer / producer warp; with run-time epilogue modes a 4x larger loop body measurably slowed
         // the MMA issue (0.24 -> 0.29 ms), and x2 / x4 unrolling of this loop measured neutral / slower
         // (profiles/r02_epilogue_unroll.txt)
-        const long long tl0 = p.prof ? clock64() : 0;
 #pragma unroll kEpiUnroll
         for (int cc = 0; cc < 4; ++cc) {
           const int c0 = sub * 64 + cc * 16;
@@ -583,7 +537,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
           float f[16];
           epi_math16_linear<kAct>(v, f, sScale, sBias, ncol0 + c0);   // ReLU deferred (see conv_common.cuh)
           __syncwarp();
-          if (c0 + 16 < ncols && !(hp.debug & 1)) {
+          if (c0 + 16 < ncols) {
             tmem_ld16(taddr + c0 + 16, v);
             if constexpr (kKS == 2) tmem_ld16(taddr + p.BN + c0 + 16, reinterpret_cast<uint32_t(&)[16]>(v2));
           }
@@ -646,7 +600,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
                 o.w = pack_bf16x2(f[g * 8 + 6], f[g * 8 + 7]);
               }
               const int chunk = cc * 2 + g;
-              if (!(hp.debug & 2) && (!strip || row_in_tile)) *reinterpret_cast<uint4*>(so_row + ((chunk ^ (srow & 7)) << 4)) = o;
+              if (!strip || row_in_tile) *reinterpret_cast<uint4*>(so_row + ((chunk ^ (srow & 7)) << 4)) = o;
               if (p.pool && !strip) {
                 // fused nn.MaxPool2d(2): the 2x2 window of pixel (tx, ty) lives in lanes ^1 (x) and ^8 (y) of this
                 // warp (row = ty*8 + tx); max of the rounded bf16 values == rounded max (rounding is monotonic)
@@ -667,8 +621,6 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
             }
           }
         }
-        const long long tl1 = p.prof ? clock64() : 0;
-        if (p.prof) e_loop += tl1 - tl0;
         if (kMode == UG_EPI_OUTC) continue;
         if ((sub + 1) * 64 >= ncols) {  // all TMEM reads of this accumulator are done: hand it back to the MMA issuer
           tc_fence_before();
@@ -717,7 +669,7 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
           }
         }
         named_bar_sync(1 + i, 128);
-        if (etid == 0 && !(hp.debug & 2)) {
+        if (etid == 0) {
           const int col = ncol0 + sub * 64;
           if (p.up == 2) {  // ConvTranspose 2x2 s2: column block -> quadrant (dy,dx) map, channel inside the quadrant
             const int qd = col / p.convt_cout;
@@ -760,7 +712,6 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
             p.stats_max[o] = mx;
           }
         }
-        if (p.prof) e_tail += clock64() - tl1;
         if (p.obufs == 2) obuf ^= 1;
       }
       if (kMode == UG_EPI_OUTC) {
@@ -784,16 +735,6 @@ __global__ void __launch_bounds__(kMultiThreads(kKS, kRT && kPair), 1) conv_mult
       }
     }
     if (p.tma_store && etid == 0) bulk_wait_group_all();
-    if (p.prof && etid == 0 && i == 0) {
-      p.prof[blockIdx.x * 16 + 12] = e_wacc;
-      p.prof[blockIdx.x * 16 + 13] = e_wobuf;
-      p.prof[blockIdx.x * 16 + 14] = clock64() - e_start;
-      p.prof[blockIdx.x * 16 + 15] = e_tiles;
-      if (hp.debug & 8) {  // finer epilogue split in the slots of issuer 1 (profiling runs only)
-        p.prof[blockIdx.x * 16 + 9] = e_loop;
-        p.prof[blockIdx.x * 16 + 10] = e_tail;
-      }
-    }
   }
 
   tc_fence_before();
@@ -996,7 +937,6 @@ int conv_multi_prepare(ug_engine* h, const ug_conv_desc* d, int BN, ConvLaunch* 
   hp.m_major = n_tiles > 1 ? 1 : 0;
   hp.d_nt = make_fastdiv(n_tiles);
   hp.d_pitch = make_fastdiv(pitch);
-  hp.debug = d->stages >= 100 ? d->stages - 100 : 0;  // profiling ablations (scripts/conv_prof.py)
   L->kernel = pair ? ConvKernel::MultiPair : ConvKernel::Multi;
   L->multi_fn = nullptr;
   for (int i = 0; i < (int)(sizeof(kMultiInstances) / sizeof(kMultiInstances[0])); ++i) {

@@ -72,7 +72,6 @@ struct ConvKParams {
   int stage_copy;  // ConvTranspose scatter: stage the tile in smem, then coalesced cooperative copy-out
   void* out2;      // second destination of a split 1x1 GEMM (see ug_conv_desc.out2): columns >= n_split
   int out2_cstride, n_split, n1;
-  long long* prof;  // optional per-CTA cycle counters [grid][8] (debug / profiling builds of the plan)
 };
 
 // Division by a launch-time constant as multiply + shift (exact for n < 2^24): the role loops decode a tile index
@@ -113,9 +112,6 @@ struct MultiParams {
                       // y0 + kc); 2: ONE box of TH + R - 1 rows per tile, tap kc reads it TW * 128 * kc bytes further in
                       // (a "row halo": the window rows of neighbouring taps are the same bytes)
   int resid_tma;      // kRT kernels: residual tiles arrive by TMA in the staging buffers (see the header comment)
-  int debug;          // ablation switches for profiling (results are wrong when set): 1 = no TMEM loads,
-                      // 2 = no staging stores / TMA store, 4 = activation TMA loads only for the first stages,
-                      // 16 = no residual loads (ADD / GATE epilogues)
 };
 
 struct StoreMaps {  // output maps: [0] for plain stores, [q] = quadrant (dy,dx) of a ConvTranspose 2x2 s2 scatter;

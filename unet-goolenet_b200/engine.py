@@ -10,7 +10,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libugnet.so")
-# UG_DEV_LIB=1 (scripts/ only): load libugnet_dev.so = the same objects + the profiling / micro-benchmark hooks of
+# UG_DEV_LIB=1 (scripts/ only): load libugnet_dev.so = the same objects + the micro-benchmark and launch-plan hooks of
 # include/ugnet_dev.h, which are not part of the product ABI
 DEV_LIB_PATH = os.path.join(_HERE, "libugnet_dev.so")
 USE_DEV_LIB = os.environ.get("UG_DEV_LIB", "0") == "1"
@@ -158,8 +158,8 @@ EXPORTED_SYMBOLS = ["ug_version", "ug_create", "ug_destroy", "ug_last_error", "u
                     "ug_wavelet_ragged_workspace_bytes",
                     "ug_plan_load", "ug_plan_num_io", "ug_plan_io_name", "ug_plan_io", "ug_plan_device_bytes",
                     "ug_plan_program", "ug_plan_copy_in", "ug_plan_copy_out", "ug_plan_run", "ug_plan_destroy"]
-DEV_SYMBOLS = ["ug_conv_profile", "ug_conv_profile16", "ug_mma_microbench", "ug_mma_microbench2",
-               "ug_mma_microbench_pair", "ug_conv_launch_info", "ug_conv_instances", "ug_memop_launch_info"]
+DEV_SYMBOLS = ["ug_mma_microbench", "ug_mma_microbench2", "ug_mma_microbench_pair", "ug_conv_launch_info",
+               "ug_conv_instances", "ug_memop_launch_info"]
 
 _lib = None
 
@@ -187,9 +187,7 @@ def load_library():
     if USE_DEV_LIB:
         lib.ug_mma_microbench.argtypes = [_vp, _i, _i, _i, _i, _i, C.POINTER(C.c_double)]
         lib.ug_mma_microbench2.argtypes = [_vp, _i, _i, _i, _i, _i, _i, _i, _i, C.POINTER(C.c_double)]
-        lib.ug_conv_profile16.argtypes = [_vp, _vp, _vp, C.POINTER(C.c_double)]
         lib.ug_mma_microbench_pair.argtypes = [_vp, _i, _i, _i, C.POINTER(C.c_double)]
-        lib.ug_conv_profile.argtypes = [_vp, _vp, _vp, C.POINTER(C.c_double)]
     lib.ug_program_create.argtypes = [_vp, _vp, _i, C.POINTER(_vp)]
     lib.ug_program_run.argtypes = [_vp, _vp, _vp]
     lib.ug_program_num_launches.argtypes = [_vp]
@@ -458,25 +456,6 @@ class Engine:
         s = stream if stream is not None else torch.cuda.current_stream().cuda_stream
         fn = getattr(self.lib, _SINGLE_ENTRY[_DESC_KIND[type(desc)]])
         self._check(fn(self.handle, C.byref(desc), s))
-
-    def conv_profile(self, desc, stream=None):
-        """Per-role cycle counters of the persistent conv kernel for one op (ugnet_dev.h; needs UG_DEV_LIB=1)."""
-        s = stream if stream is not None else torch.cuda.current_stream().cuda_stream
-        out = (C.c_double * 10)()
-        self._check(self.lib.ug_conv_profile(self.handle, C.byref(desc), s, out))
-        keys = ["prod_wait_empty", "prod_total", "mma_wait_full", "mma_wait_acc", "epi_wait_acc", "epi_wait_obuf",
-                "epi_math", "epi_store", "ctas", "tiles_per_cta"]
-        return dict(zip(keys, list(out)))
-
-    def conv_profile16(self, desc, stream=None):
-        """Per-role cycle counters of the multi-issuer 3x3 kernel for one op (ugnet_dev.h; needs UG_DEV_LIB=1)."""
-        s = stream if stream is not None else torch.cuda.current_stream().cuda_stream
-        out = (C.c_double * 16)()
-        self._check(self.lib.ug_conv_profile16(self.handle, C.byref(desc), s, out))
-        keys = ["prod_wait_a", "prod_wait_b", "prod_cycles", "prod_ns", "i0_wait_a", "i0_wait_b", "i0_wait_acc",
-                "i0_cycles", "i1_wait_a", "i1_wait_b", "i1_wait_acc", "i1_cycles", "epi_wait_acc", "epi_wait_obuf",
-                "epi_cycles", "epi_tiles"]
-        return dict(zip(keys, list(out)))
 
     def program(self, descs, keepalive=()):
         return Program(self, descs, keepalive)
