@@ -349,6 +349,34 @@ typedef struct ug_source_frame_desc {
   int B, S, Hs, Ws, h, w;
 } ug_source_frame_desc;
 
+/* Segmentation metrics against ground truth: per image i, with P = {pred != 0} and G = {gt != 0} (masks of 0/1 or
+ * 0/255 alike) of the same H x W, placed like ug_source_frame_desc's mask (index[i] for a ragged batch, else Hs x Ws at
+ * pixel offset i*Hs*Ws):
+ *   counts[i] = {tp, fp, fn} = {|P n G|, |P \ G|, |G \ P|};
+ *   the surface dX of a set X is the pixels of X with a 4-neighbour outside X (outside the image counts as outside X:
+ *   X & ~binary_erosion(X, generate_binary_structure(2, 1), border_value=0)); d_PG(p) is the Euclidean distance in
+ *   pixels from p in dP to the nearest pixel of dG, d_GP the same the other way round;
+ *   hd[i] = {HD, HD95} = {max(max d_PG, max d_GP), max(pct95(d_PG), pct95(d_GP))} in fp64, pct95 being
+ *   np.percentile(d, 95) with numpy's default linear method; both +inf when exactly one surface is empty and NaN when
+ *   both are.  Dice and IoU follow from the counts (host side).
+ * The table may come from outside the library (a plan image's host): an entry with a negative offset, a side outside
+ * [1, 8*224] or an extent past capacity_px is rejected: nothing is read or written through it, counts[i] = {0,0,0},
+ * hd[i] = {NaN, NaN} and status[i] = 1 (0 otherwise; status is optional).  The launch geometry depends on B and Hs /
+ * the largest side allowed only, never on the table.  Worst-case time is linear in the pixels (exact separable EDT
+ * restricted to the bounding box of P u G, integer radix select); the outputs are bit-identical run to run. */
+typedef struct ug_seg_metrics_desc {
+  const unsigned char* pred;       /* u8: image i at pred + px_offset (ragged) or pred + i*Hs*Ws */
+  const unsigned char* gt;         /* u8, placed like pred */
+  const ug_ragged_image* index;    /* optional device table [B]; NULL = every image is Hs x Ws */
+  int* status;                     /* optional int32 [B]: 1 = entry rejected */
+  int* counts;                     /* int32 [B][3]: tp, fp, fn */
+  double* hd;                      /* fp64 [B][2]: HD, HD95 */
+  void* workspace;                 /* >= ug_seg_metrics_workspace_bytes(B, capacity_px or B*Hs*Ws) */
+  size_t workspace_bytes;
+  long long capacity_px;           /* ragged: pixels of pred / gt; unused when index is NULL */
+  int B, Hs, Ws;
+} ug_seg_metrics_desc;
+
 enum {
   UG_OP_CONV = 1,
   /* 2 and 10 were the stand-alone im2col packs of round 1 (replaced by UG_OP_STEM); the numbers stay retired */
@@ -367,7 +395,8 @@ enum {
   UG_OP_RESIZE_RAGGED = 16,
   UG_OP_WAVELET_RAGGED = 17,
   UG_OP_CAM = 18,
-  UG_OP_SOURCE_FRAME = 19
+  UG_OP_SOURCE_FRAME = 19,
+  UG_OP_SEG_METRICS = 20
 };
 
 typedef struct ug_op {
@@ -391,6 +420,7 @@ typedef struct ug_op {
     ug_wavelet_ragged_desc wavelet_ragged;
     ug_cam_desc cam; /* smaller than ug_conv_desc as well */
     ug_source_frame_desc source_frame; /* and so is this one */
+    ug_seg_metrics_desc seg_metrics;   /* as is this one */
   } u;
 } ug_op;
 
@@ -419,8 +449,11 @@ int ug_resize_ragged(ug_handle h, const ug_resize_ragged_desc* d, void* stream);
 int ug_wavelet_ragged(ug_handle h, const ug_wavelet_ragged_desc* d, void* stream);
 int ug_cam(ug_handle h, const ug_cam_desc* d, void* stream);
 int ug_source_frame(ug_handle h, const ug_source_frame_desc* d, void* stream);
+int ug_seg_metrics(ug_handle h, const ug_seg_metrics_desc* d, void* stream);
 size_t ug_wavelet_workspace_bytes(int B, int H, int W);
 size_t ug_wavelet_ragged_workspace_bytes(int B, long long capacity_px);
+/* Workspace of ug_seg_metrics for B images in capacity_px pixels (ragged capacity, or B*Hs*Ws); 0 for bad arguments. */
+size_t ug_seg_metrics_workspace_bytes(int B, long long capacity_px);
 
 /* Programs: a validated op list with tensor maps and launch geometry prepared once; run = launches only. */
 int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out);
@@ -468,7 +501,10 @@ int ug_program_run_host_pipelined(ug_handle h, ug_program p, const ug_copy* h2d,
  * "cam" f32 [B,7,7] and "cam_map" f32 [B,224,224] (the map in the UNet input frame, inside the ROI box).  A plan
  * exported with source_frame=True (a plan with a uint8 or ragged source) also reports the outputs at each image's own
  * size (ug_source_frame_desc): "src_mask" u8 [B,Hs,Ws] (ragged: [P], image i at px_offset), "src_boxes" i32 [B,4]
- * and, with cam=True, "src_cam_map" f32 [B,Hs,Ws] (ragged: [P]). */
+ * and, with cam=True, "src_cam_map" f32 [B,Hs,Ws] (ragged: [P]).  A plan exported with seg_metrics="input" or
+ * "source" (export_plan(B, ..., seg_metrics=...)) also scores the mask against ground truth (ug_seg_metrics_desc): it
+ * takes "gt_mask" u8, [B,224,224] for "input" (against "mask") or placed like "src_mask" for "source" (against
+ * "src_mask"), and reports "seg_counts" i32 [B,3] (tp, fp, fn) and "seg_hd" f64 [B,2] (HD, HD95). */
 typedef struct ug_plan_s* ug_plan;
 /* Parses the image (host memory, may be freed afterwards), allocates ONE device arena for every buffer of the plan
  * (ug_plan_device_bytes), uploads the constants, relocates the op list and prepares the program. */

@@ -146,6 +146,83 @@ def _grade_ragged(runner, gray_images, filenames, cam_dir=None, mask_dir=None, f
     return records
 
 
+@torch.no_grad()
+def evaluate_images(pipeline, gray_images, gt_masks, labels, filenames, frame="source", save_dir=None):
+    """grade_images plus ground truth (分割/main.py val and 分类/ROI_main.py's scores on the device path): per chunk the
+    wavelet step, the pipeline program and its metrics op (PipelineRunner.plan(seg_metrics=frame)).
+
+    gray_images / filenames as grade_images (a uint8 [N,H,W] batch or a list of [H_i,W_i] images); gt_masks: one mask
+    per image, nonzero = foreground, at each image's own size (frame="source") or 224x224 (frame="input"), as a list or
+    an [N,...] array; labels: N class labels, or None.
+    Returns (rows, summary): rows are dicts name, pred, label, tp, fp, fn, dice, iou, hd, hd95 in the order of
+    result.txt; summary holds the means of dice / iou / hd95 over the images where they are finite, how many were NaN
+    (empty ground truth, or no surface at all) and inf (one surface empty) and left out, and with labels the
+    metrics.classification_metrics dict under "classification".  With save_dir, writes result.txt exactly as
+    grade_images and metrics.csv (the rows, same order)."""
+    from . import metrics
+    from .util import ragged
+    from .util.wavelet import wavelet_enhance_batch, wavelet_ragged_into
+    if frame not in ("input", "source"):
+        raise ValueError(f"frame must be 'input' or 'source', got {frame!r}")
+    runner = getattr(pipeline, "runner", pipeline)
+    n = len(gray_images)
+    if len(gt_masks) != n or len(filenames) != n or (labels is not None and len(labels) != n):
+        raise ValueError("gray_images, gt_masks, filenames and labels must have one entry per image")
+    logits, counts, hds = [], [], []
+    if isinstance(gray_images, (list, tuple)):
+        packed = ragged.pack(gray_images, 1, min_side=ragged.WAVELET_MIN_SIDE, max_side=ragged.MAX_RATIO * 224)
+        gt = metrics.gt_batch(list(gt_masks) if frame == "source" else gt_masks, gray_images, packed, frame)
+        for s, c in runner._chunks(n):
+            part = ragged.chunk(packed, s, s + c)
+            ws = runner.plan(c, source="ragged", capacity=part.n_px, source_frame=frame == "source", seg_metrics=frame)
+            gray = part.data.to(runner.dev, non_blocking=True)
+            ws["src_index"].copy_(ragged.table_tensor(part.table))
+            if frame == "source":
+                ws["gt_mask"][:part.n_px].copy_(ragged.chunk(gt, s, s + c).data, non_blocking=True)
+            else:
+                ws["gt_mask"].copy_(gt[s:s + c])
+            wavelet_ragged_into(gray, ws["src_index"], ws["src_u8"], c)
+            ws["program"].run()
+            logits.append(ws["cls_logits"].cpu())
+            counts.append(ws["seg_counts"].cpu())
+            hds.append(ws["seg_hd"].cpu())
+        res = metrics.seg_result(torch.cat(counts), torch.cat(hds))
+        cls = torch.cat(logits)
+    else:
+        g = torch.as_tensor(np.ascontiguousarray(gray_images) if isinstance(gray_images, np.ndarray) else gray_images)
+        rgb = wavelet_enhance_batch(g.to(runner.dev))
+        out = runner(rgb, gt_masks=gt_masks, metrics_frame=frame)
+        cls, res = out[2].cpu(), out[-1]
+    pred = torch.argmax(torch.softmax(cls, dim=1), dim=1).numpy()                # test.py:86
+    rows = []
+    for i, name in enumerate(filenames):
+        tp, fp, fn = (int(v) for v in res.counts[i])
+        rows.append(dict(name=name.replace(".png", ""), pred=int(pred[i]),
+                         label=None if labels is None else int(labels[i]), tp=tp, fp=fp, fn=fn,
+                         dice=float(res.dice[i]), iou=float(res.iou[i]), hd=float(res.hd[i]), hd95=float(res.hd95[i])))
+    rows.sort(key=lambda r: int(r["name"].replace(".jpg", "").replace(".png", "")))
+    summary = {}
+    for k in ("dice", "iou", "hd95"):
+        v = np.array([r[k] for r in rows])
+        ok = np.isfinite(v)
+        summary[k] = float(v[ok].mean()) if ok.any() else float("nan")
+        summary[k + "_nan"] = int(np.isnan(v).sum())
+        summary[k + "_inf"] = int(np.isinf(v).sum())
+    if labels is not None:
+        summary["classification"] = metrics.classification_metrics(cls, torch.as_tensor(np.asarray(labels)),
+                                                                   num_classes=cls.shape[1])
+    if save_dir is not None:
+        _write_records([f"{r['name']} {r['pred']}" for r in rows], save_dir)
+        import csv
+        with open(os.path.join(save_dir, "metrics.csv"), "w", newline="") as f:
+            w = csv.writer(f)
+            cols = ["name", "pred", "label", "tp", "fp", "fn", "dice", "iou", "hd", "hd95"]
+            w.writerow(cols)
+            for r in rows:
+                w.writerow(["" if r[c] is None else (repr(r[c]) if isinstance(r[c], float) else r[c]) for c in cols])
+    return rows, summary
+
+
 def _write_records(records, save_dir):
     records.sort(key=lambda x: int(x.split()[0].replace(".jpg", "").replace(".png", "")))
     if save_dir is not None:

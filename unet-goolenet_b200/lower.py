@@ -8,6 +8,7 @@ lays out the NHWC bf16 activation workspace in HBM and emits the op descriptors 
   GoogLeNetClassifier.forward (test.py:64-73)            -> GoogLeNetRunner._emit_googlenet
   Grad-CAM at inception5b (GoogLeNetClassifier.grad_cam) -> GoogLeNetRunner._emit_cam (programs built with cam=True)
   outputs at each source image's own size               -> PipelineRunner._emit_source_frame (source_frame=True)
+  Dice / IoU / Hausdorff against ground truth (分割/main.py val) -> PipelineRunner._emit_seg_metrics (seg_metrics=...)
   whole two-stage path                                   -> PipelineRunner
 
 Dead compute of the reference forward is skipped: the `x` output of the bottleneck (attention1, the first
@@ -32,6 +33,31 @@ class SourceFrame(NamedTuple):
     masks: object
     boxes: torch.Tensor
     cam_maps: Optional[object]
+
+
+class SegMetrics(NamedTuple):
+    """Per-image scores of the segmentation mask against ground truth (PipelineRunner.__call__(..., gt_masks=...),
+    metrics.seg_metrics): counts i32 [B,3] (tp, fp, fn), then f64 [B] Dice, IoU, HD and HD95 (metrics.py states the
+    definitions), all on the host."""
+    counts: torch.Tensor
+    dice: torch.Tensor
+    iou: torch.Tensor
+    hd: torch.Tensor
+    hd95: torch.Tensor
+
+
+SEG_FRAMES = ("input", "source")
+
+
+def seg_metrics_desc(pred, gt, counts, hd, workspace, B, index=None, capacity=0, Hs=0, Ws=0):
+    """ug_seg_metrics_desc over device buffers (index: the ragged table, with capacity pixels; else B images of Hs x Ws)."""
+    return E.SegMetricsDesc(pred.data_ptr(), gt.data_ptr(), E.ptr(index), None, counts.data_ptr(), hd.data_ptr(),
+                            workspace.data_ptr(), workspace.numel(), capacity if index is not None else 0, B, Hs, Ws)
+
+
+def seg_metrics_workspace(B, px, dev):
+    """The op's scratch for B images in px pixels (u8, sized by ug_seg_metrics_workspace_bytes)."""
+    return torch.empty((E.load_library().ug_seg_metrics_workspace_bytes(B, px),), device=dev, dtype=torch.uint8)
 
 
 # Plans (program + activation workspace) kept per runner: a loader with ragged / varying batch sizes would otherwise
@@ -735,7 +761,7 @@ class PipelineRunner:
         for b in [m for m in self._gpools if m not in liveb]:
             del self._gpools[b]
 
-    def plan(self, B, source=None, slot=0, capacity=None, cam=False, source_frame=False):
+    def plan(self, B, source=None, slot=0, capacity=None, cam=False, source_frame=False, seg_metrics=None):
         """Program for a batch of B images; B must be <= micro_batch or a multiple of it.  With `source` =
         (Hs, Ws) the program starts with the device front-end (PIL-exact resize of uint8 HWC sources + to_tensor,
         util/data_utils.py) writing the UNet input, and `ws["src_u8"]` is the program's input buffer.
@@ -748,9 +774,15 @@ class PipelineRunner:
         cam=True appends the Grad-CAM op (GoogLeNetRunner._emit_cam) after the classifier head: `ws["cam"]` f32
         [B,7,7] and `ws["cam_map"]` f32 [B,224,224], the map placed in each image's ROI box of the UNet input frame.
         source_frame=True appends, last, the op that carries the outputs to each source image's own size
-        (_emit_source_frame); it needs a `source`."""
+        (_emit_source_frame); it needs a `source`.
+        seg_metrics="input" / "source" appends, last, the op that scores the mask against the io buffer `ws["gt_mask"]`
+        (_emit_seg_metrics): "input" the 224x224 mask, "source" the source-frame mask (needs source_frame=True)."""
         if source_frame and source is None:
             raise ValueError("source_frame=True needs uint8 or ragged sources: float input has no source frame")
+        if seg_metrics not in (None,) + SEG_FRAMES:
+            raise ValueError(f"seg_metrics must be None, 'input' or 'source', got {seg_metrics!r}")
+        if seg_metrics == "source" and not source_frame:
+            raise ValueError("seg_metrics='source' scores the source-frame mask: it needs source_frame=True")
         if source == "ragged":
             capacity = ragged.capacity(capacity or 0)
             key = (B, slot, "ragged", capacity)
@@ -760,6 +792,8 @@ class PipelineRunner:
             key += ("cam",)
         if source_frame:
             key += ("source_frame",)
+        if seg_metrics:
+            key += ("seg_metrics", seg_metrics)
 
         def build():
             mb = min(B, self.micro_batch)
@@ -801,6 +835,8 @@ class PipelineRunner:
                 self.gnet._emit_cam(B, ws, ops, boxes=ws["boxes"])
             if source_frame:
                 self._emit_source_frame(B, source, capacity, ws, ops)
+            if seg_metrics:
+                self._emit_seg_metrics(B, source, capacity, seg_metrics, ws, ops)
             return _finish(self.engine, ops, ws, ua + ga + [v for v in ws.values() if isinstance(v, torch.Tensor)])
         return self.plans.get_or_build(key, build)
 
@@ -822,17 +858,37 @@ class PipelineRunner:
                                      E.ptr(ws.get("src_cam_map")), capacity if ragged_src else 0, B, IMG, Hs, Ws,
                                      7 if "cam" in ws else 0, 7 if "cam" in ws else 0))
 
-    def export_plan(self, B, source=None, capacity=None, cam=False, source_frame=False):
+    def _emit_seg_metrics(self, B, source, capacity, frame, ws, ops):
+        """ug_seg_metrics_desc scoring ws["mask"] ("input") or ws["src_mask"] ("source") against ws["gt_mask"] u8,
+        placed like the scored mask: ws["seg_counts"] i32 [B,3] and ws["seg_hd"] f64 [B,2].  A ragged "source" plan
+        reads the front-end's table; as in _emit_source_frame, status is not written (src_status has it)."""
+        dev = self.dev
+        pred = ws["mask"] if frame == "input" else ws["src_mask"]
+        ws["gt_mask"] = torch.empty_like(pred)
+        ws["seg_counts"] = torch.empty((B, 3), device=dev, dtype=torch.int32)
+        ws["seg_hd"] = torch.empty((B, 2), device=dev, dtype=torch.float64)
+        ws["seg_workspace"] = seg_metrics_workspace(B, pred.numel(), dev)
+        if frame == "source" and source == "ragged":
+            d = seg_metrics_desc(pred, ws["gt_mask"], ws["seg_counts"], ws["seg_hd"], ws["seg_workspace"], B,
+                                 index=ws["src_index"], capacity=capacity)
+        else:
+            Hs, Ws = (IMG, IMG) if frame == "input" else source
+            d = seg_metrics_desc(pred, ws["gt_mask"], ws["seg_counts"], ws["seg_hd"], ws["seg_workspace"], B, Hs=Hs,
+                                 Ws=Ws)
+        ops.append(d)
+
+    def export_plan(self, B, source=None, capacity=None, cam=False, source_frame=False, seg_metrics=None):
         """The whole two-stage program for a batch of B images as a relocatable plan image (bytes): op list, device
         memory layout, BN-folded packed weights of both networks.  A host in any language runs it through the C ABI
         alone (ug_plan_load / ug_plan_copy_in / ug_plan_run / ug_plan_copy_out, include/ugnet.h; examples/run_plan.c).
         source / capacity / cam / source_frame as for plan(); a ragged plan's inputs are "src_u8" and "src_index", a cam
         plan also reports "cam" and "cam_map", a source_frame plan "src_mask", "src_boxes" and (with cam)
-        "src_cam_map"."""
-        ws = self.plan(B, source=source, capacity=capacity, cam=cam, source_frame=source_frame)
+        "src_cam_map", a seg_metrics plan takes "gt_mask" and reports "seg_counts" and "seg_hd"."""
+        ws = self.plan(B, source=source, capacity=capacity, cam=cam, source_frame=source_frame, seg_metrics=seg_metrics)
         prog = ws["program"]
         io = {k: ws[k] for k in ("x_in", "src_u8", "src_index", "src_status", "logits", "mask", "boxes", "u8",
-                                 "cls_logits", "cam", "cam_map", "src_mask", "src_boxes", "src_cam_map") if k in ws}
+                                 "cls_logits", "cam", "cam_map", "src_mask", "src_boxes", "src_cam_map", "gt_mask", "seg_counts",
+                                 "seg_hd") if k in ws}
         tensors = list(prog.keepalive) + list(io.values()) + [(self.unet.w_blob, True), (self.gnet.w_blob, True)]
         return E.export_plan(prog.descs, io, tensors)
 
@@ -847,16 +903,18 @@ class PipelineRunner:
             out.append((s, n - s))
         return out
 
-    def feed_ragged(self, part, cam=False, source_frame=False):
+    def feed_ragged(self, part, cam=False, source_frame=False, seg_metrics=None):
         """The ragged plan for one chunk (a ragged.Packed of HWC images, at most one plan's batch) with its packed
         sources and table copied in (one copy each)."""
-        ws = self.plan(len(part.table), source="ragged", capacity=part.n_px, cam=cam, source_frame=source_frame)
+        ws = self.plan(len(part.table), source="ragged", capacity=part.n_px, cam=cam, source_frame=source_frame,
+                       seg_metrics=seg_metrics)
         ws["src_u8"][:part.data.numel()].copy_(part.data, non_blocking=True)
         ws["src_index"].copy_(ragged.table_tensor(part.table))
         return ws
 
     @torch.no_grad()
-    def __call__(self, imgs, return_logits=False, return_cam=False, return_source=False):
+    def __call__(self, imgs, return_logits=False, return_cam=False, return_source=False, gt_masks=None,
+                 metrics_frame="input"):
         """imgs: float [B,3,224,224] CUDA, or uint8 [B,Hs,Ws,3] CUDA source images of any size (resized on the
         device exactly as the reference's PIL transform does), or a list of uint8 [H,W,3] images of different sizes
         (CUDA tensors or numpy arrays, sides up to 8*224; one ragged batch, util/ragged.py) ->
@@ -864,8 +922,13 @@ class PipelineRunner:
         if return_logits, then the Grad-CAM map of the predicted class f32 [B,224,224] (in [0,1] inside the ROI box,
         0 outside; see plan(cam=True)) if return_cam, then a SourceFrame of the mask, box and (with return_cam) map at
         each source image's own size if return_source (uint8 sources only: tensors [B,Hs,Ws] for a uint8 batch, lists of
-        [H_i,W_i] tensors for a list; see plan(source_frame=True))."""
+        [H_i,W_i] tensors for a list; see plan(source_frame=True)), then a SegMetrics of the mask against `gt_masks` if
+        given: in the form of the input, u8 [B,224,224] (metrics_frame="input", any input) or [B,Hs,Ws] / a list of
+        [H_i,W_i] masks at each source's own size (metrics_frame="source", uint8 sources only); nonzero = foreground.
+        Every other output is the same with and without gt_masks."""
+        from . import metrics
         masks, boxes, cls, seg, cams = [], [], [], [], []
+        counts, hds = [], []
         src_masks, src_boxes, src_cams = [], [], []
         packed = None
         if isinstance(imgs, (list, tuple)):
@@ -877,17 +940,27 @@ class PipelineRunner:
             raise ValueError(f"uint8 input must be HWC [B,H,W,3], got {tuple(imgs.shape)}")
         if return_source and packed is None and not from_u8:
             raise ValueError("return_source=True needs uint8 sources: float [B,3,224,224] input has no source frame")
+        frame = None
+        if gt_masks is not None:
+            frame = metrics_frame
+            gt = metrics.gt_batch(gt_masks, imgs, packed, frame)
+        src_frame = return_source or frame == "source"
         for s, c in self._chunks(n):
             if packed is not None:
                 part = ragged.chunk(packed, s, s + c)
-                kw = {k: True for k, on in (("cam", return_cam), ("source_frame", return_source)) if on}
+                kw = {k: v for k, v in (("cam", return_cam), ("source_frame", src_frame), ("seg_metrics", frame)) if v}
                 ws = self.feed_ragged(part, **kw)
             elif from_u8:
-                ws = self.plan(c, source=(imgs.shape[1], imgs.shape[2]), cam=return_cam, source_frame=return_source)
+                ws = self.plan(c, source=(imgs.shape[1], imgs.shape[2]), cam=return_cam, source_frame=src_frame,
+                               seg_metrics=frame)
                 ws["src_u8"].copy_(imgs[s:s + c])
             else:
-                ws = self.plan(c, cam=return_cam)
+                ws = self.plan(c, cam=return_cam, seg_metrics=frame)
                 ws["x_in"].copy_(imgs[s:s + c])
+            if frame == "source" and packed is not None:
+                ws["gt_mask"][:part.n_px].copy_(ragged.chunk(gt, s, s + c).data, non_blocking=True)
+            elif frame is not None:
+                ws["gt_mask"].copy_(gt[s:s + c])
             ws["program"].run()
             masks.append(ws["mask"].clone())
             boxes.append(ws["boxes"].clone())
@@ -906,6 +979,9 @@ class PipelineRunner:
                     src_masks.append(ws["src_mask"].clone())
                     if return_cam:
                         src_cams.append(ws["src_cam_map"].clone())
+            if frame is not None:
+                counts.append(ws["seg_counts"].cpu())
+                hds.append(ws["seg_hd"].cpu())
         out = (torch.cat(masks), torch.cat(boxes), torch.cat(cls))
         if return_logits:
             out += (torch.cat(seg),)
@@ -916,4 +992,6 @@ class PipelineRunner:
                 src_masks = torch.cat(src_masks)
                 src_cams = torch.cat(src_cams) if return_cam else None
             out += (SourceFrame(src_masks, torch.cat(src_boxes), src_cams if return_cam else None),)
+        if frame is not None:
+            out += (metrics.seg_result(torch.cat(counts), torch.cat(hds)),)
         return out

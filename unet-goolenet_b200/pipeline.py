@@ -19,7 +19,8 @@ class TwoStagePipeline:
         self.runner = PipelineRunner(usd, gsd, dev, micro_batch=micro_batch, padding=padding, cls_batch=cls_batch)
 
     @torch.no_grad()
-    def __call__(self, imgs, return_logits=False, return_cam=False, return_source=False):
+    def __call__(self, imgs, return_logits=False, return_cam=False, return_source=False, gt_masks=None,
+                 metrics_frame="input"):
         """imgs: float [B,3,224,224] on the pipeline's device, or uint8 HWC sources [B,Hs,Ws,3] of any size (resized
         on the device like the reference's CDDataAugmentation.transform: PIL bilinear + to_tensor), or a list of uint8
         [H,W,3] images of different sizes (CUDA tensors or numpy arrays; run as ragged batches, util/ragged.py) ->
@@ -27,8 +28,11 @@ class TwoStagePipeline:
         segmentation logits if return_logits and by the Grad-CAM map of the predicted class (float32 [B,224,224], in
         the 224x224 frame, inside each image's box) if return_cam, and by a SourceFrame(masks, boxes, cam_maps) of the
         same outputs at each source image's own size if return_source (uint8 sources only; lists of per-image tensors
-        for a list of images; cam_maps is None without return_cam)."""
-        return self.runner(imgs, return_logits=return_logits, return_cam=return_cam, return_source=return_source)
+        for a list of images; cam_maps is None without return_cam), and by a SegMetrics(counts, dice, iou, hd, hd95) of
+        the mask against gt_masks if given (metrics_frame "input": u8 [B,224,224]; "source": masks at each source's own
+        size, a tensor [B,Hs,Ws] or a list like the input; see PipelineRunner.__call__ and metrics.py)."""
+        return self.runner(imgs, return_logits=return_logits, return_cam=return_cam, return_source=return_source,
+                           gt_masks=gt_masks, metrics_frame=metrics_frame)
 
     def predict(self, imgs):
         """argmax(softmax(logits)) as 分类/test.py:86 (softmax is monotone, so argmax of the logits)."""
