@@ -377,6 +377,41 @@ typedef struct ug_seg_metrics_desc {
   int B, Hs, Ws;
 } ug_seg_metrics_desc;
 
+/* Connected components of a mask ("lesions"): per image i, with F = {mask != 0} (0/1 and 0/255 masks alike), placed
+ * like ug_seg_metrics_desc's pred (index[i] for a ragged batch, else Hs x Ws at pixel offset i*Hs*Ws), x = column,
+ * y = row:
+ *   the components of F under `connectivity` 8 or 4, numbered 1..n in raster order of each component's first pixel
+ *   (scipy.ndimage.label(F, generate_binary_structure(2, 1 or 2))); labels[p] = that number, 0 for background;
+ *   count[i] = n (also when n > K);
+ *   lesions[i*K .. i*K+K-1]: the K largest components, area descending, ties by label ascending; rows past n are zero;
+ *   main_mask[p] = 1 where labels[p] is the label of row 0 and n > 0, else 0 (optional, u8, placed like mask).
+ * A row's integers are exact: area, the box [x0, x1) x [y0, y1), boundary (pixels of the component with a 4-neighbour
+ * outside F or outside the image, ug_seg_metrics' surface rule) and the moment sums sx = sum x, sy, sxx, sxy, syy in
+ * int64.  Centroid, axes, orientation and eccentricity follow on the host (ugnet_b200/lesions.py).
+ * connectivity must be 4 or 8 and 1 <= K <= 32 (UG_EINVAL otherwise, nothing written).  labels is required: it is
+ * the op's union-find array.  The table may come from outside the library: an entry with a negative offset, a side
+ * outside [1, 8*224] or an extent past capacity_px is rejected: nothing is read or written through it, count[i] = 0,
+ * its rows are zero and status[i] = 1 (0 otherwise; status is optional).  The launch geometry depends on B, Hs / Ws or
+ * the largest side allowed, and K only, never on the table; the outputs are bit-identical run to run. */
+typedef struct ug_lesion {
+  int label, area, x0, y0, x1, y1, boundary, reserved;
+  long long sx, sy, sxx, sxy, syy;
+} ug_lesion; /* 72 bytes */
+
+typedef struct ug_lesions_desc {
+  const unsigned char* mask;       /* u8: image i at mask + px_offset (ragged) or mask + i*Hs*Ws */
+  const ug_ragged_image* index;    /* optional device table [B]; NULL = every image is Hs x Ws */
+  int* status;                     /* optional int32 [B]: 1 = entry rejected */
+  int* labels;                     /* int32, placed like mask (required: the union-find array) */
+  unsigned char* main_mask;        /* optional u8, placed like mask */
+  ug_lesion* lesions;              /* [B][K] */
+  int* count;                      /* int32 [B] */
+  void* workspace;                 /* >= ug_lesions_workspace_bytes(B, capacity_px or B*Hs*Ws, K) */
+  size_t workspace_bytes;
+  long long capacity_px;           /* ragged: pixels of mask / labels / main_mask; unused when index is NULL */
+  int B, Hs, Ws, connectivity, K;
+} ug_lesions_desc;
+
 enum {
   UG_OP_CONV = 1,
   /* 2 and 10 were the stand-alone im2col packs of round 1 (replaced by UG_OP_STEM); the numbers stay retired */
@@ -396,7 +431,8 @@ enum {
   UG_OP_WAVELET_RAGGED = 17,
   UG_OP_CAM = 18,
   UG_OP_SOURCE_FRAME = 19,
-  UG_OP_SEG_METRICS = 20
+  UG_OP_SEG_METRICS = 20,
+  UG_OP_LESIONS = 21
 };
 
 typedef struct ug_op {
@@ -421,6 +457,7 @@ typedef struct ug_op {
     ug_cam_desc cam; /* smaller than ug_conv_desc as well */
     ug_source_frame_desc source_frame; /* and so is this one */
     ug_seg_metrics_desc seg_metrics;   /* as is this one */
+    ug_lesions_desc lesions;           /* and this one */
   } u;
 } ug_op;
 
@@ -450,10 +487,14 @@ int ug_wavelet_ragged(ug_handle h, const ug_wavelet_ragged_desc* d, void* stream
 int ug_cam(ug_handle h, const ug_cam_desc* d, void* stream);
 int ug_source_frame(ug_handle h, const ug_source_frame_desc* d, void* stream);
 int ug_seg_metrics(ug_handle h, const ug_seg_metrics_desc* d, void* stream);
+int ug_lesions(ug_handle h, const ug_lesions_desc* d, void* stream);
 size_t ug_wavelet_workspace_bytes(int B, int H, int W);
 size_t ug_wavelet_ragged_workspace_bytes(int B, long long capacity_px);
 /* Workspace of ug_seg_metrics for B images in capacity_px pixels (ragged capacity, or B*Hs*Ws); 0 for bad arguments. */
 size_t ug_seg_metrics_workspace_bytes(int B, long long capacity_px);
+/* Workspace of ug_lesions for B images in capacity_px pixels (ragged capacity, or B*Hs*Ws) and K rows per image; 0 for
+ * bad arguments. */
+size_t ug_lesions_workspace_bytes(int B, long long capacity_px, int K);
 
 /* Programs: a validated op list with tensor maps and launch geometry prepared once; run = launches only. */
 int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out);
@@ -504,7 +545,14 @@ int ug_program_run_host_pipelined(ug_handle h, ug_program p, const ug_copy* h2d,
  * and, with cam=True, "src_cam_map" f32 [B,Hs,Ws] (ragged: [P]).  A plan exported with seg_metrics="input" or
  * "source" (export_plan(B, ..., seg_metrics=...)) also scores the mask against ground truth (ug_seg_metrics_desc): it
  * takes "gt_mask" u8, [B,224,224] for "input" (against "mask") or placed like "src_mask" for "source" (against
- * "src_mask"), and reports "seg_counts" i32 [B,3] (tp, fp, fn) and "seg_hd" f64 [B,2] (HD, HD95). */
+ * "src_mask"), and reports "seg_counts" i32 [B,3] (tp, fp, fn) and "seg_hd" f64 [B,2] (HD, HD95).  A plan exported
+ * with lesions="input" or roi="largest" (export_plan(B, ..., lesions=..., roi=...)) labels the connected components
+ * of each 224x224 mask (ug_lesions_desc, connectivity 8, K = 8) and reports "lesion_labels" i32 [B,224,224],
+ * "lesion_mask" u8 [B,224,224] (the largest lesion), "lesion_count" i32 [B] and "lesions" ug_lesion [B,8]; with
+ * roi="largest" "boxes", the crops, "cls_logits" and the CAM follow the box of "lesion_mask" instead of "mask" ("mask"
+ * and "logits" do not change).  With lesions="source" (and source_frame=True) the op runs last on "src_mask" and
+ * reports "src_lesion_labels" i32 and "src_lesion_mask" u8 placed like "src_mask", "src_lesion_count" i32 [B] and
+ * "src_lesions" ug_lesion [B,8]. */
 typedef struct ug_plan_s* ug_plan;
 /* Parses the image (host memory, may be freed afterwards), allocates ONE device arena for every buffer of the plan
  * (ug_plan_device_bytes), uploads the constants, relocates the op list and prepares the program. */

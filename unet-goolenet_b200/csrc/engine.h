@@ -333,5 +333,6 @@ int launch_wavelet_ragged(ug_engine* h, const ug_wavelet_ragged_desc* d, cudaStr
 int launch_cam(ug_engine* h, const ug_cam_desc* d, cudaStream_t s);
 int launch_source_frame(ug_engine* h, const ug_source_frame_desc* d, cudaStream_t s);
 int launch_seg_metrics(ug_engine* h, const ug_seg_metrics_desc* d, cudaStream_t s);
+int launch_lesions(ug_engine* h, const ug_lesions_desc* d, cudaStream_t s);
 
 }  // namespace ug

@@ -21,7 +21,7 @@ EPI_STORE, EPI_ADD, EPI_GATE, EPI_OUTC = 0, 1, 2, 3
 # (2 and 10 were round 1's stand-alone im2col packs; the numbers stay retired, see ugnet.h)
 OP_CONV, OP_POOL, OP_LAYERNORM, OP_ATTN, OP_CHANSTATS, OP_GATE, OP_BBOX, OP_CROPRESIZE = 1, 3, 4, 5, 6, 7, 8, 9
 OP_HEAD, OP_STEM, OP_RESIZE, OP_WAVELET, OP_S2D = 11, 12, 13, 14, 15
-OP_RESIZE_RAGGED, OP_WAVELET_RAGGED, OP_CAM, OP_SOURCE_FRAME, OP_SEG_METRICS = 16, 17, 18, 19, 20
+OP_RESIZE_RAGGED, OP_WAVELET_RAGGED, OP_CAM, OP_SOURCE_FRAME, OP_SEG_METRICS, OP_LESIONS = 16, 17, 18, 19, 20, 21
 
 _vp, _i, _f, _ll = C.c_void_p, C.c_int, C.c_float, C.c_longlong
 
@@ -121,13 +121,25 @@ class SegMetricsDesc(C.Structure):
                 ("Ws", _i)]
 
 
+class Lesion(C.Structure):
+    """ug_lesion: one row of the ug_lesions table (72 bytes)."""
+    _fields_ = [("label", _i), ("area", _i), ("x0", _i), ("y0", _i), ("x1", _i), ("y1", _i), ("boundary", _i),
+                ("reserved", _i), ("sx", _ll), ("sy", _ll), ("sxx", _ll), ("sxy", _ll), ("syy", _ll)]
+
+
+class LesionsDesc(C.Structure):
+    _fields_ = [("mask", _vp), ("index", _vp), ("status", _vp), ("labels", _vp), ("main_mask", _vp),
+                ("lesions", _vp), ("count", _vp), ("workspace", _vp), ("workspace_bytes", C.c_size_t),
+                ("capacity_px", _ll), ("B", _i), ("Hs", _i), ("Ws", _i), ("connectivity", _i), ("K", _i)]
+
+
 class _OpUnion(C.Union):
     _fields_ = [("conv", ConvDesc), ("pool", PoolDesc), ("ln", LayerNormDesc),
                 ("attn", AttnDesc), ("stats", ChanStatsDesc), ("gate", GateDesc), ("bbox", BBoxDesc),
                 ("crop", CropResizeDesc), ("head", HeadDesc), ("stem", StemDesc),
                 ("resize", ResizeDesc), ("wavelet", WaveletDesc), ("s2d", S2dDesc),
                 ("resize_ragged", ResizeRaggedDesc), ("wavelet_ragged", WaveletRaggedDesc), ("cam", CamDesc),
-                ("source_frame", SourceFrameDesc), ("seg_metrics", SegMetricsDesc)]
+                ("source_frame", SourceFrameDesc), ("seg_metrics", SegMetricsDesc), ("lesions", LesionsDesc)]
 
 
 class Op(C.Structure):
@@ -142,26 +154,28 @@ _KIND_FIELD = {OP_CONV: "conv", OP_POOL: "pool", OP_LAYERNORM: "ln", OP_ATTN: "a
                OP_CHANSTATS: "stats", OP_GATE: "gate", OP_BBOX: "bbox", OP_CROPRESIZE: "crop",
                OP_HEAD: "head", OP_STEM: "stem", OP_RESIZE: "resize", OP_WAVELET: "wavelet", OP_S2D: "s2d",
                OP_RESIZE_RAGGED: "resize_ragged", OP_WAVELET_RAGGED: "wavelet_ragged", OP_CAM: "cam",
-               OP_SOURCE_FRAME: "source_frame", OP_SEG_METRICS: "seg_metrics"}
+               OP_SOURCE_FRAME: "source_frame", OP_SEG_METRICS: "seg_metrics", OP_LESIONS: "lesions"}
 _DESC_KIND = {ConvDesc: OP_CONV, PoolDesc: OP_POOL, LayerNormDesc: OP_LAYERNORM,
               AttnDesc: OP_ATTN, ChanStatsDesc: OP_CHANSTATS, GateDesc: OP_GATE, BBoxDesc: OP_BBOX,
               CropResizeDesc: OP_CROPRESIZE, HeadDesc: OP_HEAD, StemDesc: OP_STEM,
               ResizeDesc: OP_RESIZE, WaveletDesc: OP_WAVELET, S2dDesc: OP_S2D,
               ResizeRaggedDesc: OP_RESIZE_RAGGED, WaveletRaggedDesc: OP_WAVELET_RAGGED, CamDesc: OP_CAM,
-              SourceFrameDesc: OP_SOURCE_FRAME, SegMetricsDesc: OP_SEG_METRICS}
+              SourceFrameDesc: OP_SOURCE_FRAME, SegMetricsDesc: OP_SEG_METRICS, LesionsDesc: OP_LESIONS}
 _SINGLE_ENTRY = {OP_CONV: "ug_conv", OP_POOL: "ug_pool",
                  OP_LAYERNORM: "ug_layernorm", OP_ATTN: "ug_attention", OP_CHANSTATS: "ug_chanstats",
                  OP_GATE: "ug_gate", OP_BBOX: "ug_bbox", OP_CROPRESIZE: "ug_cropresize",
                  OP_HEAD: "ug_head", OP_STEM: "ug_stem",
                  OP_RESIZE: "ug_resize_u8", OP_WAVELET: "ug_wavelet", OP_S2D: "ug_s2d_pack",
                  OP_RESIZE_RAGGED: "ug_resize_ragged", OP_WAVELET_RAGGED: "ug_wavelet_ragged", OP_CAM: "ug_cam",
-                 OP_SOURCE_FRAME: "ug_source_frame", OP_SEG_METRICS: "ug_seg_metrics"}
+                 OP_SOURCE_FRAME: "ug_source_frame", OP_SEG_METRICS: "ug_seg_metrics",
+                 OP_LESIONS: "ug_lesions"}
 
 EXPORTED_SYMBOLS = ["ug_version", "ug_create", "ug_destroy", "ug_last_error", "ug_launch_count",
                     *_SINGLE_ENTRY.values(), "ug_program_create", "ug_program_run", "ug_program_num_launches",
                     "ug_program_destroy", "ug_program_run_host", "ug_program_run_host_pipelined",
                     "ug_program_run_timed", "ug_wavelet_workspace_bytes",
                     "ug_wavelet_ragged_workspace_bytes", "ug_seg_metrics_workspace_bytes",
+                    "ug_lesions_workspace_bytes",
                     "ug_plan_load", "ug_plan_num_io", "ug_plan_io_name", "ug_plan_io", "ug_plan_device_bytes",
                     "ug_plan_program", "ug_plan_copy_in", "ug_plan_copy_out", "ug_plan_run", "ug_plan_destroy"]
 DEV_SYMBOLS = ["ug_mma_microbench", "ug_mma_microbench2", "ug_mma_microbench_pair", "ug_conv_launch_info",
@@ -204,6 +218,8 @@ def load_library():
     lib.ug_wavelet_ragged_workspace_bytes.restype = C.c_size_t
     lib.ug_seg_metrics_workspace_bytes.argtypes = [_i, _ll]
     lib.ug_seg_metrics_workspace_bytes.restype = C.c_size_t
+    lib.ug_lesions_workspace_bytes.argtypes = [_i, _ll, _i]
+    lib.ug_lesions_workspace_bytes.restype = C.c_size_t
     lib.ug_program_destroy.argtypes = [_vp, _vp]
     lib.ug_program_run_host.argtypes = [_vp, _vp, _vp, _i, _vp, _i, _vp]
     lib.ug_program_run_host_pipelined.argtypes = [_vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp]

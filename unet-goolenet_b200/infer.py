@@ -56,7 +56,7 @@ def inference_all_seg(model, test_loader, device, save_dir=None):
 
 @torch.no_grad()
 def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256, cam_dir=None, mask_dir=None,
-                 frame="input"):
+                 frame="input", roi="all", lesions=None):
     """The whole of 分类/test.py:122-134 + :74-96 on the device for a batch of grayscale images:
     cv2.imread(path, 0) output (uint8 [H, W]) -> wavelet_enhance -> resize 224 + to_tensor -> UNet -> mask -> bbox ->
     ROI crop/resize -> GoogLeNet -> argmax; returns the sorted "<name> <class>" records (and writes result.txt).
@@ -73,29 +73,78 @@ def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256
     mask_dir: also write, per image, `mask_dir/<name without extension>.png`: the segmentation mask painted as
     分割/predict.py:32-45 paints it, red (255,0,0) on black.
     frame: "input" writes both at 224x224, the UNet input frame; "source" writes them at each image's own size (the
-    gray image's: the wavelet step keeps the size), carried there by the pipeline's source-frame op."""
+    gray image's: the wavelet step keeps the size), carried there by the pipeline's source-frame op.
+    roi: "all" crops the hull of every foreground pixel of the mask (roi.py); "largest" crops the largest connected
+    component only (PipelineRunner.plan(roi="largest")).
+    lesions: "input" / "source" also labels the connected components of the 224x224 / source-frame masks and, with
+    save_dir, writes `lesions.csv`: one row per table row of an image with lesions (the 8 largest, lesions.py), in the
+    order of result.txt: name, rank, count, label, area, box x0 y0 x1 y1 (end-exclusive), centroid cx cy,
+    orientation, major and minor axis, eccentricity, equivalent diameter and boundary (pixel units)."""
     from .util.wavelet import wavelet_enhance_batch
     if frame not in ("input", "source"):
         raise ValueError(f"frame must be 'input' or 'source', got {frame!r}")
+    if lesions not in (None, "input", "source"):
+        raise ValueError(f"lesions must be None, 'input' or 'source', got {lesions!r}")
     runner = getattr(pipeline, "runner", pipeline)
+    les_rows = []
     if isinstance(gray_images, (list, tuple)):
-        records = _grade_ragged(runner, gray_images, filenames, cam_dir, mask_dir, frame)
-        return _write_records(records, save_dir)
-    g = torch.as_tensor(np.ascontiguousarray(gray_images) if isinstance(gray_images, np.ndarray) else gray_images)
-    source = frame == "source" and (cam_dir is not None or mask_dir is not None)
-    records = []
-    for s in range(0, g.shape[0], batch_size):
-        rgb = wavelet_enhance_batch(g[s:s + batch_size].to(runner.dev))      # [B,H,W,3] uint8, test.py:128-129
-        out = runner(rgb, return_cam=cam_dir is not None, return_source=source)  # test.py:130-131 and :82-84
-        pred = torch.argmax(torch.softmax(out[2], dim=1), dim=1).cpu().numpy()  # test.py:86
-        names = filenames[s:s + batch_size]
-        for i, name in enumerate(names):
-            records.append(f"{name.replace('.png', '')} {int(pred[i])}")
-        if source:
-            _write_maps(out[-1].cam_maps, out[-1].masks, names, cam_dir, mask_dir)
-        else:
-            _write_maps(out[3] if cam_dir is not None else None, out[0], names, cam_dir, mask_dir)
-    return _write_records(records, save_dir)
+        records = _grade_ragged(runner, gray_images, filenames, cam_dir, mask_dir, frame, roi, lesions, les_rows)
+    else:
+        g = torch.as_tensor(np.ascontiguousarray(gray_images) if isinstance(gray_images, np.ndarray) else gray_images)
+        source = frame == "source" and (cam_dir is not None or mask_dir is not None)
+        records = []
+        for s in range(0, g.shape[0], batch_size):
+            rgb = wavelet_enhance_batch(g[s:s + batch_size].to(runner.dev))      # [B,H,W,3] uint8, test.py:128-129
+            out = runner(rgb, return_cam=cam_dir is not None, return_source=source, lesions=lesions,
+                         roi=roi)                                                  # test.py:130-131 and :82-84
+            pred = torch.argmax(torch.softmax(out[2], dim=1), dim=1).cpu().numpy()  # test.py:86
+            names = filenames[s:s + batch_size]
+            for i, name in enumerate(names):
+                records.append(f"{name.replace('.png', '')} {int(pred[i])}")
+            if lesions:
+                les = out[-1]
+                les_rows += _lesion_rows(names, les.count, les.table, les.derived)
+                out = out[:-1]
+            if source:
+                _write_maps(out[-1].cam_maps, out[-1].masks, names, cam_dir, mask_dir)
+            else:
+                _write_maps(out[3] if cam_dir is not None else None, out[0], names, cam_dir, mask_dir)
+    records = _write_records(records, save_dir)
+    if lesions and save_dir is not None:
+        _write_lesions(les_rows, save_dir)
+    return records
+
+
+LESION_COLUMNS = ["name", "rank", "count", "label", "area", "x0", "y0", "x1", "y1", "cx", "cy", "orientation",
+                  "major_axis", "minor_axis", "eccentricity", "equivalent_diameter", "boundary"]
+
+
+def _lesion_rows(names, count, table, derived):
+    """lesions.csv rows (dicts of LESION_COLUMNS) of a batch: every table row with a lesion, rank 0 = the largest."""
+    out = []
+    for i, name in enumerate(names):
+        for k in range(table.shape[1]):
+            t = table[i, k]
+            if int(t["label"]) == 0:
+                continue
+            r = dict(name=name.replace(".png", ""), rank=k, count=int(count[i]))
+            r.update({c: int(t[c]) for c in ("label", "area", "x0", "y0", "x1", "y1", "boundary")})
+            r.update(cx=float(derived.cx[i, k]), cy=float(derived.cy[i, k]))
+            r.update({c: float(getattr(derived, c)[i, k]) for c in ("orientation", "major_axis", "minor_axis",
+                                                                      "eccentricity", "equivalent_diameter")})
+            out.append(r)
+    return out
+
+
+def _write_lesions(rows, save_dir):
+    import csv
+    rows = sorted(rows, key=lambda r: (int(r["name"].replace(".jpg", "").replace(".png", "")), r["rank"]))
+    os.makedirs(save_dir, exist_ok=True)
+    with open(os.path.join(save_dir, "lesions.csv"), "w", newline="") as f:
+        w = csv.writer(f)
+        w.writerow(LESION_COLUMNS)
+        for r in rows:
+            w.writerow([repr(r[c]) if isinstance(r[c], float) else r[c] for c in LESION_COLUMNS])
 
 
 def _stem_png(d, name):
@@ -121,7 +170,9 @@ def _write_maps(cam_maps, masks, names, cam_dir, mask_dir):
             Image.fromarray(canvas, "RGB").save(_stem_png(mask_dir, name))
 
 
-def _grade_ragged(runner, gray_images, filenames, cam_dir=None, mask_dir=None, frame="input"):
+def _grade_ragged(runner, gray_images, filenames, cam_dir=None, mask_dir=None, frame="input", roi="all",
+                  lesions=None, les_rows=None):
+    from . import lesions as L
     from .util import ragged
     from .util.wavelet import wavelet_ragged_into
     packed = ragged.pack(gray_images, 1, min_side=ragged.WAVELET_MIN_SIDE, max_side=ragged.MAX_RATIO * 224)
@@ -129,7 +180,8 @@ def _grade_ragged(runner, gray_images, filenames, cam_dir=None, mask_dir=None, f
     records = []
     for s, c in runner._chunks(len(gray_images)):
         part = ragged.chunk(packed, s, s + c)
-        ws = runner.plan(c, source="ragged", capacity=part.n_px, cam=cam_dir is not None, source_frame=source)
+        ws = runner.plan(c, source="ragged", capacity=part.n_px, cam=cam_dir is not None,
+                         source_frame=source or lesions == "source", lesions=lesions, roi=roi)
         gray = part.data.to(runner.dev, non_blocking=True)
         ws["src_index"].copy_(ragged.table_tensor(part.table))
         wavelet_ragged_into(gray, ws["src_index"], ws["src_u8"], c)         # test.py:128-129, into the plan's input
@@ -138,6 +190,10 @@ def _grade_ragged(runner, gray_images, filenames, cam_dir=None, mask_dir=None, f
         names = filenames[s:s + c]
         for i, name in enumerate(names):
             records.append(f"{name.replace('.png', '')} {int(pred[i])}")
+        if lesions:
+            pre = "src_" if lesions == "source" else ""
+            table = L.rows(ws[pre + "lesions"])
+            les_rows += _lesion_rows(names, ws[pre + "lesion_count"].cpu(), table, L.derive(table))
         if source:
             cams = ragged.unpack(ws["src_cam_map"], part.table, 1) if cam_dir is not None else None
             _write_maps(cams, ragged.unpack(ws["src_mask"], part.table, 1), names, cam_dir, mask_dir)
@@ -147,7 +203,7 @@ def _grade_ragged(runner, gray_images, filenames, cam_dir=None, mask_dir=None, f
 
 
 @torch.no_grad()
-def evaluate_images(pipeline, gray_images, gt_masks, labels, filenames, frame="source", save_dir=None):
+def evaluate_images(pipeline, gray_images, gt_masks, labels, filenames, frame="source", save_dir=None, roi="all"):
     """grade_images plus ground truth (分割/main.py val and 分类/ROI_main.py's scores on the device path): per chunk the
     wavelet step, the pipeline program and its metrics op (PipelineRunner.plan(seg_metrics=frame)).
 
@@ -158,7 +214,8 @@ def evaluate_images(pipeline, gray_images, gt_masks, labels, filenames, frame="s
     result.txt; summary holds the means of dice / iou / hd95 over the images where they are finite, how many were NaN
     (empty ground truth, or no surface at all) and inf (one surface empty) and left out, and with labels the
     metrics.classification_metrics dict under "classification".  With save_dir, writes result.txt exactly as
-    grade_images and metrics.csv (the rows, same order)."""
+    grade_images and metrics.csv (the rows, same order).  roi as grade_images: "largest" grades each image's largest
+    lesion, so its scores can be set against the default's on the same labelled data."""
     from . import metrics
     from .util import ragged
     from .util.wavelet import wavelet_enhance_batch, wavelet_ragged_into
@@ -174,7 +231,8 @@ def evaluate_images(pipeline, gray_images, gt_masks, labels, filenames, frame="s
         gt = metrics.gt_batch(list(gt_masks) if frame == "source" else gt_masks, gray_images, packed, frame)
         for s, c in runner._chunks(n):
             part = ragged.chunk(packed, s, s + c)
-            ws = runner.plan(c, source="ragged", capacity=part.n_px, source_frame=frame == "source", seg_metrics=frame)
+            ws = runner.plan(c, source="ragged", capacity=part.n_px, source_frame=frame == "source", seg_metrics=frame,
+                             roi=roi)
             gray = part.data.to(runner.dev, non_blocking=True)
             ws["src_index"].copy_(ragged.table_tensor(part.table))
             if frame == "source":
@@ -191,7 +249,7 @@ def evaluate_images(pipeline, gray_images, gt_masks, labels, filenames, frame="s
     else:
         g = torch.as_tensor(np.ascontiguousarray(gray_images) if isinstance(gray_images, np.ndarray) else gray_images)
         rgb = wavelet_enhance_batch(g.to(runner.dev))
-        out = runner(rgb, gt_masks=gt_masks, metrics_frame=frame)
+        out = runner(rgb, gt_masks=gt_masks, metrics_frame=frame, roi=roi)
         cls, res = out[2].cpu(), out[-1]
     pred = torch.argmax(torch.softmax(cls, dim=1), dim=1).numpy()                # test.py:86
     rows = []

@@ -9,6 +9,7 @@ lays out the NHWC bf16 activation workspace in HBM and emits the op descriptors 
   Grad-CAM at inception5b (GoogLeNetClassifier.grad_cam) -> GoogLeNetRunner._emit_cam (programs built with cam=True)
   outputs at each source image's own size               -> PipelineRunner._emit_source_frame (source_frame=True)
   Dice / IoU / Hausdorff against ground truth (分割/main.py val) -> PipelineRunner._emit_seg_metrics (seg_metrics=...)
+  connected components of the mask, largest-lesion ROI   -> PipelineRunner._emit_lesions (lesions=..., roi="largest")
   whole two-stage path                                   -> PipelineRunner
 
 Dead compute of the reference forward is skipped: the `x` output of the bottleneck (attention1, the first
@@ -20,6 +21,7 @@ from typing import NamedTuple, Optional
 import torch
 
 from . import engine as E
+from . import lesions as L
 from . import pack
 from .util import ragged
 
@@ -47,6 +49,8 @@ class SegMetrics(NamedTuple):
 
 
 SEG_FRAMES = ("input", "source")
+ROI_RULES = ("all", "largest")
+LESION_K, LESION_CONNECTIVITY = 8, 8   # table rows per image and connectivity of the programs' lesions op
 
 
 def seg_metrics_desc(pred, gt, counts, hd, workspace, B, index=None, capacity=0, Hs=0, Ws=0):
@@ -509,9 +513,11 @@ class UNetRunner(_Builder):
         hw, hb = self.w["cls_head"]
         ops.append(E.HeadDesc(tok.data_ptr(), hw.data_ptr(), hb.data_ptr(), ws["cl_out"].data_ptr(), B, 196, 512, 1))
 
-    def _emit_bbox(self, B, ws, ops, padding=30, boxes=None):
+    def _emit_bbox(self, B, ws, ops, padding=30, boxes=None, mask=None):
+        """ug_bbox over ws["mask"], or over `mask` (the largest-lesion mask of a roi="largest" pipeline)."""
         ws["boxes"] = boxes if boxes is not None else torch.empty((B, 4), device=self.dev, dtype=torch.int32)
-        ops.append(E.BBoxDesc(ws["mask"].data_ptr(), ws["boxes"].data_ptr(), B, IMG, IMG, padding))
+        src = ws["mask"] if mask is None else mask
+        ops.append(E.BBoxDesc(src.data_ptr(), ws["boxes"].data_ptr(), B, IMG, IMG, padding))
 
     def plan(self, B, padding=30):
         def build():
@@ -761,7 +767,8 @@ class PipelineRunner:
         for b in [m for m in self._gpools if m not in liveb]:
             del self._gpools[b]
 
-    def plan(self, B, source=None, slot=0, capacity=None, cam=False, source_frame=False, seg_metrics=None):
+    def plan(self, B, source=None, slot=0, capacity=None, cam=False, source_frame=False, seg_metrics=None,
+             lesions=None, roi="all"):
         """Program for a batch of B images; B must be <= micro_batch or a multiple of it.  With `source` =
         (Hs, Ws) the program starts with the device front-end (PIL-exact resize of uint8 HWC sources + to_tensor,
         util/data_utils.py) writing the UNet input, and `ws["src_u8"]` is the program's input buffer.
@@ -776,13 +783,27 @@ class PipelineRunner:
         source_frame=True appends, last, the op that carries the outputs to each source image's own size
         (_emit_source_frame); it needs a `source`.
         seg_metrics="input" / "source" appends, last, the op that scores the mask against the io buffer `ws["gt_mask"]`
-        (_emit_seg_metrics): "input" the 224x224 mask, "source" the source-frame mask (needs source_frame=True)."""
+        (_emit_seg_metrics): "input" the 224x224 mask, "source" the source-frame mask (needs source_frame=True).
+        lesions="input" labels the connected components of each micro-batch's mask right after its UNet
+        (_emit_lesions; connectivity 8, 8 table rows): ws["lesion_labels"] i32 [B,224,224], ws["lesion_mask"] u8
+        (the largest lesion), ws["lesion_count"] i32 [B] and ws["lesions"] (ug_lesion rows as int64 [B,8,9]);
+        lesions="source" appends, last, the same op on the source-frame mask (needs source_frame=True; ws["src_lesion_*"]
+        and ws["src_lesions"], placed like src_mask).  roi="largest" crops the largest lesion instead of the hull of
+        all foreground pixels: it adds the "input" op if lesions did not and points each micro-batch's bbox at
+        ws["lesion_mask"]; the boxes, crops, classifier, CAM and source-frame boxes follow, mask / logits / src_mask do
+        not change."""
         if source_frame and source is None:
             raise ValueError("source_frame=True needs uint8 or ragged sources: float input has no source frame")
         if seg_metrics not in (None,) + SEG_FRAMES:
             raise ValueError(f"seg_metrics must be None, 'input' or 'source', got {seg_metrics!r}")
         if seg_metrics == "source" and not source_frame:
             raise ValueError("seg_metrics='source' scores the source-frame mask: it needs source_frame=True")
+        if lesions not in (None,) + SEG_FRAMES:
+            raise ValueError(f"lesions must be None, 'input' or 'source', got {lesions!r}")
+        if lesions == "source" and not source_frame:
+            raise ValueError("lesions='source' labels the source-frame mask: it needs source_frame=True")
+        if roi not in ROI_RULES:
+            raise ValueError(f"roi must be 'all' or 'largest', got {roi!r}")
         if source == "ragged":
             capacity = ragged.capacity(capacity or 0)
             key = (B, slot, "ragged", capacity)
@@ -794,6 +815,11 @@ class PipelineRunner:
             key += ("source_frame",)
         if seg_metrics:
             key += ("seg_metrics", seg_metrics)
+        if lesions:
+            key += ("lesions", lesions)
+        if roi != "all":
+            key += ("roi", roi)
+        input_lesions = lesions == "input" or roi == "largest"
 
         def build():
             mb = min(B, self.micro_batch)
@@ -819,13 +845,22 @@ class PipelineRunner:
                                         IMG))
             pool = self._pools.setdefault(mb, [])
             gpool = self._gpools.setdefault(B, [])
+            if input_lesions:
+                ws["lesion_labels"], ws["lesion_mask"], ws["lesion_count"], ws["lesions"] = \
+                    L.outputs(B, ws["mask"], LESION_K, dev)
+                ws["lesion_workspace"] = L.workspace(mb, mb * IMG * IMG, LESION_K, dev)   # shared by the micro-batches
             for s in range(0, B, mb):
                 sl = slice(s, s + mb)
                 sub = {}
                 with self.unet.sharing(pool):
                     self.unet._emit_unet(mb, sub, ops, io=dict(x_in=ws["x_in"][sl], logits=ws["logits"][sl],
                                                                mask=ws["mask"][sl]))
-                self.unet._emit_bbox(mb, sub, ops, self.padding, boxes=ws["boxes"][sl])
+                if input_lesions:
+                    ops.append(L.lesions_desc(ws["mask"][sl], ws["lesion_labels"][sl], ws["lesion_mask"][sl],
+                                              ws["lesions"][sl], ws["lesion_count"][sl], ws["lesion_workspace"], mb,
+                                              LESION_CONNECTIVITY, LESION_K, Hs=IMG, Ws=IMG))
+                self.unet._emit_bbox(mb, sub, ops, self.padding, boxes=ws["boxes"][sl],
+                                     mask=ws["lesion_mask"][sl] if roi == "largest" else None)
                 ops.append(E.CropResizeDesc(ws["x_in"][sl].data_ptr(), ws["boxes"][sl].data_ptr(),
                                             ws["u8"][sl].data_ptr(), mb, IMG, IMG, IMG))
                 ws.setdefault("sub", []).append(sub)
@@ -837,6 +872,8 @@ class PipelineRunner:
                 self._emit_source_frame(B, source, capacity, ws, ops)
             if seg_metrics:
                 self._emit_seg_metrics(B, source, capacity, seg_metrics, ws, ops)
+            if lesions == "source":
+                self._emit_lesions(B, source, capacity, ws, ops)
             return _finish(self.engine, ops, ws, ua + ga + [v for v in ws.values() if isinstance(v, torch.Tensor)])
         return self.plans.get_or_build(key, build)
 
@@ -877,18 +914,35 @@ class PipelineRunner:
                                  Ws=Ws)
         ops.append(d)
 
-    def export_plan(self, B, source=None, capacity=None, cam=False, source_frame=False, seg_metrics=None):
+    def _emit_lesions(self, B, source, capacity, ws, ops):
+        """ug_lesions_desc over ws["src_mask"]: ws["src_lesion_labels"] i32 and ws["src_lesion_mask"] u8 placed like
+        it, ws["src_lesion_count"] i32 [B] and ws["src_lesions"] int64 [B,8,9].  A ragged plan reads the front-end's
+        table; as in _emit_source_frame, status is not written (src_status has it)."""
+        m = ws["src_mask"]
+        ws["src_lesion_labels"], ws["src_lesion_mask"], ws["src_lesion_count"], ws["src_lesions"] = \
+            L.outputs(B, m, LESION_K, self.dev)
+        ws["src_lesion_workspace"] = L.workspace(B, m.numel(), LESION_K, self.dev)
+        kw = dict(index=ws["src_index"], capacity=capacity) if source == "ragged" else dict(Hs=source[0], Ws=source[1])
+        ops.append(L.lesions_desc(m, ws["src_lesion_labels"], ws["src_lesion_mask"], ws["src_lesions"],
+                                  ws["src_lesion_count"], ws["src_lesion_workspace"], B, LESION_CONNECTIVITY, LESION_K,
+                                  **kw))
+
+    def export_plan(self, B, source=None, capacity=None, cam=False, source_frame=False, seg_metrics=None,
+                    lesions=None, roi="all"):
         """The whole two-stage program for a batch of B images as a relocatable plan image (bytes): op list, device
         memory layout, BN-folded packed weights of both networks.  A host in any language runs it through the C ABI
         alone (ug_plan_load / ug_plan_copy_in / ug_plan_run / ug_plan_copy_out, include/ugnet.h; examples/run_plan.c).
         source / capacity / cam / source_frame as for plan(); a ragged plan's inputs are "src_u8" and "src_index", a cam
         plan also reports "cam" and "cam_map", a source_frame plan "src_mask", "src_boxes" and (with cam)
-        "src_cam_map", a seg_metrics plan takes "gt_mask" and reports "seg_counts" and "seg_hd"."""
-        ws = self.plan(B, source=source, capacity=capacity, cam=cam, source_frame=source_frame, seg_metrics=seg_metrics)
+        "src_cam_map", a seg_metrics plan takes "gt_mask" and reports "seg_counts" and "seg_hd", a lesions / roi="largest"
+        plan "lesion_labels", "lesion_mask", "lesion_count" and "lesions" (or with lesions="source" their "src_" forms)."""
+        ws = self.plan(B, source=source, capacity=capacity, cam=cam, source_frame=source_frame, seg_metrics=seg_metrics,
+                       lesions=lesions, roi=roi)
         prog = ws["program"]
         io = {k: ws[k] for k in ("x_in", "src_u8", "src_index", "src_status", "logits", "mask", "boxes", "u8",
                                  "cls_logits", "cam", "cam_map", "src_mask", "src_boxes", "src_cam_map", "gt_mask", "seg_counts",
-                                 "seg_hd") if k in ws}
+                                 "seg_hd", "lesion_labels", "lesion_mask", "lesion_count", "lesions", "src_lesion_labels",
+                                 "src_lesion_mask", "src_lesion_count", "src_lesions") if k in ws}
         tensors = list(prog.keepalive) + list(io.values()) + [(self.unet.w_blob, True), (self.gnet.w_blob, True)]
         return E.export_plan(prog.descs, io, tensors)
 
@@ -903,18 +957,18 @@ class PipelineRunner:
             out.append((s, n - s))
         return out
 
-    def feed_ragged(self, part, cam=False, source_frame=False, seg_metrics=None):
+    def feed_ragged(self, part, cam=False, source_frame=False, seg_metrics=None, lesions=None, roi="all"):
         """The ragged plan for one chunk (a ragged.Packed of HWC images, at most one plan's batch) with its packed
         sources and table copied in (one copy each)."""
         ws = self.plan(len(part.table), source="ragged", capacity=part.n_px, cam=cam, source_frame=source_frame,
-                       seg_metrics=seg_metrics)
+                       seg_metrics=seg_metrics, lesions=lesions, roi=roi)
         ws["src_u8"][:part.data.numel()].copy_(part.data, non_blocking=True)
         ws["src_index"].copy_(ragged.table_tensor(part.table))
         return ws
 
     @torch.no_grad()
     def __call__(self, imgs, return_logits=False, return_cam=False, return_source=False, gt_masks=None,
-                 metrics_frame="input"):
+                 metrics_frame="input", lesions=None, roi="all"):
         """imgs: float [B,3,224,224] CUDA, or uint8 [B,Hs,Ws,3] CUDA source images of any size (resized on the
         device exactly as the reference's PIL transform does), or a list of uint8 [H,W,3] images of different sizes
         (CUDA tensors or numpy arrays, sides up to 8*224; one ragged batch, util/ragged.py) ->
@@ -925,7 +979,12 @@ class PipelineRunner:
         [H_i,W_i] tensors for a list; see plan(source_frame=True)), then a SegMetrics of the mask against `gt_masks` if
         given: in the form of the input, u8 [B,224,224] (metrics_frame="input", any input) or [B,Hs,Ws] / a list of
         [H_i,W_i] masks at each source's own size (metrics_frame="source", uint8 sources only); nonzero = foreground.
-        Every other output is the same with and without gt_masks."""
+        Every other output is the same with and without gt_masks.
+        Then, with lesions="input" / "source", a lesions.Lesions(count, labels, main_masks, table, derived) of the
+        connected components of the 224x224 masks / the source-frame masks (uint8 sources only; labels and main_masks
+        in the form of SourceFrame's masks); see plan(lesions=...) and lesions.py.  roi="largest" crops each image's
+        largest lesion instead of the hull of all its foreground pixels: boxes, class logits and CAM maps change,
+        masks and segmentation logits do not; an empty mask keeps roi.py's centred box."""
         from . import metrics
         masks, boxes, cls, seg, cams = [], [], [], [], []
         counts, hds = [], []
@@ -944,18 +1003,23 @@ class PipelineRunner:
         if gt_masks is not None:
             frame = metrics_frame
             gt = metrics.gt_batch(gt_masks, imgs, packed, frame)
-        src_frame = return_source or frame == "source"
+        if lesions == "source" and packed is None and not from_u8:
+            raise ValueError("lesions='source' needs uint8 sources: float [B,3,224,224] input has no source frame")
+        src_frame = return_source or frame == "source" or lesions == "source"
+        les = dict(lesions=lesions, roi=roi)
+        les_count, les_labels, les_main, les_table = [], [], [], []
         for s, c in self._chunks(n):
             if packed is not None:
                 part = ragged.chunk(packed, s, s + c)
-                kw = {k: v for k, v in (("cam", return_cam), ("source_frame", src_frame), ("seg_metrics", frame)) if v}
+                kw = {k: v for k, v in (("cam", return_cam), ("source_frame", src_frame), ("seg_metrics", frame),
+                                        ("lesions", lesions), ("roi", roi if roi != "all" else None)) if v}
                 ws = self.feed_ragged(part, **kw)
             elif from_u8:
                 ws = self.plan(c, source=(imgs.shape[1], imgs.shape[2]), cam=return_cam, source_frame=src_frame,
-                               seg_metrics=frame)
+                               seg_metrics=frame, **les)
                 ws["src_u8"].copy_(imgs[s:s + c])
             else:
-                ws = self.plan(c, cam=return_cam, seg_metrics=frame)
+                ws = self.plan(c, cam=return_cam, seg_metrics=frame, **les)
                 ws["x_in"].copy_(imgs[s:s + c])
             if frame == "source" and packed is not None:
                 ws["gt_mask"][:part.n_px].copy_(ragged.chunk(gt, s, s + c).data, non_blocking=True)
@@ -982,6 +1046,16 @@ class PipelineRunner:
             if frame is not None:
                 counts.append(ws["seg_counts"].cpu())
                 hds.append(ws["seg_hd"].cpu())
+            if lesions:
+                pre = "src_" if lesions == "source" else ""
+                les_count.append(ws[pre + "lesion_count"].clone())
+                les_table.append(ws[pre + "lesions"].clone())
+                if lesions == "source" and packed is not None:
+                    les_labels += ragged.unpack(ws["src_lesion_labels"][:part.n_px].clone(), part.table, 1)
+                    les_main += ragged.unpack(ws["src_lesion_mask"][:part.n_px].clone(), part.table, 1)
+                else:
+                    les_labels.append(ws[pre + "lesion_labels"].clone())
+                    les_main.append(ws[pre + "lesion_mask"].clone())
         out = (torch.cat(masks), torch.cat(boxes), torch.cat(cls))
         if return_logits:
             out += (torch.cat(seg),)
@@ -994,4 +1068,8 @@ class PipelineRunner:
             out += (SourceFrame(src_masks, torch.cat(src_boxes), src_cams if return_cam else None),)
         if frame is not None:
             out += (metrics.seg_result(torch.cat(counts), torch.cat(hds)),)
+        if lesions:
+            if lesions == "input" or packed is None:
+                les_labels, les_main = torch.cat(les_labels), torch.cat(les_main)
+            out += (L.result(torch.cat(les_count), les_labels, les_main, torch.cat(les_table)),)
         return out

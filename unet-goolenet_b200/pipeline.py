@@ -20,7 +20,7 @@ class TwoStagePipeline:
 
     @torch.no_grad()
     def __call__(self, imgs, return_logits=False, return_cam=False, return_source=False, gt_masks=None,
-                 metrics_frame="input"):
+                 metrics_frame="input", lesions=None, roi="all"):
         """imgs: float [B,3,224,224] on the pipeline's device, or uint8 HWC sources [B,Hs,Ws,3] of any size (resized
         on the device like the reference's CDDataAugmentation.transform: PIL bilinear + to_tensor), or a list of uint8
         [H,W,3] images of different sizes (CUDA tensors or numpy arrays; run as ragged batches, util/ragged.py) ->
@@ -30,9 +30,13 @@ class TwoStagePipeline:
         same outputs at each source image's own size if return_source (uint8 sources only; lists of per-image tensors
         for a list of images; cam_maps is None without return_cam), and by a SegMetrics(counts, dice, iou, hd, hd95) of
         the mask against gt_masks if given (metrics_frame "input": u8 [B,224,224]; "source": masks at each source's own
-        size, a tensor [B,Hs,Ws] or a list like the input; see PipelineRunner.__call__ and metrics.py)."""
+        size, a tensor [B,Hs,Ws] or a list like the input; see PipelineRunner.__call__ and metrics.py), and by a
+        lesions.Lesions(count, labels, main_masks, table, derived) of the connected components of the mask if lesions
+        is "input" (224x224 masks) or "source" (source-frame masks, uint8 sources only).  roi="largest" crops each
+        image's largest lesion instead of the hull of all its foreground pixels (boxes, class logits and CAM follow;
+        masks do not change)."""
         return self.runner(imgs, return_logits=return_logits, return_cam=return_cam, return_source=return_source,
-                           gt_masks=gt_masks, metrics_frame=metrics_frame)
+                           gt_masks=gt_masks, metrics_frame=metrics_frame, lesions=lesions, roi=roi)
 
     def predict(self, imgs):
         """argmax(softmax(logits)) as 分类/test.py:86 (softmax is monotone, so argmax of the logits)."""
