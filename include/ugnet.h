@@ -412,6 +412,29 @@ typedef struct ug_lesions_desc {
   int B, Hs, Ws, connectivity, K;
 } ug_lesions_desc;
 
+/* Per-lesion ROI crops: the crop of ug_cropresize_desc taken around each of the R largest lesions of ug_lesions' table
+ * instead of around the whole mask, so that every lesion of an image can be graded.  Outputs are rank-major: rank r of
+ * the B images is one contiguous batch [B] of boxes, statuses and crops.  For image i and rank r < R, with
+ * row = lesions[i*K + r], the row is graded iff r < count[i], row.label >= 1, row.area >= 1, 0 <= row.x0 < row.x1 <= W,
+ * 0 <= row.y0 < row.y1 <= H and the box
+ *   {max(x0 - padding, 0), max(y0 - padding, 0), min(x1 - 1 + padding, W), min(y1 - 1 + padding, H)}
+ * (roi.py:33-36 applied to the lesion's own pixels; for rank 0 exactly ug_bbox of ug_lesions' main mask) is non-empty
+ * (it is empty only for padding 0 and a lesion one pixel wide or high).  A graded row gets that box, status 0 and the
+ * crop of ug_cropresize_desc from it (trunc(x*255), channel flip, PIL-exact bilinear resize to SxS).  A row not graded
+ * gets the box {0,0,0,0}, status 1 and a zero crop, and nothing is read through it beyond the six integers checked.
+ * The table may come from outside the library.  1 <= R <= K <= 32, padding >= 0, 1 <= S <= 512, 1 <= H, W <= 8*S and
+ * R*B <= 65535 (UG_EINVAL otherwise, nothing written).  One launch; its geometry depends on B, R, S (and H, W) only,
+ * never on the table; the outputs are bit-identical run to run. */
+typedef struct ug_lesion_crops_desc {
+  const float* img;            /* fp32 NCHW [B,3,H,W] in [0,1]: the UNet input (x_in) */
+  const ug_lesion* lesions;    /* [B][K]: ug_lesions' table */
+  const int* count;            /* int32 [B]: ug_lesions' count */
+  int* boxes;                  /* int32 [R][B][4] {x0,y0,x1,y1}, end-exclusive; {0,0,0,0} where not graded */
+  int* status;                 /* int32 [R][B]: 0 = graded, 1 = no lesion at this rank or row rejected (required) */
+  unsigned char* out_u8;       /* u8 [R][B][S][S][3]: the crops (HWC, channel order as ug_cropresize); zeros where not graded */
+  int B, H, W, S, K, R, padding;
+} ug_lesion_crops_desc;
+
 enum {
   UG_OP_CONV = 1,
   /* 2 and 10 were the stand-alone im2col packs of round 1 (replaced by UG_OP_STEM); the numbers stay retired */
@@ -432,7 +455,8 @@ enum {
   UG_OP_CAM = 18,
   UG_OP_SOURCE_FRAME = 19,
   UG_OP_SEG_METRICS = 20,
-  UG_OP_LESIONS = 21
+  UG_OP_LESIONS = 21,
+  UG_OP_LESION_CROPS = 22
 };
 
 typedef struct ug_op {
@@ -458,6 +482,7 @@ typedef struct ug_op {
     ug_source_frame_desc source_frame; /* and so is this one */
     ug_seg_metrics_desc seg_metrics;   /* as is this one */
     ug_lesions_desc lesions;           /* and this one */
+    ug_lesion_crops_desc lesion_crops; /* and this one */
   } u;
 } ug_op;
 
@@ -488,6 +513,7 @@ int ug_cam(ug_handle h, const ug_cam_desc* d, void* stream);
 int ug_source_frame(ug_handle h, const ug_source_frame_desc* d, void* stream);
 int ug_seg_metrics(ug_handle h, const ug_seg_metrics_desc* d, void* stream);
 int ug_lesions(ug_handle h, const ug_lesions_desc* d, void* stream);
+int ug_lesion_crops(ug_handle h, const ug_lesion_crops_desc* d, void* stream);
 size_t ug_wavelet_workspace_bytes(int B, int H, int W);
 size_t ug_wavelet_ragged_workspace_bytes(int B, long long capacity_px);
 /* Workspace of ug_seg_metrics for B images in capacity_px pixels (ragged capacity, or B*Hs*Ws); 0 for bad arguments. */
@@ -552,7 +578,13 @@ int ug_program_run_host_pipelined(ug_handle h, ug_program p, const ug_copy* h2d,
  * roi="largest" "boxes", the crops, "cls_logits" and the CAM follow the box of "lesion_mask" instead of "mask" ("mask"
  * and "logits" do not change).  With lesions="source" (and source_frame=True) the op runs last on "src_mask" and
  * reports "src_lesion_labels" i32 and "src_lesion_mask" u8 placed like "src_mask", "src_lesion_count" i32 [B] and
- * "src_lesions" ug_lesion [B,8]. */
+ * "src_lesions" ug_lesion [B,8].  A plan exported with grade_lesions=R (1 <= R <= 8; export_plan(B, ...,
+ * grade_lesions=R)) also labels the 224x224 masks as lesions="input" does, crops the R largest lesions of each image
+ * (ug_lesion_crops_desc, the plan's padding) and grades each crop with GoogLeNet, one batch of B crops per rank:
+ * "lesion_boxes" i32 [R,B,4], "lesion_status" i32 [R,B] (0 = graded), "lesion_u8" u8 [R,B,224,224,3] and
+ * "lesion_cls_logits" f32 [R,B,6]; with cam=True also "lesion_cam" f32 [R,B,7,7] and "lesion_cam_map" f32
+ * [R,B,224,224] (the map inside each lesion's box).  Rows not graded have zero boxes, crops and CAM; their logits are
+ * those of a zero crop.  Every other output is the same as without grade_lesions. */
 typedef struct ug_plan_s* ug_plan;
 /* Parses the image (host memory, may be freed afterwards), allocates ONE device arena for every buffer of the plan
  * (ug_plan_device_bytes), uploads the constants, relocates the op list and prepares the program. */

@@ -58,6 +58,7 @@ static int run_simple(ug_engine* h, const ug_op* op, cudaStream_t s) {
     case UG_OP_SOURCE_FRAME: return launch_source_frame(h, &op->u.source_frame, s);
     case UG_OP_SEG_METRICS: return launch_seg_metrics(h, &op->u.seg_metrics, s);
     case UG_OP_LESIONS: return launch_lesions(h, &op->u.lesions, s);
+    case UG_OP_LESION_CROPS: return launch_lesion_crops(h, &op->u.lesion_crops, s);
     default: return set_error(h, UG_EINVAL, "unknown op kind %d", op->kind);
   }
 }
@@ -145,6 +146,7 @@ UG_SIMPLE_ENTRY(ug_cam, ug_cam_desc, launch_cam)
 UG_SIMPLE_ENTRY(ug_source_frame, ug_source_frame_desc, launch_source_frame)
 UG_SIMPLE_ENTRY(ug_seg_metrics, ug_seg_metrics_desc, launch_seg_metrics)
 UG_SIMPLE_ENTRY(ug_lesions, ug_lesions_desc, launch_lesions)
+UG_SIMPLE_ENTRY(ug_lesion_crops, ug_lesion_crops_desc, launch_lesion_crops)
 
 int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out) {
   if (!h || !ops || n_ops <= 0 || !out) return UG_EINVAL;
@@ -172,7 +174,7 @@ int ug_program_create(ug_handle h, const ug_op* ops, int n_ops, ug_program* out)
         delete p;
         return rc;
       }
-    } else if (po.kind < UG_OP_CONV || po.kind > UG_OP_LESIONS) {
+    } else if (po.kind < UG_OP_CONV || po.kind > UG_OP_LESION_CROPS) {
       delete p;
       return set_error(h, UG_EINVAL, "op %d: unknown kind %d", i, po.kind);
     }

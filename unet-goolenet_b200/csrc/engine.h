@@ -21,7 +21,7 @@ struct ug_engine {
   // "already raised" flags are per handle (= per device), not process-wide
   bool attr_gemm = false, attr_multi = false, attr_pair = false, attr_stem = false, attr_attn = false;
   int max_pairs = -1;  // co-resident clusters of two ~200 KB CTAs on this device (cudaOccupancyMaxActiveClusters), -1 = not queried
-  size_t attr_resize = 0, attr_crop = 0, attr_ragged = 0;
+  size_t attr_resize = 0, attr_crop = 0, attr_ragged = 0, attr_lesion_crop = 0;
 };
 
 namespace ug {
@@ -334,5 +334,6 @@ int launch_cam(ug_engine* h, const ug_cam_desc* d, cudaStream_t s);
 int launch_source_frame(ug_engine* h, const ug_source_frame_desc* d, cudaStream_t s);
 int launch_seg_metrics(ug_engine* h, const ug_seg_metrics_desc* d, cudaStream_t s);
 int launch_lesions(ug_engine* h, const ug_lesions_desc* d, cudaStream_t s);
+int launch_lesion_crops(ug_engine* h, const ug_lesion_crops_desc* d, cudaStream_t s);
 
 }  // namespace ug

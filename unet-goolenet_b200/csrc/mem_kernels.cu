@@ -822,16 +822,44 @@ __device__ void pil_coef_general(int in_size, int out_size, int xx, RsCoef* c) {
 // NCHW image in [0,1], quantised as (x*255).astype(uint8) with the channel order reversed (roi.py:39-44), i.e. the
 // ROI stage (ug_cropresize_desc); d.src is unused, `img` / `boxes` / `IH` / `IW` describe the float image.  kRagged:
 // uint8 HWC images of different sizes (ug_resize_ragged_desc); image n's size and offset come from rg.index[n].
-enum { kUniform = 0, kCrop = 1, kRagged = 2 };
+// kLesionCrop: kCrop around the lesions of ug_lesions' table (ug_lesion_crops_desc); block row n is rank n / B of
+// image n % B, its box is derived from that table row (ls) and written out with the row's status.
+enum { kUniform = 0, kCrop = 1, kRagged = 2, kLesionCrop = 3 };
 struct RaggedSrc {
   const ug_ragged_image* index;
   int* status;
   long long src_bytes;
 };
+struct LesionSrc {
+  const ug_lesion* lesions;
+  const int* count;
+  int* boxes;
+  int* status;
+  int K, padding;
+};
+
+// The box of rank n / B of image n % B (ug_lesion_crops_desc): false (box zero) when the row is not graded.  The table
+// may come from outside the library: the row is read only for r < count, and only its six checked integers are used
+// (the box arithmetic is 64-bit: padding may be as large as INT_MAX).
+__device__ __forceinline__ bool lesion_crop_box(const LesionSrc& ls, int n, int B, int H, int W, int* box) {
+  const int i = n % B, r = n / B;
+  box[0] = box[1] = box[2] = box[3] = 0;
+  if (r >= ls.count[i]) return false;
+  const ug_lesion& row = ls.lesions[(long long)i * ls.K + r];
+  const int x0 = row.x0, y0 = row.y0, x1 = row.x1, y1 = row.y1;
+  if (row.label < 1 || row.area < 1 || x0 < 0 || x0 >= x1 || x1 > W || y0 < 0 || y0 >= y1 || y1 > H) return false;
+  const int bx0 = max(x0 - ls.padding, 0), by0 = max(y0 - ls.padding, 0);   // roi.py:33-36 on the lesion's pixels
+  const int bx1 = (int)min((long long)x1 - 1 + ls.padding, (long long)W);
+  const int by1 = (int)min((long long)y1 - 1 + ls.padding, (long long)H);
+  if (bx0 >= bx1 || by0 >= by1) return false;
+  box[0] = bx0, box[1] = by0, box[2] = bx1, box[3] = by1;
+  return true;
+}
 
 template <int kMode>
 __global__ void __launch_bounds__(256) resize_u8_kernel(ug_resize_desc d, int max_src_rows, const float* __restrict__ img,
-                                                        const int* __restrict__ boxes, int IH, int IW, RaggedSrc rg) {
+                                                        const int* __restrict__ boxes, int IH, int IW, RaggedSrc rg,
+                                                        LesionSrc ls) {
   pdl_wait();  // programmatic dependent launch: see common.cuh
   pdl_launch_dependents();
   extern __shared__ unsigned char rs_smem[];
@@ -843,6 +871,24 @@ __global__ void __launch_bounds__(256) resize_u8_kernel(ug_resize_desc d, int ma
   const int rows = min(kRsRows, d.S - oy0);
   int bx0 = 0, by0 = 0;
   long long src_off = (long long)n * d.Hs * d.Ws * 3;
+  constexpr bool kFloatSrc = kMode == kCrop || kMode == kLesionCrop;
+  if (kMode == kLesionCrop) {
+    int box[4];
+    const bool ok = lesion_crop_box(ls, n, d.B, IH, IW, box);
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+      for (int k = 0; k < 4; ++k) ls.boxes[n * 4 + k] = box[k];
+      ls.status[n] = ok ? 0 : 1;
+    }
+    if (!ok) {  // this block's output rows of a row not graded are zeros
+      for (int t = threadIdx.x; t < rows * d.S; t += blockDim.x) {
+        unsigned char* o = d.out_u8 + (((long long)n * d.S + oy0 + t / d.S) * d.S + t % d.S) * 3;
+        o[0] = o[1] = o[2] = 0;
+      }
+      return;
+    }
+    d.Ws = box[2] - box[0];   // the box corner is derived again after the coefficients (fewer live registers)
+    d.Hs = box[3] - box[1];
+  }
   if (kMode == kCrop) {
     bx0 = boxes[n * 4 + 0];
     by0 = boxes[n * 4 + 1];
@@ -877,14 +923,20 @@ __global__ void __launch_bounds__(256) resize_u8_kernel(ug_resize_desc d, int ma
   __syncthreads();
   const int sy0 = s_v[0].xmin;                                          // first / one-past-last source row needed
   const int sy1 = s_v[rows - 1].xmin + s_v[rows - 1].n;
-  const unsigned char* src = kMode == kCrop ? nullptr : d.src + src_off;
-  const float* fimg = kMode == kCrop ? img + (long long)n * 3 * IH * IW : nullptr;
+  const unsigned char* src = kFloatSrc ? nullptr : d.src + src_off;
+  const float* fimg = kFloatSrc ? img + (long long)(kMode == kLesionCrop ? n % d.B : n) * 3 * IH * IW : nullptr;
+  if (kMode == kLesionCrop) {
+    int box[4];
+    lesion_crop_box(ls, n, d.B, IH, IW, box);
+    bx0 = box[0];
+    by0 = box[1];
+  }
   const int row_elems = d.S * 3;
   for (int t = threadIdx.x; t < (sy1 - sy0) * d.S; t += blockDim.x) {   // horizontal pass (one output pixel, 3 ch)
     const int r = t / d.S, ox = t - r * d.S;
     const RsCoef& hc = s_h[ox];
     int a0 = 1 << (kPrecBits - 1), a1 = a0, a2 = a0;
-    if (kMode == kCrop) {
+    if (kFloatSrc) {
       // (roi*255).astype(uint8): fp32 multiply, truncate; output channel c reads plane 2-c (cv2.COLOR_BGR2RGB)
       const float* p0 = fimg + ((long long)(by0 + sy0 + r)) * IW + bx0 + hc.xmin;
       const long long plane = (long long)IH * IW;
@@ -953,7 +1005,7 @@ int launch_resize_u8(ug_engine* h, const ug_resize_desc* d, cudaStream_t s) {
     h->attr_resize = smem;
   }
   launch_pdl(resize_u8_kernel<kUniform>, dim3(ceil_div(d->S, kRsRows), d->B), 256, smem, s, *d, max_rows, nullptr, nullptr,
-             0, 0, RaggedSrc{});
+             0, 0, RaggedSrc{}, LesionSrc{});
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "resize_u8 launch");
 }
@@ -975,7 +1027,7 @@ int launch_resize_ragged(ug_engine* h, const ug_resize_ragged_desc* d, cudaStrea
   ug_resize_desc r;
   r.src = d->src; r.out_f32 = d->out_f32; r.out_u8 = d->out_u8; r.B = d->B; r.Hs = 0; r.Ws = 0; r.S = d->S;
   launch_pdl(resize_u8_kernel<kRagged>, dim3(ceil_div(d->S, kRsRows), d->B), 256, smem, s, r, max_rows, nullptr, nullptr,
-             0, 0, RaggedSrc{d->index, d->status, d->src_bytes});
+             0, 0, RaggedSrc{d->index, d->status, d->src_bytes}, LesionSrc{});
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "resize_ragged launch");
 }
@@ -1008,9 +1060,35 @@ int launch_cropresize(ug_engine* h, const ug_cropresize_desc* d, cudaStream_t s)
   ug_resize_desc r;
   r.src = nullptr; r.out_f32 = nullptr; r.out_u8 = d->out_u8; r.B = d->B; r.Hs = d->H; r.Ws = d->W; r.S = d->S;
   launch_pdl(resize_u8_kernel<kCrop>, L.grid, L.block, L.smem, s, r, L.max_rows, d->img, d->boxes, d->H, d->W,
-             RaggedSrc{});
+             RaggedSrc{}, LesionSrc{});
   h->launches++;
   return check_cuda(h, cudaGetLastError(), "cropresize launch");
+}
+
+// Per-lesion ROI crops (ug_lesion_crops_desc): the kCrop kernel with one block row per (rank, image), each deriving
+// its box from the lesion table.  Shared memory is sized as plan_cropresize's for the whole H x W image (a box is
+// never larger), so the launch depends on B, R, S, H and W only.
+int launch_lesion_crops(ug_engine* h, const ug_lesion_crops_desc* d, cudaStream_t s) {
+  if (!d->img || !d->lesions || !d->count || !d->boxes || !d->status || !d->out_u8 || d->B <= 0 || d->R < 1 ||
+      d->R > d->K || d->K > 32 || d->padding < 0 || d->S < 1 || d->S > 512 || d->H < 1 || d->W < 1 ||
+      d->H > kRsMaxSide * d->S || d->W > kRsMaxSide * d->S || (long long)d->R * d->B > 65535)
+    return set_error(h, UG_EINVAL, "lesion_crops: bad args (1 <= R <= K <= 32, padding >= 0, S <= 512, H, W <= 8*S)");
+  const double sc = std::max(std::max((double)d->H / d->S, (double)d->W / d->S), 1.0);
+  const int max_rows = std::min(d->H, (int)ceil((kRsRows - 1) * sc + 2.0 * sc + 3.0));
+  const size_t smem = (size_t)(d->S + kRsRows) * sizeof(RsCoef) + (size_t)max_rows * d->S * 3;
+  if (smem > h->attr_lesion_crop) {
+    cudaError_t e = cudaFuncSetAttribute((const void*)resize_u8_kernel<kLesionCrop>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return check_cuda(h, e, "cudaFuncSetAttribute(resize_u8_kernel<lesion crop>)");
+    h->attr_lesion_crop = smem;
+  }
+  ug_resize_desc r;
+  r.src = nullptr; r.out_f32 = nullptr; r.out_u8 = d->out_u8; r.B = d->B; r.Hs = d->H; r.Ws = d->W; r.S = d->S;
+  launch_pdl(resize_u8_kernel<kLesionCrop>, dim3(ceil_div(d->S, kRsRows), d->R * d->B), 256, smem, s, r, max_rows,
+             d->img, nullptr, d->H, d->W, RaggedSrc{}, LesionSrc{d->lesions, d->count, d->boxes, d->status, d->K,
+                                                                 d->padding});
+  h->launches++;
+  return check_cuda(h, cudaGetLastError(), "lesion_crops launch");
 }
 
 // ------------------------------------------------------------------------------------------------

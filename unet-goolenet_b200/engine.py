@@ -22,6 +22,7 @@ EPI_STORE, EPI_ADD, EPI_GATE, EPI_OUTC = 0, 1, 2, 3
 OP_CONV, OP_POOL, OP_LAYERNORM, OP_ATTN, OP_CHANSTATS, OP_GATE, OP_BBOX, OP_CROPRESIZE = 1, 3, 4, 5, 6, 7, 8, 9
 OP_HEAD, OP_STEM, OP_RESIZE, OP_WAVELET, OP_S2D = 11, 12, 13, 14, 15
 OP_RESIZE_RAGGED, OP_WAVELET_RAGGED, OP_CAM, OP_SOURCE_FRAME, OP_SEG_METRICS, OP_LESIONS = 16, 17, 18, 19, 20, 21
+OP_LESION_CROPS = 22
 
 _vp, _i, _f, _ll = C.c_void_p, C.c_int, C.c_float, C.c_longlong
 
@@ -133,13 +134,19 @@ class LesionsDesc(C.Structure):
                 ("capacity_px", _ll), ("B", _i), ("Hs", _i), ("Ws", _i), ("connectivity", _i), ("K", _i)]
 
 
+class LesionCropsDesc(C.Structure):
+    _fields_ = [("img", _vp), ("lesions", _vp), ("count", _vp), ("boxes", _vp), ("status", _vp), ("out_u8", _vp),
+                ("B", _i), ("H", _i), ("W", _i), ("S", _i), ("K", _i), ("R", _i), ("padding", _i)]
+
+
 class _OpUnion(C.Union):
     _fields_ = [("conv", ConvDesc), ("pool", PoolDesc), ("ln", LayerNormDesc),
                 ("attn", AttnDesc), ("stats", ChanStatsDesc), ("gate", GateDesc), ("bbox", BBoxDesc),
                 ("crop", CropResizeDesc), ("head", HeadDesc), ("stem", StemDesc),
                 ("resize", ResizeDesc), ("wavelet", WaveletDesc), ("s2d", S2dDesc),
                 ("resize_ragged", ResizeRaggedDesc), ("wavelet_ragged", WaveletRaggedDesc), ("cam", CamDesc),
-                ("source_frame", SourceFrameDesc), ("seg_metrics", SegMetricsDesc), ("lesions", LesionsDesc)]
+                ("source_frame", SourceFrameDesc), ("seg_metrics", SegMetricsDesc), ("lesions", LesionsDesc),
+                ("lesion_crops", LesionCropsDesc)]
 
 
 class Op(C.Structure):
@@ -154,13 +161,15 @@ _KIND_FIELD = {OP_CONV: "conv", OP_POOL: "pool", OP_LAYERNORM: "ln", OP_ATTN: "a
                OP_CHANSTATS: "stats", OP_GATE: "gate", OP_BBOX: "bbox", OP_CROPRESIZE: "crop",
                OP_HEAD: "head", OP_STEM: "stem", OP_RESIZE: "resize", OP_WAVELET: "wavelet", OP_S2D: "s2d",
                OP_RESIZE_RAGGED: "resize_ragged", OP_WAVELET_RAGGED: "wavelet_ragged", OP_CAM: "cam",
-               OP_SOURCE_FRAME: "source_frame", OP_SEG_METRICS: "seg_metrics", OP_LESIONS: "lesions"}
+               OP_SOURCE_FRAME: "source_frame", OP_SEG_METRICS: "seg_metrics", OP_LESIONS: "lesions",
+               OP_LESION_CROPS: "lesion_crops"}
 _DESC_KIND = {ConvDesc: OP_CONV, PoolDesc: OP_POOL, LayerNormDesc: OP_LAYERNORM,
               AttnDesc: OP_ATTN, ChanStatsDesc: OP_CHANSTATS, GateDesc: OP_GATE, BBoxDesc: OP_BBOX,
               CropResizeDesc: OP_CROPRESIZE, HeadDesc: OP_HEAD, StemDesc: OP_STEM,
               ResizeDesc: OP_RESIZE, WaveletDesc: OP_WAVELET, S2dDesc: OP_S2D,
               ResizeRaggedDesc: OP_RESIZE_RAGGED, WaveletRaggedDesc: OP_WAVELET_RAGGED, CamDesc: OP_CAM,
-              SourceFrameDesc: OP_SOURCE_FRAME, SegMetricsDesc: OP_SEG_METRICS, LesionsDesc: OP_LESIONS}
+              SourceFrameDesc: OP_SOURCE_FRAME, SegMetricsDesc: OP_SEG_METRICS, LesionsDesc: OP_LESIONS,
+              LesionCropsDesc: OP_LESION_CROPS}
 _SINGLE_ENTRY = {OP_CONV: "ug_conv", OP_POOL: "ug_pool",
                  OP_LAYERNORM: "ug_layernorm", OP_ATTN: "ug_attention", OP_CHANSTATS: "ug_chanstats",
                  OP_GATE: "ug_gate", OP_BBOX: "ug_bbox", OP_CROPRESIZE: "ug_cropresize",
@@ -168,7 +177,7 @@ _SINGLE_ENTRY = {OP_CONV: "ug_conv", OP_POOL: "ug_pool",
                  OP_RESIZE: "ug_resize_u8", OP_WAVELET: "ug_wavelet", OP_S2D: "ug_s2d_pack",
                  OP_RESIZE_RAGGED: "ug_resize_ragged", OP_WAVELET_RAGGED: "ug_wavelet_ragged", OP_CAM: "ug_cam",
                  OP_SOURCE_FRAME: "ug_source_frame", OP_SEG_METRICS: "ug_seg_metrics",
-                 OP_LESIONS: "ug_lesions"}
+                 OP_LESIONS: "ug_lesions", OP_LESION_CROPS: "ug_lesion_crops"}
 
 EXPORTED_SYMBOLS = ["ug_version", "ug_create", "ug_destroy", "ug_last_error", "ug_launch_count",
                     *_SINGLE_ENTRY.values(), "ug_program_create", "ug_program_run", "ug_program_num_launches",

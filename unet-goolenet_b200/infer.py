@@ -56,7 +56,7 @@ def inference_all_seg(model, test_loader, device, save_dir=None):
 
 @torch.no_grad()
 def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256, cam_dir=None, mask_dir=None,
-                 frame="input", roi="all", lesions=None):
+                 frame="input", roi="all", lesions=None, grade_lesions=0):
     """The whole of 分类/test.py:122-134 + :74-96 on the device for a batch of grayscale images:
     cv2.imread(path, 0) output (uint8 [H, W]) -> wavelet_enhance -> resize 224 + to_tensor -> UNet -> mask -> bbox ->
     ROI crop/resize -> GoogLeNet -> argmax; returns the sorted "<name> <class>" records (and writes result.txt).
@@ -79,31 +79,46 @@ def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256
     lesions: "input" / "source" also labels the connected components of the 224x224 / source-frame masks and, with
     save_dir, writes `lesions.csv`: one row per table row of an image with lesions (the 8 largest, lesions.py), in the
     order of result.txt: name, rank, count, label, area, box x0 y0 x1 y1 (end-exclusive), centroid cx cy,
-    orientation, major and minor axis, eccentricity, equivalent diameter and boundary (pixel units)."""
+    orientation, major and minor axis, eccentricity, equivalent diameter and boundary (pixel units).
+    grade_lesions: R in 1..8 also grades each of the R largest lesions of an image on its own crop
+    (PipelineRunner.plan(grade_lesions=R)) and implies lesions="input": lesions.csv gains the columns pred (the class
+    of the lesion's crop, test.py:86) and prob (its softmax probability), both empty for ranks >= R and for lesions
+    whose padded box is empty.  result.txt keeps the per-image grade."""
+    from . import lesions as L
     from .util.wavelet import wavelet_enhance_batch
     if frame not in ("input", "source"):
         raise ValueError(f"frame must be 'input' or 'source', got {frame!r}")
     if lesions not in (None, "input", "source"):
         raise ValueError(f"lesions must be None, 'input' or 'source', got {lesions!r}")
+    L.check_grade_lesions(grade_lesions, 8)
+    if grade_lesions and lesions == "source":
+        raise ValueError("grade_lesions grades the lesions of the 224x224 mask: the source-frame table (lesions='source') "
+                         "numbers the components of a different mask")
+    if grade_lesions:
+        lesions = "input"
     runner = getattr(pipeline, "runner", pipeline)
     les_rows = []
     if isinstance(gray_images, (list, tuple)):
-        records = _grade_ragged(runner, gray_images, filenames, cam_dir, mask_dir, frame, roi, lesions, les_rows)
+        records = _grade_ragged(runner, gray_images, filenames, cam_dir, mask_dir, frame, roi, lesions, les_rows,
+                                grade_lesions)
     else:
         g = torch.as_tensor(np.ascontiguousarray(gray_images) if isinstance(gray_images, np.ndarray) else gray_images)
         source = frame == "source" and (cam_dir is not None or mask_dir is not None)
         records = []
         for s in range(0, g.shape[0], batch_size):
             rgb = wavelet_enhance_batch(g[s:s + batch_size].to(runner.dev))      # [B,H,W,3] uint8, test.py:128-129
-            out = runner(rgb, return_cam=cam_dir is not None, return_source=source, lesions=lesions,
-                         roi=roi)                                                  # test.py:130-131 and :82-84
+            out = runner(rgb, return_cam=cam_dir is not None, return_source=source, lesions=lesions, roi=roi,
+                         grade_lesions=grade_lesions)                              # test.py:130-131 and :82-84
             pred = torch.argmax(torch.softmax(out[2], dim=1), dim=1).cpu().numpy()  # test.py:86
             names = filenames[s:s + batch_size]
             for i, name in enumerate(names):
                 records.append(f"{name.replace('.png', '')} {int(pred[i])}")
+            gr = None
+            if grade_lesions:
+                gr, out = out[-1], out[:-1]
             if lesions:
                 les = out[-1]
-                les_rows += _lesion_rows(names, les.count, les.table, les.derived)
+                les_rows += _lesion_rows(names, les.count, les.table, les.derived, gr)
                 out = out[:-1]
             if source:
                 _write_maps(out[-1].cam_maps, out[-1].masks, names, cam_dir, mask_dir)
@@ -111,16 +126,20 @@ def grade_images(pipeline, gray_images, filenames, save_dir=None, batch_size=256
                 _write_maps(out[3] if cam_dir is not None else None, out[0], names, cam_dir, mask_dir)
     records = _write_records(records, save_dir)
     if lesions and save_dir is not None:
-        _write_lesions(les_rows, save_dir)
+        _write_lesions(les_rows, save_dir, LESION_COLUMNS + (GRADE_COLUMNS if grade_lesions else []))
     return records
 
 
 LESION_COLUMNS = ["name", "rank", "count", "label", "area", "x0", "y0", "x1", "y1", "cx", "cy", "orientation",
                   "major_axis", "minor_axis", "eccentricity", "equivalent_diameter", "boundary"]
+GRADE_COLUMNS = ["pred", "prob"]
 
 
-def _lesion_rows(names, count, table, derived):
-    """lesions.csv rows (dicts of LESION_COLUMNS) of a batch: every table row with a lesion, rank 0 = the largest."""
+def _lesion_rows(names, count, table, derived, grades=None):
+    """lesions.csv rows (dicts of LESION_COLUMNS, and GRADE_COLUMNS with `grades`, a lesions.LesionGrades) of a batch:
+    every table row with a lesion, rank 0 = the largest."""
+    if grades is not None:
+        probs = torch.softmax(grades.logits, dim=2)
     out = []
     for i, name in enumerate(names):
         for k in range(table.shape[1]):
@@ -132,19 +151,23 @@ def _lesion_rows(names, count, table, derived):
             r.update(cx=float(derived.cx[i, k]), cy=float(derived.cy[i, k]))
             r.update({c: float(getattr(derived, c)[i, k]) for c in ("orientation", "major_axis", "minor_axis",
                                                                       "eccentricity", "equivalent_diameter")})
+            if grades is not None:
+                graded = k < grades.status.shape[1] and int(grades.status[i, k]) == 0
+                p = int(grades.pred[i, k]) if graded else None
+                r.update(pred=p, prob=float(probs[i, k, p]) if graded else None)
             out.append(r)
     return out
 
 
-def _write_lesions(rows, save_dir):
+def _write_lesions(rows, save_dir, columns):
     import csv
     rows = sorted(rows, key=lambda r: (int(r["name"].replace(".jpg", "").replace(".png", "")), r["rank"]))
     os.makedirs(save_dir, exist_ok=True)
     with open(os.path.join(save_dir, "lesions.csv"), "w", newline="") as f:
         w = csv.writer(f)
-        w.writerow(LESION_COLUMNS)
+        w.writerow(columns)
         for r in rows:
-            w.writerow([repr(r[c]) if isinstance(r[c], float) else r[c] for c in LESION_COLUMNS])
+            w.writerow(["" if r[c] is None else (repr(r[c]) if isinstance(r[c], float) else r[c]) for c in columns])
 
 
 def _stem_png(d, name):
@@ -171,7 +194,7 @@ def _write_maps(cam_maps, masks, names, cam_dir, mask_dir):
 
 
 def _grade_ragged(runner, gray_images, filenames, cam_dir=None, mask_dir=None, frame="input", roi="all",
-                  lesions=None, les_rows=None):
+                  lesions=None, les_rows=None, grade_lesions=0):
     from . import lesions as L
     from .util import ragged
     from .util.wavelet import wavelet_ragged_into
@@ -181,7 +204,8 @@ def _grade_ragged(runner, gray_images, filenames, cam_dir=None, mask_dir=None, f
     for s, c in runner._chunks(len(gray_images)):
         part = ragged.chunk(packed, s, s + c)
         ws = runner.plan(c, source="ragged", capacity=part.n_px, cam=cam_dir is not None,
-                         source_frame=source or lesions == "source", lesions=lesions, roi=roi)
+                         source_frame=source or lesions == "source", lesions=lesions, roi=roi,
+                         grade_lesions=grade_lesions)
         gray = part.data.to(runner.dev, non_blocking=True)
         ws["src_index"].copy_(ragged.table_tensor(part.table))
         wavelet_ragged_into(gray, ws["src_index"], ws["src_u8"], c)         # test.py:128-129, into the plan's input
@@ -193,7 +217,11 @@ def _grade_ragged(runner, gray_images, filenames, cam_dir=None, mask_dir=None, f
         if lesions:
             pre = "src_" if lesions == "source" else ""
             table = L.rows(ws[pre + "lesions"])
-            les_rows += _lesion_rows(names, ws[pre + "lesion_count"].cpu(), table, L.derive(table))
+            gr = None
+            if grade_lesions:
+                gr = L.grades(ws["lesion_count"], ws["lesion_status"].t(), ws["lesion_boxes"].transpose(0, 1),
+                              ws["lesion_cls_logits"].transpose(0, 1))
+            les_rows += _lesion_rows(names, ws[pre + "lesion_count"].cpu(), table, L.derive(table), gr)
         if source:
             cams = ragged.unpack(ws["src_cam_map"], part.table, 1) if cam_dir is not None else None
             _write_maps(cams, ragged.unpack(ws["src_mask"], part.table, 1), names, cam_dir, mask_dir)

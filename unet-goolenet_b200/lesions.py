@@ -68,6 +68,38 @@ class Lesions(NamedTuple):
     derived: Shape
 
 
+class LesionGrades(NamedTuple):
+    """A grade for each of the R largest lesions of every image (PipelineRunner.plan(grade_lesions=R)), image-major:
+    count i32 [B] (the image's number of lesions, also when it exceeds R); status i32 [B,R] (0 = graded, 1 = no lesion
+    at that rank, or a box empty after padding); boxes i32 [B,R,4] {x0,y0,x1,y1} of the 224x224 frame (end-exclusive,
+    roi.py's padding around the lesion's own pixels; zero where not graded); logits f32 [B,R,ncls] (NaN where not
+    graded); pred i64 [B,R] argmax(softmax(logits)) as 分类/test.py:86 (-1 where not graded), all on the host; cam_maps
+    f32 [B,R,224,224] on the device (the Grad-CAM map of each lesion's predicted class inside its box) or None."""
+    count: torch.Tensor
+    status: torch.Tensor
+    boxes: torch.Tensor
+    logits: torch.Tensor
+    pred: torch.Tensor
+    cam_maps: object
+
+
+def check_grade_lesions(R, max_r):
+    if isinstance(R, bool) or not isinstance(R, (int, np.integer)) or not 0 <= R <= max_r:
+        raise ValueError(f"grade_lesions must be an int in [0, {max_r}], got {R!r}")
+
+
+def grades(count, status, boxes, logits, cam_maps=None):
+    """LesionGrades from a grade_lesions program's outputs, already image-major: count [B], status [B,R], boxes
+    [B,R,4], logits [B,R,ncls] and cam_maps [B,R,224,224] or None."""
+    status = status.cpu()
+    bad = status != 0
+    logits = logits.cpu().clone()
+    logits[bad] = float("nan")
+    pred = torch.argmax(torch.softmax(logits, dim=2), dim=2)           # test.py:86
+    pred[bad] = -1
+    return LesionGrades(count.cpu(), status, boxes.cpu(), logits, pred, cam_maps)
+
+
 def rows(buf):
     """The device table buffer (int64 [B,K,ROW_WORDS]) as a LESION_DTYPE [B,K] array on the host."""
     a = buf.detach().cpu().contiguous().numpy()

@@ -10,6 +10,7 @@ lays out the NHWC bf16 activation workspace in HBM and emits the op descriptors 
   outputs at each source image's own size               -> PipelineRunner._emit_source_frame (source_frame=True)
   Dice / IoU / Hausdorff against ground truth (分割/main.py val) -> PipelineRunner._emit_seg_metrics (seg_metrics=...)
   connected components of the mask, largest-lesion ROI   -> PipelineRunner._emit_lesions (lesions=..., roi="largest")
+  a grade per lesion (crops of the R largest lesions)    -> PipelineRunner._emit_lesion_grades (grade_lesions=R)
   whole two-stage path                                   -> PipelineRunner
 
 Dead compute of the reference forward is skipped: the `x` output of the bottleneck (attention1, the first
@@ -609,8 +610,9 @@ class GoogLeNetRunner(_Builder):
         self.w["fc"] = (_f32(sd["fc.weight"], dev), _f32(sd["fc.bias"], dev))
         self.ncls = self.w["fc"][0].shape[0]
 
-    def _emit_googlenet(self, B, ws, ops, u8=None, f32=None):
-        """u8: [B,224,224,3] uint8 crops (HWC, channel order as the reference's roi_rgb), or f32: float NCHW."""
+    def _emit_googlenet(self, B, ws, ops, u8=None, f32=None, logits=None):
+        """u8: [B,224,224,3] uint8 crops (HWC, channel order as the reference's roi_rgb), or f32: float NCHW.  The head
+        writes ws["cls_logits"]: `logits` (f32 [B,ncls]) when given, else a workspace buffer."""
         buf = self.buf
         c1 = buf(B, 112, 112, 64)
         # conv1 7x7 s2 as a TMA implicit GEMM: space-to-depth pack of the crop (to_tensor + _transform_input folded,
@@ -652,17 +654,18 @@ class GoogLeNetRunner(_Builder):
             self.conv(ops, self.w[name + ".branch4.1"], View(pl), flat, View(out, pp, c1x1 + c3x3 + c5x5))
             ws[name] = out
             cur = out
-        ws["cls_logits"] = buf(B, self.ncls, dtype=torch.float32)
+        ws["cls_logits"] = logits if logits is not None else buf(B, self.ncls, dtype=torch.float32)
         ops.append(E.HeadDesc(cur.data_ptr(), self.w["fc"][0].data_ptr(), self.w["fc"][1].data_ptr(),
                               ws["cls_logits"].data_ptr(), B, 49, 1024, self.ncls))
 
-    def _emit_cam(self, B, ws, ops, boxes=None):
+    def _emit_cam(self, B, ws, ops, boxes=None, cam=None, cam_map=None):
         """Grad-CAM of the predicted class at inception5b (ug_cam_desc), appended after the head: ws["cam"] f32 [B,7,7]
         and ws["cam_map"] f32 [B,224,224], the map normalised and resized into `boxes` (int32 [B,4] of the 224x224
-        frame) or over the whole frame.  Both are fresh per call (outputs, never shared with another plan)."""
+        frame) or over the whole frame.  Both are `cam` / `cam_map` when given, else fresh per call (outputs, never
+        shared with another plan)."""
         feat = ws["inception5b"]
-        ws["cam"] = self.buf(B, 7, 7, dtype=torch.float32)
-        ws["cam_map"] = self.buf(B, IMG, IMG, dtype=torch.float32)
+        ws["cam"] = cam if cam is not None else self.buf(B, 7, 7, dtype=torch.float32)
+        ws["cam_map"] = cam_map if cam_map is not None else self.buf(B, IMG, IMG, dtype=torch.float32)
         ops.append(E.CamDesc(feat.data_ptr(), self.w["fc"][0].data_ptr(), ws["cls_logits"].data_ptr(), None,
                              E.ptr(boxes), None, ws["cam"].data_ptr(), ws["cam_map"].data_ptr(), B, 7, 7,
                              feat.shape[-1], self.ncls, IMG))
@@ -768,7 +771,7 @@ class PipelineRunner:
             del self._gpools[b]
 
     def plan(self, B, source=None, slot=0, capacity=None, cam=False, source_frame=False, seg_metrics=None,
-             lesions=None, roi="all"):
+             lesions=None, roi="all", grade_lesions=0):
         """Program for a batch of B images; B must be <= micro_batch or a multiple of it.  With `source` =
         (Hs, Ws) the program starts with the device front-end (PIL-exact resize of uint8 HWC sources + to_tensor,
         util/data_utils.py) writing the UNet input, and `ws["src_u8"]` is the program's input buffer.
@@ -791,7 +794,13 @@ class PipelineRunner:
         and ws["src_lesions"], placed like src_mask).  roi="largest" crops the largest lesion instead of the hull of
         all foreground pixels: it adds the "input" op if lesions did not and points each micro-batch's bbox at
         ws["lesion_mask"]; the boxes, crops, classifier, CAM and source-frame boxes follow, mask / logits / src_mask do
-        not change."""
+        not change.
+        grade_lesions=R (1..8) grades each of the R largest lesions of every image on its own (_emit_lesion_grades): it
+        adds the "input" lesions op if lesions / roi did not, crops each lesion after the last UNet micro-batch and
+        runs R more GoogLeNet passes of B crops (and, with cam, R more CAM ops) after the per-image ones:
+        ws["lesion_boxes"] i32 [R,B,4], ws["lesion_status"] i32 [R,B], ws["lesion_u8"] u8 [R,B,224,224,3],
+        ws["lesion_cls_logits"] f32 [R,B,6] and with cam ws["lesion_cam"] f32 [R,B,7,7] and ws["lesion_cam_map"] f32
+        [R,B,224,224].  Every per-image output is the same as without it."""
         if source_frame and source is None:
             raise ValueError("source_frame=True needs uint8 or ragged sources: float input has no source frame")
         if seg_metrics not in (None,) + SEG_FRAMES:
@@ -804,6 +813,7 @@ class PipelineRunner:
             raise ValueError("lesions='source' labels the source-frame mask: it needs source_frame=True")
         if roi not in ROI_RULES:
             raise ValueError(f"roi must be 'all' or 'largest', got {roi!r}")
+        L.check_grade_lesions(grade_lesions, LESION_K)
         if source == "ragged":
             capacity = ragged.capacity(capacity or 0)
             key = (B, slot, "ragged", capacity)
@@ -819,7 +829,9 @@ class PipelineRunner:
             key += ("lesions", lesions)
         if roi != "all":
             key += ("roi", roi)
-        input_lesions = lesions == "input" or roi == "largest"
+        if grade_lesions:
+            key += ("grade_lesions", grade_lesions)
+        input_lesions = lesions == "input" or roi == "largest" or grade_lesions > 0
 
         def build():
             mb = min(B, self.micro_batch)
@@ -864,10 +876,14 @@ class PipelineRunner:
                 ops.append(E.CropResizeDesc(ws["x_in"][sl].data_ptr(), ws["boxes"][sl].data_ptr(),
                                             ws["u8"][sl].data_ptr(), mb, IMG, IMG, IMG))
                 ws.setdefault("sub", []).append(sub)
+            if grade_lesions:
+                self._emit_lesion_crops(B, grade_lesions, ws, ops)
             with self.gnet.sharing(gpool):
                 self.gnet._emit_googlenet(B, ws, ops, u8=ws["u8"])
             if cam:
                 self.gnet._emit_cam(B, ws, ops, boxes=ws["boxes"])
+            if grade_lesions:
+                self._emit_lesion_grades(B, grade_lesions, cam, gpool, ws, ops)
             if source_frame:
                 self._emit_source_frame(B, source, capacity, ws, ops)
             if seg_metrics:
@@ -876,6 +892,36 @@ class PipelineRunner:
                 self._emit_lesions(B, source, capacity, ws, ops)
             return _finish(self.engine, ops, ws, ua + ga + [v for v in ws.values() if isinstance(v, torch.Tensor)])
         return self.plans.get_or_build(key, build)
+
+    def _emit_lesion_crops(self, B, R, ws, ops):
+        """ug_lesion_crops_desc over the whole batch: the crops of the R largest lesions of ws["lesions"] from ws["x_in"]
+        with the runner's padding, rank-major (rank r of the B images is one contiguous batch)."""
+        dev = self.dev
+        ws["lesion_boxes"] = torch.empty((R, B, 4), device=dev, dtype=torch.int32)
+        ws["lesion_status"] = torch.empty((R, B), device=dev, dtype=torch.int32)
+        ws["lesion_u8"] = torch.empty((R, B, IMG, IMG, 3), device=dev, dtype=torch.uint8)
+        ops.append(E.LesionCropsDesc(ws["x_in"].data_ptr(), ws["lesions"].data_ptr(), ws["lesion_count"].data_ptr(),
+                                     ws["lesion_boxes"].data_ptr(), ws["lesion_status"].data_ptr(),
+                                     ws["lesion_u8"].data_ptr(), B, IMG, IMG, IMG, LESION_K, R, self.padding))
+
+    def _emit_lesion_grades(self, B, R, cam, gpool, ws, ops):
+        """One GoogLeNet pass per rank over ws["lesion_u8"][r] in the per-image stage's activation workspace (`gpool`),
+        its head writing ws["lesion_cls_logits"][r], and with cam one ug_cam into that rank's boxes.  Each pass keeps
+        its own ws entries (ws["lesion_sub"][r]), so the per-image cls_logits, cam and cam_map are left alone."""
+        dev = self.dev
+        ws["lesion_cls_logits"] = torch.empty((R, B, self.gnet.ncls), device=dev, dtype=torch.float32)
+        if cam:
+            ws["lesion_cam"] = torch.empty((R, B, 7, 7), device=dev, dtype=torch.float32)
+            ws["lesion_cam_map"] = torch.empty((R, B, IMG, IMG), device=dev, dtype=torch.float32)
+        ws["lesion_sub"] = []
+        for r in range(R):
+            sub = {}
+            with self.gnet.sharing(gpool):
+                self.gnet._emit_googlenet(B, sub, ops, u8=ws["lesion_u8"][r], logits=ws["lesion_cls_logits"][r])
+            if cam:
+                self.gnet._emit_cam(B, sub, ops, boxes=ws["lesion_boxes"][r], cam=ws["lesion_cam"][r],
+                                    cam_map=ws["lesion_cam_map"][r])
+            ws["lesion_sub"].append(sub)
 
     def _emit_source_frame(self, B, source, capacity, ws, ops):
         """ug_source_frame_desc over the plan's logits, boxes and (cam plans) raw cam: ws["src_mask"] u8 and
@@ -928,21 +974,24 @@ class PipelineRunner:
                                   **kw))
 
     def export_plan(self, B, source=None, capacity=None, cam=False, source_frame=False, seg_metrics=None,
-                    lesions=None, roi="all"):
+                    lesions=None, roi="all", grade_lesions=0):
         """The whole two-stage program for a batch of B images as a relocatable plan image (bytes): op list, device
         memory layout, BN-folded packed weights of both networks.  A host in any language runs it through the C ABI
         alone (ug_plan_load / ug_plan_copy_in / ug_plan_run / ug_plan_copy_out, include/ugnet.h; examples/run_plan.c).
         source / capacity / cam / source_frame as for plan(); a ragged plan's inputs are "src_u8" and "src_index", a cam
         plan also reports "cam" and "cam_map", a source_frame plan "src_mask", "src_boxes" and (with cam)
         "src_cam_map", a seg_metrics plan takes "gt_mask" and reports "seg_counts" and "seg_hd", a lesions / roi="largest"
-        plan "lesion_labels", "lesion_mask", "lesion_count" and "lesions" (or with lesions="source" their "src_" forms)."""
+        plan "lesion_labels", "lesion_mask", "lesion_count" and "lesions" (or with lesions="source" their "src_" forms),
+        a grade_lesions plan also "lesion_boxes", "lesion_status", "lesion_u8", "lesion_cls_logits" and (with cam)
+        "lesion_cam" and "lesion_cam_map"."""
         ws = self.plan(B, source=source, capacity=capacity, cam=cam, source_frame=source_frame, seg_metrics=seg_metrics,
-                       lesions=lesions, roi=roi)
+                       lesions=lesions, roi=roi, grade_lesions=grade_lesions)
         prog = ws["program"]
         io = {k: ws[k] for k in ("x_in", "src_u8", "src_index", "src_status", "logits", "mask", "boxes", "u8",
                                  "cls_logits", "cam", "cam_map", "src_mask", "src_boxes", "src_cam_map", "gt_mask", "seg_counts",
                                  "seg_hd", "lesion_labels", "lesion_mask", "lesion_count", "lesions", "src_lesion_labels",
-                                 "src_lesion_mask", "src_lesion_count", "src_lesions") if k in ws}
+                                 "src_lesion_mask", "src_lesion_count", "src_lesions", "lesion_boxes", "lesion_status",
+                                 "lesion_u8", "lesion_cls_logits", "lesion_cam", "lesion_cam_map") if k in ws}
         tensors = list(prog.keepalive) + list(io.values()) + [(self.unet.w_blob, True), (self.gnet.w_blob, True)]
         return E.export_plan(prog.descs, io, tensors)
 
@@ -957,18 +1006,19 @@ class PipelineRunner:
             out.append((s, n - s))
         return out
 
-    def feed_ragged(self, part, cam=False, source_frame=False, seg_metrics=None, lesions=None, roi="all"):
+    def feed_ragged(self, part, cam=False, source_frame=False, seg_metrics=None, lesions=None, roi="all",
+                    grade_lesions=0):
         """The ragged plan for one chunk (a ragged.Packed of HWC images, at most one plan's batch) with its packed
         sources and table copied in (one copy each)."""
         ws = self.plan(len(part.table), source="ragged", capacity=part.n_px, cam=cam, source_frame=source_frame,
-                       seg_metrics=seg_metrics, lesions=lesions, roi=roi)
+                       seg_metrics=seg_metrics, lesions=lesions, roi=roi, grade_lesions=grade_lesions)
         ws["src_u8"][:part.data.numel()].copy_(part.data, non_blocking=True)
         ws["src_index"].copy_(ragged.table_tensor(part.table))
         return ws
 
     @torch.no_grad()
     def __call__(self, imgs, return_logits=False, return_cam=False, return_source=False, gt_masks=None,
-                 metrics_frame="input", lesions=None, roi="all"):
+                 metrics_frame="input", lesions=None, roi="all", grade_lesions=0):
         """imgs: float [B,3,224,224] CUDA, or uint8 [B,Hs,Ws,3] CUDA source images of any size (resized on the
         device exactly as the reference's PIL transform does), or a list of uint8 [H,W,3] images of different sizes
         (CUDA tensors or numpy arrays, sides up to 8*224; one ragged batch, util/ragged.py) ->
@@ -984,8 +1034,12 @@ class PipelineRunner:
         connected components of the 224x224 masks / the source-frame masks (uint8 sources only; labels and main_masks
         in the form of SourceFrame's masks); see plan(lesions=...) and lesions.py.  roi="largest" crops each image's
         largest lesion instead of the hull of all its foreground pixels: boxes, class logits and CAM maps change,
-        masks and segmentation logits do not; an empty mask keeps roi.py's centred box."""
+        masks and segmentation logits do not; an empty mask keeps roi.py's centred box.
+        Last, with grade_lesions=R (1..8), a lesions.LesionGrades(count, status, boxes, logits, pred, cam_maps): a
+        grade for each of the R largest lesions of every image (see plan(grade_lesions=...) and lesions.py); every
+        other output is the same as without it."""
         from . import metrics
+        L.check_grade_lesions(grade_lesions, LESION_K)
         masks, boxes, cls, seg, cams = [], [], [], [], []
         counts, hds = [], []
         src_masks, src_boxes, src_cams = [], [], []
@@ -1006,13 +1060,15 @@ class PipelineRunner:
         if lesions == "source" and packed is None and not from_u8:
             raise ValueError("lesions='source' needs uint8 sources: float [B,3,224,224] input has no source frame")
         src_frame = return_source or frame == "source" or lesions == "source"
-        les = dict(lesions=lesions, roi=roi)
+        les = dict(lesions=lesions, roi=roi, grade_lesions=grade_lesions)
         les_count, les_labels, les_main, les_table = [], [], [], []
+        grades = []
         for s, c in self._chunks(n):
             if packed is not None:
                 part = ragged.chunk(packed, s, s + c)
                 kw = {k: v for k, v in (("cam", return_cam), ("source_frame", src_frame), ("seg_metrics", frame),
-                                        ("lesions", lesions), ("roi", roi if roi != "all" else None)) if v}
+                                        ("lesions", lesions), ("roi", roi if roi != "all" else None),
+                                        ("grade_lesions", grade_lesions)) if v}
                 ws = self.feed_ragged(part, **kw)
             elif from_u8:
                 ws = self.plan(c, source=(imgs.shape[1], imgs.shape[2]), cam=return_cam, source_frame=src_frame,
@@ -1056,6 +1112,10 @@ class PipelineRunner:
                 else:
                     les_labels.append(ws[pre + "lesion_labels"].clone())
                     les_main.append(ws[pre + "lesion_mask"].clone())
+            if grade_lesions:                              # [R,B,...] -> image-major copies
+                grades.append([ws["lesion_count"].clone()] +
+                              [ws[k].transpose(0, 1).contiguous() if k in ws else None
+                               for k in ("lesion_status", "lesion_boxes", "lesion_cls_logits", "lesion_cam_map")])
         out = (torch.cat(masks), torch.cat(boxes), torch.cat(cls))
         if return_logits:
             out += (torch.cat(seg),)
@@ -1072,4 +1132,6 @@ class PipelineRunner:
             if lesions == "input" or packed is None:
                 les_labels, les_main = torch.cat(les_labels), torch.cat(les_main)
             out += (L.result(torch.cat(les_count), les_labels, les_main, torch.cat(les_table)),)
+        if grade_lesions:
+            out += (L.grades(*[torch.cat(parts) if parts[0] is not None else None for parts in zip(*grades)]),)
         return out

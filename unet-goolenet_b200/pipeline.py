@@ -20,7 +20,7 @@ class TwoStagePipeline:
 
     @torch.no_grad()
     def __call__(self, imgs, return_logits=False, return_cam=False, return_source=False, gt_masks=None,
-                 metrics_frame="input", lesions=None, roi="all"):
+                 metrics_frame="input", lesions=None, roi="all", grade_lesions=0):
         """imgs: float [B,3,224,224] on the pipeline's device, or uint8 HWC sources [B,Hs,Ws,3] of any size (resized
         on the device like the reference's CDDataAugmentation.transform: PIL bilinear + to_tensor), or a list of uint8
         [H,W,3] images of different sizes (CUDA tensors or numpy arrays; run as ragged batches, util/ragged.py) ->
@@ -34,9 +34,11 @@ class TwoStagePipeline:
         lesions.Lesions(count, labels, main_masks, table, derived) of the connected components of the mask if lesions
         is "input" (224x224 masks) or "source" (source-frame masks, uint8 sources only).  roi="largest" crops each
         image's largest lesion instead of the hull of all its foreground pixels (boxes, class logits and CAM follow;
-        masks do not change)."""
+        masks do not change), and last, with grade_lesions=R (1..8), by a lesions.LesionGrades(count, status, boxes,
+        logits, pred, cam_maps) grading each of the R largest lesions of every image on its own crop."""
         return self.runner(imgs, return_logits=return_logits, return_cam=return_cam, return_source=return_source,
-                           gt_masks=gt_masks, metrics_frame=metrics_frame, lesions=lesions, roi=roi)
+                           gt_masks=gt_masks, metrics_frame=metrics_frame, lesions=lesions, roi=roi,
+                           grade_lesions=grade_lesions)
 
     def predict(self, imgs):
         """argmax(softmax(logits)) as 分类/test.py:86 (softmax is monotone, so argmax of the logits)."""
